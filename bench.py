@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark of the memory-bank anomaly-scoring hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1|2|3|4|5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1|2|3|4|5] [--dump-outputs DIR]
 
 Default (--config 1, BASELINE cfg 5 headline).  A "step" scores one batch (--batch, default 16) of synthetic 784-patch
 images (DINO ViT-B/8 shaped, 768-d) against an un-subsampled 200 000 x 768 float32 bank through the full path: distance
@@ -17,7 +17,7 @@ GEMM + min/argmin, s*/m*/top-3 re-weighting, bilinear upsample and Gaussian blur
 N > 1 (torchrun, one rank per GPU): the bank is row-sharded; every step runs one round of the three-phase sharded
 protocol (two small exchanges over peer-mapped memory fused into the kernels) with three rounds outstanding on two compute lanes (strong scaling: the job is still one 200k bank).
 `--impl reference` times the CPU restatement of the reference path (oracle/, the one place it may be executed from here)
-on ALL host cores with a bounded sample.
+on ALL host cores, --steps images.
 """
 import argparse
 import json
@@ -32,6 +32,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree as it found it (it may be read-only)
 
 BANK_ROWS, DIM, P, FMAP, OUT_HW = 200_000, 768, 784, 28, 224
 PIPELINE_DEPTH = 3   # submitted calls outstanding per handle (three result slots, two compute lanes)
@@ -196,13 +197,12 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    # one step = one 784-patch image on the host cores (~0.3 s on 16 cores): the step count is bounded so that the arm ends
-    # within a few minutes; the warm-up count is the driver's.  value = ALL host cores at every N; the reference's own
-    # default of 6 threads (main.py:149 --cpu_core_num) is timed beside it.
-    steps = max(1, min(args.steps, 20))
+    # one step = one 784-patch image on the host cores (~0.3 s on 16 cores).  value = ALL host cores at every N; the
+    # reference's own default of 6 threads (main.py:149 --cpu_core_num) is timed beside it over the same step count.
+    steps = args.steps
     warm = args.warmup
     val, ms, cores = cpu_reference_leg(steps, warm)
-    val6, ms6, _ = cpu_reference_leg(max(1, min(steps, 5)), 1, threads=min(6, cores))
+    val6, ms6, _ = cpu_reference_leg(steps, 1, threads=min(6, cores))
     line = {"metric": METRIC, "value": val, "unit": "patch-NN scores/s", "n_gpus": args.gpus, "steps": steps, "warmup": warm,
             "ms_per_step": ms, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32",
             "data": "synthetic", "impl": "reference",
@@ -293,6 +293,29 @@ def parity_vs_oracle(results, patches_host, n_images=2, exact_bank=None):
 
 def results_equal(a, b, names=("min_idx", "min_val", "s", "s_star", "s_idx", "nn_idx", "m_star_knn", "w", "s_map")):
     return all(bool((getattr(a, n) == getattr(b, n)).all()) for n in names)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory, result):
+    """Writes every array of a BatchResult (what the caller of score_batch_async receives) as <directory>/<name>.npy, so
+    that two builds run with the same arguments can be compared output for output.  float32 arrays are written as they
+    are; integer arrays (indices) as float64, which holds them exactly.  Every array is indexed by image first; when
+    the batch would exceed DUMP_LIMIT_BYTES, a fixed seeded sample of the images is written.  image_index.npy lists the
+    images written."""
+    arrays = {n: np.asarray(a) for n, a in result.arrays.items() if a is not None}
+    arrays = {n: a if a.dtype == np.float32 else a.astype(np.float64) for n, a in arrays.items()}
+    n_img = len(result)
+    per_image = sum(a.nbytes for a in arrays.values()) // n_img + 8
+    keep = np.arange(n_img)
+    if n_img * per_image > DUMP_LIMIT_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n_img, DUMP_LIMIT_BYTES // per_image, replace=False))
+        arrays = {n: a[keep] for n, a in arrays.items()}
+    arrays["image_index"] = keep.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -511,6 +534,8 @@ def run_ours(args):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the results of one GPU: run it without torchrun")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     if world > 1:
@@ -564,17 +589,18 @@ def run_ours(args):
     def timed(patches, steps, collect_stage=False, pipelined=True):
         """K steps between barriers; device time from CUDA events on the bank's stream, max over ranks.  pipelined: up to
         PIPELINE_DEPTH batches outstanding -- every step still copies its inputs from the host block and its results back inside the timed
-        region, the copies just overlap the other batch's kernels."""
+        region, the copies just overlap the other batch's kernels.  Also returns the results of the last step."""
         stage_ms = []
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(st)
         w0 = time.perf_counter()
         pending = []
+        last = None
         for i in range(steps):
             t = submit(patches[i % len(patches)])
             if not pipelined:
-                t.wait()
+                last = t.wait()
                 if collect_stage:
                     stage_ms.append(bank.timings())
                 continue
@@ -582,13 +608,13 @@ def run_ours(args):
             if len(pending) >= PIPELINE_DEPTH:
                 pending.pop(0).wait()
         while pending:
-            pending.pop(0).wait()
+            last = pending.pop(0).wait()
         e1.record(st)
         e1.synchronize()
         wall = time.perf_counter() - w0
         barrier()
         ms, wall_ms = max_over_ranks(e0.elapsed_time(e1), wall * 1e3)
-        return ms, wall_ms, stage_ms
+        return ms, wall_ms, stage_ms, last
 
     for i in range(args.warmup):
         submit(devb[i % n_img]).wait()
@@ -606,15 +632,17 @@ def run_ours(args):
         single_stage = bank.timings()
     # the plain synchronous call, for the per-stage times and as a reference point beside the pipelined numbers
     n_s = max(5, args.steps // 2)
-    ms_s, wall_s, stages = timed(devb, n_s, collect_stage=(world == 1), pipelined=False)
-    ms_h, wall_h, _ = timed(host, n_s, pipelined=False)
+    ms_s, wall_s, stages, _ = timed(devb, n_s, collect_stage=(world == 1), pipelined=False)
+    ms_h, wall_h, _, _ = timed(host, n_s, pipelined=False)
     sync_call = {"value": B * P * n_s / (max(ms_s, wall_s) * 1e-3), "e2e": B * P * n_s / (max(ms_h, wall_h) * 1e-3),
                  "unit": "patch-NN scores/s", "note": "one batch / round at a time (the host waits for every batch)"}
     for i in range(3):
         timed(host, 2)
     with ClockSampler(local) as clk:
-        ms_dev, wall_dev, _ = timed(devb, args.steps)
-        ms_e2e, wall_e2e, _ = timed(host, args.steps)
+        ms_dev, wall_dev, _, last = timed(devb, args.steps)
+        ms_e2e, wall_e2e, _, _ = timed(host, args.steps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
     # results are host-visible when the loop ends, so the event span equals the wall span; report the larger (safer) one
     t_dev, t_e2e = max(ms_dev, wall_dev), max(ms_e2e, wall_e2e)
     value = B * P * args.steps / (t_dev * 1e-3)
@@ -780,7 +808,7 @@ def run_ours(args):
         for i in range(3):
             submit(devb[i % n_img]).wait()
         n_full = max(5, args.steps // 2)
-        ms_full, wall_full, st_full = timed(devb, n_full, collect_stage=True, pipelined=False)
+        ms_full, wall_full, st_full, _ = timed(devb, n_full, collect_stage=True, pipelined=False)
         bank.set_prefilter_terms(0)
         g3 = float(np.mean([x["gemm"] for x in st_full]))
         line["fp32_equivalent_3term_mode"] = {"value": B * P * n_full / (max(ms_full, wall_full) * 1e-3), "unit": "patch-NN scores/s",
@@ -952,7 +980,14 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-extras", action="store_true", help="skip the 1M-row bank and the bounded cfg 2 / cfg 4 legs")
     ap.add_argument("--skip-dropin", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the results of the last step of the headline loop to DIR/<name>.npy "
+                         "(one GPU, --config 1, --impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config != 1):
+        ap.error("--dump-outputs needs --impl ours and --config 1")
     args.warmup = max(3, args.warmup)
     if args.impl == "reference":
         return run_reference(args)

@@ -1,6 +1,7 @@
 """TEST INFRASTRUCTURE ONLY -- freezes golden vectors from the UNMODIFIED reference (run in the build container).
 
-    python -m oracle.make_golden        # writes tests/golden/*.npz
+    python -m oracle.make_golden                       # writes tests/golden/*.npz
+    python -m oracle.make_golden --from-restatement    # only au_pro_case / fresh_seed_case, without the reference
 
 The reference ships no tests, fixtures or golden vectors (SURVEY.md section 4), so parity is pinned on outputs of the
 reference's own code (feature_extractors/features.py, multiple_features.py, utils/utils.py) imported through
@@ -108,7 +109,81 @@ def golden_dual():
     print("dual_case:", {k: getattr(v, "shape", v) for k, v in out.items()})
 
 
+# --------------------------------------------------------------------------------------------------------------------
+# outputs of the live-reference comparisons of tests/test_metrics.py and tests/test_oracle.py, frozen so that those
+# comparisons also run where the reference is absent.  Both tests assert bit-identity between the reference and
+# cmdiad_b200.metrics / oracle.restate on exactly these inputs, so --from-restatement computes the same values without
+# the reference.  The committed files were made that way, from code that passed both live tests (commit 03de1db; the
+# metrics and oracle code is unchanged since).
+# --------------------------------------------------------------------------------------------------------------------
+AU_PRO_CASES = ((0, False), (1, True), (2, False), (3, True))   # (seed, quantised) of test_metrics._maps
+AU_PRO_SETTINGS = ((0.3, 100), (0.01, 100), (0.3, 37))         # (integration_limit, num_thresholds)
+FRESH_SEED_CASE = dict(n_train=3, P=784, D=768, seed=77, patch_seed=5, fmap=28)
+
+
+def au_pro_key(seed, limit, nth):
+    return f"seed{seed}_limit{limit}_n{nth}"
+
+
+def golden_au_pro(use_reference=True):
+    """calculate_au_pro (utils/au_pro_util.py) on the seeded maps of tests/test_metrics.py: value and curve"""
+    from tests.test_metrics import _maps
+    if use_reference:
+        from tests.test_metrics import _reference_au_pro
+        calc, source = _reference_au_pro().calculate_au_pro, "reference utils/au_pro_util.py"
+    else:
+        from cmdiad_b200 import metrics
+        calc, source = metrics.au_pro, "cmdiad_b200.metrics.au_pro (bit-identical to the reference on these inputs)"
+    out = {"source": np.str_(source)}
+    for seed, quantised in AU_PRO_CASES:
+        gts, preds = _maps(seed, quantised=quantised)
+        for limit, nth in AU_PRO_SETTINGS:
+            au, (fprs, pros) = calc(gts, preds, integration_limit=limit, num_thresholds=nth)
+            k = au_pro_key(seed, limit, nth)
+            out[f"{k}_au_pro"] = np.float64(au)
+            out[f"{k}_fprs"] = np.asarray(fprs, dtype=np.float64)
+            out[f"{k}_pros"] = np.asarray(pros, dtype=np.float64)
+    np.savez_compressed(os.path.join(OUT, "au_pro_case.npz"), **out)
+    print("au_pro_case:", len(out) - 1, "arrays from", source)
+
+
+def golden_fresh_seed(use_reference=True):
+    """RGBFeatures run_coreset (TF32 mode) + calculate_dist + compute_single_s_s_map on a seed none of the other golden
+    cases uses; the statistics come from oracle.restate as in tests/test_oracle.py"""
+    from oracle import restate as O
+    c = FRESH_SEED_CASE
+    train = synth.image_bank(c["n_train"], c["P"], c["D"], seed=c["seed"])
+    cat = torch.cat([_t(x) for x in train], 0)
+    mean, std = O.bank_stats_restated(cat)
+    patch = (_t(synth.patches(c["P"], c["D"], c["patch_seed"], anomalous_frac=0.01)) - mean) / std
+    fmap = (c["fmap"], c["fmap"])
+    if use_reference:
+        m = R.make_method("RGBFeatures", coreset_dtype="TF32", random_state=0)
+        for x in train:
+            m.patch_rgb_lib.append(_t(x))
+        with R.cuda_to_cpu_if_needed():
+            m.run_coreset()
+        idx = m.coreset_idx.numpy()
+        s, s_map = m.compute_single_s_s_map(patch, m.calculate_dist(patch, m.patch_rgb_lib), fmap, modal="rgb")
+        s, s_map, source = np.float32(s), s_map[0].numpy(), "reference RGBFeatures"
+    else:
+        lib = O.normalize_restated(cat, mean, std).numpy()
+        z = O.project_restated(lib, *O.sparse_components(lib.shape[0], c["D"], 0.9, 0))
+        idx = O.coreset_restated(z, int(0.1 * lib.shape[0]), "TF32")
+        r = O.score_restated(patch.numpy(), lib[idx], fmap, 224)
+        s, s_map, source = np.float32(r["s"]), r["s_map"], "oracle.restate (bit-identical to the reference on these inputs)"
+    np.savez_compressed(os.path.join(OUT, "fresh_seed_case.npz"), coreset_idx=np.asarray(idx, dtype=np.int64), s=s,
+                        s_map=np.asarray(s_map, dtype=np.float32), source=np.str_(source))
+    print("fresh_seed_case: from", source)
+
+
 if __name__ == "__main__":
     os.makedirs(OUT, exist_ok=True)
-    golden_rgb()
-    golden_dual()
+    if "--from-restatement" in sys.argv[1:]:
+        golden_au_pro(use_reference=False)
+        golden_fresh_seed(use_reference=False)
+    else:
+        golden_rgb()
+        golden_dual()
+        golden_au_pro()
+        golden_fresh_seed()

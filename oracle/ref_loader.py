@@ -1,8 +1,9 @@
 """TEST INFRASTRUCTURE ONLY -- loads the UNMODIFIED reference (evenrose/CMDIAD) in-process.
 
-Only usable in the build container, where /root/reference exists; nothing under -m gpu tests, smoke() or bench.py
-may call this (the GPU box has no /root/reference).  It is used by oracle/make_golden.py to freeze golden vectors
-under tests/golden/ and by the CPU test-suite to validate oracle/restate.py against the real reference code.
+The repository does not contain the reference: place a checkout of it at oracle/_ref/ (git-ignored) or point
+CMDIAD_REFERENCE_ROOT at one.  Nothing under -m gpu tests, smoke() or bench.py may call this.  It is used by
+oracle/make_golden.py to freeze golden vectors under tests/golden/ and by the CPU test-suite to validate
+oracle/restate.py against the real reference code; those tests skip where the reference is absent.
 
 Recipe (SURVEY.md Appendix C): register empty stand-in modules for the seven imports this image lacks
 (cupy, cupyx.scipy.spatial.distance, matplotlib.pyplot, timm, knn_cuda, pointnet2_ops, tifffile), import
@@ -17,7 +18,8 @@ from argparse import Namespace
 
 import torch
 
-REFERENCE_ROOT = os.environ.get("CMDIAD_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("CMDIAD_REFERENCE_ROOT", os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref"))
+SKIP_REASON = "needs the unmodified reference tree (oracle/_ref/ or CMDIAD_REFERENCE_ROOT), which the repository does not ship"
 
 
 def reference_available() -> bool:

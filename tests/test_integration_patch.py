@@ -1,7 +1,7 @@
 """CPU suite: integration/cmdiad_b200.patch applies to the reference and the patched reference is a working drop-in.
 
-Needs /root/reference (build container).  The patched tree is a scratch copy under tmp_path; nothing is copied into
-the repository."""
+Needs the reference tree (oracle/ref_loader.py).  The patched tree is a scratch copy under tmp_path; nothing is copied
+into the repository."""
 import os
 import shutil
 import subprocess
@@ -15,7 +15,7 @@ from oracle import ref_loader as R
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PATCH = os.path.join(ROOT, "integration", "cmdiad_b200.patch")
 
-pytestmark = pytest.mark.skipif(not R.reference_available(), reason="needs /root/reference (build container only)")
+pytestmark = pytest.mark.skipif(not R.reference_available(), reason=R.SKIP_REASON)
 
 
 def _scratch_copy(tmp_path):

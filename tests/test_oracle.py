@@ -1,5 +1,5 @@
 """CPU suite, part 1: the oracle (oracle/restate.py + coreset_oracle.c) against the golden vectors frozen from the
-unmodified reference, and -- when /root/reference is present -- against the reference itself."""
+unmodified reference, and -- when the reference tree is present -- against the reference itself."""
 import numpy as np
 import pytest
 import torch
@@ -104,26 +104,32 @@ def test_projection_against_sklearn(built):
         O.sparse_components(10 ** 7, 64, 0.9, 0)  # d' > D: sklearn raises, the reference skips the projection
 
 
-@pytest.mark.skipif(not R.reference_available(), reason="needs /root/reference (build container only)")
-def test_oracle_against_live_reference(built):
-    """restatement vs the unmodified reference classes on a fresh seed (not just the frozen golden inputs)"""
+def test_oracle_against_live_reference(built, golden):
+    """restatement vs the unmodified reference classes on a fresh seed (not just the inputs of rgb_case): the
+    reference's outputs are frozen in tests/golden/fresh_seed_case.npz (oracle/make_golden.py); where the reference
+    tree is present it is also run live"""
     from cmdiad_b200 import synth
-    m = R.make_method("RGBFeatures", coreset_dtype="TF32", random_state=0)
+    frozen = golden["fresh_seed_case"]
     train = synth.image_bank(3, 784, 768, seed=77)
-    for x in train:
-        m.patch_rgb_lib.append(torch.from_numpy(x))
-    with R.cuda_to_cpu_if_needed():
-        m.run_coreset()
     cat = torch.cat([torch.from_numpy(x) for x in train], 0)
     mean, std = O.bank_stats_restated(cat)
     lib = O.normalize_restated(cat, mean, std).numpy()
     z = O.project_restated(lib, *O.sparse_components(lib.shape[0], 768, 0.9, 0))
     idx = O.coreset_restated(z, int(0.1 * lib.shape[0]), "TF32")
-    assert (idx == m.coreset_idx.numpy()).all()
+    assert (idx == frozen["coreset_idx"]).all()
     patch = ((torch.from_numpy(synth.patches(784, 768, 5, anomalous_frac=0.01)) - mean) / std)
+    r = O.score_restated(patch.numpy(), lib[idx], (28, 28), 224)
+    assert np.float32(r["s"]) == frozen["s"] and (r["s_map"] == frozen["s_map"]).all()
+    if not R.reference_available():
+        return
+    m = R.make_method("RGBFeatures", coreset_dtype="TF32", random_state=0)
+    for x in train:
+        m.patch_rgb_lib.append(torch.from_numpy(x))
+    with R.cuda_to_cpu_if_needed():
+        m.run_coreset()
+    assert (idx == m.coreset_idx.numpy()).all()
     dist = m.calculate_dist(patch, m.patch_rgb_lib)
     s, s_map = m.compute_single_s_s_map(patch, dist, (28, 28), modal="rgb")
-    r = O.score_restated(patch.numpy(), lib[idx], (28, 28), 224)
     assert np.float32(r["s"]) == np.float32(s) and (r["s_map"] == s_map[0].numpy()).all()
 
 
