@@ -134,6 +134,7 @@ SYMBOLS = {
 # test hook exported by the library but deliberately not part of the public header
 DEBUG_SYMBOLS = {
     "cmdb_debug_exact_min": (_I, [_VP, _VP, _I, _VP, _VP]),
+    "cmdb_debug_eval_load": (_I, [_VP, _VP, _I64]),
     "cmdb_coreset_select_debug": (_I, [_VP, _I64, _VP, _VP, _VP, _I, _I, _VP, _VP, _VP]),
 }
 

@@ -146,8 +146,9 @@ static int blur_batch(cmdb_bank *b, int B, int fh, int fw, int out_hw, int img_f
 
 // ---------------------------------------------------------------------------------------------------------------
 // late-fusion head (multiple_features.py:986-994): lambda scaling in float32, SGDOneClassSVM.score_samples in float64
-//   X @ coef_ on 2 columns: dgemv evaluates fma(x0, c0, x1 * c1) for the [npix, 2] map matrix and the ddot of a single
-//   row fma(x1, c1, x0 * c0) (OpenBLAS as shipped with numpy/scipy in this image; pinned by tests against sklearn).
+//   X @ coef_: dgemv evaluates fma(x0, c0, x1 * c1) for the [npix, 2] map matrix and fma(x2, c2, fma(x0, c0, x1 * c1))
+//   for [npix, 3]; the ddot of a single row is a sequential fma over the columns, fma(x1, c1, x0 * c0) and
+//   fma(x2, c2, fma(x1, c1, x0 * c0)) (OpenBLAS as shipped with numpy/scipy; pinned by tests against sklearn).
 // grid (pixel blocks, images)
 // ---------------------------------------------------------------------------------------------------------------
 struct FuseParams {
@@ -181,7 +182,7 @@ __global__ void __launch_bounds__(256) fuse_head_kernel(FuseParams p) {
                 v = __fma_rn(x0, p.seg_coef[0], __dmul_rn(x1, p.seg_coef[1]));
             } else {
                 const double x2 = (double)__fmul_rn(p.smap_lambda[2], m2[i]);
-                v = __fma_rn(x0, p.seg_coef[0], __fma_rn(x1, p.seg_coef[1], __dmul_rn(x2, p.seg_coef[2])));
+                v = __fma_rn(x2, p.seg_coef[2], __fma_rn(x0, p.seg_coef[0], __dmul_rn(x1, p.seg_coef[1])));
             }
         }
         v = __dadd_rn(__dsub_rn(v, p.seg_off), p.seg_off);  // decision_function(X) + offset_

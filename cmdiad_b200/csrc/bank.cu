@@ -19,47 +19,56 @@ void set_error(const char *fmt, ...) {
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// statistics: sum and sum of squares in float64 (one pass, float4 loads), grid sized to the SM count
+// statistics in float64, two passes over the bank (float4 loads, grid sized to the SM count): pass 1 sums x, pass 2
+// sums (x - mean)^2 with mean = sum / n, so the variance does not cancel when |mean| >> std.  Every block writes one
+// partial and a single block adds the partials in index order: no atomics, the result does not depend on the order
+// in which blocks finish, and repeated calls are bit-identical.
 // ---------------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(512) stats_kernel(const float *__restrict__ x, int64_t n, double *__restrict__ out) {
-    double s = 0.0, ss = 0.0;
+template <bool kSqDev>
+__global__ void __launch_bounds__(512) stats_pass_kernel(const float *__restrict__ x, int64_t n, const double *__restrict__ sum,
+                                                         double *__restrict__ partial) {
+    const double mean = kSqDev ? *sum / (double)n : 0.0;
+    double s = 0.0;
     const int64_t n4 = n >> 2;
     const float4 *x4 = reinterpret_cast<const float4 *>(x);
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
         float4 v = __ldg(x4 + i);
         // per-vector partial in float64 keeps the dependent chain short
-        double a = (double)v.x + (double)v.y + (double)v.z + (double)v.w;
-        double b = (double)v.x * v.x + (double)v.y * v.y + (double)v.z * v.z + (double)v.w * v.w;
-        s += a;
-        ss += b;
+        if (kSqDev) {
+            const double a = v.x - mean, b = v.y - mean, c = v.z - mean, d = v.w - mean;
+            s += a * a + b * b + c * c + d * d;
+        } else {
+            s += (double)v.x + (double)v.y + (double)v.z + (double)v.w;
+        }
     }
     if (blockIdx.x == 0 && threadIdx.x < (n & 3)) {
-        double v = x[(n4 << 2) + threadIdx.x];
-        s += v;
-        ss += v * v;
+        const double v = (double)x[(n4 << 2) + threadIdx.x] - mean;
+        s += kSqDev ? v * v : v;
     }
-    for (int o = 16; o > 0; o >>= 1) {
-        s += __shfl_xor_sync(0xffffffffu, s, o);
-        ss += __shfl_xor_sync(0xffffffffu, ss, o);
-    }
-    __shared__ double sh[2][16];
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    __shared__ double sh[16];
     const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
-    if (l == 0) {
-        sh[0][w] = s;
-        sh[1][w] = ss;
-    }
+    if (l == 0) sh[w] = s;
     __syncthreads();
     if (w == 0) {
-        s = l < (blockDim.x >> 5) ? sh[0][l] : 0.0;
-        ss = l < (blockDim.x >> 5) ? sh[1][l] : 0.0;
-        for (int o = 8; o > 0; o >>= 1) {
-            s += __shfl_xor_sync(0xffffffffu, s, o);
-            ss += __shfl_xor_sync(0xffffffffu, ss, o);
-        }
-        if (l == 0) {
-            atomicAdd(out, s);
-            atomicAdd(out + 1, ss);
-        }
+        s = l < (blockDim.x >> 5) ? sh[l] : 0.0;
+        for (int o = 8; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+        if (l == 0) partial[blockIdx.x] = s;
+    }
+}
+
+// one block: *out = sum of partial[0 .. n_part) in a fixed order
+__global__ void __launch_bounds__(256) stats_reduce_kernel(const double *__restrict__ partial, int n_part, double *__restrict__ out) {
+    double s = 0.0;
+    for (int i = threadIdx.x; i < n_part; i += blockDim.x) s += partial[i];
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    __shared__ double sh[8];
+    if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = s;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        s = 0.0;
+        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) s += sh[w];
+        *out = s;
     }
 }
 
@@ -272,7 +281,7 @@ int cmdb_bank_create(int device, int dim, int64_t capacity_rows, cmdb_bank **out
     for (auto &e : b->ev_chunk)
         if (err == cudaSuccess) err = cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
     if (err == cudaSuccess) err = cudaMalloc(&b->data, sizeof(float) * (size_t)capacity_rows * dim);
-    if (err == cudaSuccess) err = cudaMalloc(&b->stats_buf, 2 * sizeof(double));
+    if (err == cudaSuccess) err = cudaMalloc(&b->stats_buf, sizeof(double) * (2 + (size_t)b->num_sms * 4));
     if (err == cudaSuccess) err = cudaMalloc(&b->absmax_buf, sizeof(unsigned int));
     if (err != cudaSuccess) {
         set_error("cmdb_bank_create: allocation of %lld x %d floats failed: %s", (long long)capacity_rows, dim,
@@ -529,20 +538,23 @@ int cmdb_bank_stats(cmdb_bank *b, double *out_mean, double *out_std, double *out
     CMDB_REQUIRE(b->rows > 0, CMDB_ERR_STATE, "cmdb_bank_stats: bank is empty");
     CMDB_CUDA(cudaSetDevice(b->device));
     const int64_t n = b->rows * b->dim;
-    CMDB_CUDA(cudaMemsetAsync(b->stats_buf, 0, 2 * sizeof(double), b->stream));
-    int grid = (int)std::min<int64_t>((n / 4 + 511) / 512 + 1, (int64_t)b->num_sms * 4);
-    stats_kernel<<<grid, 512, 0, b->stream>>>(b->data, n, b->stats_buf);
+    // stats_buf: [0] sum, [1] sum of squared deviations, [2 ..) one partial per block (sized for num_sms * 4 blocks)
+    const int grid = (int)std::min<int64_t>((n / 4 + 511) / 512 + 1, (int64_t)b->num_sms * 4);
+    double *part = b->stats_buf + 2;
+    stats_pass_kernel<false><<<grid, 512, 0, b->stream>>>(b->data, n, nullptr, part);
+    stats_reduce_kernel<<<1, 256, 0, b->stream>>>(part, grid, b->stats_buf);
+    stats_pass_kernel<true><<<grid, 512, 0, b->stream>>>(b->data, n, b->stats_buf, part);
+    stats_reduce_kernel<<<1, 256, 0, b->stream>>>(part, grid, b->stats_buf + 1);
     CMDB_CUDA(cudaGetLastError());
     double h[2];
     CMDB_CUDA(cudaMemcpyAsync(h, b->stats_buf, sizeof(h), cudaMemcpyDeviceToHost, b->stream));
     CMDB_CUDA(cudaStreamSynchronize(b->stream));
     const double mean = h[0] / (double)n;
-    double var = n > 1 ? (h[1] - h[0] * mean) / (double)(n - 1) : NAN;  // unbiased, like torch.std
-    if (var < 0) var = 0;
+    const double var = n > 1 ? h[1] / (double)(n - 1) : NAN;  // unbiased, like torch.std
     if (out_mean) *out_mean = mean;
     if (out_std) *out_std = sqrt(var);
     if (out_sum) *out_sum = h[0];
-    if (out_sumsq) *out_sumsq = h[1];
+    if (out_sumsq) *out_sumsq = h[1] + h[0] * mean;  // sum of squares, rebuilt from the deviations
     return CMDB_OK;
 }
 

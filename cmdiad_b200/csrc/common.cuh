@@ -233,7 +233,7 @@ struct cmdb_bank {
     cudaEvent_t ev_base = nullptr;
     cudaEvent_t ev_dbg[2][4] = {};   // inside the refine stage: before / after the certificate kernel, after the rescan, after the tier-2 launches
     int cur_slot = 0;
-    double *stats_buf = nullptr;  // 2 doubles on device
+    double *stats_buf = nullptr;  // 2 + num_sms * 4 doubles on device (cmdb_bank_stats)
     unsigned int *absmax_buf = nullptr;
 };
 

@@ -238,6 +238,26 @@ using namespace cmdb;
 
 extern "C" {
 
+// test hook (not in the public header): appends n_images maps of acc_npix float64 values to the device-side result store
+// under the checks of the fused submit (store reserved, room for the images, no batch outstanding), so that the metrics
+// can be driven with chosen values -- ties, sign mixes, 10 M-pixel stores -- instead of whatever scoring produces.  The
+// image scores of the loaded images are set to 0.
+int cmdb_debug_eval_load(cmdb_bank *b, const double *maps_host, int64_t n_images) {
+    CMDB_REQUIRE(b && maps_host && n_images >= 1, CMDB_ERR_INVALID, "cmdb_debug_eval_load: bad arguments");
+    cmdb_bank::Fused &f = b->fused;
+    CMDB_REQUIRE(!f.active[0] && !f.active[1], CMDB_ERR_STATE, "cmdb_debug_eval_load: a submitted batch is outstanding");
+    CMDB_REQUIRE(f.acc_maps && f.acc_n + n_images <= f.acc_cap, CMDB_ERR_CAPACITY,
+                 "cmdb_debug_eval_load: device-side result store missing or full (%lld + %lld > %lld); call cmdb_eval_reserve",
+                 f.acc_n, (long long)n_images, f.acc_cap);
+    CMDB_CUDA(cudaSetDevice(b->device));
+    CMDB_CUDA(cudaMemcpyAsync(f.acc_maps + (size_t)f.acc_n * f.acc_npix, maps_host, sizeof(double) * (size_t)n_images * f.acc_npix,
+                              cudaMemcpyHostToDevice, b->stream));
+    CMDB_CUDA(cudaMemsetAsync(f.acc_scores + f.acc_n, 0, sizeof(double) * (size_t)n_images, b->stream));
+    CMDB_CUDA(cudaStreamSynchronize(b->stream));
+    f.acc_n += n_images;
+    return CMDB_OK;
+}
+
 int cmdb_eval_pixel_metrics(cmdb_bank *b, const int32_t *labels_host, int64_t n_components, const int64_t *ok_rank_pos_host,
                             int n_thresholds, double *out_thresholds, int64_t *out_component_le_counts,
                             int64_t *out_component_sizes, uint64_t *out_two_u, int64_t *out_n_pos, int64_t *out_n_neg) {

@@ -104,7 +104,9 @@ def device_pixel_metrics(fusion, gts, num_thresholds=100, limits=(0.3, 0.01)):
     from . import _lib as L
     lib = L.load()
     labels, n_comp = label_components(gts)
-    assert fusion.eval_count() == labels.shape[0], "one ground-truth mask per stored map"
+    hw = fusion._eval_hw
+    if labels.shape != (fusion.eval_count(), hw * hw):   # the library reads one label per stored pixel
+        raise ValueError(f"one {hw}x{hw} ground-truth mask per stored map: {fusion.eval_count()} maps, masks {labels.shape}")
     labels = np.ascontiguousarray(labels)
     n_ok = int((labels == 0).sum())
     pos = np.linspace(0, n_ok - 1, num=num_thresholds, dtype=int).astype(np.int64)

@@ -96,8 +96,10 @@ int cmdb_bank_dim(const cmdb_bank *bank, int *out_dim);
 /* Row-sharding (SURVEY 8e): this handle holds global rows [row_offset, row_offset + rows). Default offset 0. */
 int cmdb_bank_set_row_offset(cmdb_bank *bank, int64_t row_offset);
 int cmdb_bank_set_option(cmdb_bank *bank, int option, int value);
-/* torch.mean / torch.std (unbiased) over ALL elements (multiple_features.py:39-40): float64 accumulation on the GPU.
- * out_sum / out_sumsq (optional) return the raw float64 sums so that shards can be combined on the host. */
+/* torch.mean / torch.std (unbiased) over ALL elements (multiple_features.py:39-40): float64 accumulation on the GPU, two
+ * passes (sum, then sum of squared deviations from the mean) reduced in a fixed order, so repeated calls are bit-identical.
+ * out_sum / out_sumsq (optional) return the float64 sum and sum of squares (the latter rebuilt as
+ * sum((x - mean)^2) + sum * mean) so that shards can be combined on the host. */
 int cmdb_bank_stats(cmdb_bank *bank, double *out_mean, double *out_std_unbiased, double *out_sum, double *out_sumsq);
 /* lib = (lib - mean) / std in float32, in place (multiple_features.py:41); one IEEE subtract and one IEEE divide. */
 int cmdb_bank_normalize(cmdb_bank *bank, float mean, float std);
