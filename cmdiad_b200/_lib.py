@@ -102,10 +102,6 @@ SYMBOLS = {
     "cmdb_score_batch_submit": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _I, ctypes.c_uint, ctypes.POINTER(ctypes.c_int64)]),
     "cmdb_score_batch_wait": (_I, [_VP, ctypes.c_int64, ctypes.POINTER(ScoreOut)]),
     "cmdb_score_shard_min": (_I, [_VP, _VP, _I, _I, _I, _I, _VP]),
-    "cmdb_score_shard_select": (_I, [_VP, _VP, _I, _I, _VP]),
-    "cmdb_score_shard_topk": (_I, [_VP, _VP, _I, _I, _VP]),
-    "cmdb_score_shard_nn": (_I, [_VP, _VP, _I, _I, _VP]),
-    "cmdb_score_shard_finish": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _I, _I, ctypes.POINTER(ScoreOut)]),
     "cmdb_upsample_blur": (_I, [_I, _VP, _I, _I, _I, _VP, _VP, _VP]),
     "cmdb_bank_set_query_norm": (_I, [_VP, ctypes.c_float, ctypes.c_float, _I]),
     "cmdb_bank_build_knn_rows": (_I, [_VP, _I64, _I64]),
@@ -114,7 +110,6 @@ SYMBOLS = {
     "cmdb_score_shard_lookup": (_I, [_VP, _VP, _I, _I, _VP]),
     "cmdb_score_shard_finish_submit": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _I, _I, ctypes.c_uint, ctypes.POINTER(ctypes.c_int64)]),
     "cmdb_score_shard_wait": (_I, [_VP, ctypes.c_int64, ctypes.POINTER(ScoreOut)]),
-    "cmdb_bank_stage_h2d": (_I, [_VP, _VP, _VP, ctypes.c_size_t]),
     "cmdb_bank_attach_comm": (_I, [_VP, _VP]),
     "cmdb_score_shard_round_submit": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _I, _I, _I, ctypes.c_uint, ctypes.POINTER(ctypes.c_int64)]),
     "cmdb_bank_read_device": (_I, [_VP, _I64, _I64, _VP]),

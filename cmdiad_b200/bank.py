@@ -214,8 +214,9 @@ class Bank:
         """Row-sharded bank: builds the REPLICATED neighbour table (SURVEY 8f-1 for sharded banks).  Collective: the fp32
         shards are all-gathered over NVLink into a temporary un-sharded handle on every rank, each rank computes the table
         entries of the rows it owns (R/world x R distance work per rank, through the same certified GEMM), and the
-        24-byte-per-row slices are all-gathered.  Afterwards score_sharded_batch needs two small collectives per round
-        instead of four and no re-weighting pass over the bank."""
+        24-byte-per-row slices are all-gathered.  score_sharded_batch / score_sharded_async look the neighbours of
+        m_star up in this table, so a round needs two small collectives and no re-weighting pass over the bank.
+        finalize() drops the table."""
         import torch.distributed as dist
         world, rank = dist.get_world_size(group), dist.get_rank(group)
         dev = torch.device("cuda", self.device)
@@ -323,6 +324,7 @@ class Bank:
 
     def finalize(self):
         L.check(self._lib.cmdb_bank_finalize(self._h))
+        self._knn_replicated = False   # cmdb_bank_finalize frees the neighbour table
 
     # ---- persistence (SURVEY 8f: the reference rebuilds its banks on every run and never saves them) -------------------
     def save(self, path, **meta):
@@ -573,65 +575,29 @@ class Bank:
     def score_sharded_batch(self, patches, feature_map_dims, out_hw=224, full=False, group=None, distribute=False,
                             phase_events=None):
         """Row-sharded scoring: one process per GPU, each holding a contiguous block of bank rows; torch.distributed
-        (NCCL over NVLink) collectives between the phases of include/cmdiad_b200.h.  Kernels and collectives are all
-        enqueued on the handle's stream: nothing synchronises the host between the phases, and the collectives are per
-        round of up to 32 images, not per image.
-        With the replicated neighbour table (build_knn_sharded): three phases / two collectives per round, and two
-        rounds are kept in flight (score_sharded_async).  Without it: the five-phase protocol with the re-weighting
-        sweep over the shards, one round at a time.
+        (NCCL over NVLink) collectives between the phases of include/cmdiad_b200.h.  Rounds of up to max_shard_batch()
+        images go through score_sharded_async with two rounds kept in flight.  Collective: without a replicated
+        neighbour table (build_knn_sharded) on this handle, the first call builds it.
         distribute=False: every rank returns all maps.  distribute=True: rank r finishes (blur, device->host) only images
         r, r+world, ... and returns None for the others.
-        phase_events (table path): optional list; gets one list of torch events per round, recorded on the handle's
-        stream around the phases named in Bank.PHASES."""
-        import torch.distributed as dist
+        phase_events: optional list; gets one list of torch events per round, recorded on the handle's stream around the
+        phases named in Bank.PHASES."""
+        if not getattr(self, "_knn_replicated", False):
+            self.build_knn_sharded(group)
         patches = _as_f32(patches)
-        Btot, P = patches.shape[0], patches.shape[1]
-        fh, fw = feature_map_dims
-        world, rank = dist.get_world_size(group), dist.get_rank(group)
         results = []
         step = self.max_shard_batch()
-        if getattr(self, "_knn_replicated", False):
-            pending = None
-            for b0 in range(0, Btot, step):
-                evs = [] if phase_events is not None else None
-                t = self.score_sharded_async(patches[b0:b0 + step], feature_map_dims, out_hw, full, group, distribute, b0, evs)
-                if phase_events is not None:
-                    phase_events.append(evs)
-                if pending is not None:
-                    results.extend(pending.wait())
-                pending = t
+        pending = None
+        for b0 in range(0, patches.shape[0], step):
+            evs = [] if phase_events is not None else None
+            t = self.score_sharded_async(patches[b0:b0 + step], feature_map_dims, out_hw, full, group, distribute, b0, evs)
+            if phase_events is not None:
+                phase_events.append(evs)
             if pending is not None:
                 results.extend(pending.wait())
-            return results
-        self._order_after_producer(patches)
-        with torch.cuda.stream(self.stream()):
-            for k, b0 in enumerate(range(0, Btot, step)):
-                chunk = patches[b0:b0 + step]
-                B = chunk.shape[0]
-                slot = k & 1
-                res, outs, _ = self._alloc_out(B, P, out_hw, full)
-                if not chunk.is_cuda and world > 1 and B * P >= 1024:
-                    chunk = self._stage_sharded(chunk, slot, world, rank, group, torch.cuda.current_stream(chunk.device if chunk.is_cuda else torch.device('cuda', self.device)))
-                keys = self._shard_buf("keys", slot, (B * P,), torch.int64)
-                L.check(self._lib.cmdb_score_shard_min(self._h, _ptr(chunk), B, P, int(chunk.is_cuda), int(out_hw), _ptr(keys)))
-                dist.all_reduce(keys, op=dist.ReduceOp.MIN, group=group)
-                m_star = self._shard_buf("m_star", slot, (B * self.dim,), torch.float32)
-                L.check(self._lib.cmdb_score_shard_select(self._h, _ptr(keys), B, P, _ptr(m_star)))
-                dist.all_reduce(m_star, op=dist.ReduceOp.SUM, group=group)
-                top = self._shard_buf("top", slot, (B * 3,), torch.int64)
-                L.check(self._lib.cmdb_score_shard_topk(self._h, _ptr(m_star), B, P, _ptr(top)))
-                gathered = self._shard_buf("gathered", slot, (world * B * 3,), torch.int64)
-                dist.all_gather_into_tensor(gathered, top, group=group)
-                nn_rows = self._shard_buf("nn_rows", slot, (B * 3 * self.dim,), torch.float32)
-                L.check(self._lib.cmdb_score_shard_nn(self._h, _ptr(gathered), world, B, _ptr(nn_rows)))
-                dist.all_reduce(nn_rows, op=dist.ReduceOp.SUM, group=group)
-                # image i of this round has global index b0 + i and belongs to rank (b0 + i) % world
-                first, stride = ((rank - b0) % world, world) if distribute else (0, 1)
-                L.check(self._lib.cmdb_score_shard_finish(self._h, _ptr(nn_rows), B, P, int(fh), int(fw), int(out_hw),
-                                                          int(first), int(stride), outs))
-                if distribute:
-                    res.owned = set(range(first, B, stride))
-                results.extend(res)
+            pending = t
+        if pending is not None:
+            results.extend(pending.wait())
         return results
 
 

@@ -34,24 +34,12 @@ __global__ void unpack_keys_kernel(const long long *__restrict__ keys, int P, in
         atomicMax(s_key + i / P_img, ((unsigned long long)__float_as_uint(v) << 32) | (0xffffffffu - (unsigned int)(i % P_img)));
     }
 }
-// out[c] = bank[global_row - offset][c] if this shard owns the row, else 0
-__global__ void contrib_rows_kernel(const float *__restrict__ bank, long long rows, long long row_offset, int dim,
-                                    const long long *__restrict__ global_rows, const unsigned long long *__restrict__ keys,
-                                    int n, float *__restrict__ out) {
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n * dim; i += gridDim.x * blockDim.x) {
-        const int r = i / dim, c = i - r * dim;
-        long long g = global_rows ? global_rows[r] : (keys[r] == ~0ULL ? -1 : (long long)(keys[r] & 0xffffffffULL));
-        const long long l = g - row_offset;
-        out[i] = (g >= 0 && l >= 0 && l < rows) ? bank[(size_t)l * dim + c] : 0.f;
-    }
-}
 
 void api_prefer_carveout_fuse();
 void api_prefer_carveout() {
     api_prefer_carveout_fuse();
     CMDB_PREFER_MAX_SMEM(pack_keys_kernel);
     CMDB_PREFER_MAX_SMEM(unpack_keys_kernel);
-    CMDB_PREFER_MAX_SMEM(contrib_rows_kernel);
     (void)cudaGetLastError();
 }
 
@@ -68,9 +56,6 @@ static int stage_alloc(cmdb_bank *b, int B, int P, int out_hw) {
     return score_scratch_alloc(b, B, P, out_hw);
 }
 
-// device->host copy of the result block of a sub-batch, then scatter into the caller's buffers.  All images: ONE copy.
-// A strided subset (sharded finish: this rank owns images img_first, img_first + img_step, ...): the scalar / per-patch
-// prefix in one copy plus one map copy per owned image.
 // bytes of the result block that a full-batch copy has to move (want: bit 0 = pre-blur maps, bit 1 = 8-bit maps)
 static size_t out_block_extent(const cmdb_bank *b, int B, unsigned want) {
     const ScoreScratch &s = b->ss;
@@ -79,14 +64,14 @@ static size_t out_block_extent(const cmdb_bank *b, int B, unsigned want) {
     if (want & 2u) bytes = s.off_map_u8 + s.map_stride * B;
     return bytes;
 }
-static unsigned want_mask_of(const cmdb_score_out *outs, int B, int first = 0, int step = 1) {
+static unsigned want_mask_of(const cmdb_score_out *outs, int B) {
     unsigned w = 0;
-    for (int i = first; i < B; i += step) w |= (outs[i].s_map_pre ? 1u : 0u) | (outs[i].s_map_u8 ? 2u : 0u);
+    for (int i = 0; i < B; ++i) w |= (outs[i].s_map_pre ? 1u : 0u) | (outs[i].s_map_u8 ? 2u : 0u);
     return w;
 }
 
 // host block of a slot -> the caller's buffers (maps = false: only the scalars and per-patch arrays of image i)
-static void scatter_one(const cmdb_bank *b, const unsigned char *h, int i, int P, int out_hw, cmdb_score_out *out, bool maps = true) {
+static void scatter_one(const cmdb_bank *b, const unsigned char *h, int i, int P, int out_hw, cmdb_score_out *out, bool maps) {
     const ScoreScratch &s = b->ss;
     const size_t npix = (size_t)out_hw * out_hw;
     TailResult tr;
@@ -105,35 +90,6 @@ static void scatter_one(const cmdb_bank *b, const unsigned char *h, int i, int P
     if (out->m_star_knn) out->m_star_knn[0] = tr.knn0, out->m_star_knn[1] = tr.knn1;
     if (out->nn_idx)
         for (int k = 0; k < 3; ++k) out->nn_idx[k] = tr.nn_idx[k];
-}
-static void scatter_outputs(const cmdb_bank *b, const unsigned char *h, int B, int P, int out_hw, cmdb_score_out *outs,
-                            int img_first = 0, int img_step = 1) {
-    for (int i = img_first; i < B; i += img_step) scatter_one(b, h, i, P, out_hw, outs + i);
-}
-
-// sharded finish: device->host copy of the result block (all images: ONE copy; a strided subset -- this rank owns images
-// img_first, img_first + img_step, ... -- the scalar / per-patch prefix in one copy plus one map copy per owned image),
-// then scatter into the caller's buffers
-static int copy_outputs(cmdb_bank *b, int B, int P, int out_hw, cmdb_score_out *outs, int img_first, int img_step) {
-    ScoreScratch &s = b->ss;
-    cudaStream_t st = b->stream;
-    const size_t npix = (size_t)out_hw * out_hw;
-    const unsigned want = want_mask_of(outs, B, img_first, img_step);
-    if (img_step == 1 && img_first == 0) {
-        CMDB_CUDA(cudaMemcpyAsync(s.out_block_host, s.out_block, out_block_extent(b, B, want), cudaMemcpyDeviceToHost, st));
-    } else {
-        CMDB_CUDA(cudaMemcpyAsync(s.out_block_host, s.out_block, s.off_map_out, cudaMemcpyDeviceToHost, st));
-        for (int i = img_first; i < B; i += img_step) {
-            const size_t o1 = s.off_map_out + sizeof(float) * s.map_stride * i, o2 = s.off_map_pre + sizeof(float) * s.map_stride * i;
-            const size_t o3 = s.off_map_u8 + s.map_stride * i;
-            CMDB_CUDA(cudaMemcpyAsync(s.out_block_host + o1, s.out_block + o1, sizeof(float) * npix, cudaMemcpyDeviceToHost, st));
-            if (want & 1u) CMDB_CUDA(cudaMemcpyAsync(s.out_block_host + o2, s.out_block + o2, sizeof(float) * npix, cudaMemcpyDeviceToHost, st));
-            if (want & 2u) CMDB_CUDA(cudaMemcpyAsync(s.out_block_host + o3, s.out_block + o3, npix, cudaMemcpyDeviceToHost, st));
-        }
-    }
-    CMDB_CUDA(cudaStreamSynchronize(st));
-    scatter_outputs(b, s.out_block_host, B, P, out_hw, outs, img_first, img_step);
-    return CMDB_OK;
 }
 
 static int blur_batch(cmdb_bank *b, int B, int fh, int fw, int out_hw, int img_first = 0, int img_step = 1) {
@@ -344,7 +300,7 @@ static int submit_sub_batch(cmdb_bank *b, const float *src, int is_device, int b
                               (host_maps ? out_block_extent(b, bc, want) : s.off_map_out) - s.off_min_val, cudaMemcpyDeviceToHost,
                               b->d2h_stream));
     CMDB_MARK(CMDB_T_REWEIGHT);
-    CMDB_CHECK(score_reweight(b, bc, P, true));
+    CMDB_CHECK(score_reweight(b, bc, P));
     CMDB_MARK(CMDB_T_OUT);
     CMDB_CUDA(cudaEventRecord(b->ev_compute[slot], st));
     CMDB_CUDA(cudaStreamWaitEvent(b->d2h_stream, b->ev_compute[slot], 0));
@@ -352,17 +308,28 @@ static int submit_sub_batch(cmdb_bank *b, const float *src, int is_device, int b
     CMDB_CUDA(cudaEventRecord(b->ev_done[slot], b->d2h_stream));
     if (b->timing) CMDB_CUDA(cudaEventRecord(b->timing == 2 ? b->ev_tl[lane][CMDB_T_COUNT] : b->ev[CMDB_T_COUNT], b->d2h_stream));
 #undef CMDB_MARK
+    if (b->timing == 1) b->ev_valid = true;  // only batches record the stage events, sharded rounds do not
     cmdb_bank::Pending &pd = b->pending[slot];
     pd.active = true, pd.B = bc, pd.P = P, pd.out_hw = out_hw, pd.want = want, pd.host_maps = host_maps;
+    pd.img_first = 0, pd.img_step = 1;
     return CMDB_OK;
 }
 
+// Waits for a submitted batch or sharded round and fills outs[0 .. B): the scalars and per-patch arrays of every image,
+// the maps of images img_first, img_first + img_step, ... (all of them for a batch; a sharded round only finished those).
 static int wait_slot(cmdb_bank *b, int slot, cmdb_score_out *outs) {
     cmdb_bank::Pending &pd = b->pending[slot];
     CMDB_CUDA(cudaEventSynchronize(b->ev_done[slot]));
     pd.active = false;
-    scatter_outputs(b, b->ss.out_block_host_buf[slot], pd.B, pd.P, pd.out_hw, outs);
-    if (b->timing == 1) b->ev_valid = true;
+    if (b->shard_abort_host && *b->shard_abort_host) {
+        set_error("a peer rank did not arrive at the exchange of a sharded round within the timeout (all ranks must submit "
+                  "the same rounds in the same order)");
+        return CMDB_ERR_CUDA;
+    }
+    for (int i = 0; i < pd.B; ++i) {
+        const bool maps = i >= pd.img_first && (i - pd.img_first) % pd.img_step == 0;
+        scatter_one(b, b->ss.out_block_host_buf[slot], i, pd.P, pd.out_hw, outs + i, maps);
+    }
     return CMDB_OK;
 }
 
@@ -417,15 +384,19 @@ int cmdb_score_batch_submit(cmdb_bank *b, const float *patches, int B, int P, in
     return CMDB_OK;
 }
 
-int cmdb_score_batch_wait(cmdb_bank *b, int64_t ticket, cmdb_score_out *outs) {
-    CMDB_REQUIRE(b && outs, CMDB_ERR_INVALID, "cmdb_score_batch_wait: NULL argument");
+static int wait_ticket(cmdb_bank *b, int64_t ticket, cmdb_score_out *outs, const char *fn) {
+    CMDB_REQUIRE(b && outs, CMDB_ERR_INVALID, "%s: NULL argument", fn);
     for (int slot = 0; slot < kResultSlots; ++slot)
         if (b->pending[slot].active && b->pending[slot].ticket == ticket) {
             CMDB_CUDA(cudaSetDevice(b->device));
             return wait_slot(b, slot, outs);
         }
-    set_error("cmdb_score_batch_wait: ticket %lld is not outstanding", (long long)ticket);
+    set_error("%s: ticket %lld is not outstanding", fn, (long long)ticket);
     return CMDB_ERR_STATE;
+}
+
+int cmdb_score_batch_wait(cmdb_bank *b, int64_t ticket, cmdb_score_out *outs) {
+    return wait_ticket(b, ticket, outs, "cmdb_score_batch_wait");
 }
 
 int cmdb_score(cmdb_bank *b, const float *patch, int P, int fh, int fw, int out_hw, int patch_is_device,
@@ -466,64 +437,6 @@ int cmdb_score_shard_min(cmdb_bank *b, const float *patches, int B, int P, int p
     return CMDB_OK;  // stream-ordered on the handle's stream (cmdb_bank_stream): run the collective there
 }
 
-int cmdb_score_shard_select(cmdb_bank *b, const int64_t *reduced_keys_device, int B, int P, float *m_star_contrib_device) {
-    CMDB_CHECK(check_score_args(b, reduced_keys_device, B, P, "cmdb_score_shard_select"));
-    CMDB_REQUIRE(m_star_contrib_device && B * P <= b->ss.cap_p && B <= b->ss.cap_b, CMDB_ERR_INVALID,
-                 "cmdb_score_shard_select: bad arguments (call cmdb_score_shard_min first)");
-    CMDB_CUDA(cudaSetDevice(b->device));
-    cudaStream_t st = b->stream;
-    CMDB_CUDA(cudaMemsetAsync(b->ss.s_key, 0, sizeof(unsigned long long) * B, st));
-    unpack_keys_kernel<<<(B * P + 255) / 256, 256, 0, st>>>((const long long *)reduced_keys_device, B * P, P, b->ss.min_val,
-                                                            b->ss.min_idx, b->ss.s_key);
-    CMDB_CHECK(score_select(b, B, P, true));  // m_star rows this rank owns, zeros elsewhere
-    CMDB_CUDA(cudaMemcpyAsync(m_star_contrib_device, b->ss.m_star, sizeof(float) * (size_t)B * b->dim, cudaMemcpyDeviceToDevice, st));
-    return CMDB_OK;
-}
-
-int cmdb_score_shard_topk(cmdb_bank *b, const float *m_star_device, int B, int P, int64_t *topk_keys_device) {
-    CMDB_CHECK(check_score_args(b, m_star_device, B, P, "cmdb_score_shard_topk"));
-    CMDB_REQUIRE(topk_keys_device && B <= b->ss.cap_b, CMDB_ERR_INVALID, "cmdb_score_shard_topk: bad arguments");
-    CMDB_CUDA(cudaSetDevice(b->device));
-    cudaStream_t st = b->stream;
-    CMDB_CUDA(cudaMemcpyAsync(b->ss.m_star, m_star_device, sizeof(float) * (size_t)B * b->dim, cudaMemcpyDeviceToDevice, st));
-    CMDB_CHECK(score_reweight(b, B, P, false));
-    CMDB_CUDA(cudaMemcpyAsync(topk_keys_device, b->ss.top3, sizeof(long long) * 3 * B, cudaMemcpyDeviceToDevice, st));
-    return CMDB_OK;
-}
-
-int cmdb_score_shard_nn(cmdb_bank *b, const int64_t *gathered_keys_device, int n_ranks, int B, float *nn_rows_contrib_device) {
-    CMDB_CHECK(check_score_args(b, gathered_keys_device, B, 1, "cmdb_score_shard_nn"));
-    CMDB_REQUIRE(nn_rows_contrib_device && n_ranks >= 1 && n_ranks <= b->ss.n_topk_blocks && B <= b->ss.cap_b, CMDB_ERR_INVALID,
-                 "cmdb_score_shard_nn: bad arguments");
-    CMDB_CUDA(cudaSetDevice(b->device));
-    cudaStream_t st = b->stream;
-    CMDB_CUDA(cudaMemcpyAsync(b->ss.topk_keys, gathered_keys_device, sizeof(long long) * 3 * (size_t)n_ranks * B,
-                              cudaMemcpyDeviceToDevice, st));
-    CMDB_CHECK(score_merge_top3(b, n_ranks, B));
-    contrib_rows_kernel<<<8 * B, 256, 0, st>>>(b->data, b->fin_rows, b->row_offset, b->dim, nullptr, b->ss.top3, 3 * B,
-                                               nn_rows_contrib_device);
-    CMDB_CUDA(cudaGetLastError());
-    return CMDB_OK;
-}
-
-int cmdb_score_shard_finish(cmdb_bank *b, const float *nn_rows_device, int B, int P, int fh, int fw, int out_hw,
-                            int img_first, int img_step, cmdb_score_out *outs) {
-    CMDB_CHECK(check_score_args(b, nn_rows_device, B, P, "cmdb_score_shard_finish"));
-    CMDB_REQUIRE(outs && fh > 0 && fw > 0 && fh * fw == P && B * P <= b->ss.cap_p && B <= b->ss.cap_b, CMDB_ERR_INVALID,
-                 "cmdb_score_shard_finish: bad arguments");
-    CMDB_REQUIRE((size_t)out_hw * out_hw == b->ss.map_stride, CMDB_ERR_INVALID,
-                 "cmdb_score_shard_finish: out_hw differs from cmdb_score_shard_min");
-    CMDB_REQUIRE(img_first >= 0 && img_step >= 1, CMDB_ERR_INVALID, "cmdb_score_shard_finish: bad image subset");
-    CMDB_CUDA(cudaSetDevice(b->device));
-    CMDB_CUDA(cudaMemcpyAsync(b->ss.nn_rows, nn_rows_device, sizeof(float) * 3 * (size_t)B * b->dim, cudaMemcpyDeviceToDevice,
-                              b->stream));
-    CMDB_CHECK(score_final(b, B));
-    CMDB_CHECK(blur_batch(b, B, fh, fw, out_hw, img_first, img_step));
-    return copy_outputs(b, B, P, out_hw, outs, img_first, img_step);
-}
-
-// ---- sharded rounds with the replicated neighbour table: min -> [MIN all-reduce] -> lookup -> [SUM all-reduce] -> finish ----
-
 int cmdb_score_shard_lookup(cmdb_bank *b, const int64_t *reduced_keys_device, int B, int P, float *knn_d2_contrib_device) {
     CMDB_CHECK(check_score_args(b, reduced_keys_device, B, P, "cmdb_score_shard_lookup"));
     CMDB_REQUIRE(knn_d2_contrib_device && B * P <= b->ss.cap_p && B <= b->ss.cap_b, CMDB_ERR_INVALID,
@@ -539,16 +452,8 @@ int cmdb_score_shard_lookup(cmdb_bank *b, const int64_t *reduced_keys_device, in
     return score_shard_lookup(b, B, knn_d2_contrib_device);
 }
 
-static int shard_finish_enqueue(cmdb_bank *b, const float *knn_d2_sum_device, int B, int P, int fh, int fw, int out_hw,
-                                int img_first, int img_step, unsigned want_maps, int64_t *out_ticket);
-
 int cmdb_score_shard_finish_submit(cmdb_bank *b, const float *knn_d2_sum_device, int B, int P, int fh, int fw, int out_hw,
                                    int img_first, int img_step, unsigned want_maps, int64_t *out_ticket) {
-    return shard_finish_enqueue(b, knn_d2_sum_device, B, P, fh, fw, out_hw, img_first, img_step, want_maps, out_ticket);
-}
-
-static int shard_finish_enqueue(cmdb_bank *b, const float *knn_d2_sum_device, int B, int P, int fh, int fw, int out_hw,
-                                int img_first, int img_step, unsigned want_maps, int64_t *out_ticket) {
     CMDB_CHECK(check_score_args(b, knn_d2_sum_device, B, P, "cmdb_score_shard_finish_submit"));
     CMDB_REQUIRE(out_ticket && fh > 0 && fw > 0 && fh * fw == P && B * P <= b->ss.cap_p && B <= b->ss.cap_b, CMDB_ERR_INVALID,
                  "cmdb_score_shard_finish_submit: bad arguments");
@@ -633,7 +538,7 @@ int cmdb_score_shard_round_submit(cmdb_bank *b, const float *patches, int B, int
     if (!busy && (size_t)out_hw * out_hw != b->ss.map_stride) score_scratch_free(b);
     CMDB_REQUIRE(!busy || (size_t)out_hw * out_hw == b->ss.map_stride, CMDB_ERR_STATE,
                  "cmdb_score_shard_round_submit: out_hw changes while a submitted round is outstanding; wait for it first");
-    const int slot = b->next_slot, lane = b->next_lane;   // advanced by shard_finish_enqueue
+    const int slot = b->next_slot, lane = b->next_lane;   // advanced by cmdb_score_shard_finish_submit
     CMDB_REQUIRE(!b->pending[slot].active, CMDB_ERR_STATE,
                  "cmdb_score_shard_round_submit: three submitted rounds are outstanding on this handle; wait for one first");
     CMDB_CHECK(stage_alloc(b, B, P, out_hw));
@@ -647,45 +552,11 @@ int cmdb_score_shard_round_submit(cmdb_bank *b, const float *patches, int B, int
     float *contrib = b->shard_d2 + xslot * kShardD2Cap, *d2_sum = b->shard_d2 + (kShardSlots + xslot) * kShardD2Cap;
     CMDB_CHECK(score_shard_lookup(b, B, contrib));
     CMDB_CHECK(score_shard_exchange_d2(b, B, peers, world, rank, xslot, epoch, contrib, d2_sum));
-    return shard_finish_enqueue(b, d2_sum, B, P, fh, fw, out_hw, img_first, img_step, want_maps, out_ticket);
+    return cmdb_score_shard_finish_submit(b, d2_sum, B, P, fh, fw, out_hw, img_first, img_step, want_maps, out_ticket);
 }
 
 int cmdb_score_shard_wait(cmdb_bank *b, int64_t ticket, cmdb_score_out *outs) {
-    CMDB_REQUIRE(b && outs, CMDB_ERR_INVALID, "cmdb_score_shard_wait: NULL argument");
-    for (int slot = 0; slot < kResultSlots; ++slot) {
-        cmdb_bank::Pending &pd = b->pending[slot];
-        if (!pd.active || pd.ticket != ticket) continue;
-        CMDB_CUDA(cudaSetDevice(b->device));
-        CMDB_CUDA(cudaEventSynchronize(b->ev_done[slot]));
-        pd.active = false;
-        if (b->shard_abort_host && *b->shard_abort_host) {
-            set_error("cmdb_score_shard_wait: a peer rank did not arrive at the exchange of this round within the timeout (all ranks "
-                      "must submit the same rounds in the same order)");
-            return CMDB_ERR_CUDA;
-        }
-        // maps: the images this rank finished; the scalars and per-patch arrays are replicated, so every image gets those
-        for (int i = 0; i < pd.B; ++i) {
-            const bool mine = i >= pd.img_first && (i - pd.img_first) % pd.img_step == 0;
-            scatter_one(b, b->ss.out_block_host_buf[slot], i, pd.P, pd.out_hw, outs + i, mine);
-        }
-        return CMDB_OK;
-    }
-    set_error("cmdb_score_shard_wait: ticket %lld is not outstanding", (long long)ticket);
-    return CMDB_ERR_STATE;
-}
-
-// plain host -> device copy on the handle's stream (stream-ordered with the phases that follow); used by the Python side to
-// stage its slice of a round's queries without involving torch's pinned-memory bookkeeping
-int cmdb_bank_stage_h2d(cmdb_bank *b, void *dst_device, const void *src_host, size_t bytes) {
-    CMDB_REQUIRE(b && dst_device && src_host, CMDB_ERR_INVALID, "cmdb_bank_stage_h2d: NULL argument");
-    if (bytes == 0) return CMDB_OK;
-    CMDB_CUDA(cudaSetDevice(b->device));
-    // on the copy stream, so that it overlaps the kernels already queued on the compute stream; the compute stream picks the
-    // data up through an event.  (The caller guarantees that dst_device is not read by earlier, still running work.)
-    CMDB_CUDA(cudaMemcpyAsync(dst_device, src_host, bytes, cudaMemcpyHostToDevice, b->copy_stream));
-    CMDB_CUDA(cudaEventRecord(b->ev_stage, b->copy_stream));
-    for (auto st : b->lane_stream) CMDB_CUDA(cudaStreamWaitEvent(st, b->ev_stage, 0));  // whichever lane runs the round
-    return CMDB_OK;
+    return wait_ticket(b, ticket, outs, "cmdb_score_shard_wait");
 }
 
 int cmdb_bank_read_device(cmdb_bank *b, int64_t row0, int64_t n_rows, float *out_device) {

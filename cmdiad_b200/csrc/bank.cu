@@ -277,7 +277,6 @@ int cmdb_bank_create(int device, int dim, int64_t capacity_rows, cmdb_bank **out
     for (auto &e : b->ev_compute)
         if (err == cudaSuccess) err = cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
     if (err == cudaSuccess) err = cudaEventCreateWithFlags(&b->ev_fail, cudaEventDisableTiming);
-    if (err == cudaSuccess) err = cudaEventCreateWithFlags(&b->ev_stage, cudaEventDisableTiming);
     for (auto &e : b->ev_chunk)
         if (err == cudaSuccess) err = cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
     if (err == cudaSuccess) err = cudaMalloc(&b->data, sizeof(float) * (size_t)capacity_rows * dim);
@@ -356,7 +355,6 @@ void cmdb_bank_destroy(cmdb_bank *b) {
     for (auto &e : b->ev_compute)
         if (e) cudaEventDestroy(e);
     if (b->ev_fail) cudaEventDestroy(b->ev_fail);
-    if (b->ev_stage) cudaEventDestroy(b->ev_stage);
     for (auto &e : b->ev_chunk)
         if (e) cudaEventDestroy(e);
     delete b;

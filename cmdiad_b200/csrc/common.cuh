@@ -88,7 +88,6 @@ struct ScoreScratch {
     void *tmap_qlo = nullptr;
     float *m_test = nullptr;        // [D] patch[s_idx]
     float *m_star = nullptr;        // [D] bank[min_idx[s_idx]]
-    float *nn_rows = nullptr;       // [3, D] rows of the 3 nearest neighbours (sharded mode)
     unsigned long long *top3 = nullptr;  // merged 3 smallest w_dist keys
     int n_topk_blocks = 0;
     unsigned int *done_counter = nullptr;  // last-block-done counter of reweight_kernel
@@ -163,13 +162,12 @@ struct cmdb_bank {
     cudaEvent_t ev_done[cmdb::kResultSlots] = {};   // result slot's block is in the pinned host memory
     cudaEvent_t ev_compute[cmdb::kResultSlots] = {};   // the kernels of the call that used the slot are done (its q_f32 may be overwritten)
     cudaEvent_t ev_fail = nullptr;        // the certificate counters of the last certified call are on the host
-    cudaEvent_t ev_stage = nullptr;       // cmdb_bank_stage_h2d: the staged bytes are on the device
     struct Pending {
         bool active = false;
         int B = 0, P = 0, out_hw = 0;
         unsigned want = 0;
         bool host_maps = true;   // false: the per-modality maps stay in HBM (fused late-fusion head), only scalars travel
-        int img_first = 0, img_step = 1;  // sharded rounds: the images whose maps this rank finished
+        int img_first = 0, img_step = 1;  // images whose maps were finished (a sharded round's rank: its share; a batch: all)
         long long ticket = 0;
     } pending[cmdb::kResultSlots];
     bool any_pending() const {
@@ -329,7 +327,7 @@ int score_simt_candidates(cmdb_bank *b, int P, int *n_cand_out);
 int score_refine(cmdb_bank *b, int B, int P_img, int n_cand, bool compact);
 int score_refine_certified(cmdb_bank *b, int B, int P_img, int n_cand);
 int score_select(cmdb_bank *b, int B, int P_img, bool local_m_star);
-int score_reweight(cmdb_bank *b, int B, int P_img, bool fused);
+int score_reweight(cmdb_bank *b, int B, int P_img);
 int score_build_knn_table(cmdb_bank *b, long long row_first, long long row_count);
 int score_exact_scan(cmdb_bank *b, const float *q_dev, int P, unsigned long long *keys_dev);
 int score_shard_lookup(cmdb_bank *b, int B, float *contrib_dev);
@@ -341,8 +339,6 @@ struct PeerPtrs {
 int score_shard_exchange_keys(cmdb_bank *b, int B, int P_img, const PeerPtrs &peers, int world, int rank, int slot, unsigned long long epoch);
 int score_shard_exchange_d2(cmdb_bank *b, int B, const PeerPtrs &peers, int world, int rank, int slot, unsigned long long epoch,
                             const float *contrib_dev, float *d2_sum_dev);
-int score_merge_top3(cmdb_bank *b, int n_ranks, int B);
-int score_final(cmdb_bank *b, int B);
 int upsample_blur_launch(cudaStream_t stream, int n_img, int img_first, int img_step, size_t map_stride, const float *map_dev,
                          int fh, int fw, int out_hw, float *pre_dev, float *out_dev, unsigned char *u8_dev,
                          unsigned char *tmp_dev, float *mx_dev, float *mx_part_dev /* [n images][16] band maxima */);

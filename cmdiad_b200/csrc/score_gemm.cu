@@ -606,7 +606,7 @@ void gemm_prefer_carveout() {
 static void free_lane(ScoreScratch &s) {
     cudaFree(s.q_hi), cudaFree(s.q_lo), cudaFree(s.q_scale_exp);
     cudaFree(s.cand), cudaFree(s.topk_keys);   // s_key lives inside the fail_ctl allocation
-    cudaFree(s.map_tmp), cudaFree(s.map_max), cudaFree(s.m_test), cudaFree(s.m_star), cudaFree(s.nn_rows);
+    cudaFree(s.map_tmp), cudaFree(s.map_max), cudaFree(s.m_test), cudaFree(s.m_star);
     cudaFree(s.top3), cudaFree(s.done_counter);
     cudaFree(s.q_norm), cudaFree(s.q_eps), cudaFree(s.fail_list), cudaFree(s.fail_ctl);
     cudaFree(s.work_list), cudaFree(s.best_key);
@@ -745,7 +745,6 @@ int score_scratch_alloc(cmdb_bank *b, int B, int P_img, int out_hw) {
         CMDB_CUDA(cudaMalloc(&s.top3, sizeof(unsigned long long) * 3 * cap_b));
         CMDB_CUDA(cudaMalloc(&s.m_test, sizeof(float) * D * cap_b));
         CMDB_CUDA(cudaMalloc(&s.m_star, sizeof(float) * D * cap_b));
-        CMDB_CUDA(cudaMalloc(&s.nn_rows, sizeof(float) * 3 * D * cap_b));
         s.cap_p = cap_p, s.cap_b = cap_b, s.map_cap = map_cap;
         CMDB_CHECK(make_map(&s.tmap_qhi, s.q_hi, cap_p, b->dim, BM));
         CMDB_CHECK(make_map(&s.tmap_qlo, s.q_lo, cap_p, b->dim, BM));

@@ -801,18 +801,16 @@ struct ReweightParams {
     const float *q;                  // [B*P_img, dim] normalised patches
     const unsigned long long *s_key; // [B] packed argmax of min_val
     const long long *min_idx;        // [B*P_img] global rows
-    const float *m_star_explicit;    // sharded mode: replicated m_star rows [B, dim]; NULL = take them from the local bank
     unsigned long long *block_keys;  // [B][gridDim.x * 3]
     unsigned long long *top3;        // [B][3] merged result
     unsigned int *done_counter;      // last-block-done counter (self resetting)
     TailResult *res;                 // [B]
-    int fuse_final;                  // 1: the last block also computes m_star_knn, w, s (single-GPU path)
 };
 
 // w_dist pass (features.py:239-254) for a batch of B images in ONE sweep over the bank: every warp keeps a bank row in
 // registers and evaluates its exact squared distance to all B m_star rows (shared memory), so the bank is read once
 // per batch (rows*dim*4 bytes).  Prologue = "select" (decode s*, s_idx, locate m_star); epilogue = last-block-done
-// merge (+ final re-weighting), so the whole re-weighting stage is one launch.
+// merge + final re-weighting, so the whole re-weighting stage is one launch.
 template <int DV>  // float4 vectors per lane: ceil(dim / 128)
 __global__ void __launch_bounds__(256) reweight_kernel(ReweightParams p) {
     extern __shared__ __align__(16) float ms[];  // [B][dim] m_star rows, then wtop [8][B][3]
@@ -832,7 +830,7 @@ __global__ void __launch_bounds__(256) reweight_kernel(ReweightParams p) {
     __syncthreads();
     for (int i = threadIdx.x; i < B * dim; i += blockDim.x) {
         const int b = i / dim, c = i - b * dim;
-        ms[i] = p.m_star_explicit ? p.m_star_explicit[i] : p.bank[(size_t)(g_sh[b] - p.row_offset) * dim + c];
+        ms[i] = p.bank[(size_t)(g_sh[b] - p.row_offset) * dim + c];
     }
     __syncthreads();
     const float4 *ms4 = reinterpret_cast<const float4 *>(ms);
@@ -906,7 +904,7 @@ __global__ void __launch_bounds__(256) reweight_kernel(ReweightParams p) {
     if (threadIdx.x == 0) is_last = atomicAdd(p.done_counter, 1u) == gridDim.x - 1;
     __syncthreads();
     if (!is_last) return;
-    // ---- last block: one warp per image merges every block's keys, then (single-GPU path) finishes the re-weighting ----
+    // ---- last block: one warp per image merges every block's keys, then finishes the re-weighting ----
     __threadfence();
     if (threadIdx.x == 0) *p.done_counter = 0;
     for (int b = warp; b < B; b += 8) {
@@ -917,15 +915,13 @@ __global__ void __launch_bounds__(256) reweight_kernel(ReweightParams p) {
         const unsigned long long skey = p.s_key[b];
         const float s_star = __uint_as_float((unsigned int)(skey >> 32));
         const int s_idx = s_idx_sh[b];
-        float knn[2] = {NAN, NAN};
-        if (p.fuse_final) {  // features.py:275-283: m_star_knn = ||m_test - bank[nn_idx[1:]]||, m_test = patch[s_idx]
+        float knn[2] = {NAN, NAN};  // features.py:275-283: m_star_knn = ||m_test - bank[nn_idx[1:]]||, m_test = patch[s_idx]
 #pragma unroll
-            for (int k = 0; k < 2; ++k)
-                if (f[1 + k] != ~0ULL)
-                    knn[k] = sqrtf(warp_sqdist(p.q + ((size_t)b * p.P_img + s_idx) * dim,
-                                               p.bank + (size_t)((long long)(f[1 + k] & 0xffffffffULL) - p.row_offset) * dim,
-                                               dim4, lane));
-        }
+        for (int k = 0; k < 2; ++k)
+            if (f[1 + k] != ~0ULL)
+                knn[k] = sqrtf(warp_sqdist(p.q + ((size_t)b * p.P_img + s_idx) * dim,
+                                           p.bank + (size_t)((long long)(f[1 + k] & 0xffffffffULL) - p.row_offset) * dim,
+                                           dim4, lane));
         if (lane == 0) {
             TailResult *res = p.res + b;
             p.top3[b * 3 + 0] = f[0], p.top3[b * 3 + 1] = f[1], p.top3[b * 3 + 2] = f[2];
@@ -933,14 +929,12 @@ __global__ void __launch_bounds__(256) reweight_kernel(ReweightParams p) {
             res->s_star = s_star;
             res->m_star_row = g_sh[b];
             for (int k = 0; k < 3; ++k) res->nn_idx[k] = f[k] == ~0ULL ? -1 : (long long)(f[k] & 0xffffffffULL);
-            if (p.fuse_final) {
-                const float Dn = sqrtf((float)dim);  // torch.sqrt(torch.tensor(patch.shape[1]))  (features.py:285)
-                const float den = expf(knn[0] / Dn) + expf(knn[1] / Dn);
-                const float w = 1.f - expf(s_star / Dn) / den;  // features.py:287
-                res->w = w;
-                res->s = w * s_star;  // features.py:290
-                res->knn0 = knn[0], res->knn1 = knn[1];
-            }
+            const float Dn = sqrtf((float)dim);  // torch.sqrt(torch.tensor(patch.shape[1]))  (features.py:285)
+            const float den = expf(knn[0] / Dn) + expf(knn[1] / Dn);
+            const float w = 1.f - expf(s_star / Dn) / den;  // features.py:287
+            res->w = w;
+            res->s = w * s_star;  // features.py:290
+            res->knn0 = knn[0], res->knn1 = knn[1];
         }
     }
 }
@@ -1302,42 +1296,6 @@ int score_shard_exchange_d2(cmdb_bank *b, int B, const PeerPtrs &peers, int worl
     return CMDB_OK;
 }
 
-// sharded mode, after the all-gather: image b = blockIdx.x merges the keys of all ranks ([rank][B][3] layout)
-__global__ void __launch_bounds__(32) merge_top3_kernel(const unsigned long long *__restrict__ gathered, int n_ranks, int B,
-                                                        unsigned long long *__restrict__ out3) {
-    const int b = blockIdx.x, lane = threadIdx.x;
-    unsigned long long t[3] = {~0ULL, ~0ULL, ~0ULL}, f[3];
-    for (int i = lane; i < n_ranks * 3; i += 32) top3_insert(t, gathered[((size_t)(i / 3) * B + b) * 3 + i % 3]);
-    warp_top3(t, f);
-    if (lane == 0) out3[b * 3 + 0] = f[0], out3[b * 3 + 1] = f[1], out3[b * 3 + 2] = f[2];
-}
-
-// final (sharded mode): image b = blockIdx.x.  m_star_knn = ||m_test - nn_rows[1:]|| (features.py:275-283), w and s
-// (:285-290); nn_rows [B][3][dim] are the replicated neighbour rows.
-__global__ void __launch_bounds__(64) final_kernel(const unsigned long long *__restrict__ top3, const float *__restrict__ m_test,
-                                                   const float *__restrict__ nn_rows, int dim, TailResult *res_all) {
-    const int b = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;  // 2 warps: one per neighbour
-    __shared__ float knn[2];
-    const unsigned long long *keys3 = top3 + b * 3;
-    TailResult *res = res_all + b;
-    const unsigned long long key = keys3[1 + warp];
-    const bool valid = key != ~0ULL;
-    float d2 = 0.f;
-    if (valid) d2 = warp_sqdist(m_test + (size_t)b * dim, nn_rows + ((size_t)b * 3 + 1 + warp) * dim, dim >> 2, lane);
-    if (lane == 0) knn[warp] = valid ? sqrtf(d2) : NAN;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        const float Dn = sqrtf((float)dim);
-        const float s_star = res->s_star;
-        const float den = expf(knn[0] / Dn) + expf(knn[1] / Dn);
-        const float w = 1.f - expf(s_star / Dn) / den;
-        res->w = w;
-        res->s = w * s_star;
-        res->knn0 = knn[0], res->knn1 = knn[1];
-        for (int k = 0; k < 3; ++k) res->nn_idx[k] = keys3[k] == ~0ULL ? -1 : (long long)(keys3[k] & 0xffffffffULL);
-    }
-}
-
 // ---------------------------------------------------------------------------------------------------------------
 // upsample + blur in two small multi-CTA kernels (the image is split into 16 row bands, then 16 column bands):
 //   K0  every CTA takes the max of its row band of the upsampled map (the global max is needed before the 8-bit
@@ -1505,13 +1463,11 @@ int score_select(cmdb_bank *b, int B, int P_img, bool local_m_star) {
     return CMDB_OK;
 }
 
-// fused = single-GPU path (select prologue + merge + final in one launch); otherwise the m_star rows come from
-// ss.m_star and only the merged top-3 keys (+ s*, s_idx) are produced
-// tensor-core variant: (select ->) fp16 split of the m_star rows -> hi.hi GEMM with one M tile -> reweight_cert_kernel
-static int score_reweight_tensor(cmdb_bank *b, int B, int P_img, bool fused) {
+// tensor-core variant: select -> fp16 split of the m_star rows -> hi.hi GEMM with one M tile -> reweight_cert_kernel
+static int score_reweight_tensor(cmdb_bank *b, int B, int P_img) {
     ScoreScratch &s = b->ss;
     cudaStream_t st = b->stream;
-    if (fused) CMDB_CHECK(score_select(b, B, P_img, true));  // m_test, m_star, s*, s_idx, m_star_row
+    CMDB_CHECK(score_select(b, B, P_img, true));  // m_test, m_star, s*, s_idx, m_star_row
     // the min/argmin phase is complete: its query operand buffers and candidate lists are free again
     q_split_rows(b, s.m_star, B);
     CMDB_CUDA(cudaGetLastError());
@@ -1526,7 +1482,7 @@ static int score_reweight_tensor(cmdb_bank *b, int B, int P_img, bool fused) {
     p.stride = score_tile_stride(1, p.n_units);
     p.nt = (int)(b->fin_rows_pad / kScoreBN);
     p.run = s.sched_run_last;
-    p.s_key = s.s_key, p.top3 = s.top3, p.res = reinterpret_cast<TailResult *>(s.tail), p.fuse_final = fused ? 1 : 0;
+    p.s_key = s.s_key, p.top3 = s.top3, p.res = reinterpret_cast<TailResult *>(s.tail), p.fuse_final = 1;
     CMDB_REQUIRE(n_cand <= 320, CMDB_ERR_UNSUPPORTED, "scoring: %d GEMM producers exceed reweight_cert_kernel's limit", n_cand);
     reweight_cert_kernel<<<B, 256, 0, st>>>(p);
     CMDB_CUDA(cudaGetLastError());
@@ -1576,8 +1532,8 @@ int score_build_knn_table(cmdb_bank *b, long long row_first, long long row_count
     return CMDB_OK;
 }
 
-int score_reweight(cmdb_bank *b, int B, int P_img, bool fused) {
-    if (fused && b->knn_table && b->row_offset == 0 && b->knn_rows == b->fin_rows) {  // the bank's neighbour table: the w_dist pass is a lookup
+int score_reweight(cmdb_bank *b, int B, int P_img) {
+    if (b->knn_table && b->row_offset == 0 && b->knn_rows == b->fin_rows) {  // the bank's neighbour table: the w_dist pass is a lookup
         CMDB_CHECK(score_select(b, B, P_img, true));
         reweight_lookup_kernel<<<B, 64, 0, b->stream>>>(b->knn_table, b->ss.m_test, b->data, b->dim, b->ss.s_key, b->ss.top3,
                                                         reinterpret_cast<TailResult *>(b->ss.tail));
@@ -1591,14 +1547,12 @@ int score_reweight(cmdb_bank *b, int B, int P_img, bool fused) {
         return e ? atoi(e) : -1;
     }();
     if (b->score_impl == CMDB_SCORE_TCGEN05 && b->prefilter_terms == 0 && B <= kScoreBM && (force == 1 || (force < 0 && B >= 2)))
-        return score_reweight_tensor(b, B, P_img, fused);
+        return score_reweight_tensor(b, B, P_img);
     ReweightParams p{};
     p.bank = b->data, p.rows = b->fin_rows, p.row_offset = b->row_offset, p.dim = b->dim, p.B = B, p.P_img = P_img;
     p.q = b->ss.q_f32, p.s_key = b->ss.s_key, p.min_idx = b->ss.min_idx;
-    p.m_star_explicit = fused ? nullptr : b->ss.m_star;
     p.block_keys = b->ss.topk_keys, p.top3 = b->ss.top3, p.done_counter = b->ss.done_counter;
     p.res = reinterpret_cast<TailResult *>(b->ss.tail);
-    p.fuse_final = fused ? 1 : 0;
     const size_t smem = sizeof(float) * (size_t)B * b->dim + sizeof(unsigned long long) * 8 * B * 3;
     const int blocks = b->ss.n_topk_blocks;
 #define CMDB_RW(DVV)                                                                                              \
@@ -1640,8 +1594,6 @@ void tail_prefer_carveout() {
     CMDB_PREFER_MAX_SMEM(select_kernel);
     CMDB_PREFER_MAX_SMEM(reweight_cert_kernel);
     CMDB_PREFER_MAX_SMEM(reweight_lookup_kernel);
-    CMDB_PREFER_MAX_SMEM(merge_top3_kernel);
-    CMDB_PREFER_MAX_SMEM(final_kernel);
     CMDB_PREFER_MAX_SMEM(shard_lookup_kernel);
     CMDB_PREFER_MAX_SMEM(shard_final_kernel);
     CMDB_PREFER_MAX_SMEM(shard_push_keys_kernel);
@@ -1652,19 +1604,6 @@ void tail_prefer_carveout() {
     CMDB_PREFER_MAX_SMEM(upsample_hblur_kernel);
     CMDB_PREFER_MAX_SMEM(vblur_kernel);
     (void)cudaGetLastError();
-}
-
-int score_merge_top3(cmdb_bank *b, int n_ranks, int B) {
-    merge_top3_kernel<<<B, 32, 0, b->stream>>>(b->ss.topk_keys, n_ranks, B, b->ss.top3);
-    CMDB_CUDA(cudaGetLastError());
-    return CMDB_OK;
-}
-
-int score_final(cmdb_bank *b, int B) {
-    final_kernel<<<B, 64, 0, b->stream>>>(b->ss.top3, b->ss.m_test, b->ss.nn_rows, b->dim,
-                                          reinterpret_cast<TailResult *>(b->ss.tail));
-    CMDB_CUDA(cudaGetLastError());
-    return CMDB_OK;
 }
 
 // images img_first, img_first + img_step, ... (n_img of them); per-image stride of the map buffers = map_stride pixels

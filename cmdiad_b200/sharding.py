@@ -34,17 +34,6 @@ def unpack_keys(keys):
     return d, keys & 0xFFFFFFFF
 
 
-def contribution(rows_local, row_offset, wanted_global_rows):
-    """[len(wanted), D] array holding the wanted rows this shard owns and zeros elsewhere: summing the contributions
-    of all ranks reproduces the rows exactly (x + 0 + ... + 0)."""
-    wanted = np.asarray(wanted_global_rows, dtype=np.int64)
-    out = np.zeros((len(wanted), rows_local.shape[1]), dtype=rows_local.dtype)
-    loc = wanted - row_offset
-    ok = (loc >= 0) & (loc < rows_local.shape[0])
-    out[ok] = rows_local[loc[ok]]
-    return out
-
-
 def stage_slice(n_rows, world, rank):
     """cooperative staging of a round's host queries (Bank._stage_sharded): rank r copies rows [lo, hi) over PCIe into
     a `per`-row block (zero padded), the blocks are all-gathered and cut back to n_rows.  Returns (per, lo, hi)."""

@@ -241,33 +241,6 @@ int cmdb_score_batch(cmdb_bank *bank, const float *patches, int B, int P, int fh
                      cmdb_score_out *outs);
 
 /*
- * Row-sharded scoring (one process per GPU, SURVEY 8e).  Every rank holds a contiguous block of bank rows
- * (cmdb_bank_set_row_offset) and the full, replicated batch of patches.  All buffers named *_device are device memory on
- * the bank's GPU, owned by the caller (torch tensors), so the collectives between the phases run on them directly.
- * B images per round (B <= 32 and B*dim*4 <= 160 KB); all five phases of one round use the same B, P, out_hw:
- *   1. cmdb_score_shard_min     keys[b*P+p] = (float_bits(local min distance) << 32) | global_row  -> all-reduce MIN (int64)
- *      (non-negative, so integer MIN == argmin with lowest-global-row tie-break)
- *   2. cmdb_score_shard_select  decodes the reduced keys (min_val, min_idx, s_star, s_idx per image); writes m_star[b] =
- *      the winning bank row if this rank owns it, zeros otherwise                                  -> all-reduce SUM (float[B*dim])
- *   3. cmdb_score_shard_topk    3 smallest local w_dist keys per image for the replicated m_star   -> all-gather (int64[B*3])
- *   4. cmdb_score_shard_nn      merges the gathered keys ([rank][B][3]); writes the neighbour rows this rank owns, zeros
- *      otherwise                                                                                   -> all-reduce SUM (float[B*3*dim])
- *   5. cmdb_score_shard_finish  m_star_knn, w, s, upsample + blur for images img_first, img_first + img_step, ... of the
- *      round (0, 1 = all images, identical results on every rank; rank, world = each rank finishes and returns only its
- *      share, the other outs[] entries are left untouched).
- * Phases 1-4 only enqueue work on the handle's stream (cmdb_bank_stream) and return; run the collectives on that same
- * stream (or synchronise it first).  Phase 5 returns when its host outputs are complete.
- */
-int cmdb_score_shard_min(cmdb_bank *bank, const float *patches, int B, int P, int patch_is_device, int out_hw,
-                         int64_t *keys_device);
-int cmdb_score_shard_select(cmdb_bank *bank, const int64_t *reduced_keys_device, int B, int P, float *m_star_contrib_device);
-int cmdb_score_shard_topk(cmdb_bank *bank, const float *m_star_device, int B, int P, int64_t *topk_keys_device);
-int cmdb_score_shard_nn(cmdb_bank *bank, const int64_t *gathered_keys_device, int n_ranks, int B,
-                        float *nn_rows_contrib_device);
-int cmdb_score_shard_finish(cmdb_bank *bank, const float *nn_rows_device, int B, int P, int fh, int fw, int out_hw,
-                            int img_first, int img_step, cmdb_score_out *outs);
-
-/*
  * Query normalisation on the device: with enabled != 0 every scoring entry point of this handle takes RAW patches and
  * applies (patch - mean) / std in float32 (one IEEE subtract, one IEEE divide == torch's CPU result) right after staging
  * them, i.e. the first line of compute_s_s_map (multiple_features.py:90, 976-977) moves behind the ABI.
@@ -333,19 +306,29 @@ int cmdb_eval_read(cmdb_bank *bank, int64_t first, int64_t n, double *maps_host 
                    double *scores_host /* [n] or NULL */);
 
 /*
- * Row-sharded scoring with the replicated neighbour table (cmdb_bank_set_knn_table): three phases and TWO small collectives
- * per round, and a submit / wait finish so that three rounds can be outstanding per handle (the result copy of round k and
- * the host work for the next rounds overlap the kernels of the other lane; nothing synchronises the host between the phases):
- *   1. cmdb_score_shard_min            as above                                                     -> all-reduce MIN (int64[B*P])
+ * Row-sharded scoring (one process per GPU, SURVEY 8e).  Every rank holds a contiguous block of bank rows
+ * (cmdb_bank_set_row_offset), the REPLICATED neighbour table of all global rows (cmdb_bank_set_knn_table) and the full
+ * batch of patches.  All buffers named *_device are device memory on the bank's GPU, owned by the caller (torch tensors),
+ * so the collectives between the phases run on them directly.  A round scores B images (B <= 32 and B*dim*4 <= 160 KB)
+ * in three phases with TWO small collectives; all phases of one round use the same B, P, out_hw:
+ *   1. cmdb_score_shard_min            keys[b*P+p] = (float_bits(local min distance) << 32) | global_row
+ *      (non-negative, so integer MIN == argmin with lowest-global-row tie-break)               -> all-reduce MIN (int64[B*P])
  *   2. cmdb_score_shard_lookup         decodes the reduced keys (min_val, min_idx, s*, s_idx, m_star row), reads the three
  *      nearest rows of m_star from the table and writes, per image, the exact SQUARED distances ||m_test - bank[nn_k]||^2
  *      (k = 1, 2; features.py:275-283) for the neighbour rows this rank owns, 0 for the others     -> all-reduce SUM (float[B*2])
  *   3. cmdb_score_shard_finish_submit  m_star_knn = sqrt(sum), w, s for all images; upsample + blur + device->host copy of
- *      the maps of images img_first, img_first + img_step, ...; returns a ticket without waiting.
+ *      the maps of images img_first, img_first + img_step, ... (0, 1 = all images; rank, world = each rank finishes only
+ *      its share); returns a ticket without waiting.
  *      cmdb_score_shard_wait(ticket, outs[B]) blocks until the round is complete: every outs[i] gets the scalars and
- *      per-patch arrays (replicated on all ranks), the maps are filled for the images this rank finished.
+ *      per-patch arrays (replicated on all ranks), the maps are filled for the images this rank finished (the map buffers
+ *      of the other outs[] entries are left untouched).
+ * Phases 1 and 2 only enqueue work on the handle's stream (cmdb_bank_stream) and return; run the collectives on that same
+ * stream.  Nothing synchronises the host between the phases, and three rounds can be outstanding per handle (the result
+ * copy of round k and the host work for the next rounds overlap the kernels of the other lane).
  * Results are bit-identical to cmdb_score_batch on the un-sharded bank.
  */
+int cmdb_score_shard_min(cmdb_bank *bank, const float *patches, int B, int P, int patch_is_device, int out_hw,
+                         int64_t *keys_device);
 int cmdb_score_shard_lookup(cmdb_bank *bank, const int64_t *reduced_keys_device, int B, int P, float *knn_d2_contrib_device);
 int cmdb_score_shard_finish_submit(cmdb_bank *bank, const float *knn_d2_sum_device, int B, int P, int fh, int fw, int out_hw,
                                    int img_first, int img_step, unsigned want_maps, int64_t *out_ticket);
@@ -357,14 +340,12 @@ int cmdb_score_shard_wait(cmdb_bank *bank, int64_t ticket, cmdb_score_out *outs)
  * round's slot of ALL ranks' buffers over NVLink and raises a flag (threadfence_system + release store by its last
  * block); the decode kernel waits for the world flags in its local buffer and takes the MIN while unpacking.  ~10 us per
  * exchange instead of two launches + an NCCL all-reduce (60 us at 8 ranks for the 98 KB of keys).  Collective: every
- * rank submits the same rounds in the same order; cmdb_score_shard_wait returns CMDB_ERR_CUDA if a peer never arrived.
+ * rank submits the same rounds in the same order; if a peer never arrived, cmdb_score_shard_wait and every later wait on
+ * the handle return CMDB_ERR_CUDA.
  */
 int cmdb_bank_attach_comm(cmdb_bank *bank, cmdb_comm *comm);
 int cmdb_score_shard_round_submit(cmdb_bank *bank, const float *patches, int B, int P, int fh, int fw, int out_hw,
                                   int patch_is_device, int img_first, int img_step, unsigned want_maps, int64_t *out_ticket);
-/* cudaMemcpyAsync(host -> device) on the handle's copy stream; everything enqueued on the handle afterwards sees the data.
- * dst_device must not be in use by work queued earlier (double-buffer it across rounds). */
-int cmdb_bank_stage_h2d(cmdb_bank *bank, void *dst_device, const void *src_host, size_t bytes);
 
 /*
  * Pixel-level evaluation of everything in the result store, on the device (features.py:321-324: pixel AUROC and the two

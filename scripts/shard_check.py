@@ -1,7 +1,8 @@
 """torchrun --nproc-per-node N scripts/shard_check.py : row-sharded scoring == single-GPU scoring, bit for bit.
 
-Covers both sharded protocols (five phases with the re-weighting sweep; three phases with the replicated neighbour
-table, pipelined rounds), replicated and distributed finishing, host and device queries, several rounds per call.
+Covers both transports of the sharded round with the replicated neighbour table (NCCL collectives; exchanges over
+peer-mapped memory), the table itself, replicated and distributed finishing, host and device queries, several rounds per
+call and pipelined rounds.
 Prints one line per check and a final SHARD CHECK OK / FAILED (rank 0); exit code 1 on failure."""
 import os
 import sys
@@ -47,8 +48,7 @@ pb = np.stack([synth.patches(P, D, seed=80 + t, anomalous_frac=0.01, cent=cent) 
 bb = full.score_batch(pb, (28, 28), 224, full=True)
 from cmdiad_b200 import Comm  # noqa: E402
 comm = Comm(local)
-for mode in ("five-phase", "table/nccl", "table/peer-memory"):
-    table = mode != "five-phase"
+for mode in ("table/nccl", "table/peer-memory"):
     if mode == "table/nccl":
         shard.build_knn_sharded()
         keys_sh = shard.read_knn(0, R).numpy()
@@ -66,23 +66,23 @@ for mode in ("five-phase", "table/nccl", "table/peer-memory"):
         mine = t % world == rank
         ok &= (dd[t] is not None) == mine and (not mine or same(dd[t], bb[t]))
     report(f"[{tag}] distributed finish (rank r returns images r, r+{world}, ...)", ok)
-    if table:  # scalars of the images finished elsewhere are replicated
-        arr = shard.score_sharded_batch(pb[:5], (28, 28), 224, distribute=True)
-        ok = all(float(arr[0].s[0]) == float(bb[0].s[0]) for _ in range(1)) if rank == 0 else True
-        report(f"[{tag}] scalars available on every rank", ok)
+    # scalars of the images finished elsewhere are replicated
+    arr = shard.score_sharded_batch(pb[:5], (28, 28), 224, distribute=True)
+    ok = all(float(arr[0].s[0]) == float(bb[0].s[0]) for _ in range(1)) if rank == 0 else True
+    report(f"[{tag}] scalars available on every rank", ok)
     for t in range(2):
         a = shard.score_sharded(pb[t], (28, 28), 224, full=True)
         report(f"[{tag}] single image {t}", same(a, bb[t]))
-    if table:  # three rounds outstanding (three result slots on two compute lanes), 8 rounds of 8 images
-        for src_name, src in (("host", torch.from_numpy(pb).pin_memory()), ("device", torch.from_numpy(pb).cuda())):
-            pending, got = [], []
-            for k in range(8):
-                pending.append(shard.score_sharded_async(src[8 * k:8 * k + 8], (28, 28), 224, full=True))
-                if len(pending) == 3:
-                    got.extend(pending.pop(0).wait())
-            while pending:
+    # three rounds outstanding (three result slots on two compute lanes), 8 rounds of 8 images
+    for src_name, src in (("host", torch.from_numpy(pb).pin_memory()), ("device", torch.from_numpy(pb).cuda())):
+        pending, got = [], []
+        for k in range(8):
+            pending.append(shard.score_sharded_async(src[8 * k:8 * k + 8], (28, 28), 224, full=True))
+            if len(pending) == 3:
                 got.extend(pending.pop(0).wait())
-            report(f"[{tag}] 8 rounds, three outstanding, {src_name} queries", all(same(got[t], bb[t]) for t in range(64)))
+        while pending:
+            got.extend(pending.pop(0).wait())
+        report(f"[{tag}] 8 rounds, three outstanding, {src_name} queries", all(same(got[t], bb[t]) for t in range(64)))
 t = torch.tensor([bad], device="cuda")
 dist.all_reduce(t)
 if rank == 0:

@@ -130,8 +130,8 @@ def test_projection_error_branch_keeps_unprojected_bank(env, capsys):
 
 
 def test_sharded_entry_points_with_one_rank(env):
-    """the five-phase sharded scoring and the sharded coreset entry points on a 1-rank NCCL group must reproduce the
-    plain single-GPU calls (the multi-rank exchange itself is checked by scripts/shard_check.py and
+    """the sharded scoring and the sharded coreset entry points on a 1-rank NCCL group must reproduce the plain
+    single-GPU calls (the multi-rank exchange itself is checked by scripts/shard_check.py and
     scripts/coreset_shard_check.py under torchrun, and by tests/test_sharding_gloo.py on the host side)"""
     import torch.distributed as dist
     from cmdiad_b200 import Bank, Comm
@@ -151,12 +151,20 @@ def test_sharded_entry_points_with_one_rank(env):
         comm.close()
         b.finalize()
         patches = np.stack([env["synth"].patches(784, 768, 70 + i, anomalous_frac=0.01, k=64) for i in range(3)])
-        a = b.score_sharded_batch(patches, (28, 28), 224, full=True)
+        # no neighbour table yet: score_batch sweeps the bank, and the first sharded call builds the replicated table
         c = b.score_batch(patches, (28, 28), 224, full=True)
+        a = b.score_sharded_batch(patches, (28, 28), 224, full=True)
         for i in range(3):
             for name in ("s", "s_idx", "min_val", "min_idx", "nn_idx", "m_star_knn", "w", "s_map"):
                 assert (getattr(a[i], name) == getattr(c[i], name)).all(), (i, name)
-        # replicated neighbour table + pipelined rounds (three phases, two collectives per round); 40 images = 2 rounds
+        # finalize frees the table: the next sharded call has to build it again
+        b.finalize()
+        c = b.score_batch(patches, (28, 28), 224, full=True)
+        a = b.score_sharded_batch(patches, (28, 28), 224, full=True)
+        for i in range(3):
+            for name in ("s", "s_idx", "min_val", "min_idx", "nn_idx", "m_star_knn", "w", "s_map"):
+                assert (getattr(a[i], name) == getattr(c[i], name)).all(), (i, name)
+        # explicit build + pipelined rounds (three phases, two collectives per round); 40 images = 2 rounds
         b.build_knn_sharded()
         many = np.stack([env["synth"].patches(784, 768, 170 + i, anomalous_frac=0.01, k=64) for i in range(40)])
         a = b.score_sharded_batch(many, (28, 28), 224, full=True)

@@ -1,7 +1,7 @@
-"""CPU suite, part 3: the N > 1 path.  The five-phase row-sharded scoring protocol (include/cmdiad_b200.h) is run over
-gloo with world_size 2: local work is done by the CPU oracle on each rank's shard, the collectives and the key /
-ownership encodings are the ones the GPU path uses (cmdiad_b200/sharding.py), and the result must equal the unsharded
-oracle exactly."""
+"""CPU suite, part 3: the N > 1 path.  The row-sharded scoring protocol (include/cmdiad_b200.h) is run over gloo with
+world_size 2: local work is done by the CPU oracle on each rank's shard, the collectives and the key / ownership
+encodings are the ones the GPU path uses (cmdiad_b200/sharding.py), and the result must equal the unsharded oracle
+exactly."""
 import os
 import socket
 
@@ -20,79 +20,6 @@ def _free_port():
         return s.getsockname()[1]
 
 
-def _worker(rank, world, port, R, P, D, ret):
-    os.environ["MASTER_ADDR"] = "127.0.0.1"
-    os.environ["MASTER_PORT"] = str(port)
-    dist.init_process_group("gloo", rank=rank, world_size=world)
-    torch.set_num_threads(2)
-    cent = synth.centroids(D, 64)
-    lib = synth.patches(R, D, seed=1, cent=cent)
-    lib[R // 2 + 3] = lib[5]  # an exact duplicate across the two shards: the lower global row must win
-    patch = synth.patches(P, D, seed=2, anomalous_frac=0.02, cent=cent)
-    patch[7] = lib[5] + 1e-3
-    lo, hi = sharding.shard_range(R, rank, world)
-    mine = lib[lo:hi]
-    # phase 1: local exact (min, argmin) -> packed keys -> all-reduce MIN
-    d = torch.cdist(torch.from_numpy(patch), torch.from_numpy(mine), compute_mode="donot_use_mm_for_euclid_dist")
-    mv, mi = torch.min(d, dim=1)
-    keys = torch.from_numpy(sharding.pack_keys(mv.numpy(), mi.numpy() + lo))
-    dist.all_reduce(keys, op=dist.ReduceOp.MIN)
-    min_val, min_idx = sharding.unpack_keys(keys.numpy())
-    # phase 2: s*, s_idx, m_star row (owner contributes, others zeros) -> all-reduce SUM
-    s_idx = int(np.argmax(min_val))
-    m_star = torch.from_numpy(sharding.contribution(mine, lo, [min_idx[s_idx]]))
-    dist.all_reduce(m_star, op=dist.ReduceOp.SUM)
-    # phase 3: local w_dist top-3 keys -> all-gather
-    wd = ((torch.from_numpy(mine) - m_star) ** 2).sum(1)
-    k = min(3, mine.shape[0])
-    tv, ti = torch.topk(wd, k, largest=False)
-    top = np.full(3, np.iinfo(np.int64).max, dtype=np.int64)
-    top[:k] = sharding.pack_keys(tv.numpy(), ti.numpy() + lo)
-    gathered = [torch.zeros(3, dtype=torch.int64) for _ in range(world)]
-    dist.all_gather(gathered, torch.from_numpy(top))
-    # phase 4: merge, neighbour rows by contribution -> all-reduce SUM
-    merged = np.sort(torch.cat(gathered).numpy())[:3]
-    _, nn = sharding.unpack_keys(merged)
-    nn_rows = torch.from_numpy(sharding.contribution(mine, lo, nn))
-    dist.all_reduce(nn_rows, op=dist.ReduceOp.SUM)
-    if rank == 0:
-        ret.put(dict(min_val=min_val.copy(), min_idx=min_idx.copy(), s_idx=s_idx, m_star=m_star.numpy().copy(), nn=nn.copy(),
-                     nn_rows=nn_rows.numpy().copy(), owner=sharding.owner_of(min_idx, R, world)))
-    dist.barrier()
-    dist.destroy_process_group()
-
-
-@pytest.mark.timeout(300)
-def test_sharded_protocol_over_gloo_matches_unsharded():
-    R, P, D, world = 1501, 96, 64, 2
-    ctx = mp.get_context("spawn")
-    ret = ctx.Queue()
-    port = _free_port()
-    procs = [ctx.Process(target=_worker, args=(r, world, port, R, P, D, ret)) for r in range(world)]
-    for p in procs:
-        p.start()
-    got = ret.get(timeout=240)
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
-    cent = synth.centroids(D, 64)
-    lib = synth.patches(R, D, seed=1, cent=cent)
-    lib[R // 2 + 3] = lib[5]
-    patch = synth.patches(P, D, seed=2, anomalous_frac=0.02, cent=cent)
-    patch[7] = lib[5] + 1e-3
-    d = torch.cdist(torch.from_numpy(patch), torch.from_numpy(lib), compute_mode="donot_use_mm_for_euclid_dist")
-    mv, mi = torch.min(d, dim=1)
-    assert (got["min_idx"] == mi.numpy()).all() and (got["min_val"] == mv.numpy()).all()
-    assert got["min_idx"][7] == 5  # duplicate rows 5 and R//2+3 live on different shards: lowest global row wins
-    s_idx = int(torch.argmax(mv))
-    assert got["s_idx"] == s_idx and (got["m_star"][0] == lib[mi[s_idx]]).all()
-    wd = ((torch.from_numpy(lib) - torch.from_numpy(lib[mi[s_idx]])) ** 2).sum(1)
-    ref_nn = np.lexsort((np.arange(R), wd.numpy()))[:3]
-    assert (got["nn"] == ref_nn).all() and (got["nn_rows"] == lib[ref_nn]).all()
-    lo1, _ = sharding.shard_range(R, 1, world)
-    assert (got["owner"] == (got["min_idx"] >= lo1)).all()
-
-
 def _table_worker(rank, world, port, R, P, D, ret):
     """three-phase protocol with the replicated neighbour table: MIN over packed keys, lookup, SUM of squared distances"""
     os.environ["MASTER_ADDR"] = "127.0.0.1"
@@ -101,7 +28,9 @@ def _table_worker(rank, world, port, R, P, D, ret):
     torch.set_num_threads(2)
     cent = synth.centroids(D, 64)
     lib = synth.patches(R, D, seed=3, cent=cent)
+    lib[R // 2 + 3] = lib[5]  # an exact duplicate across the two shards: the lower global row must win
     patch = synth.patches(P, D, seed=4, anomalous_frac=0.02, cent=cent)
+    patch[7] = lib[5] + 1e-3
     lo, hi = sharding.shard_range(R, rank, world)
     mine = lib[lo:hi]
     # the replicated table: every rank computes the entries of ITS rows against the whole bank, slices are all-gathered
@@ -127,7 +56,8 @@ def _table_worker(rank, world, port, R, P, D, ret):
     d2 = torch.from_numpy(sharding.knn_d2_contribution(mine, lo, patch[s_idx], nn[1:]))
     dist.all_reduce(d2, op=dist.ReduceOp.SUM)
     if rank == 0:
-        ret.put(dict(min_idx=min_idx.copy(), s_idx=s_idx, nn=nn.copy(), d2=d2.numpy().copy()))
+        ret.put(dict(min_val=min_val.copy(), min_idx=min_idx.copy(), s_idx=s_idx, nn=nn.copy(), d2=d2.numpy().copy(),
+                     owner=sharding.owner_of(min_idx, R, world)))
     dist.barrier()
     dist.destroy_process_group()
 
@@ -147,17 +77,22 @@ def test_three_phase_table_protocol_over_gloo():
         assert p.exitcode == 0
     cent = synth.centroids(D, 64)
     lib = synth.patches(R, D, seed=3, cent=cent)
+    lib[R // 2 + 3] = lib[5]
     patch = synth.patches(P, D, seed=4, anomalous_frac=0.02, cent=cent)
+    patch[7] = lib[5] + 1e-3
     d = torch.cdist(torch.from_numpy(patch), torch.from_numpy(lib), compute_mode="donot_use_mm_for_euclid_dist")
     mv, mi = torch.min(d, dim=1)
     s_idx = int(torch.argmax(mv))
-    assert (got["min_idx"] == mi.numpy()).all() and got["s_idx"] == s_idx
+    assert (got["min_idx"] == mi.numpy()).all() and (got["min_val"] == mv.numpy()).all() and got["s_idx"] == s_idx
+    assert got["min_idx"][7] == 5  # duplicate rows 5 and R//2+3 live on different shards: lowest global row wins
     wd = torch.cdist(torch.from_numpy(lib[mi[s_idx]:mi[s_idx] + 1]), torch.from_numpy(lib),
                      compute_mode="donot_use_mm_for_euclid_dist")[0] ** 2
     ref_nn = np.lexsort((np.arange(R), wd.numpy()))[:3]
     assert (got["nn"] == ref_nn).all()
     want = sharding.knn_d2_contribution(lib, 0, patch[s_idx], ref_nn[1:])
     assert (got["d2"] == want).all()  # x + 0 == x: the SUM all-reduce returns the owner's value exactly
+    lo1, _ = sharding.shard_range(R, 1, world)
+    assert (got["owner"] == (got["min_idx"] >= lo1)).all()
 
 
 def test_key_packing_properties():
@@ -183,7 +118,7 @@ def _stage_worker(rank, world, port, B, P, D, ret):
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     dist.init_process_group("gloo", rank=rank, world_size=world)
-    # host logic of Bank._stage_sharded (the device copy itself is cmdb_bank_stage_h2d): slice, pad, all-gather, cut
+    # host logic of Bank._stage_sharded (the device copy itself is a torch copy): slice, pad, all-gather, cut
     x = torch.from_numpy(np.stack([synth.patches(P, D, seed=40 + i, dist="G") for i in range(B)]))
     rows = B * P
     per, lo, hi = sharding.stage_slice(rows, world, rank)
