@@ -260,10 +260,7 @@ int cmdb_bank_create(int device, int dim, int64_t capacity_rows, cmdb_bank **out
     b->capacity = capacity_rows;
     cudaDeviceGetAttribute(&b->num_sms, cudaDevAttrMultiProcessorCount, device);
     cudaError_t err = cudaStreamCreateWithFlags(&b->lane_stream[0], cudaStreamNonBlocking);
-    // CMDB_SINGLE_LANE=1 (diagnostics): both lanes share one stream, i.e. batches never overlap each other
-    const char *single = getenv("CMDB_SINGLE_LANE");
-    if (single && single[0] == '1') b->lane_stream[1] = b->lane_stream[0];
-    else if (err == cudaSuccess) err = cudaStreamCreateWithFlags(&b->lane_stream[1], cudaStreamNonBlocking);
+    if (err == cudaSuccess) err = cudaStreamCreateWithFlags(&b->lane_stream[1], cudaStreamNonBlocking);
     b->stream = b->lane_stream[0];
     if (err == cudaSuccess) err = cudaStreamCreateWithFlags(&b->copy_stream, cudaStreamNonBlocking);
     if (err == cudaSuccess) err = cudaStreamCreateWithFlags(&b->d2h_stream, cudaStreamNonBlocking);
@@ -341,7 +338,7 @@ void cmdb_bank_destroy(cmdb_bank *b) {
     for (auto &l : b->ev_dbg)
         for (auto &e : l)
             if (e) cudaEventDestroy(e);
-    if (b->lane_stream[1] && b->lane_stream[1] != b->lane_stream[0]) cudaStreamDestroy(b->lane_stream[1]);
+    if (b->lane_stream[1]) cudaStreamDestroy(b->lane_stream[1]);
     if (b->lane_stream[0]) cudaStreamDestroy(b->lane_stream[0]);
     if (b->copy_stream) cudaStreamDestroy(b->copy_stream);
     if (b->d2h_stream) cudaStreamDestroy(b->d2h_stream);

@@ -42,6 +42,7 @@ constexpr int kNumSMsDefault = 148;
 constexpr int kMaxRanks = 8;         // GPUs of one NVSwitch box
 constexpr int kScoreBN = 256;        // bank rows per GEMM tile
 constexpr int kScoreBM = 128;        // query rows per GEMM tile
+constexpr int kGemmEpiGroups = 2;    // epilogue warp groups per GEMM CTA: producers = groups * CTAs
 constexpr int kResultSlots = 3;      // result blocks / outstanding submitted calls per handle (the compute lanes stay two)
 constexpr int kMaxStageChunks = 4;   // host query batches are staged and multiplied in up to this many chunks
 constexpr int kWorkCap = 16384;      // capacity of ScoreScratch::work_list
@@ -92,8 +93,6 @@ struct ScoreScratch {
     int n_topk_blocks = 0;
     unsigned int *done_counter = nullptr;  // last-block-done counter of reweight_kernel
     float4 *cand = nullptr;         // [n_ctas, cap_p] per-CTA running top-2 (val1, idx1, val2, idx2) of the GEMM epilogue
-    size_t cand_window_bytes = 0;   // L2 access-policy window over cand (0 = persistence not available / disabled)
-    float cand_hit_ratio = 0.f;
     float *min_val = nullptr;       // [cap_p]
     long long *min_idx = nullptr;   // [cap_p]
     unsigned long long *s_key = nullptr;    // packed argmax key of min_val
@@ -298,7 +297,6 @@ int score_query_prep(cmdb_bank *b, int P, bool compact, int row0 = 0);  // rows 
 // device-side fail count
 int score_gemm_candidates(cmdb_bank *b, int P, int terms, bool compact, int *n_cand_out, int row0 = 0);
 void q_split_rows(cmdb_bank *b, const float *rows_dev, int n);
-int score_gemm_groups();              // epilogue warp groups per CTA: producers = groups * CTAs
 int score_tile_stride(int mt, int G); // host copy of the GEMM's tile schedule stride
 int score_gemm_run(int nt, int mt_units, int G);  // N tiles per visit of an M tile for a launch of that shape
 // stage the queries (src: host or device, [B*P_img, dim]) + candidates + refine, all modes

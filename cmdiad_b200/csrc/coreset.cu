@@ -5,8 +5,7 @@
 //   * the projected bank z ([N,d'] half or double, natural row-major layout) is streamed once per pick
 //     (N*d'*sizeof(T) algorithmic bytes per pick) and pinned in L2 as far as the persisting carve-out allows; rows are
 //     statically split CTA -> 4-warp group -> warp (a warp owns one alignment class of its group's chunk), so the
-//     running min-distance vector never leaves shared memory (a grid-wide chunk queue exists as a template variant,
-//     CMDB_CORESET_DYNAMIC=1; it measured slower);
+//     running min-distance vector never leaves shared memory as long as the CTA's rows fit there;
 //   * the distance ||z_i - last|| is evaluated in the CANONICAL reduction order documented in
 //     oracle/coreset_oracle.c (the order of ATen's CUDA reduction for torch.linalg.norm on a contiguous [N,d'] tensor:
 //     32 lanes per row, aligned 4-element vectors round-robin over lanes, 4 accumulators per lane, fma accumulate,
@@ -21,15 +20,12 @@
 //     mailboxes with plain NVLink stores of self-flagged 8-byte words (CUDA-IPC mapped peer memory, csrc/comm.cu); all
 //     CTAs spin on their LOCAL mailbox -- no NCCL call, no system fence per pick; bounded spins turn a missing peer
 //     into an error instead of a hang.
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace cmdb {
 
 constexpr int kCsThreads = 512;
 constexpr int kCsWarps = kCsThreads / 32;
-constexpr int kCoresetDynamicDefault = 0;  // grid-wide chunk queue (1) or static CTA->warp row split (0)
 
 struct __align__(16) PickSlot {
     unsigned long long val;  // value bits (non-negative half/double order like unsigned integers)
@@ -277,8 +273,6 @@ struct CoresetParams {
     unsigned char *mb_peer[kMaxRanks];  // mailbox of every rank (mb_peer[rank] is local memory)
     unsigned int mb_keys_off;           // byte offset of the key slots inside a mailbox: [parity][source rank][source CTA]
     const void *z_full;                 // replica of the WHOLE projected bank [n_total, d] (storage type); local rows are a slice
-    unsigned int *chunk_ctr;            // [3] dynamic scheduling: per-pick work counters (rotating, reset by CTA 0)
-    int dynamic;                        // 1: warps pull 32-row chunks from a grid-wide queue instead of a static split
     unsigned int mb_ready_off;          // byte offset of the per-rank "shard has arrived in your replica" flags (8 bytes each)
     unsigned long long ready_epoch;     // value those flags take for this call
     unsigned int *abort_flag;           // set when a peer did not answer in time
@@ -329,7 +323,7 @@ struct Batch<double> {
     static constexpr int rows = 2;  // 32-byte vectors: keep the register footprint of two batches in flight below 128
 };
 
-template <typename T, int NV, bool DYN>
+template <typename T, int NV>
 __global__ void __launch_bounds__(kCsThreads, 1) coreset_kernel(CoresetParams p) {
     using acc_t = typename Traits<T>::acc_t;
     constexpr int RB = Batch<T>::rows;
@@ -348,10 +342,10 @@ __global__ void __launch_bounds__(kCsThreads, 1) coreset_kernel(CoresetParams p)
     const bool vectorized = d >= 128;
     acc_t *tile = tile_all + warp * 32 * 33;
 
-    // static mode: this CTA owns rows [cta_row0, cta_row1) and keeps their min-distances in shared memory;
-    // dynamic mode: rows are pulled from a grid-wide queue, min-distances live in global memory (L2, .cg accesses)
-    const long long cta_row0 = DYN ? 0 : (long long)blockIdx.x * p.rows_per_cta;
-    const long long cta_row1 = DYN ? p.N : min(p.N, cta_row0 + p.rows_per_cta);
+    // this CTA owns rows [cta_row0, cta_row1) and keeps their min-distances in shared memory when they fit, else in
+    // global memory (L2, .cg accesses)
+    const long long cta_row0 = (long long)blockIdx.x * p.rows_per_cta;
+    const long long cta_row1 = min(p.N, cta_row0 + p.rows_per_cta);
     const long long cta_rows = max(0LL, cta_row1 - cta_row0);
     T *mind = p.mind_in_smem ? mind_sh : reinterpret_cast<T *>(p.mind) + cta_row0;
     const bool mind_global = !p.mind_in_smem;
@@ -371,7 +365,7 @@ __global__ void __launch_bounds__(kCsThreads, 1) coreset_kernel(CoresetParams p)
 #pragma unroll
         for (int t = 0; t < NV; ++t) wp.vmain[t] = lane + 32 * t < wp.g.nfull;
     };
-    if (!DYN) {
+    {
         constexpr int kGroups = kCsWarps / 4;
         const long long rows_per_group = (cta_rows + kGroups - 1) / kGroups;
         const long long g_row0 = cta_row0 + (warp >> 2) * rows_per_group;
@@ -383,7 +377,6 @@ __global__ void __launch_bounds__(kCsThreads, 1) coreset_kernel(CoresetParams p)
         wp.n_rows = wp.first < g_row1 ? (g_row1 - wp.first + 3) >> 2 : 0;
         plan_class(c);
     }
-    const long long n_chunks = ((p.N + 127) >> 7) * 4;  // dynamic mode: (128-row block, class) pairs
     const size_t rstride_b = (size_t)4 * d * sizeof(T);  // bytes between consecutive rows of this warp
 
     long long sel = 0;  // features.py:372 -- pick 0 is (global) row 0
@@ -418,17 +411,14 @@ __global__ void __launch_bounds__(kCsThreads, 1) coreset_kernel(CoresetParams p)
         }
         {
             const long long sl = sel - p.row_offset;  // local row of the previous pick, if this shard owns it
-            if (threadIdx.x == 0 && pick > 1 && sl >= cta_row0 && sl < cta_row1 && (!DYN || blockIdx.x == 0)) {
+            if (threadIdx.x == 0 && pick > 1 && sl >= cta_row0 && sl < cta_row1) {
                 if (mind_global) st_cg(mind + (sl - cta_row0), Traits<T>::zero());
                 else mind[sl - cta_row0] = Traits<T>::zero();
             }
-            // the counter of the NEXT pick was last used two picks ago and nobody can touch it before this CTA
-            // publishes its slot for the current pick
-            if (DYN && blockIdx.x == 0 && threadIdx.x == 0) p.chunk_ctr[(pick + 1) % 3] = 0u;
         }
         __syncthreads();
         LastRegs<T, NV> L;
-        if (!DYN) load_last<T, NV>(L, last_sh, wp.g, lane, d, vectorized);
+        load_last<T, NV>(L, last_sh, wp.g, lane, d, vectorized);
 
         T best_val = Traits<T>::zero();
         long long best_row = -1;
@@ -517,29 +507,7 @@ __global__ void __launch_bounds__(kCsThreads, 1) coreset_kernel(CoresetParams p)
             }
         }
         };
-        if constexpr (!DYN) {
-            run_rows();
-        } else {
-            // grid-wide work queue: chunk id -> (128-row block, alignment class); the next id is fetched while the
-            // current chunk is processed
-            unsigned int *ctr = p.chunk_ctr + pick % 3;
-            unsigned int nxt = 0;
-            if (lane == 0) nxt = atomicAdd(ctr, 1u);
-            for (;;) {
-                const unsigned int cur = __shfl_sync(0xffffffffu, nxt, 0);
-                if (cur >= n_chunks) break;
-                if (lane == 0) nxt = atomicAdd(ctr, 1u);
-                const long long blk0 = (long long)(cur >> 2) << 7;
-                const int c = (int)(cur & 3);  // global row % 4 of this chunk's rows
-                wp.first = blk0 + ((c - (int)((blk0 + p.row_offset) & 3)) & 3);
-                const long long blk1 = min(p.N, blk0 + 128);
-                wp.n_rows = wp.first < blk1 ? (blk1 - wp.first + 3) >> 2 : 0;
-                if (wp.n_rows == 0) continue;
-                plan_class(c);
-                load_last<T, NV>(L, last_sh, wp.g, lane, d, vectorized);
-                run_rows();
-            }
-        }
+        run_rows();
         // ---- CTA argmax: warp shuffle, then shared memory ----
         unsigned long long bv = best_row < 0 ? 0ULL : Traits<T>::bits(best_val);
         unsigned long long br = best_row < 0 ? ~0ULL : (unsigned long long)best_row;
@@ -776,13 +744,10 @@ static int launch_coreset(cmdb_bank *b, CoresetParams p) {
     const int nv = d >= 128 ? (d / 4 + 31) / 32 : 1;
     int grid = b->num_sms;
     const size_t fixed = sizeof(typename Traits<T>::acc_t) * kCsWarps * 32 * 33 + sizeof(T) * (size_t)d + 16 + 64 * 8;
-    const char *dyn = getenv("CMDB_CORESET_DYNAMIC");
-    const bool dynamic = dyn ? (dyn[0] != '0') : (kCoresetDynamicDefault != 0);
     auto run = [&](auto kern) -> int {
         p.rows_per_cta = (p.N + grid - 1) / grid;
         size_t smem = fixed + sizeof(T) * (size_t)p.rows_per_cta;
-        p.dynamic = dynamic;
-        p.mind_in_smem = !p.dynamic && smem <= 200 * 1024;
+        p.mind_in_smem = smem <= 200 * 1024;
         if (!p.mind_in_smem) smem = fixed;
         CMDB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         int per_sm = 0;
@@ -792,15 +757,13 @@ static int launch_coreset(cmdb_bank *b, CoresetParams p) {
         // The projected bank is re-read once per pick.  B200's L2 (126 MB) cannot hold a 120 MB cyclic sweep under its
         // default replacement (measured: 20 % hit rate), so pin as much of it as the persisting carve-out allows and
         // stream the rest: DRAM traffic per pick drops to roughly (1 - hitRatio) of the bank.
-        const char *env = getenv("CMDB_CORESET_L2PERSIST");
-        const bool want_persist = !(env && env[0] == '0');
         int max_persist = 0, max_window = 0;
         cudaDeviceGetAttribute(&max_persist, cudaDevAttrMaxPersistingL2CacheSize, b->device);
         cudaDeviceGetAttribute(&max_window, cudaDevAttrMaxAccessPolicyWindowSize, b->device);
         const size_t z_bytes = sizeof(T) * (size_t)p.N * p.d;
         bool persisting = false;
         cudaStreamAttrValue attr{};
-        if (want_persist && max_persist > 0 && max_window > 0) {
+        if (max_persist > 0 && max_window > 0) {
             const size_t carve = std::min<size_t>(z_bytes, (size_t)max_persist);
             // the carve-out is process-wide device state: only ever GROW it here (another component of the host program
             // may have configured its own) and let coreset_greedy_dev restore the previous value when the loop is done
@@ -818,10 +781,6 @@ static int launch_coreset(cmdb_bank *b, CoresetParams p) {
             }
             (void)cudaGetLastError();
         }
-        if (getenv("CMDB_TRACE"))
-            fprintf(stderr, "[cmdb] coreset: N=%lld d=%d grid=%d smem=%zu dynamic=%d mind_in_smem=%d z=%.1f MB L2 persist=%d (max %d MB, window %d MB, hitRatio %.2f)\n",
-                    p.N, p.d, grid, smem, p.dynamic, p.mind_in_smem, z_bytes / 1e6, (int)persisting, max_persist >> 20, max_window >> 20,
-                    persisting ? attr.accessPolicyWindow.hitRatio : 0.f);
         void *args[] = {&p};
         cudaError_t le = cudaLaunchCooperativeKernel((void *)kern, dim3(grid), dim3(kCsThreads), args, smem, b->stream);
         if (persisting) {
@@ -832,9 +791,9 @@ static int launch_coreset(cmdb_bank *b, CoresetParams p) {
         CMDB_CUDA(le);
         return CMDB_OK;
     };
-#define CMDB_CS(NVV)                                            \
-    case NVV:                                                   \
-        return dynamic ? run(coreset_kernel<T, NVV, true>) : run(coreset_kernel<T, NVV, false>);
+#define CMDB_CS(NVV) \
+    case NVV:        \
+        return run(coreset_kernel<T, NVV>);
     switch (nv) {
         CMDB_CS(1) CMDB_CS(2) CMDB_CS(3) CMDB_CS(4) CMDB_CS(5) CMDB_CS(6) CMDB_CS(7) CMDB_CS(8)
         default:
@@ -891,20 +850,14 @@ int coreset_greedy_dev(cmdb_bank *b, const double *z_dev, int64_t N, int d, int6
     } while (0)
     CS_TRY(cudaMalloc(&idx_dev, sizeof(long long) * (size_t)n_select));
     CS_TRY(cudaMalloc(&slots, sizeof(PickSlot) * 2 * (size_t)b->num_sms));
-    CS_TRY(cudaMalloc(&abort_dev, 4 * sizeof(unsigned int)));  // abort flag + 3 rotating chunk counters
-    CS_TRY(cudaMemsetAsync(abort_dev, 0, 4 * sizeof(unsigned int), st));
+    CS_TRY(cudaMalloc(&abort_dev, sizeof(unsigned int)));
+    CS_TRY(cudaMemsetAsync(abort_dev, 0, sizeof(unsigned int), st));
     if (force_idx_host) {
         CS_TRY(cudaMalloc(&force_dev, sizeof(long long) * (size_t)n_select));
         CS_TRY(cudaMemcpyAsync(force_dev, force_idx_host, sizeof(long long) * (size_t)n_select, cudaMemcpyHostToDevice, st));
     }
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    if (getenv("CMDB_TRACE")) {
-        cudaEventCreate(&ev0), cudaEventCreate(&ev1);
-        cudaEventRecord(ev0, st);
-    }
     CoresetParams p{};
     p.N = N, p.d = d, p.n_select = n_select, p.out_idx = idx_dev, p.force_idx = force_dev, p.slots = slots;
-    p.chunk_ctr = abort_dev + 1;
     p.l2_prev_limit = &l2_prev, p.l2_changed = &l2_changed;
     p.world = 1, p.rank = 0, p.row_offset = 0, p.abort_flag = abort_dev, p.spin_limit = 20LL * 1000 * 1000 * 1000;  // ~10 s
     const double *first_row = z_dev;  // pick 0 = global row 0
@@ -973,14 +926,6 @@ int coreset_greedy_dev(cmdb_bank *b, const double *z_dev, int64_t N, int d, int6
         return rc;
     }
     unsigned int aborted = 0;
-    if (getenv("CMDB_TRACE")) {
-        cudaEventRecord(ev1, st);
-        cudaEventSynchronize(ev1);
-        float ms = 0.f;
-        cudaEventElapsedTime(&ms, ev0, ev1);
-        fprintf(stderr, "[cmdb] coreset: init + greedy kernel %.3f ms for %lld picks (%.2f us/pick)\n", ms, (long long)n_select,
-                ms * 1e3 / (double)std::max<int64_t>(1, n_select - 1));
-    }
     CS_TRY(cudaMemcpyAsync(out_idx_host, idx_dev, sizeof(long long) * (size_t)n_select, cudaMemcpyDeviceToHost, st));
     CS_TRY(cudaMemcpyAsync(&aborted, abort_dev, sizeof(aborted), cudaMemcpyDeviceToHost, st));
     if (out_min_last_host)

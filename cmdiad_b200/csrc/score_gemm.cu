@@ -12,7 +12,8 @@
 //   * warp-specialised persistent CTAs (one per SM): warp 0 = TMA producer (SWIZZLE_128B tiles into a 4- / 2-stage
 //     ring), warp 1 = single-thread tcgen05.mma issuer (M=128 queries x N=256 bank rows, accumulators double-buffered in
 //     all 512 TMEM columns), warp 2 = TMEM allocation, warps 4-11 = two epilogue groups (column halves);
-//     CG = 2: CTA pairs (cluster of 2, cta_group::2, M = 256), each CTA stages its query tile and half of the bank tile;
+//     CG = 2 (TERMS = 3 only): CTA pairs (cluster of 2, cta_group::2, M = 256), each CTA stages its query tile and half
+//     of the bank tile;
 //   * epilogue: tcgen05.ld 32 columns at a time, val = ||b||^2 - 2 a.b (the per-query ||a||^2 is constant under argmin),
 //     two branch-free top-2 chains per thread (value, bank row), carried across all tiles of the producer in a list in
 //     L2 (296 producers x P x 16 B); one thread == one query row, so no cross-lane reduction is needed;
@@ -717,28 +718,6 @@ int score_scratch_alloc(cmdb_bank *b, int B, int P_img, int out_hw) {
         CMDB_CUDA(cudaMemset(s.done_counter, 0, sizeof(unsigned int)));
         const size_t cand_bytes = sizeof(float4) * (size_t)cap_p * 2 * b->num_sms;
         CMDB_CUDA(cudaMalloc(&s.cand, cand_bytes));
-        {
-            // optional L2 persistence for the candidate lists (CMDB_CAND_L2PERSIST=1; measured: no effect once the lists are
-            // touched once per run of tiles, see DESIGN.md 4.1).  The carve-out is process-wide device state: only ever GROWN.
-            static const bool enabled = [] {
-                const char *e = getenv("CMDB_CAND_L2PERSIST");
-                return e && e[0] == '1';
-            }();
-            int max_persist = 0, max_window = 0;
-            cudaDeviceGetAttribute(&max_persist, cudaDevAttrMaxPersistingL2CacheSize, b->device);
-            cudaDeviceGetAttribute(&max_window, cudaDevAttrMaxAccessPolicyWindowSize, b->device);
-            s.cand_window_bytes = 0, s.cand_hit_ratio = 0.f;
-            if (enabled && max_persist > 0 && max_window > 0) {
-                const size_t want = std::min<size_t>(cand_bytes, (size_t)max_persist);
-                size_t cur = 0;
-                (void)cudaDeviceGetLimit(&cur, cudaLimitPersistingL2CacheSize);
-                if (cur >= want || cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want) == cudaSuccess) {
-                    s.cand_window_bytes = std::min<size_t>(cand_bytes, (size_t)max_window);
-                    s.cand_hit_ratio = (float)std::min(1.0, (double)std::max(cur, want) / (double)s.cand_window_bytes);
-                }
-                (void)cudaGetLastError();
-            }
-        }
         CMDB_CUDA(cudaMalloc(&s.map_tmp, (size_t)map_cap * cap_b));
         CMDB_CUDA(cudaMalloc(&s.map_max, sizeof(float) * cap_b * 17));  // [cap_b] maxima, then [cap_b][16] band maxima
         CMDB_CUDA(cudaMalloc(&s.topk_keys, sizeof(unsigned long long) * 3 * s.n_topk_blocks * cap_b));
@@ -773,14 +752,6 @@ void q_split_rows(cmdb_bank *b, const float *rows_dev, int n) {
                                                                               s.q_norm, s.q_eps, nullptr, nullptr);
 }
 
-int score_gemm_groups() {
-    static const int eg = [] {
-        const char *e = getenv("CMDB_GEMM_EPI_GROUPS");
-        return (e && atoi(e) == 1) ? 1 : 2;
-    }();
-    return eg;
-}
-
 int score_tile_stride(int mt, int G) {  // == tile_stride() of the kernel
     for (int s = mt;; ++s) {
         int a = s % G, b = G;
@@ -796,11 +767,6 @@ int score_tile_stride(int mt, int G) {  // == tile_stride() of the kernel
 // N tiles per visit of an M tile.  Longer runs cut the traffic of the candidate lists (read + written once per run instead of
 // once per tile) but coarsen the work units: take the longest run whose busiest unit stays within 2 % of the ideal share.
 int score_gemm_run(int nt, int mt_units, int G) {
-    static const int forced = [] {
-        const char *e = getenv("CMDB_GEMM_RUN");
-        return e ? atoi(e) : 0;
-    }();
-    if (forced >= 1) return std::min(forced, 8);
     // at least G runs per M tile, so that EVERY producer keeps seeing a share of every query's rows (the certificate wants the
     // rows near a query's minimum spread over many producers; idle producers made 1.7x more queries need a rescan)
     const double ideal = (double)nt * mt_units / G;
@@ -828,16 +794,10 @@ int score_gemm_candidates(cmdb_bank *b, int P, int terms, bool compact, int *n_c
     p.mt = p_pad / BM;
     p.m_base = row0 / BM;
     p.m_count = compact ? s.fail_ctl + 2 : nullptr;
-    const int eg_env = score_gemm_groups();
-    // CTA pairs (cta_group::2): CMDB_GEMM_PAIR=0/1 forces a choice for every launch with >= 2 M tiles
-    static const int pair_env = [] {
-        const char *e = getenv("CMDB_GEMM_PAIR");
-        return e ? atoi(e) : -1;
-    }();
-    // measured at 16 images x 200k x 768: the 3-term kernel gains 5 % from pairs (7.84 -> 7.42 ms), the 1-term pre-filter
-    // loses 3 % (2.81 -> 2.90 ms; it is not limited by shared-memory reads, and a pair halves the producers per query)
-    const bool pair = !compact && eg_env == 2 && b->num_sms % 2 == 0 &&
-                      ((p.mt >= 2 && pair_env == 1) || (pair_env < 0 && terms == 3 && p.mt >= 8));
+    // CTA pairs (cta_group::2), measured at 16 images x 200k x 768: the 3-term kernel gains 5 % from pairs (7.84 -> 7.42 ms),
+    // the 1-term pre-filter loses 3 % (2.81 -> 2.90 ms; it is not limited by shared-memory reads, and a pair halves the
+    // producers per query)
+    const bool pair = !compact && b->num_sms % 2 == 0 && terms == 3 && p.mt >= 8;
     {
         const int cg = pair ? 2 : 1;
         // compact launches size themselves on the device (m_count): single tiles there
@@ -846,27 +806,15 @@ int score_gemm_candidates(cmdb_bank *b, int P, int terms, bool compact, int *n_c
     if (!compact && row0 == 0) s.sched_pair = pair;   // the first-pass schedule (the exact rescan needs it)
     s.sched_pair_last = pair;
     s.sched_run_last = p.run;
-    const int threads = kGemmCtlThreads + 128 * eg_env;
+    const int threads = kGemmCtlThreads + 128 * kGemmEpiGroups;
     auto launch = [&](auto kern, size_t smem, bool cluster2) -> int {
         CMDB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         cudaLaunchConfig_t cfg{};
         cfg.gridDim = dim3(b->num_sms), cfg.blockDim = dim3(threads), cfg.dynamicSmemBytes = smem, cfg.stream = st;
-        cudaLaunchAttribute attr[2] = {};
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = cluster2 ? 2 : 1, attr[0].val.clusterDim.y = 1, attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr, cfg.numAttrs = 1;
-        if (s.cand_window_bytes > 0) {
-            // the producers' running top-2 lists are read and written once per tile (2 x 8 KB) while the bank streams through
-            // L2: without help they are evicted between two visits and spill to DRAM (r1: 961 MB of DRAM traffic per launch
-            // against 326 MB of input).  Mark them persisting for this launch; everything else keeps the normal policy.
-            attr[1].id = cudaLaunchAttributeAccessPolicyWindow;
-            attr[1].val.accessPolicyWindow.base_ptr = s.cand;
-            attr[1].val.accessPolicyWindow.num_bytes = s.cand_window_bytes;
-            attr[1].val.accessPolicyWindow.hitRatio = s.cand_hit_ratio;
-            attr[1].val.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-            attr[1].val.accessPolicyWindow.missProp = cudaAccessPropertyNormal;
-            cfg.numAttrs = 2;
-        }
+        cudaLaunchAttribute attr{};
+        attr.id = cudaLaunchAttributeClusterDimension;
+        attr.val.clusterDim.x = cluster2 ? 2 : 1, attr.val.clusterDim.y = 1, attr.val.clusterDim.z = 1;
+        cfg.attrs = &attr, cfg.numAttrs = 1;
         // the pair kernels load HALF bank tiles (box of 128 rows)
         const CUtensorMap &mh = *reinterpret_cast<CUtensorMap *>(cluster2 ? b->tmap_hi2 : b->tmap_hi);
         const CUtensorMap &ml = *reinterpret_cast<CUtensorMap *>(cluster2 ? b->tmap_lo2 : b->tmap_lo);
@@ -874,14 +822,10 @@ int score_gemm_candidates(cmdb_bank *b, int P, int terms, bool compact, int *n_c
                                      *reinterpret_cast<CUtensorMap *>(s.tmap_qlo), mh, ml, p));
         return CMDB_OK;
     };
-    if (pair) {
-        if (terms == 1) CMDB_CHECK(launch(score_gemm_kernel<1, 2, 2>, GemmSmem<1, 2>::total + 1024, true));
-        else CMDB_CHECK(launch(score_gemm_kernel<3, 2, 2>, GemmSmem<3, 2>::total + 1024, true));
-    } else if (terms == 1 && eg_env == 2) CMDB_CHECK(launch(score_gemm_kernel<1, 2, 1>, GemmSmem<1, 1>::total + 1024, false));
-    else if (terms == 1) CMDB_CHECK(launch(score_gemm_kernel<1, 1, 1>, GemmSmem<1, 1>::total + 1024, false));
-    else if (eg_env == 2) CMDB_CHECK(launch(score_gemm_kernel<3, 2, 1>, GemmSmem<3, 1>::total + 1024, false));
-    else CMDB_CHECK(launch(score_gemm_kernel<3, 1, 1>, GemmSmem<3, 1>::total + 1024, false));
-    *n_cand_out = eg_env * b->num_sms;  // (CTA, column group) producers
+    if (pair) CMDB_CHECK(launch(score_gemm_kernel<3, kGemmEpiGroups, 2>, GemmSmem<3, 2>::total + 1024, true));
+    else if (terms == 1) CMDB_CHECK(launch(score_gemm_kernel<1, kGemmEpiGroups, 1>, GemmSmem<1, 1>::total + 1024, false));
+    else CMDB_CHECK(launch(score_gemm_kernel<3, kGemmEpiGroups, 1>, GemmSmem<3, 1>::total + 1024, false));
+    *n_cand_out = kGemmEpiGroups * b->num_sms;  // (CTA, column group) producers
     return CMDB_OK;
 }
 

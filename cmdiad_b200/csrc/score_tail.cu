@@ -11,8 +11,6 @@
 //               truncation, Pillow's 3+3 pass integer box blur, /255, *max -- 16 row bands / 16 column bands per image
 #include <math.h>
 
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace cmdb {
@@ -165,7 +163,7 @@ __global__ void __launch_bounds__(256) refine_kernel(const float4 *__restrict__ 
 // this would cost more than a GEMM (fallback_use_rescan; banks full of near-duplicates), the uncertified queries are
 // redone with the FP32-equivalent 3-term GEMM.  Either way min_val / min_idx equal those of an exact scan of the whole bank.
 // ---------------------------------------------------------------------------------------------------------------
-// One block per QB consecutive queries (QB = 8 by default), three phases:
+// One block per QB consecutive queries (launched with QB = 8), three phases:
 //   (1) the producers' lists are read with the QUERY index along the lanes (a warp-wide load is 32 / QB contiguous runs of
 //       QB x 16 bytes of cand[c][q0 ...]; round 1 read them one query per warp, 32 sectors of 32 producers per request,
 //       which was two thirds of the kernel's time); every thread keeps its share in registers; smallest first value per
@@ -198,7 +196,7 @@ __device__ __forceinline__ void cert_recheck(const int *list, int n_list, const 
     }
 }
 
-template <int QB>  // queries per block: 32 (large batches), 16 or 8 (single images: more blocks, one query per warp)
+template <int QB>  // queries per block: 8, 16 or 32 (8: more blocks, one query per warp in phase 3)
 __global__ void __launch_bounds__(kCertThreads) refine_cert_kernel(const float4 *__restrict__ cand, int n_cand, int cand_stride,
                                                           const float *__restrict__ q, const float *__restrict__ bank, int dim,
                                                           int P, int P_img, long long row_offset,
@@ -571,22 +569,12 @@ static int score_certify(cmdb_bank *b, int B, int P_img, int n_cand) {
     CMDB_CUDA(cudaMemsetAsync(s.fail_ctl, 0, 8 * sizeof(int) + sizeof(unsigned long long) * B, st));  // control block + s_key
     const float acc_model = (float)(b->dim / 16 + 1) * 17.f * 1.1920929e-7f;
     if (b->timing == 2) CMDB_CUDA(cudaEventRecord(b->ev_dbg[b->cur_slot][0], st));
-    // queries per block: 8 = one query per warp in phase 3 and 10 list entries per thread held in registers (measured best;
-    // CMDB_CERT_QB = 16 / 32 select the wider variants)
-    static const int qb_env = [] {
-        const char *e = getenv("CMDB_CERT_QB");
-        return e ? atoi(e) : 0;
-    }();
-    const int qb = qb_env == 8 || qb_env == 16 || qb_env == 32 ? qb_env : 8;
-#define CMDB_CERT(QB)                                                                                                       \
-    refine_cert_kernel<QB><<<(P + QB - 1) / QB, kCertThreads, 0, st>>>(s.cand, n_cand, s.cap_p, s.q_f32, b->data, b->dim, P, P_img,    \
-                                                                       b->row_offset, s.q_norm, s.q_eps, b->cert_bmax, b->cert_eb_max, \
-                                                                       acc_model, s.min_val, s.min_idx, s.s_key, s.fail_list,          \
-                                                                       s.fail_ctl, s.work_list, s.best_key)
-    if (qb == 32) CMDB_CERT(32);
-    else if (qb == 16) CMDB_CERT(16);
-    else CMDB_CERT(8);
-#undef CMDB_CERT
+    // queries per block: 8 = one query per warp in phase 3 and 10 list entries per thread held in registers (measured best)
+    constexpr int QB = 8;
+    refine_cert_kernel<QB><<<(P + QB - 1) / QB, kCertThreads, 0, st>>>(s.cand, n_cand, s.cap_p, s.q_f32, b->data, b->dim, P, P_img,
+                                                                       b->row_offset, s.q_norm, s.q_eps, b->cert_bmax, b->cert_eb_max,
+                                                                       acc_model, s.min_val, s.min_idx, s.s_key, s.fail_list,
+                                                                       s.fail_ctl, s.work_list, s.best_key);
     if (b->timing == 2) CMDB_CUDA(cudaEventRecord(b->ev_dbg[b->cur_slot][1], st));
     CMDB_CUDA(cudaGetLastError());
     return CMDB_OK;
@@ -597,7 +585,7 @@ static int score_rescan(cmdb_bank *b, int P_img) {
     cudaStream_t st = b->stream;
     CMDB_CUDA(cudaGetLastError());
     // tier 1: few uncertified (query, producer) pairs -> exact rescan of those producers' rows
-    const int cg = s.sched_pair ? 2 : 1, n_units = b->num_sms / cg, EG = score_gemm_groups();
+    const int cg = s.sched_pair ? 2 : 1, n_units = b->num_sms / cg, EG = kGemmEpiGroups;
     const int last_tiles = s.mt_total - (s.mt_total - 1) / s.chunk_tiles * s.chunk_tiles;
     const int nt = (int)(b->fin_rows_pad / kScoreBN);
     rescan_kernel<<<b->num_sms * 8, 256, 0, st>>>(s.work_list, s.fail_ctl + 3, s.q_f32, b->data, b->dim, b->fin_rows, n_units, cg, EG,
@@ -659,16 +647,12 @@ int score_local_min(cmdb_bank *b, const float *src, int src_is_device, int B, in
     }
     b->last_mode = mode;
     const int mt_total = (P + kScoreBM - 1) / kScoreBM;
-    static const int env_chunks = [] {
-        const char *e = getenv("CMDB_STAGE_CHUNKS");
-        return e ? atoi(e) : 0;
-    }();
     // another batch in flight on this handle (submit / wait pipeline): the whole copy already overlaps that batch's
     // kernels, so one chunk -- and one GEMM launch -- is best
     const bool overlapped = b->any_pending();
     const bool via_copy_stream = !src_is_device && (overlapped || mt_total >= 16);
     int n_chunks = 1;
-    if (via_copy_stream && !overlapped) n_chunks = env_chunks > 0 ? env_chunks : (mt_total >= 64 ? 4 : 2);
+    if (via_copy_stream && !overlapped) n_chunks = mt_total >= 64 ? 4 : 2;
     n_chunks = std::max(1, std::min(std::min(n_chunks, kMaxStageChunks), mt_total));
     const int chunk_tiles = (mt_total + n_chunks - 1) / n_chunks;
     n_chunks = (mt_total + chunk_tiles - 1) / chunk_tiles;
@@ -1478,7 +1462,7 @@ static int score_reweight_tensor(cmdb_bank *b, int B, int P_img) {
     p.m_star = s.m_star, p.m_test = s.m_test, p.bank = b->data, p.rows = b->fin_rows, p.row_offset = b->row_offset;
     p.dim = b->dim, p.q_norm = s.q_norm, p.q_eps = s.q_eps;
     p.bmax = b->cert_bmax, p.eb_max = b->cert_eb_max, p.acc_model = (float)(b->dim / 16 + 1) * 17.f * 1.1920929e-7f;
-    p.cg = s.sched_pair_last ? 2 : 1, p.n_units = b->num_sms / p.cg, p.EG = score_gemm_groups();
+    p.cg = s.sched_pair_last ? 2 : 1, p.n_units = b->num_sms / p.cg, p.EG = kGemmEpiGroups;
     p.stride = score_tile_stride(1, p.n_units);
     p.nt = (int)(b->fin_rows_pad / kScoreBN);
     p.run = s.sched_run_last;
@@ -1518,7 +1502,7 @@ int score_build_knn_table(cmdb_bank *b, long long row_first, long long row_count
         p.m_star = rows, p.m_test = nullptr, p.bank = b->data, p.rows = b->fin_rows, p.row_offset = 0;
         p.dim = b->dim, p.q_norm = s.q_norm, p.q_eps = s.q_eps;
         p.bmax = b->cert_bmax, p.eb_max = b->cert_eb_max, p.acc_model = (float)(b->dim / 16 + 1) * 17.f * 1.1920929e-7f;
-        p.cg = s.sched_pair_last ? 2 : 1, p.n_units = b->num_sms / p.cg, p.EG = score_gemm_groups();
+        p.cg = s.sched_pair_last ? 2 : 1, p.n_units = b->num_sms / p.cg, p.EG = kGemmEpiGroups;
         const int mt = (n + kScoreBM - 1) / kScoreBM;
         p.stride = score_tile_stride((mt + p.cg - 1) / p.cg, p.n_units);
         p.nt = (int)(b->fin_rows_pad / kScoreBN);
@@ -1541,12 +1525,8 @@ int score_reweight(cmdb_bank *b, int B, int P_img) {
         return CMDB_OK;
     }
     // a single image: the one-launch CUDA-core sweep is as fast as a one-tile GEMM over the whole bank; batches go to the
-    // tensor cores, whose cost does not grow with B (identical keys either way).  CMDB_REWEIGHT_TENSOR=0/1 forces one path (tests).
-    static const int force = [] {
-        const char *e = getenv("CMDB_REWEIGHT_TENSOR");
-        return e ? atoi(e) : -1;
-    }();
-    if (b->score_impl == CMDB_SCORE_TCGEN05 && b->prefilter_terms == 0 && B <= kScoreBM && (force == 1 || (force < 0 && B >= 2)))
+    // tensor cores, whose cost does not grow with B (identical keys either way).
+    if (b->score_impl == CMDB_SCORE_TCGEN05 && b->prefilter_terms == 0 && B >= 2 && B <= kScoreBM)
         return score_reweight_tensor(b, B, P_img);
     ReweightParams p{};
     p.bank = b->data, p.rows = b->fin_rows, p.row_offset = b->row_offset, p.dim = b->dim, p.B = B, p.P_img = P_img;
@@ -1587,8 +1567,6 @@ int score_shard_final(cmdb_bank *b, int B, const float *d2_sum_dev) {
 
 void tail_prefer_carveout() {
     CMDB_PREFER_MAX_SMEM(refine_kernel);
-    CMDB_PREFER_MAX_SMEM(refine_cert_kernel<32>);
-    CMDB_PREFER_MAX_SMEM(refine_cert_kernel<16>);
     CMDB_PREFER_MAX_SMEM(refine_cert_kernel<8>);
     CMDB_PREFER_MAX_SMEM(rescan_kernel);
     CMDB_PREFER_MAX_SMEM(select_kernel);
