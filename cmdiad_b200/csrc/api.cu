@@ -51,14 +51,38 @@ static int check_score_args(cmdb_bank *b, const void *patch, int B, int P, const
     return CMDB_OK;
 }
 
-static int stage_alloc(cmdb_bank *b, int B, int P, int out_hw) {
+// Opens a scoring call on b: takes the next compute lane and result slot and sizes the scratch for B images (at most
+// score_max_batch) of P patches with out_hw x out_hw maps.  The map stride is fixed per scratch: another out_hw frees the
+// scratch first, which needs every submitted call waited for.
+static int begin_call(cmdb_bank *b, int B, int P, int out_hw, const char *fn, ScoreCall *c) {
+    CMDB_REQUIRE(B <= score_max_batch(b), CMDB_ERR_INVALID, "%s: batch=%d exceeds the per-call limit %d", fn, B, score_max_batch(b));
     CMDB_CUDA(cudaSetDevice(b->device));
-    return score_scratch_alloc(b, B, P, out_hw);
+    if (b->layout.map_stride && (size_t)out_hw * out_hw != b->layout.map_stride) {
+        CMDB_REQUIRE(!b->any_pending(), CMDB_ERR_STATE, "%s: out_hw changes while a submitted call is outstanding; wait for it first",
+                     fn);
+        score_scratch_free(b);
+    }
+    CMDB_REQUIRE(!b->slot[b->next_slot].pending.active, CMDB_ERR_STATE,
+                 "%s: all %d result slots hold submitted calls; wait for one first", fn, kResultSlots);
+    CMDB_CHECK(score_scratch_alloc(b, B, P, out_hw));  // fails with CMDB_ERR_STATE if the scratch would have to grow
+    *c = score_call(b, b->next_lane, b->next_slot);
+    b->next_lane ^= 1;
+    b->next_slot = (b->next_slot + 1) % kResultSlots;
+    return CMDB_OK;
+}
+
+// Hands a call to the caller once its result copies are enqueued on the d2h stream: the slot holds the results of B images
+// (maps of images img_first, img_first + img_step, ...) until the caller waits for the call's ticket.
+static int publish_call(const ScoreCall &c, int B, int P, int out_hw, unsigned want, bool host_maps, int img_first, int img_step) {
+    cmdb_bank *b = c.b;
+    CMDB_CUDA(cudaEventRecord(c.slot->ev_done, b->d2h_stream));
+    c.slot->pending = ResultSlot::Pending{true, B, P, out_hw, want, host_maps, img_first, img_step, ++b->ticket_counter};
+    return CMDB_OK;
 }
 
 // bytes of the result block that a full-batch copy has to move (want: bit 0 = pre-blur maps, bit 1 = 8-bit maps)
 static size_t out_block_extent(const cmdb_bank *b, int B, unsigned want) {
-    const ScoreScratch &s = b->ss;
+    const ScoreLayout &s = b->layout;
     size_t bytes = s.off_map_out + sizeof(float) * s.map_stride * B;
     if (want & 1u) bytes = s.off_map_pre + sizeof(float) * s.map_stride * B;
     if (want & 2u) bytes = s.off_map_u8 + s.map_stride * B;
@@ -72,7 +96,7 @@ static unsigned want_mask_of(const cmdb_score_out *outs, int B) {
 
 // host block of a slot -> the caller's buffers (maps = false: only the scalars and per-patch arrays of image i)
 static void scatter_one(const cmdb_bank *b, const unsigned char *h, int i, int P, int out_hw, cmdb_score_out *out, bool maps) {
-    const ScoreScratch &s = b->ss;
+    const ScoreLayout &s = b->layout;
     const size_t npix = (size_t)out_hw * out_hw;
     TailResult tr;
     memcpy(&tr, h + sizeof(TailResult) * i, sizeof(tr));
@@ -92,12 +116,13 @@ static void scatter_one(const cmdb_bank *b, const unsigned char *h, int i, int P
         for (int k = 0; k < 3; ++k) out->nn_idx[k] = tr.nn_idx[k];
 }
 
-static int blur_batch(cmdb_bank *b, int B, int fh, int fw, int out_hw, int img_first = 0, int img_step = 1) {
-    ScoreScratch &s = b->ss;
+static int blur_batch(const ScoreCall &c, int B, int fh, int fw, int out_hw, int img_first = 0, int img_step = 1) {
+    const ScoreLayout &s = c.b->layout;
+    const Lane &l = *c.lane;
     CMDB_REQUIRE((size_t)out_hw * out_hw <= s.map_stride, CMDB_ERR_INVALID, "scoring: out_hw=%d larger than the scratch maps", out_hw);
     const int n_img = img_first < B ? (B - img_first + img_step - 1) / img_step : 0;
-    return upsample_blur_launch(b->stream, n_img, img_first, img_step, s.map_stride, s.min_val, fh, fw, out_hw, s.map_pre,
-                                s.map_out, s.map_u8, s.map_tmp, s.map_max, s.map_max + s.cap_b);
+    return upsample_blur_launch(c.stream, n_img, img_first, img_step, s.map_stride, c.min_val, fh, fw, out_hw, c.map_pre,
+                                c.map_out, c.map_u8, l.map_tmp, l.map_max, l.map_max + s.cap_b);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -208,7 +233,7 @@ static int coreset_impl(cmdb_bank *b, int64_t n_select, const int32_t *indptr, c
         rc = project_rows(b, b->data, b->rows, b->dim, indptr, indices, data, d_proj, z);
     } else {
         // features.py:369-370: projection skipped, the float32 bank itself is used
-        f32_to_f64_kernel<<<b->num_sms * 4, 512, 0, b->stream>>>(b->data, (long long)b->rows * d, z);
+        f32_to_f64_kernel<<<b->num_sms * 4, 512, 0, b->handle_stream()>>>(b->data, (long long)b->rows * d, z);
         rc = cudaGetLastError() == cudaSuccess ? CMDB_OK : CMDB_ERR_CUDA;
     }
     if (rc == CMDB_OK) rc = coreset_greedy_dev(b, z, b->rows, d, n_select, dtype_mode, out_idx_host, force_idx, out_min_last, sh);
@@ -264,62 +289,44 @@ int cmdb_coreset_rownorms(int device, const void *z_host, const void *last_host,
     return coreset_rownorms(device, z_host, last_host, n_rows, d, dtype_mode, out_host);
 }
 
-// Enqueue one sub-batch (<= score_max_batch images) on buffer slot `slot`: staging, GEMM + certificate, maps, re-weighting
-// and the device->host copies of the results (on the d2h stream, the maps as soon as the blur is done).  No host sync.
-// A submitted call takes the next result slot (kResultSlots of them) and the next compute lane (two, alternating).
-struct SlotPick {
-    int lane, rslot;
-};
-static SlotPick take_slot(cmdb_bank *b) {
-    const SlotPick p{b->next_lane, b->next_slot};
-    b->next_lane ^= 1;
-    b->next_slot = (b->next_slot + 1) % kResultSlots;
-    return p;
-}
-
-static int submit_sub_batch(cmdb_bank *b, const float *src, int is_device, int bc, int P, int fh, int fw, int out_hw,
-                            unsigned want, SlotPick pick, bool host_maps = true) {
-    const int slot = pick.rslot, lane = pick.lane;
-#define CMDB_MARK(i)                                                   \
-    do {                                                               \
-        if (b->timing) CMDB_CUDA(cudaEventRecord(b->timing == 2 ? b->ev_tl[lane][i] : b->ev[i], b->stream)); \
-    } while (0)
-    ScoreScratch &s = b->ss;
-    CMDB_CHECK(stage_alloc(b, bc, P, out_hw));
-    score_select_slot(b, lane, slot);
-    cudaStream_t st = b->stream;  // the lane's stream (only valid after the selection)
-    CMDB_MARK(CMDB_T_STAGE_IN);
+// Enqueue one sub-batch (<= score_max_batch images) of an opened call: staging, GEMM + certificate, maps, re-weighting and
+// the device->host copies of the results (on the d2h stream, the maps as soon as the blur is done), then publish it.  No
+// host sync.
+static int submit_sub_batch(ScoreCall &c, const float *src, int is_device, int bc, int P, int fh, int fw, int out_hw,
+                            unsigned want, bool host_maps = true) {
+    cmdb_bank *b = c.b;
+    const ScoreLayout &L = b->layout;
+    ResultSlot &s = *c.slot;
+    cudaStream_t st = c.stream;
+    CMDB_CHECK(score_mark(c, CMDB_T_STAGE_IN, st));
     // this slot's q_f32 was last read by the batch submitted three calls ago
-    CMDB_CHECK(score_local_min(b, src, is_device, bc, P, CMDB_T_GEMM, CMDB_T_REFINE, b->ev_compute[slot]));
-    CMDB_MARK(CMDB_T_MAP);
-    CMDB_CHECK(blur_batch(b, bc, fh, fw, out_hw));
+    CMDB_CHECK(score_local_min(c, src, is_device, bc, P, CMDB_T_GEMM, CMDB_T_REFINE, s.ev_compute));
+    CMDB_CHECK(score_mark(c, CMDB_T_MAP, st));
+    CMDB_CHECK(blur_batch(c, bc, fh, fw, out_hw));
     // min_val / min_idx / maps do not depend on the re-weighting: their copy overlaps it
     CMDB_CUDA(cudaEventRecord(b->ev_chunk[0], st));
     CMDB_CUDA(cudaStreamWaitEvent(b->d2h_stream, b->ev_chunk[0], 0));
-    CMDB_CUDA(cudaMemcpyAsync(s.out_block_host + s.off_min_val, s.out_block + s.off_min_val,
-                              (host_maps ? out_block_extent(b, bc, want) : s.off_map_out) - s.off_min_val, cudaMemcpyDeviceToHost,
+    CMDB_CUDA(cudaMemcpyAsync(s.out_block_host + L.off_min_val, s.out_block + L.off_min_val,
+                              (host_maps ? out_block_extent(b, bc, want) : L.off_map_out) - L.off_min_val, cudaMemcpyDeviceToHost,
                               b->d2h_stream));
-    CMDB_MARK(CMDB_T_REWEIGHT);
-    CMDB_CHECK(score_reweight(b, bc, P));
-    CMDB_MARK(CMDB_T_OUT);
-    CMDB_CUDA(cudaEventRecord(b->ev_compute[slot], st));
-    CMDB_CUDA(cudaStreamWaitEvent(b->d2h_stream, b->ev_compute[slot], 0));
-    CMDB_CUDA(cudaMemcpyAsync(s.out_block_host, s.out_block, s.off_min_val, cudaMemcpyDeviceToHost, b->d2h_stream));
-    CMDB_CUDA(cudaEventRecord(b->ev_done[slot], b->d2h_stream));
-    if (b->timing) CMDB_CUDA(cudaEventRecord(b->timing == 2 ? b->ev_tl[lane][CMDB_T_COUNT] : b->ev[CMDB_T_COUNT], b->d2h_stream));
-#undef CMDB_MARK
+    CMDB_CHECK(score_mark(c, CMDB_T_REWEIGHT, st));
+    CMDB_CHECK(score_reweight(c, bc, P));
+    CMDB_CHECK(score_mark(c, CMDB_T_OUT, st));
+    CMDB_CUDA(cudaEventRecord(s.ev_compute, st));
+    CMDB_CUDA(cudaStreamWaitEvent(b->d2h_stream, s.ev_compute, 0));
+    CMDB_CUDA(cudaMemcpyAsync(s.out_block_host, s.out_block, L.off_min_val, cudaMemcpyDeviceToHost, b->d2h_stream));
+    CMDB_CHECK(publish_call(c, bc, P, out_hw, want, host_maps, 0, 1));
+    CMDB_CHECK(score_mark(c, CMDB_T_COUNT, b->d2h_stream));
     if (b->timing == 1) b->ev_valid = true;  // only batches record the stage events, sharded rounds do not
-    cmdb_bank::Pending &pd = b->pending[slot];
-    pd.active = true, pd.B = bc, pd.P = P, pd.out_hw = out_hw, pd.want = want, pd.host_maps = host_maps;
-    pd.img_first = 0, pd.img_step = 1;
     return CMDB_OK;
 }
 
 // Waits for a submitted batch or sharded round and fills outs[0 .. B): the scalars and per-patch arrays of every image,
 // the maps of images img_first, img_first + img_step, ... (all of them for a batch; a sharded round only finished those).
 static int wait_slot(cmdb_bank *b, int slot, cmdb_score_out *outs) {
-    cmdb_bank::Pending &pd = b->pending[slot];
-    CMDB_CUDA(cudaEventSynchronize(b->ev_done[slot]));
+    ResultSlot &s = b->slot[slot];
+    ResultSlot::Pending &pd = s.pending;
+    CMDB_CUDA(cudaEventSynchronize(s.ev_done));
     pd.active = false;
     if (b->shard_abort_host && *b->shard_abort_host) {
         set_error("a peer rank did not arrive at the exchange of a sharded round within the timeout (all ranks must submit "
@@ -328,7 +335,7 @@ static int wait_slot(cmdb_bank *b, int slot, cmdb_score_out *outs) {
     }
     for (int i = 0; i < pd.B; ++i) {
         const bool maps = i >= pd.img_first && (i - pd.img_first) % pd.img_step == 0;
-        scatter_one(b, b->ss.out_block_host_buf[slot], i, pd.P, pd.out_hw, outs + i, maps);
+        scatter_one(b, s.out_block_host, i, pd.P, pd.out_hw, outs + i, maps);
     }
     return CMDB_OK;
 }
@@ -337,12 +344,6 @@ static int check_batch_args(cmdb_bank *b, const float *patches, int B, int P, in
     CMDB_CHECK(check_score_args(b, patches, B, P, fn));
     CMDB_REQUIRE(fh > 0 && fw > 0 && fh * fw == P, CMDB_ERR_INVALID, "%s: feature_map_dims %dx%d != P=%d", fn, fh, fw, P);
     CMDB_REQUIRE(out_hw >= 8 && out_hw <= 256, CMDB_ERR_INVALID, "%s: out_hw=%d not in [8,256]", fn, out_hw);
-    CMDB_CUDA(cudaSetDevice(b->device));
-    if (b->ss.map_stride && (size_t)out_hw * out_hw != b->ss.map_stride) {  // map stride is fixed per scratch
-        CMDB_REQUIRE(!b->any_pending(), CMDB_ERR_STATE,
-                     "%s: out_hw changes while a submitted batch is outstanding; wait for it first", fn);
-        score_scratch_free(b);
-    }
     return CMDB_OK;
 }
 
@@ -355,14 +356,12 @@ int cmdb_score_batch(cmdb_bank *b, const float *patches, int B, int P, int fh, i
     int prev_slot = -1, prev_b0 = 0;
     for (int b0 = 0; b0 < B; b0 += bc_max) {
         const int bc = std::min(bc_max, B - b0);
-        CMDB_REQUIRE(!b->pending[b->next_slot].active, CMDB_ERR_STATE,
-                     "cmdb_score_batch: all result slots hold submitted batches; wait for one first");
-        const SlotPick pick = take_slot(b);
-        const int slot = pick.rslot;
-        CMDB_CHECK(submit_sub_batch(b, patches + (size_t)b0 * P * b->dim, patch_is_device, bc, P, fh, fw, out_hw,
-                                    want_mask_of(outs + b0, bc), pick));
+        ScoreCall c{};
+        CMDB_CHECK(begin_call(b, bc, P, out_hw, "cmdb_score_batch", &c));
+        CMDB_CHECK(submit_sub_batch(c, patches + (size_t)b0 * P * b->dim, patch_is_device, bc, P, fh, fw, out_hw,
+                                    want_mask_of(outs + b0, bc)));
         if (prev_slot >= 0) CMDB_CHECK(wait_slot(b, prev_slot, outs + prev_b0));
-        prev_slot = slot, prev_b0 = b0;
+        prev_slot = c.slot_idx, prev_b0 = b0;
     }
     if (prev_slot >= 0) CMDB_CHECK(wait_slot(b, prev_slot, outs + prev_b0));
     return CMDB_OK;
@@ -372,22 +371,17 @@ int cmdb_score_batch_submit(cmdb_bank *b, const float *patches, int B, int P, in
                             unsigned want_maps, int64_t *out_ticket) {
     CMDB_REQUIRE(out_ticket, CMDB_ERR_INVALID, "cmdb_score_batch_submit: out_ticket is NULL");
     CMDB_CHECK(check_batch_args(b, patches, B, P, fh, fw, out_hw, "cmdb_score_batch_submit"));
-    CMDB_REQUIRE(B <= score_max_batch(b), CMDB_ERR_INVALID, "cmdb_score_batch_submit: batch=%d exceeds the per-call limit %d", B,
-                 score_max_batch(b));
-    CMDB_REQUIRE(!b->pending[b->next_slot].active, CMDB_ERR_STATE,
-                 "cmdb_score_batch_submit: three batches are already outstanding; call cmdb_score_batch_wait first");
-    const SlotPick pick = take_slot(b);
-    const int slot = pick.rslot;
-    CMDB_CHECK(submit_sub_batch(b, patches, patch_is_device, B, P, fh, fw, out_hw, want_maps & 3u, pick));
-    b->pending[slot].ticket = ++b->ticket_counter;
-    *out_ticket = b->pending[slot].ticket;
+    ScoreCall c{};
+    CMDB_CHECK(begin_call(b, B, P, out_hw, "cmdb_score_batch_submit", &c));
+    CMDB_CHECK(submit_sub_batch(c, patches, patch_is_device, B, P, fh, fw, out_hw, want_maps & 3u));
+    *out_ticket = c.slot->pending.ticket;
     return CMDB_OK;
 }
 
 static int wait_ticket(cmdb_bank *b, int64_t ticket, cmdb_score_out *outs, const char *fn) {
     CMDB_REQUIRE(b && outs, CMDB_ERR_INVALID, "%s: NULL argument", fn);
     for (int slot = 0; slot < kResultSlots; ++slot)
-        if (b->pending[slot].active && b->pending[slot].ticket == ticket) {
+        if (b->slot[slot].pending.active && b->slot[slot].pending.ticket == ticket) {
             CMDB_CUDA(cudaSetDevice(b->device));
             return wait_slot(b, slot, outs);
         }
@@ -404,93 +398,84 @@ int cmdb_score(cmdb_bank *b, const float *patch, int P, int fh, int fw, int out_
     return cmdb_score_batch(b, patch, 1, P, fh, fw, out_hw, patch_is_device, out);
 }
 
-static int check_shard_batch(cmdb_bank *b, int B, const char *fn) {
-    CMDB_REQUIRE(B >= 1 && B <= score_max_batch(b), CMDB_ERR_INVALID, "%s: batch=%d exceeds the per-call limit %d", fn, B,
-                 score_max_batch(b));
-    return CMDB_OK;
-}
-
-int cmdb_score_shard_min(cmdb_bank *b, const float *patches, int B, int P, int patch_is_device, int out_hw,
-                         int64_t *keys_device) {
-    CMDB_CHECK(check_score_args(b, patches, B, P, "cmdb_score_shard_min"));
-    CMDB_CHECK(check_shard_batch(b, B, "cmdb_score_shard_min"));
-    CMDB_REQUIRE(keys_device, CMDB_ERR_INVALID, "cmdb_score_shard_min: keys_device is NULL");
-    CMDB_REQUIRE(out_hw >= 8 && out_hw <= 256, CMDB_ERR_INVALID, "cmdb_score_shard_min: out_hw=%d not in [8,256]", out_hw);
-    CMDB_CUDA(cudaSetDevice(b->device));
-    {
-        // the round runs on lane next_lane (what cmdb_bank_stream returns before this call) with result slot next_slot; with
-        // the submit / wait finish up to three rounds may be outstanding (three result slots on the two lanes)
-        const bool busy = b->any_pending();
-        CMDB_REQUIRE(!busy || (size_t)out_hw * out_hw == b->ss.map_stride, CMDB_ERR_STATE,
-                     "cmdb_score_shard_min: out_hw changes while a submitted round is outstanding; wait for it first");
-        if (!busy && (size_t)out_hw * out_hw != b->ss.map_stride) score_scratch_free(b);
-        const int slot = b->next_slot, lane = b->next_lane;   // advanced by the finish call of the round
-        CMDB_REQUIRE(!b->pending[slot].active, CMDB_ERR_STATE,
-                     "cmdb_score_shard_min: all result slots hold submitted rounds; wait for one first");
-        CMDB_CHECK(stage_alloc(b, B, P, out_hw));  // fails with CMDB_ERR_STATE if the scratch would have to grow
-        score_select_slot(b, lane, slot);
-        b->shard_slot = slot, b->shard_lane = lane;
-        CMDB_CHECK(score_local_min(b, patches, patch_is_device, B, P, -1, -1, b->ev_compute[slot]));
-    }
-    pack_keys_kernel<<<(B * P + 255) / 256, 256, 0, b->stream>>>(b->ss.min_val, b->ss.min_idx, B * P, (long long *)keys_device);
-    CMDB_CUDA(cudaGetLastError());
-    return CMDB_OK;  // stream-ordered on the handle's stream (cmdb_bank_stream): run the collective there
-}
-
-int cmdb_score_shard_lookup(cmdb_bank *b, const int64_t *reduced_keys_device, int B, int P, float *knn_d2_contrib_device) {
-    CMDB_CHECK(check_score_args(b, reduced_keys_device, B, P, "cmdb_score_shard_lookup"));
-    CMDB_REQUIRE(knn_d2_contrib_device && B * P <= b->ss.cap_p && B <= b->ss.cap_b, CMDB_ERR_INVALID,
-                 "cmdb_score_shard_lookup: bad arguments (call cmdb_score_shard_min first)");
-    CMDB_REQUIRE(b->knn_table && b->knn_rows >= b->row_offset + b->fin_rows, CMDB_ERR_STATE,
-                 "cmdb_score_shard_lookup: install the replicated neighbour table first (cmdb_bank_set_knn_table)");
-    CMDB_CUDA(cudaSetDevice(b->device));
-    cudaStream_t st = b->stream;
-    CMDB_CUDA(cudaMemsetAsync(b->ss.s_key, 0, sizeof(unsigned long long) * B, st));
-    unpack_keys_kernel<<<(B * P + 255) / 256, 256, 0, st>>>((const long long *)reduced_keys_device, B * P, P, b->ss.min_val,
-                                                            b->ss.min_idx, b->ss.s_key);
-    CMDB_CHECK(score_select(b, B, P, false));  // m_test, s*, s_idx, m_star_row (a global row: no bank access needed)
-    return score_shard_lookup(b, B, knn_d2_contrib_device);
-}
-
-int cmdb_score_shard_finish_submit(cmdb_bank *b, const float *knn_d2_sum_device, int B, int P, int fh, int fw, int out_hw,
-                                   int img_first, int img_step, unsigned want_maps, int64_t *out_ticket) {
-    CMDB_CHECK(check_score_args(b, knn_d2_sum_device, B, P, "cmdb_score_shard_finish_submit"));
-    CMDB_REQUIRE(out_ticket && fh > 0 && fw > 0 && fh * fw == P && B * P <= b->ss.cap_p && B <= b->ss.cap_b, CMDB_ERR_INVALID,
-                 "cmdb_score_shard_finish_submit: bad arguments");
-    CMDB_REQUIRE((size_t)out_hw * out_hw == b->ss.map_stride, CMDB_ERR_INVALID,
-                 "cmdb_score_shard_finish_submit: out_hw differs from cmdb_score_shard_min");
-    CMDB_REQUIRE(img_first >= 0 && img_step >= 1, CMDB_ERR_INVALID, "cmdb_score_shard_finish_submit: bad image subset");
-    const int slot = b->shard_slot, lane = b->shard_lane;
-    CMDB_REQUIRE(!b->pending[slot].active, CMDB_ERR_STATE, "cmdb_score_shard_finish_submit: this round's slot is still outstanding");
-    CMDB_CUDA(cudaSetDevice(b->device));
-    ScoreScratch &s = b->ss;
-    cudaStream_t st = b->stream;
-    CMDB_CHECK(score_shard_final(b, B, knn_d2_sum_device));
-    CMDB_CHECK(blur_batch(b, B, fh, fw, out_hw, img_first, img_step));
-    CMDB_CUDA(cudaEventRecord(b->ev_compute[slot], st));
-    CMDB_CUDA(cudaStreamWaitEvent(b->d2h_stream, b->ev_compute[slot], 0));
+// Last phase of a sharded round (both forms): final scores from the summed neighbour distances, the maps of this rank's
+// images, the result copies; publishes the round.
+static int finish_round(const ScoreCall &c, const float *knn_d2_sum_device, int B, int P, int fh, int fw, int out_hw,
+                        int img_first, int img_step, unsigned want_maps, int64_t *out_ticket) {
+    cmdb_bank *b = c.b;
+    const ScoreLayout &L = b->layout;
+    ResultSlot &s = *c.slot;
+    CMDB_CHECK(score_shard_final(c, B, knn_d2_sum_device));
+    CMDB_CHECK(blur_batch(c, B, fh, fw, out_hw, img_first, img_step));
+    CMDB_CUDA(cudaEventRecord(s.ev_compute, c.stream));
+    CMDB_CUDA(cudaStreamWaitEvent(b->d2h_stream, s.ev_compute, 0));
     // scalar / per-patch prefix of ALL images in one copy, then the maps of the images this rank finished
     const size_t npix = (size_t)out_hw * out_hw;
     want_maps &= 3u;
     if (img_first == 0 && img_step == 1) {
         CMDB_CUDA(cudaMemcpyAsync(s.out_block_host, s.out_block, out_block_extent(b, B, want_maps), cudaMemcpyDeviceToHost, b->d2h_stream));
     } else {
-        CMDB_CUDA(cudaMemcpyAsync(s.out_block_host, s.out_block, s.off_map_out, cudaMemcpyDeviceToHost, b->d2h_stream));
+        CMDB_CUDA(cudaMemcpyAsync(s.out_block_host, s.out_block, L.off_map_out, cudaMemcpyDeviceToHost, b->d2h_stream));
         for (int i = img_first; i < B; i += img_step) {
-            const size_t o1 = s.off_map_out + sizeof(float) * s.map_stride * i, o2 = s.off_map_pre + sizeof(float) * s.map_stride * i;
-            const size_t o3 = s.off_map_u8 + s.map_stride * i;
+            const size_t o1 = L.off_map_out + sizeof(float) * L.map_stride * i, o2 = L.off_map_pre + sizeof(float) * L.map_stride * i;
+            const size_t o3 = L.off_map_u8 + L.map_stride * i;
             CMDB_CUDA(cudaMemcpyAsync(s.out_block_host + o1, s.out_block + o1, sizeof(float) * npix, cudaMemcpyDeviceToHost, b->d2h_stream));
             if (want_maps & 1u) CMDB_CUDA(cudaMemcpyAsync(s.out_block_host + o2, s.out_block + o2, sizeof(float) * npix, cudaMemcpyDeviceToHost, b->d2h_stream));
             if (want_maps & 2u) CMDB_CUDA(cudaMemcpyAsync(s.out_block_host + o3, s.out_block + o3, npix, cudaMemcpyDeviceToHost, b->d2h_stream));
         }
     }
-    CMDB_CUDA(cudaEventRecord(b->ev_done[slot], b->d2h_stream));
-    cmdb_bank::Pending &pd = b->pending[slot];
-    pd.active = true, pd.B = B, pd.P = P, pd.out_hw = out_hw, pd.want = want_maps, pd.host_maps = true;
-    pd.img_first = img_first, pd.img_step = img_step;
-    pd.ticket = ++b->ticket_counter;
-    b->next_slot = (slot + 1) % kResultSlots, b->next_lane = lane ^ 1;
-    *out_ticket = pd.ticket;
+    CMDB_CHECK(publish_call(c, B, P, out_hw, want_maps, true, img_first, img_step));
+    *out_ticket = s.pending.ticket;
+    return CMDB_OK;
+}
+
+int cmdb_score_shard_min(cmdb_bank *b, const float *patches, int B, int P, int patch_is_device, int out_hw,
+                         int64_t *keys_device) {
+    CMDB_CHECK(check_score_args(b, patches, B, P, "cmdb_score_shard_min"));
+    CMDB_REQUIRE(keys_device, CMDB_ERR_INVALID, "cmdb_score_shard_min: keys_device is NULL");
+    CMDB_REQUIRE(out_hw >= 8 && out_hw <= 256, CMDB_ERR_INVALID, "cmdb_score_shard_min: out_hw=%d not in [8,256]", out_hw);
+    // the round runs on the lane that cmdb_bank_stream returns before this call; with the submit / wait finish up to three
+    // rounds may be outstanding (three result slots on the two lanes)
+    ScoreCall c{};
+    CMDB_CHECK(begin_call(b, B, P, out_hw, "cmdb_score_shard_min", &c));
+    CMDB_CHECK(score_local_min(c, patches, patch_is_device, B, P, -1, -1, c.slot->ev_compute));
+    pack_keys_kernel<<<(B * P + 255) / 256, 256, 0, c.stream>>>(c.min_val, c.min_idx, B * P, (long long *)keys_device);
+    CMDB_CUDA(cudaGetLastError());
+    b->round = cmdb_bank::Round{true, c.lane_idx, c.slot_idx};
+    return CMDB_OK;  // stream-ordered on the round's lane (cmdb_bank_stream): run the collective there
+}
+
+int cmdb_score_shard_lookup(cmdb_bank *b, const int64_t *reduced_keys_device, int B, int P, float *knn_d2_contrib_device) {
+    CMDB_CHECK(check_score_args(b, reduced_keys_device, B, P, "cmdb_score_shard_lookup"));
+    CMDB_REQUIRE(b->round.open, CMDB_ERR_STATE, "cmdb_score_shard_lookup: no open round (call cmdb_score_shard_min first)");
+    CMDB_REQUIRE(knn_d2_contrib_device && B * P <= b->layout.cap_p && B <= b->layout.cap_b, CMDB_ERR_INVALID,
+                 "cmdb_score_shard_lookup: bad arguments");
+    CMDB_REQUIRE(b->knn_table && b->knn_rows >= b->row_offset + b->fin_rows, CMDB_ERR_STATE,
+                 "cmdb_score_shard_lookup: install the replicated neighbour table first (cmdb_bank_set_knn_table)");
+    CMDB_CUDA(cudaSetDevice(b->device));
+    const ScoreCall c = score_call(b, b->round.lane, b->round.slot);
+    CMDB_CUDA(cudaMemsetAsync(c.lane->s_key, 0, sizeof(unsigned long long) * B, c.stream));
+    unpack_keys_kernel<<<(B * P + 255) / 256, 256, 0, c.stream>>>((const long long *)reduced_keys_device, B * P, P, c.min_val,
+                                                                  c.min_idx, c.lane->s_key);
+    CMDB_CHECK(score_select(c, B, P, false));  // m_test, s*, s_idx, m_star_row (a global row: no bank access needed)
+    return score_shard_lookup(c, B, knn_d2_contrib_device);
+}
+
+int cmdb_score_shard_finish_submit(cmdb_bank *b, const float *knn_d2_sum_device, int B, int P, int fh, int fw, int out_hw,
+                                   int img_first, int img_step, unsigned want_maps, int64_t *out_ticket) {
+    CMDB_CHECK(check_score_args(b, knn_d2_sum_device, B, P, "cmdb_score_shard_finish_submit"));
+    CMDB_REQUIRE(b->round.open, CMDB_ERR_STATE, "cmdb_score_shard_finish_submit: no open round (call cmdb_score_shard_min first)");
+    CMDB_REQUIRE(out_ticket && fh > 0 && fw > 0 && fh * fw == P && B * P <= b->layout.cap_p && B <= b->layout.cap_b, CMDB_ERR_INVALID,
+                 "cmdb_score_shard_finish_submit: bad arguments");
+    CMDB_REQUIRE((size_t)out_hw * out_hw == b->layout.map_stride, CMDB_ERR_INVALID,
+                 "cmdb_score_shard_finish_submit: out_hw differs from cmdb_score_shard_min");
+    CMDB_REQUIRE(img_first >= 0 && img_step >= 1, CMDB_ERR_INVALID, "cmdb_score_shard_finish_submit: bad image subset");
+    CMDB_REQUIRE(!b->slot[b->round.slot].pending.active, CMDB_ERR_STATE,
+                 "cmdb_score_shard_finish_submit: this round's slot is still outstanding");
+    CMDB_CUDA(cudaSetDevice(b->device));
+    CMDB_CHECK(finish_round(score_call(b, b->round.lane, b->round.slot), knn_d2_sum_device, B, P, fh, fw, out_hw, img_first,
+                            img_step, want_maps, out_ticket));
+    b->round.open = false;
     return CMDB_OK;
 }
 
@@ -522,37 +507,27 @@ int cmdb_bank_attach_comm(cmdb_bank *b, cmdb_comm *comm) {
 int cmdb_score_shard_round_submit(cmdb_bank *b, const float *patches, int B, int P, int fh, int fw, int out_hw, int patch_is_device,
                                   int img_first, int img_step, unsigned want_maps, int64_t *out_ticket) {
     CMDB_CHECK(check_score_args(b, patches, B, P, "cmdb_score_shard_round_submit"));
-    CMDB_CHECK(check_shard_batch(b, B, "cmdb_score_shard_round_submit"));
     CMDB_REQUIRE(b->comm, CMDB_ERR_STATE, "cmdb_score_shard_round_submit: attach the peer buffers first (cmdb_bank_attach_comm)");
     CMDB_REQUIRE(b->knn_table && b->knn_rows >= b->row_offset + b->fin_rows, CMDB_ERR_STATE,
                  "cmdb_score_shard_round_submit: install the replicated neighbour table first (cmdb_bank_set_knn_table)");
-    CMDB_REQUIRE(out_ticket && fh > 0 && fw > 0 && fh * fw == P && out_hw >= 8 && out_hw <= 256, CMDB_ERR_INVALID,
-                 "cmdb_score_shard_round_submit: bad arguments");
+    CMDB_REQUIRE(out_ticket && fh > 0 && fw > 0 && fh * fw == P && out_hw >= 8 && out_hw <= 256 && img_first >= 0 && img_step >= 1,
+                 CMDB_ERR_INVALID, "cmdb_score_shard_round_submit: bad arguments");
     int rank = 0, world = 1;
     size_t bytes = 0;
     unsigned char *local = nullptr;
     PeerPtrs peers{};
     CMDB_CHECK(comm_info(b->comm, &rank, &world, &local, peers.p, &bytes));
-    CMDB_CUDA(cudaSetDevice(b->device));
-    const bool busy = b->any_pending();
-    if (!busy && (size_t)out_hw * out_hw != b->ss.map_stride) score_scratch_free(b);
-    CMDB_REQUIRE(!busy || (size_t)out_hw * out_hw == b->ss.map_stride, CMDB_ERR_STATE,
-                 "cmdb_score_shard_round_submit: out_hw changes while a submitted round is outstanding; wait for it first");
-    const int slot = b->next_slot, lane = b->next_lane;   // advanced by cmdb_score_shard_finish_submit
-    CMDB_REQUIRE(!b->pending[slot].active, CMDB_ERR_STATE,
-                 "cmdb_score_shard_round_submit: three submitted rounds are outstanding on this handle; wait for one first");
-    CMDB_CHECK(stage_alloc(b, B, P, out_hw));
-    score_select_slot(b, lane, slot);
-    b->shard_slot = slot, b->shard_lane = lane;
-    CMDB_CHECK(score_local_min(b, patches, patch_is_device, B, P, -1, -1, b->ev_compute[slot]));
+    ScoreCall c{};
+    CMDB_CHECK(begin_call(b, B, P, out_hw, "cmdb_score_shard_round_submit", &c));
+    CMDB_CHECK(score_local_min(c, patches, patch_is_device, B, P, -1, -1, c.slot->ev_compute));
     const unsigned long long epoch = comm_next_score_epoch(b->comm);  // per buffer, not per bank: several banks may share it
     const int xslot = (int)(epoch % kShardSlots);
-    CMDB_CHECK(score_shard_exchange_keys(b, B, P, peers, world, rank, xslot, epoch));
-    CMDB_CHECK(score_select(b, B, P, false));
+    CMDB_CHECK(score_shard_exchange_keys(c, B, P, peers, world, rank, xslot, epoch));
+    CMDB_CHECK(score_select(c, B, P, false));
     float *contrib = b->shard_d2 + xslot * kShardD2Cap, *d2_sum = b->shard_d2 + (kShardSlots + xslot) * kShardD2Cap;
-    CMDB_CHECK(score_shard_lookup(b, B, contrib));
-    CMDB_CHECK(score_shard_exchange_d2(b, B, peers, world, rank, xslot, epoch, contrib, d2_sum));
-    return cmdb_score_shard_finish_submit(b, d2_sum, B, P, fh, fw, out_hw, img_first, img_step, want_maps, out_ticket);
+    CMDB_CHECK(score_shard_lookup(c, B, contrib));
+    CMDB_CHECK(score_shard_exchange_d2(c, B, peers, world, rank, xslot, epoch, contrib, d2_sum));
+    return finish_round(c, d2_sum, B, P, fh, fw, out_hw, img_first, img_step, want_maps, out_ticket);
 }
 
 int cmdb_score_shard_wait(cmdb_bank *b, int64_t ticket, cmdb_score_out *outs) {
@@ -566,18 +541,19 @@ int cmdb_bank_read_device(cmdb_bank *b, int64_t row0, int64_t n_rows, float *out
     if (n_rows == 0) return CMDB_OK;
     CMDB_CUDA(cudaSetDevice(b->device));
     CMDB_CUDA(cudaMemcpyAsync(out_device, b->data + row0 * b->dim, sizeof(float) * (size_t)n_rows * b->dim, cudaMemcpyDeviceToDevice,
-                              b->stream));
-    CMDB_CUDA(cudaStreamSynchronize(b->stream));
+                              b->handle_stream()));
+    CMDB_CUDA(cudaStreamSynchronize(b->handle_stream()));
     return CMDB_OK;
 }
 
 // test hook (not in the public header): the GEMM epilogue's per-CTA top-2 lists of the last call, [n_cta][n_q][4] floats
 int cmdb_debug_read_candidates(cmdb_bank *b, float *out_host, int n_cta, int n_q) {
-    CMDB_REQUIRE(b && out_host && b->ss.cand && n_cta >= 1 && n_cta <= 2 * b->num_sms && n_q >= 1 && n_q <= b->ss.cap_p,
-                 CMDB_ERR_INVALID, "cmdb_debug_read_candidates: bad arguments");
+    CMDB_REQUIRE(b && out_host && n_cta >= 1 && n_cta <= 2 * b->num_sms && n_q >= 1 && n_q <= b->layout.cap_p, CMDB_ERR_INVALID,
+                 "cmdb_debug_read_candidates: bad arguments");
+    const Lane &l = b->lane[b->last_lane];   // the lists of the most recent call
     CMDB_CUDA(cudaSetDevice(b->device));
-    CMDB_CUDA(cudaStreamSynchronize(b->stream));
-    CMDB_CUDA(cudaMemcpy2D(out_host, sizeof(float4) * n_q, b->ss.cand, sizeof(float4) * b->ss.cap_p, sizeof(float4) * n_q, n_cta,
+    CMDB_CUDA(cudaStreamSynchronize(l.stream));
+    CMDB_CUDA(cudaMemcpy2D(out_host, sizeof(float4) * n_q, l.cand, sizeof(float4) * b->layout.cap_p, sizeof(float4) * n_q, n_cta,
                            cudaMemcpyDeviceToHost));
     return CMDB_OK;
 }
@@ -592,12 +568,13 @@ int cmdb_debug_exact_min(cmdb_bank *b, const float *patch_host, int P, float *mi
     std::vector<unsigned long long> h((size_t)P);
     cudaError_t e = cudaMalloc(&q, sizeof(float) * (size_t)P * b->dim);
     if (e == cudaSuccess) e = cudaMalloc(&keys, sizeof(unsigned long long) * (size_t)P);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(q, patch_host, sizeof(float) * (size_t)P * b->dim, cudaMemcpyHostToDevice, b->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(keys, 0xff, sizeof(unsigned long long) * (size_t)P, b->stream);
+    cudaStream_t st = b->handle_stream();
+    if (e == cudaSuccess) e = cudaMemcpyAsync(q, patch_host, sizeof(float) * (size_t)P * b->dim, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(keys, 0xff, sizeof(unsigned long long) * (size_t)P, st);
     int rc = CMDB_OK;
     if (e == cudaSuccess) rc = score_exact_scan(b, q, P, keys);
-    if (e == cudaSuccess && rc == CMDB_OK) e = cudaMemcpyAsync(h.data(), keys, sizeof(unsigned long long) * (size_t)P, cudaMemcpyDeviceToHost, b->stream);
-    if (e == cudaSuccess && rc == CMDB_OK) e = cudaStreamSynchronize(b->stream);
+    if (e == cudaSuccess && rc == CMDB_OK) e = cudaMemcpyAsync(h.data(), keys, sizeof(unsigned long long) * (size_t)P, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess && rc == CMDB_OK) e = cudaStreamSynchronize(st);
     cudaFree(q), cudaFree(keys);
     if (rc != CMDB_OK) return rc;
     CMDB_CUDA(e);
@@ -622,7 +599,7 @@ int cmdb_debug_lane_timeline(cmdb_bank *b, float *out) {
     constexpr int kN = CMDB_T_COUNT + 1 + 4;
     for (int l = 0; l < 2; ++l)
         for (int i = 0; i < kN; ++i) {
-            cudaEvent_t e = i <= CMDB_T_COUNT ? b->ev_tl[l][i] : b->ev_dbg[l][i - CMDB_T_COUNT - 1];
+            cudaEvent_t e = i <= CMDB_T_COUNT ? b->lane[l].ev_tl[i] : b->lane[l].ev_dbg[i - CMDB_T_COUNT - 1];
             if (cudaEventElapsedTime(out + l * kN + i, b->ev_base, e) != cudaSuccess) {
                 (void)cudaGetLastError();
                 out[l * kN + i] = -1.f;
@@ -681,8 +658,6 @@ int cmdb_score_fused_batch_submit(cmdb_bank *const *banks, const float *const *p
         CMDB_CHECK(check_batch_args(banks[m], patches[m], B, P[m], fh[m], fw[m], out_hw, "cmdb_score_fused_batch_submit"));
         CMDB_REQUIRE(B <= score_max_batch(banks[m]) && B <= kFusedCapB, CMDB_ERR_INVALID,
                      "cmdb_score_fused_batch_submit: batch=%d exceeds the per-call limit %d", B, std::min(kFusedCapB, score_max_batch(banks[m])));
-        CMDB_REQUIRE(!banks[m]->pending[banks[m]->next_slot].active, CMDB_ERR_STATE,
-                     "cmdb_score_fused_batch_submit: two batches are already outstanding; wait for one first");
     }
     cmdb_bank *b0 = banks[0];
     cmdb_bank::Fused &f = b0->fused;
@@ -690,7 +665,6 @@ int cmdb_score_fused_batch_submit(cmdb_bank *const *banks, const float *const *p
     CMDB_CHECK(fused_alloc(b0, out_hw));
     const int fs = f.next_fs;   // two fused blocks: at most two fused batches are outstanding
     CMDB_REQUIRE(!f.active[fs], CMDB_ERR_STATE, "cmdb_score_fused_batch_submit: two fused batches are already outstanding; wait for one first");
-    f.next_fs ^= 1;
     const int npix = out_hw * out_hw;
     const bool keep = (flags & CMDB_FUSED_KEEP_ON_DEVICE) != 0, host_maps = (flags & CMDB_FUSED_NO_HOST_MAPS) == 0;
     if (keep) {
@@ -698,21 +672,22 @@ int cmdb_score_fused_batch_submit(cmdb_bank *const *banks, const float *const *p
                      "cmdb_score_fused_batch_submit: device-side result store missing or full (%lld + %d > %lld); call cmdb_eval_reserve",
                      f.acc_n, B, f.acc_cap);
     }
+    // every modality's lane and result slot first, so that a refused one leaves nothing enqueued
+    ScoreCall calls[3] = {};
+    for (int m = 0; m < M; ++m) CMDB_CHECK(begin_call(banks[m], B, P[m], out_hw, "cmdb_score_fused_batch_submit", &calls[m]));
+    cudaStream_t st = calls[0].stream;   // the head runs on modality 0's lane
     FuseParams fp{};
     fp.n_modal = M, fp.B = B, fp.npix = npix;
     for (int m = 0; m < M; ++m) {
-        cmdb_bank *bm = banks[m];
-        const SlotPick pick = take_slot(bm);
-        const int slot = pick.rslot;
-        CMDB_CHECK(submit_sub_batch(bm, patches[m], patch_is_device, B, P[m], fh[m], fw[m], out_hw, 0u, pick, false));
-        bm->pending[slot].ticket = ++bm->ticket_counter;
-        f.banks[fs][m] = bm, f.slots[fs][m] = slot;
-        fp.maps[m] = reinterpret_cast<const float *>(bm->ss.out_block_buf[slot] + bm->ss.off_map_out);
-        fp.map_stride[m] = bm->ss.map_stride;
-        fp.tails[m] = reinterpret_cast<const TailResult *>(bm->ss.out_block_buf[slot]);
+        ScoreCall &c = calls[m];
+        CMDB_CHECK(submit_sub_batch(c, patches[m], patch_is_device, B, P[m], fh[m], fw[m], out_hw, 0u, false));
+        f.banks[fs][m] = banks[m], f.slots[fs][m] = c.slot_idx;
+        fp.maps[m] = c.map_out;
+        fp.map_stride[m] = banks[m]->layout.map_stride;
+        fp.tails[m] = c.tail;
         fp.s_lambda[m] = head->s_lambda[m], fp.smap_lambda[m] = head->smap_lambda[m];
         fp.det_coef[m] = head->detect_coef[m], fp.seg_coef[m] = head->seg_coef[m];
-        if (m > 0) CMDB_CUDA(cudaStreamWaitEvent(b0->stream, bm->ev_compute[slot], 0));
+        if (m > 0) CMDB_CUDA(cudaStreamWaitEvent(st, c.slot->ev_compute, 0));
     }
     fp.det_off = head->detect_offset, fp.seg_off = head->seg_offset;
     unsigned char *blk = f.dev[fs];
@@ -724,10 +699,10 @@ int cmdb_score_fused_batch_submit(cmdb_bank *const *banks, const float *const *p
         fp.acc_s = f.acc_scores + f.acc_n;
         f.acc_n += B;
     }
-    fuse_head_kernel<<<dim3((npix + 1023) / 1024, B), 256, 0, b0->stream>>>(fp);
+    fuse_head_kernel<<<dim3((npix + 1023) / 1024, B), 256, 0, st>>>(fp);
     CMDB_CUDA(cudaGetLastError());
     // results of this slot: scalars (+ maps) on the d2h stream; the next batch's kernels may already run meanwhile
-    CMDB_CUDA(cudaEventRecord(b0->ev_chunk[1], b0->stream));
+    CMDB_CUDA(cudaEventRecord(b0->ev_chunk[1], st));
     CMDB_CUDA(cudaStreamWaitEvent(b0->d2h_stream, b0->ev_chunk[1], 0));
     const size_t bytes = host_maps ? fused_off_map(kFusedCapB) + sizeof(double) * (size_t)npix * B : fused_off_map(kFusedCapB);
     CMDB_CUDA(cudaMemcpyAsync(f.host[fs], blk, bytes, cudaMemcpyDeviceToHost, b0->d2h_stream));
@@ -735,7 +710,8 @@ int cmdb_score_fused_batch_submit(cmdb_bank *const *banks, const float *const *p
     // the fuse kernel read the other banks' result blocks: their slots may only be reused after it (they wait on it through
     // the ticket: a slot is busy until cmdb_score_fused_batch_wait returned)
     f.active[fs] = true, f.n_modal[fs] = M, f.B[fs] = B, f.out_hw[fs] = out_hw;
-    f.ticket[fs] = b0->pending[f.slots[fs][0]].ticket;
+    f.next_fs ^= 1;
+    f.ticket[fs] = calls[0].slot->pending.ticket;
     *out_ticket = f.ticket[fs];
     return CMDB_OK;
 }
@@ -808,7 +784,7 @@ int cmdb_eval_reserve(cmdb_bank *b, int64_t n_images, int out_hw) {
     cmdb_bank::Fused &f = b->fused;
     CMDB_REQUIRE(!f.active[0] && !f.active[1], CMDB_ERR_STATE, "cmdb_eval_reserve: a submitted batch is outstanding");
     CMDB_CUDA(cudaSetDevice(b->device));
-    CMDB_CUDA(cudaStreamSynchronize(b->stream));
+    CMDB_CUDA(cudaStreamSynchronize(b->handle_stream()));
     cudaFree(f.acc_maps), cudaFree(f.acc_scores);
     f.acc_maps = f.acc_scores = nullptr, f.acc_cap = f.acc_n = 0, f.acc_npix = out_hw * out_hw;
     CMDB_CUDA(cudaMalloc(&f.acc_maps, sizeof(double) * (size_t)n_images * f.acc_npix));
@@ -838,10 +814,11 @@ int cmdb_eval_read(cmdb_bank *b, int64_t first, int64_t n, double *maps_host, do
     CMDB_CUDA(cudaSetDevice(b->device));
     if (maps_host)
         CMDB_CUDA(cudaMemcpyAsync(maps_host, f.acc_maps + (size_t)first * f.acc_npix, sizeof(double) * (size_t)n * f.acc_npix,
-                                  cudaMemcpyDeviceToHost, b->stream));
+                                  cudaMemcpyDeviceToHost, b->handle_stream()));
     if (scores_host)
-        CMDB_CUDA(cudaMemcpyAsync(scores_host, f.acc_scores + first, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, b->stream));
-    CMDB_CUDA(cudaStreamSynchronize(b->stream));
+        CMDB_CUDA(cudaMemcpyAsync(scores_host, f.acc_scores + first, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost,
+                                  b->handle_stream()));
+    CMDB_CUDA(cudaStreamSynchronize(b->handle_stream()));
     return CMDB_OK;
 }
 

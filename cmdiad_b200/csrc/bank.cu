@@ -184,13 +184,13 @@ void launch_split_rows(cudaStream_t stream, int num_sms, const float *x, int64_t
 }
 
 int bank_max_abs(cmdb_bank *b, const float *x, int64_t n, float *out_host) {
-    CMDB_CUDA(cudaMemsetAsync(b->absmax_buf, 0, sizeof(unsigned int), b->stream));
+    CMDB_CUDA(cudaMemsetAsync(b->absmax_buf, 0, sizeof(unsigned int), b->handle_stream()));
     int grid = (int)std::min<int64_t>((n / 4 + 511) / 512 + 1, (int64_t)b->num_sms * 4);
-    absmax_kernel<<<grid, 512, 0, b->stream>>>(x, n, b->absmax_buf);
+    absmax_kernel<<<grid, 512, 0, b->handle_stream()>>>(x, n, b->absmax_buf);
     CMDB_CUDA(cudaGetLastError());
     unsigned int bits = 0;
-    CMDB_CUDA(cudaMemcpyAsync(&bits, b->absmax_buf, sizeof(bits), cudaMemcpyDeviceToHost, b->stream));
-    CMDB_CUDA(cudaStreamSynchronize(b->stream));
+    CMDB_CUDA(cudaMemcpyAsync(&bits, b->absmax_buf, sizeof(bits), cudaMemcpyDeviceToHost, b->handle_stream()));
+    CMDB_CUDA(cudaStreamSynchronize(b->handle_stream()));
     memcpy(out_host, &bits, sizeof(float));
     return CMDB_OK;
 }
@@ -259,20 +259,18 @@ int cmdb_bank_create(int device, int dim, int64_t capacity_rows, cmdb_bank **out
     b->dim = dim;
     b->capacity = capacity_rows;
     cudaDeviceGetAttribute(&b->num_sms, cudaDevAttrMultiProcessorCount, device);
-    cudaError_t err = cudaStreamCreateWithFlags(&b->lane_stream[0], cudaStreamNonBlocking);
-    if (err == cudaSuccess) err = cudaStreamCreateWithFlags(&b->lane_stream[1], cudaStreamNonBlocking);
-    b->stream = b->lane_stream[0];
-    if (err == cudaSuccess) err = cudaStreamCreateWithFlags(&b->copy_stream, cudaStreamNonBlocking);
+    cudaError_t err = cudaStreamCreateWithFlags(&b->copy_stream, cudaStreamNonBlocking);
     if (err == cudaSuccess) err = cudaStreamCreateWithFlags(&b->d2h_stream, cudaStreamNonBlocking);
-    for (int i = 0; i < 2; ++i) {
-        if (err == cudaSuccess) err = cudaStreamCreateWithFlags(&b->lane_aux[i], cudaStreamNonBlocking);
-        if (err == cudaSuccess) err = cudaEventCreateWithFlags(&b->ev_fork[i], cudaEventDisableTiming);
-        if (err == cudaSuccess) err = cudaEventCreateWithFlags(&b->ev_join[i], cudaEventDisableTiming);
+    for (Lane &l : b->lane) {
+        if (err == cudaSuccess) err = cudaStreamCreateWithFlags(&l.stream, cudaStreamNonBlocking);
+        if (err == cudaSuccess) err = cudaStreamCreateWithFlags(&l.aux, cudaStreamNonBlocking);
+        if (err == cudaSuccess) err = cudaEventCreateWithFlags(&l.ev_fork, cudaEventDisableTiming);
+        if (err == cudaSuccess) err = cudaEventCreateWithFlags(&l.ev_join, cudaEventDisableTiming);
     }
-    for (auto &e : b->ev_done)
-        if (err == cudaSuccess) err = cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
-    for (auto &e : b->ev_compute)
-        if (err == cudaSuccess) err = cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
+    for (ResultSlot &s : b->slot) {
+        if (err == cudaSuccess) err = cudaEventCreateWithFlags(&s.ev_done, cudaEventDisableTiming);
+        if (err == cudaSuccess) err = cudaEventCreateWithFlags(&s.ev_compute, cudaEventDisableTiming);
+    }
     if (err == cudaSuccess) err = cudaEventCreateWithFlags(&b->ev_fail, cudaEventDisableTiming);
     for (auto &e : b->ev_chunk)
         if (err == cudaSuccess) err = cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
@@ -310,13 +308,7 @@ static void free_scoring_layout(cmdb_bank *b) {
 void cmdb_bank_destroy(cmdb_bank *b) {
     if (!b) return;
     cudaSetDevice(b->device);
-    for (auto st : b->lane_stream)
-        if (st) cudaStreamSynchronize(st);
-    for (auto st : b->lane_aux)
-        if (st) cudaStreamSynchronize(st);
-    if (b->copy_stream) cudaStreamSynchronize(b->copy_stream);
-    if (b->d2h_stream) cudaStreamSynchronize(b->d2h_stream);
-    free_scoring_layout(b);
+    free_scoring_layout(b);   // synchronises every stream of the handle first
     for (int i = 0; i < 2; ++i) {
         cudaFree(b->fused.dev[i]);
         if (b->fused.host[i]) cudaFreeHost(b->fused.host[i]);
@@ -331,26 +323,23 @@ void cmdb_bank_destroy(cmdb_bank *b) {
     cudaFree(b->cert_buf);
     for (auto &e : b->ev)
         if (e) cudaEventDestroy(e);
-    for (auto &l : b->ev_tl)
-        for (auto &e : l)
-            if (e) cudaEventDestroy(e);
     if (b->ev_base) cudaEventDestroy(b->ev_base);
-    for (auto &l : b->ev_dbg)
-        for (auto &e : l)
+    for (Lane &l : b->lane) {
+        for (auto &e : l.ev_tl)
             if (e) cudaEventDestroy(e);
-    if (b->lane_stream[1]) cudaStreamDestroy(b->lane_stream[1]);
-    if (b->lane_stream[0]) cudaStreamDestroy(b->lane_stream[0]);
+        for (auto &e : l.ev_dbg)
+            if (e) cudaEventDestroy(e);
+        if (l.stream) cudaStreamDestroy(l.stream);
+        if (l.aux) cudaStreamDestroy(l.aux);
+        if (l.ev_fork) cudaEventDestroy(l.ev_fork);
+        if (l.ev_join) cudaEventDestroy(l.ev_join);
+    }
     if (b->copy_stream) cudaStreamDestroy(b->copy_stream);
     if (b->d2h_stream) cudaStreamDestroy(b->d2h_stream);
-    for (int i = 0; i < 2; ++i) {
-        if (b->lane_aux[i]) cudaStreamDestroy(b->lane_aux[i]);
-        if (b->ev_fork[i]) cudaEventDestroy(b->ev_fork[i]);
-        if (b->ev_join[i]) cudaEventDestroy(b->ev_join[i]);
+    for (ResultSlot &s : b->slot) {
+        if (s.ev_done) cudaEventDestroy(s.ev_done);
+        if (s.ev_compute) cudaEventDestroy(s.ev_compute);
     }
-    for (auto &e : b->ev_done)
-        if (e) cudaEventDestroy(e);
-    for (auto &e : b->ev_compute)
-        if (e) cudaEventDestroy(e);
     if (b->ev_fail) cudaEventDestroy(b->ev_fail);
     for (auto &e : b->ev_chunk)
         if (e) cudaEventDestroy(e);
@@ -364,9 +353,9 @@ int cmdb_bank_append(cmdb_bank *b, const float *rows, int64_t n_rows, int rows_i
     if (n_rows == 0) return CMDB_OK;
     CMDB_CUDA(cudaSetDevice(b->device));
     CMDB_CUDA(cudaMemcpyAsync(b->data + b->rows * b->dim, rows, sizeof(float) * (size_t)n_rows * b->dim,
-                              rows_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, b->stream));
+                              rows_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, b->handle_stream()));
     // the caller may reuse / free its buffer as soon as we return (pageable host memory is staged synchronously anyway)
-    CMDB_CUDA(cudaStreamSynchronize(b->stream));
+    CMDB_CUDA(cudaStreamSynchronize(b->handle_stream()));
     b->rows += n_rows;
     b->finalized = false;
     return CMDB_OK;
@@ -416,13 +405,13 @@ int cmdb_bank_set_option(cmdb_bank *b, int option, int value) {
             CMDB_CUDA(cudaSetDevice(b->device));
             if (!b->ev_base) {
                 CMDB_CUDA(cudaEventCreate(&b->ev_base));
-                for (auto &l : b->ev_tl)
-                    for (auto &e : l) CMDB_CUDA(cudaEventCreate(&e));
-                for (auto &l : b->ev_dbg)
-                    for (auto &e : l) CMDB_CUDA(cudaEventCreate(&e));
+                for (Lane &l : b->lane) {
+                    for (auto &e : l.ev_tl) CMDB_CUDA(cudaEventCreate(&e));
+                    for (auto &e : l.ev_dbg) CMDB_CUDA(cudaEventCreate(&e));
+                }
             }
             CMDB_CUDA(cudaDeviceSynchronize());
-            CMDB_CUDA(cudaEventRecord(b->ev_base, b->lane_stream[0]));
+            CMDB_CUDA(cudaEventRecord(b->ev_base, b->lane[0].stream));
         }
         b->ev_valid = false;
         return CMDB_OK;
@@ -442,13 +431,14 @@ int cmdb_bank_set_query_norm(cmdb_bank *b, float mean, float stdv, int enabled) 
 
 int cmdb_bank_stream(cmdb_bank *b, void **out_stream) {
     CMDB_REQUIRE(b && out_stream, CMDB_ERR_INVALID, "cmdb_bank_stream: bad arguments");
-    *out_stream = (void *)b->lane_stream[b->next_lane];  // the lane the NEXT scoring call of this handle runs on
+    // the lane of the open sharded round (its collectives), else the lane the NEXT scoring call of this handle runs on
+    *out_stream = (void *)b->lane[b->round.open ? b->round.lane : b->next_lane].stream;
     return CMDB_OK;
 }
 
 int cmdb_bank_lane_streams(cmdb_bank *b, void **out_streams2) {
     CMDB_REQUIRE(b && out_streams2, CMDB_ERR_INVALID, "cmdb_bank_lane_streams: bad arguments");
-    out_streams2[0] = (void *)b->lane_stream[0], out_streams2[1] = (void *)b->lane_stream[1];
+    out_streams2[0] = (void *)b->lane[0].stream, out_streams2[1] = (void *)b->lane[1].stream;
     return CMDB_OK;
 }
 
@@ -490,8 +480,8 @@ int cmdb_bank_read_knn(cmdb_bank *b, int64_t row_first, int64_t n_rows, uint64_t
     if (n_rows == 0) return CMDB_OK;
     CMDB_CUDA(cudaSetDevice(b->device));
     CMDB_CUDA(cudaMemcpyAsync(out_keys, b->knn_table + (size_t)row_first * 3, sizeof(uint64_t) * 3 * (size_t)n_rows,
-                              out_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, b->stream));
-    CMDB_CUDA(cudaStreamSynchronize(b->stream));
+                              out_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, b->handle_stream()));
+    CMDB_CUDA(cudaStreamSynchronize(b->handle_stream()));
     return CMDB_OK;
 }
 
@@ -503,13 +493,13 @@ int cmdb_bank_set_knn_table(cmdb_bank *b, const uint64_t *keys, int64_t n_rows_t
                  (long long)(b->row_offset + b->fin_rows), (long long)n_rows_total);
     CMDB_REQUIRE(!b->any_pending(), CMDB_ERR_STATE, "cmdb_bank_set_knn_table: a submitted batch is outstanding");
     CMDB_CUDA(cudaSetDevice(b->device));
-    CMDB_CUDA(cudaStreamSynchronize(b->stream));
+    CMDB_CUDA(cudaStreamSynchronize(b->handle_stream()));
     cudaFree(b->knn_table);
     b->knn_table = nullptr, b->knn_rows = 0;
     CMDB_CUDA(cudaMalloc(&b->knn_table, sizeof(uint64_t) * 3 * (size_t)n_rows_total));
     CMDB_CUDA(cudaMemcpyAsync(b->knn_table, keys, sizeof(uint64_t) * 3 * (size_t)n_rows_total,
-                              keys_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, b->stream));
-    CMDB_CUDA(cudaStreamSynchronize(b->stream));
+                              keys_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, b->handle_stream()));
+    CMDB_CUDA(cudaStreamSynchronize(b->handle_stream()));
     b->knn_rows = n_rows_total;
     return CMDB_OK;
 }
@@ -517,7 +507,7 @@ int cmdb_bank_set_knn_table(cmdb_bank *b, const uint64_t *keys, int64_t n_rows_t
 int cmdb_bank_score_stats(cmdb_bank *b, int64_t *out6) {
     CMDB_REQUIRE(b && out6, CMDB_ERR_INVALID, "cmdb_bank_score_stats: bad arguments");
     CMDB_CUDA(cudaSetDevice(b->device));
-    for (auto st : b->lane_stream) CMDB_CUDA(cudaStreamSynchronize(st));
+    for (const Lane &l : b->lane) CMDB_CUDA(cudaStreamSynchronize(l.stream));
     const bool cert = b->last_mode == 0 && b->last_fail_host;
     out6[0] = b->last_queries;
     out6[1] = b->last_mode;
@@ -536,14 +526,14 @@ int cmdb_bank_stats(cmdb_bank *b, double *out_mean, double *out_std, double *out
     // stats_buf: [0] sum, [1] sum of squared deviations, [2 ..) one partial per block (sized for num_sms * 4 blocks)
     const int grid = (int)std::min<int64_t>((n / 4 + 511) / 512 + 1, (int64_t)b->num_sms * 4);
     double *part = b->stats_buf + 2;
-    stats_pass_kernel<false><<<grid, 512, 0, b->stream>>>(b->data, n, nullptr, part);
-    stats_reduce_kernel<<<1, 256, 0, b->stream>>>(part, grid, b->stats_buf);
-    stats_pass_kernel<true><<<grid, 512, 0, b->stream>>>(b->data, n, b->stats_buf, part);
-    stats_reduce_kernel<<<1, 256, 0, b->stream>>>(part, grid, b->stats_buf + 1);
+    stats_pass_kernel<false><<<grid, 512, 0, b->handle_stream()>>>(b->data, n, nullptr, part);
+    stats_reduce_kernel<<<1, 256, 0, b->handle_stream()>>>(part, grid, b->stats_buf);
+    stats_pass_kernel<true><<<grid, 512, 0, b->handle_stream()>>>(b->data, n, b->stats_buf, part);
+    stats_reduce_kernel<<<1, 256, 0, b->handle_stream()>>>(part, grid, b->stats_buf + 1);
     CMDB_CUDA(cudaGetLastError());
     double h[2];
-    CMDB_CUDA(cudaMemcpyAsync(h, b->stats_buf, sizeof(h), cudaMemcpyDeviceToHost, b->stream));
-    CMDB_CUDA(cudaStreamSynchronize(b->stream));
+    CMDB_CUDA(cudaMemcpyAsync(h, b->stats_buf, sizeof(h), cudaMemcpyDeviceToHost, b->handle_stream()));
+    CMDB_CUDA(cudaStreamSynchronize(b->handle_stream()));
     const double mean = h[0] / (double)n;
     const double var = n > 1 ? h[1] / (double)(n - 1) : NAN;  // unbiased, like torch.std
     if (out_mean) *out_mean = mean;
@@ -555,13 +545,14 @@ int cmdb_bank_stats(cmdb_bank *b, double *out_mean, double *out_std, double *out
 
 int cmdb_bank_normalize(cmdb_bank *b, float mean, float stdv) {
     CMDB_REQUIRE(b, CMDB_ERR_INVALID, "cmdb_bank_normalize: bank is NULL");
+    CMDB_REQUIRE(!b->any_pending(), CMDB_ERR_STATE, "cmdb_bank_normalize: a submitted call still reads the rows; wait for it first");
     if (b->rows == 0) return CMDB_OK;
     CMDB_CUDA(cudaSetDevice(b->device));
     const int64_t n = b->rows * b->dim;
     int grid = (int)std::min<int64_t>((n / 4 + 511) / 512 + 1, (int64_t)b->num_sms * 4);
-    normalize_kernel<<<grid, 512, 0, b->stream>>>(b->data, n, mean, stdv);
+    normalize_kernel<<<grid, 512, 0, b->handle_stream()>>>(b->data, n, mean, stdv);
     CMDB_CUDA(cudaGetLastError());
-    CMDB_CUDA(cudaStreamSynchronize(b->stream));
+    CMDB_CUDA(cudaStreamSynchronize(b->handle_stream()));
     b->finalized = false;
     return CMDB_OK;
 }
@@ -573,6 +564,7 @@ int cmdb_bank_gather(cmdb_bank *b, const int64_t *idx_host, int64_t n) {
         CMDB_REQUIRE(idx_host[i] >= 0 && idx_host[i] < b->rows, CMDB_ERR_INVALID,
                      "cmdb_bank_gather: idx[%lld]=%lld out of range [0,%lld)", (long long)i, (long long)idx_host[i],
                      (long long)b->rows);
+    CMDB_REQUIRE(!b->any_pending(), CMDB_ERR_STATE, "cmdb_bank_gather: a submitted call still reads the rows; wait for it first");
     CMDB_CUDA(cudaSetDevice(b->device));
     long long *idx_dev = nullptr;
     float *tmp = nullptr;
@@ -582,15 +574,15 @@ int cmdb_bank_gather(cmdb_bank *b, const int64_t *idx_host, int64_t n) {
         cudaFree(idx_dev);
         CMDB_CUDA(e);
     }
-    e = cudaMemcpyAsync(idx_dev, idx_host, sizeof(long long) * (size_t)n, cudaMemcpyHostToDevice, b->stream);
+    e = cudaMemcpyAsync(idx_dev, idx_host, sizeof(long long) * (size_t)n, cudaMemcpyHostToDevice, b->handle_stream());
     if (e == cudaSuccess) {
         int grid = (int)std::min<int64_t>((n + 7) / 8, (int64_t)b->num_sms * 8);
-        gather_rows_kernel<<<grid, 256, 0, b->stream>>>(b->data, tmp, idx_dev, n, b->dim / 4);
+        gather_rows_kernel<<<grid, 256, 0, b->handle_stream()>>>(b->data, tmp, idx_dev, n, b->dim / 4);
         e = cudaGetLastError();
     }
     if (e == cudaSuccess)
-        e = cudaMemcpyAsync(b->data, tmp, sizeof(float) * (size_t)n * b->dim, cudaMemcpyDeviceToDevice, b->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(b->stream);
+        e = cudaMemcpyAsync(b->data, tmp, sizeof(float) * (size_t)n * b->dim, cudaMemcpyDeviceToDevice, b->handle_stream());
+    if (e == cudaSuccess) e = cudaStreamSynchronize(b->handle_stream());
     cudaFree(idx_dev);
     cudaFree(tmp);
     CMDB_CUDA(e);
@@ -606,8 +598,8 @@ int cmdb_bank_read(cmdb_bank *b, int64_t row0, int64_t n_rows, float *out_host) 
     if (n_rows == 0) return CMDB_OK;
     CMDB_CUDA(cudaSetDevice(b->device));
     CMDB_CUDA(cudaMemcpyAsync(out_host, b->data + row0 * b->dim, sizeof(float) * (size_t)n_rows * b->dim,
-                              cudaMemcpyDeviceToHost, b->stream));
-    CMDB_CUDA(cudaStreamSynchronize(b->stream));
+                              cudaMemcpyDeviceToHost, b->handle_stream()));
+    CMDB_CUDA(cudaStreamSynchronize(b->handle_stream()));
     return CMDB_OK;
 }
 
@@ -616,6 +608,8 @@ int cmdb_bank_finalize(cmdb_bank *b) {
     CMDB_REQUIRE(b->rows > 0, CMDB_ERR_STATE, "cmdb_bank_finalize: bank is empty");
     CMDB_REQUIRE(b->rows + b->row_offset < (1LL << 31), CMDB_ERR_UNSUPPORTED,
                  "cmdb_bank_finalize: global row numbers must fit 31 bits for the packed (distance,row) keys");
+    CMDB_REQUIRE(!b->any_pending(), CMDB_ERR_STATE,
+                 "cmdb_bank_finalize: a submitted call still uses the scoring layout; wait for it first");
     CMDB_CUDA(cudaSetDevice(b->device));
     free_scoring_layout(b);
     const int64_t pad = (b->rows + kScoreBN - 1) / kScoreBN * kScoreBN;
@@ -627,13 +621,13 @@ int cmdb_bank_finalize(cmdb_bank *b) {
     CMDB_REQUIRE(isfinite(absmax), CMDB_ERR_INVALID, "cmdb_bank_finalize: bank contains non-finite values");
     b->scale_exp = pick_scale_exp(absmax);
     if (!b->cert_buf) CMDB_CUDA(cudaMalloc(&b->cert_buf, 2 * sizeof(unsigned int)));
-    CMDB_CUDA(cudaMemsetAsync(b->cert_buf, 0, 2 * sizeof(unsigned int), b->stream));
-    launch_split_rows(b->stream, b->num_sms, b->data, b->rows, pad, b->dim, b->scale_exp, b->hi, b->lo, b->norm, INFINITY,
+    CMDB_CUDA(cudaMemsetAsync(b->cert_buf, 0, 2 * sizeof(unsigned int), b->handle_stream()));
+    launch_split_rows(b->handle_stream(), b->num_sms, b->data, b->rows, pad, b->dim, b->scale_exp, b->hi, b->lo, b->norm, INFINITY,
                       b->cert_buf);
     CMDB_CUDA(cudaGetLastError());
     float cert[2] = {0.f, 0.f};
-    CMDB_CUDA(cudaMemcpyAsync(cert, b->cert_buf, sizeof(cert), cudaMemcpyDeviceToHost, b->stream));
-    CMDB_CUDA(cudaStreamSynchronize(b->stream));
+    CMDB_CUDA(cudaMemcpyAsync(cert, b->cert_buf, sizeof(cert), cudaMemcpyDeviceToHost, b->handle_stream()));
+    CMDB_CUDA(cudaStreamSynchronize(b->handle_stream()));
     b->cert_bmax = cert[0], b->cert_eb_max = cert[1];
     b->direct_calls_left = 0, b->fail_pending = false;
     b->fin_rows = b->rows;

@@ -45,7 +45,7 @@ constexpr int kScoreBM = 128;        // query rows per GEMM tile
 constexpr int kGemmEpiGroups = 2;    // epilogue warp groups per GEMM CTA: producers = groups * CTAs
 constexpr int kResultSlots = 3;      // result blocks / outstanding submitted calls per handle (the compute lanes stay two)
 constexpr int kMaxStageChunks = 4;   // host query batches are staged and multiplied in up to this many chunks
-constexpr int kWorkCap = 16384;      // capacity of ScoreScratch::work_list
+constexpr int kWorkCap = 16384;      // capacity of Lane::work_list
 // Fallback tiers of the certified pre-filter.  Tier 1, exact rescan: ~R/296 rows x D x 4 B per (query, producer) pair, HBM
 // bound (~0.32 us per pair at 200k x 768) -- RIGOROUS: the result equals the exact float32 scan, lowest row on ties.
 // Tier 2, 3-term GEMM over the compacted uncertified queries + exact re-check of the 4 best candidates: at least one sweep
@@ -60,12 +60,28 @@ __host__ __device__ inline bool fallback_use_rescan(int fails, int pairs) {
 }
 constexpr int kScoreBK = 64;         // fp16 K elements per pipeline stage (one 128-byte swizzle row)
 
-// device scratch of one scoring call, sized at finalize time
-struct ScoreScratch {
-    int cap_p = 0;                  // padded query-row capacity of a sub-batch (multiple of 128)
-    int cap_b = 0;                  // image capacity of a sub-batch
-    float *q_f32 = nullptr;         // [cap_p, D]  normalised query patches (the slot selected by score_select_slot)
-    float *q_f32_buf[kResultSlots] = {};   // per result slot: batches k+1 and k+2 are staged while batch k is still scored
+// Sizes of the scoring scratch of a handle (score_scratch_alloc), common to both lanes and all result slots.  The results
+// of a call live in ONE device block (tail | min_val | min_idx | map_out | map_pre | map_u8) mirrored by a pinned host
+// block, so a scoring call ends with a single device->host copy; the offsets below locate the sections.
+struct ScoreLayout {
+    int cap_p = 0;          // padded query-row capacity of a sub-batch (multiple of 128)
+    int cap_b = 0;          // image capacity of a sub-batch
+    size_t map_stride = 0;  // pixels reserved per image in the map sections
+    size_t off_min_val = 0, off_min_idx = 0, off_map_out = 0, off_map_pre = 0, off_map_u8 = 0, out_block_bytes = 0;
+    int n_topk_blocks = 0;  // blocks of reweight_kernel
+};
+
+// A compute lane: the streams a call runs on and every device buffer that lives only while a call computes.  Call k runs on
+// lane k & 1, so the tail of a batch / round -- certificate, rescans, exchanges, re-weighting, maps -- overlaps the
+// distance GEMM of the next one (the GEMM is one persistent CTA per SM; the small tail kernels fit beside it).
+struct Lane {
+    cudaStream_t stream = nullptr;
+    cudaStream_t aux = nullptr;     // side stream of the (normally empty) tier-2 launches and the counters copy, beside the rescan
+    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
+    // CMDB_OPT_TIMING = 2 (diagnostics): this lane's stage marks and the four marks inside the refine stage (before / after
+    // the certificate kernel, after the rescan, after the tier-2 launches), read by cmdb_debug_lane_timeline
+    cudaEvent_t ev_tl[CMDB_T_COUNT + 1] = {};
+    cudaEvent_t ev_dbg[4] = {};
     __half *q_hi = nullptr;         // [cap_p, D]  split-fp16 query operand
     __half *q_lo = nullptr;
     int *q_scale_exp = nullptr;     // device [cap_p]: per-row exponent e_q with q_hi + q_lo = q * 2^e_q
@@ -78,42 +94,39 @@ struct ScoreScratch {
     // GEMM), [5] / [6] last-block tickets of the certificate / rescan kernels; the per-image argmax keys (s_key) follow at
     // fail_ctl + 8 in the same allocation so that one memset clears both
     int *fail_ctl = nullptr;
+    unsigned long long *s_key = nullptr;    // [cap_b] packed argmax key of min_val
     int *fail_count_host = nullptr; // pinned copy of [0..1] (statistics / adaptive mode)
-    bool sched_pair = false;            // the last first-pass GEMM ran on CTA pairs (cta_group::2)
-    bool sched_pair_last = false;       // ... and the most recent GEMM launch of any kind
-    int sched_run_last = 1;             // N tiles per visit (score_gemm_run) of the most recent GEMM launch
-    int chunk_tiles = 0, mt_total = 0;  // M-tile layout of the last first-pass GEMM: chunks of chunk_tiles tiles (rescan needs it)
     int2 *work_list = nullptr;      // [kWorkCap] (query row, producer) pairs whose producer may hide rows inside the band
     unsigned long long *best_key = nullptr;  // [cap_p] running exact (d^2 bits << 32 | row) of the uncertified queries
-    void *tmap_qhi = nullptr;       // host CUtensorMap objects for q_hi / q_lo
-    void *tmap_qlo = nullptr;
-    float *m_test = nullptr;        // [D] patch[s_idx]
-    float *m_star = nullptr;        // [D] bank[min_idx[s_idx]]
-    unsigned long long *top3 = nullptr;  // merged 3 smallest w_dist keys
-    int n_topk_blocks = 0;
     unsigned int *done_counter = nullptr;  // last-block-done counter of reweight_kernel
     float4 *cand = nullptr;         // [n_ctas, cap_p] per-CTA running top-2 (val1, idx1, val2, idx2) of the GEMM epilogue
-    float *min_val = nullptr;       // [cap_p]
-    long long *min_idx = nullptr;   // [cap_p]
-    unsigned long long *s_key = nullptr;    // packed argmax key of min_val
+    unsigned char *map_tmp = nullptr;  // horizontally blurred 8-bit images between the two blur kernels
+    float *map_max = nullptr;       // [cap_b] map maxima, then [cap_b][16] band maxima
     unsigned long long *topk_keys = nullptr;  // [n_blocks*3] per-block w_dist top-3 packed keys
-    void *tail = nullptr;           // TailResult
-    // results live in ONE device block (tail | min_val | min_idx | map_out | map_pre | map_u8) mirrored by a pinned
-    // host block, so a scoring call ends with a single device->host copy
-    unsigned char *out_block = nullptr;       // (current slot)
-    unsigned char *out_block_host = nullptr;  // cudaMallocHost
-    // per RESULT SLOT (kResultSlots of them, cycled independently of the two lanes): the results of batches k - 1 and k
-    // travel to the host / wait for the caller while batch k + 1 is already enqueued behind batch k - 1 on its lane
-    unsigned char *out_block_buf[kResultSlots] = {};
-    unsigned char *out_block_host_buf[kResultSlots] = {};
-    size_t off_min_val = 0, off_min_idx = 0, off_map_out = 0, off_map_pre = 0, off_map_u8 = 0, out_block_bytes = 0;
-    size_t map_stride = 0;  // pixels reserved per image in the map sections
-    float *map_pre = nullptr;       // [out_hw^2]
-    float *map_out = nullptr;
-    unsigned char *map_u8 = nullptr;
-    unsigned char *map_tmp = nullptr;  // horizontally blurred 8-bit image between the two blur kernels
-    float *map_max = nullptr;
-    int map_cap = 0;
+    unsigned long long *top3 = nullptr;  // merged 3 smallest w_dist keys
+    float *m_test = nullptr;        // [cap_b, D] patch[s_idx]
+    float *m_star = nullptr;        // [cap_b, D] bank[min_idx[s_idx]]
+    void *tmap_qhi = nullptr;       // host CUtensorMap objects for q_hi / q_lo
+    void *tmap_qlo = nullptr;
+};
+
+// A result slot: what a submitted call holds until the caller has waited for it.  The slots cycle independently of the
+// lanes (call k uses slot k % kResultSlots), so the results of calls k - 1 and k travel to the host / wait for the caller
+// while call k + 1 is already enqueued, and its queries are staged while call k is still scored.
+struct ResultSlot {
+    float *q_f32 = nullptr;                 // [cap_p, D] normalised query patches
+    unsigned char *out_block = nullptr;     // device result block (ScoreLayout)
+    unsigned char *out_block_host = nullptr;  // its pinned mirror
+    cudaEvent_t ev_done = nullptr;          // the block is in the pinned host memory
+    cudaEvent_t ev_compute = nullptr;       // the kernels of the call that used the slot are done (q_f32 may be overwritten)
+    struct Pending {
+        bool active = false;
+        int B = 0, P = 0, out_hw = 0;
+        unsigned want = 0;
+        bool host_maps = true;   // false: the per-modality maps stay in HBM (fused late-fusion head), only scalars travel
+        int img_first = 0, img_step = 1;  // images whose maps were finished (a sharded round's rank: its share; a batch: all)
+        long long ticket = 0;
+    } pending;
 };
 
 }  // namespace cmdb
@@ -144,35 +157,27 @@ struct cmdb_bank {
     int last_mode = 0;           // GEMM mode the last call actually ran
     bool fail_pending = false;   // fail_count_host holds the count of a finished-or-in-flight call
     int direct_calls_left = 0;   // certified mode: calls to run directly with 3 terms before probing the pre-filter again
-    // Two compute LANES: scoring call k runs on lane k & 1 (its own stream and its own copy of every scratch buffer, ss_store),
-    // so the tail of a batch / round -- certificate, rescans, exchanges, re-weighting, maps -- overlaps the distance GEMM of
-    // the next one (the GEMM is one persistent CTA per SM; the small tail kernels fit beside it).  `stream` and `ss` are the
-    // lane currently selected (score_select_slot); everything that is not scoring runs on whichever lane is current.
-    cudaStream_t stream = nullptr;
-    cudaStream_t lane_stream[2] = {nullptr, nullptr};
-    // per lane: side stream for the (normally empty) tier-2 launches and the counters copy, which run beside the rescan
-    cudaStream_t lane_aux[2] = {nullptr, nullptr};
-    cudaEvent_t ev_fork[2] = {}, ev_join[2] = {};
-    cmdb::ScoreScratch ss_store[2];
+    // Scoring calls take the next of the two compute lanes and the next of the kResultSlots result slots (cmdb::ScoreCall,
+    // api.cu).  Everything else -- append, read, statistics, normalize, gather, finalize, coreset, projection, evaluation --
+    // runs on lane 0's stream (handle_stream()).
+    cmdb::ScoreLayout layout;
+    cmdb::Lane lane[2];
+    cmdb::ResultSlot slot[cmdb::kResultSlots];
+    int next_lane = 0;    // compute lane of the next scoring call (alternates)
+    int next_slot = 0;    // result slot of the next scoring call (cycles through kResultSlots)
+    int last_lane = 0;    // lane of the most recent scoring call or table build (cmdb_debug_read_candidates)
+    // the sharded round opened by cmdb_score_shard_min and closed by cmdb_score_shard_finish_submit
+    struct Round { bool open = false; int lane = 0, slot = 0; } round;
     int *last_fail_host = nullptr;   // pinned certificate counters of the most recent certified call (either lane)
     cudaStream_t copy_stream = nullptr;   // host -> device staging of query chunks, overlapped with the GEMM of earlier chunks
     cudaEvent_t ev_chunk[cmdb::kMaxStageChunks] = {};
     cudaStream_t d2h_stream = nullptr;    // device -> host copies of the results
-    cudaEvent_t ev_done[cmdb::kResultSlots] = {};   // result slot's block is in the pinned host memory
-    cudaEvent_t ev_compute[cmdb::kResultSlots] = {};   // the kernels of the call that used the slot are done (its q_f32 may be overwritten)
     cudaEvent_t ev_fail = nullptr;        // the certificate counters of the last certified call are on the host
-    struct Pending {
-        bool active = false;
-        int B = 0, P = 0, out_hw = 0;
-        unsigned want = 0;
-        bool host_maps = true;   // false: the per-modality maps stay in HBM (fused late-fusion head), only scalars travel
-        int img_first = 0, img_step = 1;  // images whose maps were finished (a sharded round's rank: its share; a batch: all)
-        long long ticket = 0;
-    } pending[cmdb::kResultSlots];
-    bool any_pending() const {
-        for (const auto &p : pending)
-            if (p.active) return true;
-        return false;
+    cudaStream_t handle_stream() const { return lane[0].stream; }
+    bool any_pending() const {  // a submitted call (batch, round, fused batch) still uses the handle's buffers
+        for (const auto &s : slot)
+            if (s.pending.active) return true;
+        return fused.active[0] || fused.active[1];
     }
     // queries are normalised on the device right after staging: (q - q_mean) / q_std, one IEEE subtract + one IEEE divide
     // like the reference's torch expression (multiple_features.py:90, 976-977); cmdb_bank_set_query_norm
@@ -198,10 +203,6 @@ struct cmdb_bank {
         int acc_npix = 0;
     } fused;
     long long ticket_counter = 0;
-    int next_slot = 0;    // result slot of the next submitted call (cycles through kResultSlots)
-    int next_lane = 0;    // compute lane of the next submitted call (alternates)
-    int shard_lane = 0;   // lane of the sharded round in progress
-    int shard_slot = 0;   // result slot of the sharded round in progress (cmdb_score_shard_min .. finish)
     cmdb_comm *comm = nullptr;             // peer buffers for NCCL-free sharded rounds (cmdb_bank_attach_comm; not owned)
     unsigned int *shard_ctr = nullptr;     // [0] device: last-block counter of the push kernels
     unsigned int *shard_abort_host = nullptr;  // pinned + mapped: set by a kernel whose peers never arrived
@@ -220,16 +221,12 @@ struct cmdb_bank {
     void *tmap_lo = nullptr;
     void *tmap_hi2 = nullptr;  // box of 128 bank rows (CTA-pair kernels)
     void *tmap_lo2 = nullptr;
-    cmdb::ScoreScratch ss;
     int timing = 0;
     cudaEvent_t ev[CMDB_T_COUNT + 1] = {};
     bool ev_valid = false;
-    // CMDB_OPT_TIMING = 2 (diagnostics): per-lane copies of the stage events and a common time base, so that the
-    // overlap of the two lanes can be read (cmdb_debug_lane_timeline)
-    cudaEvent_t ev_tl[2][CMDB_T_COUNT + 1] = {};
+    // CMDB_OPT_TIMING = 2 (diagnostics): common time base of the lanes' stage events (Lane::ev_tl), so that the overlap of
+    // the two lanes can be read (cmdb_debug_lane_timeline)
     cudaEvent_t ev_base = nullptr;
-    cudaEvent_t ev_dbg[2][4] = {};   // inside the refine stage: before / after the certificate kernel, after the rescan, after the tier-2 launches
-    int cur_slot = 0;
     double *stats_buf = nullptr;  // 2 + num_sms * 4 doubles on device (cmdb_bank_stats)
     unsigned int *absmax_buf = nullptr;
 };
@@ -284,24 +281,56 @@ int coreset_greedy(cmdb_bank *b, const double *z_dev, int64_t N, int d, int64_t 
 int coreset_rownorms(int device, const void *z_host, const void *last_host, int64_t n_rows, int d, int dtype_mode,
                      void *out_host);
 
+struct TailResult {  // head of a result block (ScoreCall::tail), one per image
+    float s, s_star, w, knn0, knn1;
+    int s_idx;
+    long long nn_idx[3];
+    long long m_star_row;  // global row of m_star
+};
+
+// One scoring call: the handle, the compute lane and result slot it uses, and where in the slot's result block its
+// results go.  The submit paths take the next lane and slot (api.cu); the neighbour-table build uses lane 0.
+struct ScoreCall {
+    cmdb_bank *b;
+    int lane_idx, slot_idx;
+    Lane *lane;
+    ResultSlot *slot;
+    cudaStream_t stream;   // the lane's stream
+    TailResult *tail;      // [cap_b]
+    float *min_val;        // [cap_p]
+    long long *min_idx;    // [cap_p]
+    float *map_out, *map_pre;   // [cap_b][map_stride]
+    unsigned char *map_u8;
+    // first-pass GEMM schedule of score_local_min (the exact rescan walks it): M tiles, chunks of chunk_tiles tiles, CTA pairs
+    int mt_total = 0, chunk_tiles = 0;
+    bool pair = false;
+};
+// launch schedule of one distance-GEMM launch
+struct GemmSched {
+    int producers;  // (CTA, column group) candidate lists
+    bool pair;      // CTA pairs (cta_group::2)
+    int run;        // N tiles per visit of an M tile (score_gemm_run)
+};
+
 // score_gemm.cu
 int score_scratch_alloc(cmdb_bank *b, int B, int P_img, int out_hw);
-void score_select_slot(cmdb_bank *b, int lane, int rslot);  // lane's stream / scratch / q_f32, result pointers at block `rslot`
+ScoreCall score_call(cmdb_bank *b, int lane, int slot);  // call on that lane with its results in that slot's block
+int score_mark(const ScoreCall &c, int stage, cudaStream_t st);  // timing event of `stage` (< 0: none) on st
 int score_max_batch(const cmdb_bank *b);  // images per internal sub-batch (shared-memory bound of reweight_kernel)
 void score_scratch_free(cmdb_bank *b);
 int score_make_tensor_maps(cmdb_bank *b);
-// q_f32 -> q_hi / q_lo (device-side scale selection).  compact = true: only the rows of ss.fail_list (count on the
+// q_f32 -> q_hi / q_lo (device-side scale selection) on st.  compact = true: only the rows of fail_list (count on the
 // device), written to rows 0..count-1
-int score_query_prep(cmdb_bank *b, int P, bool compact, int row0 = 0);  // rows [row0, row0 + P) (row0 % 128 == 0)
-// q_hi / q_lo -> cand via the tcgen05 distance GEMM with `terms` MMAs per K step; compact = true: the M extent is the
-// device-side fail count
-int score_gemm_candidates(cmdb_bank *b, int P, int terms, bool compact, int *n_cand_out, int row0 = 0);
-void q_split_rows(cmdb_bank *b, const float *rows_dev, int n);
+int score_query_prep(const ScoreCall &c, cudaStream_t st, int P, bool compact, int row0 = 0);  // rows [row0, row0 + P) (row0 % 128 == 0)
+// q_hi / q_lo -> cand via the tcgen05 distance GEMM with `terms` MMAs per K step on st; compact = true: the M extent is
+// the device-side fail count
+int score_gemm_candidates(const ScoreCall &c, cudaStream_t st, int P, int terms, bool compact, GemmSched *sched, int row0 = 0);
+void q_split_rows(const ScoreCall &c, const float *rows_dev, int n);
 int score_tile_stride(int mt, int G); // host copy of the GEMM's tile schedule stride
 int score_gemm_run(int nt, int mt_units, int G);  // N tiles per visit of an M tile for a launch of that shape
 // stage the queries (src: host or device, [B*P_img, dim]) + candidates + refine, all modes
 // stage_after: event the copy stream waits for before it overwrites q_f32 (nullptr: everything queued so far)
-int score_local_min(cmdb_bank *b, const float *src, int src_is_device, int B, int P_img, int ev_gemm, int ev_refine,
+int score_local_min(ScoreCall &c, const float *src, int src_is_device, int B, int P_img, int ev_gemm, int ev_refine,
                     cudaEvent_t stage_after = nullptr);
 
 // The distance GEMM keeps one persistent CTA per SM with ~200 KB of dynamic shared memory, i.e. the SM runs in its largest
@@ -315,27 +344,20 @@ void api_prefer_carveout();    // api.cu
 void bank_prefer_carveout();   // bank.cu
 
 // score_tail.cu
-struct TailResult {  // device-side result block (ScoreScratch::tail)
-    float s, s_star, w, knn0, knn1;
-    int s_idx;
-    long long nn_idx[3];
-    long long m_star_row;  // global row of m_star
-};
-int score_simt_candidates(cmdb_bank *b, int P, int *n_cand_out);
-int score_refine(cmdb_bank *b, int B, int P_img, int n_cand, bool compact);
-int score_refine_certified(cmdb_bank *b, int B, int P_img, int n_cand);
-int score_select(cmdb_bank *b, int B, int P_img, bool local_m_star);
-int score_reweight(cmdb_bank *b, int B, int P_img);
+int score_simt_candidates(const ScoreCall &c, int P, int *n_cand_out);
+int score_refine(const ScoreCall &c, cudaStream_t st, int B, int P_img, int n_cand, bool compact);
+int score_select(const ScoreCall &c, int B, int P_img, bool local_m_star);
+int score_reweight(const ScoreCall &c, int B, int P_img);
 int score_build_knn_table(cmdb_bank *b, long long row_first, long long row_count);
 int score_exact_scan(cmdb_bank *b, const float *q_dev, int P, unsigned long long *keys_dev);
-int score_shard_lookup(cmdb_bank *b, int B, float *contrib_dev);
-int score_shard_final(cmdb_bank *b, int B, const float *d2_sum_dev);
+int score_shard_lookup(const ScoreCall &c, int B, float *contrib_dev);
+int score_shard_final(const ScoreCall &c, int B, const float *d2_sum_dev);
 // peer-memory form of the two exchanges of a sharded round (no NCCL): see score_tail.cu
 struct PeerPtrs {
     unsigned char *p[kMaxRanks];
 };
-int score_shard_exchange_keys(cmdb_bank *b, int B, int P_img, const PeerPtrs &peers, int world, int rank, int slot, unsigned long long epoch);
-int score_shard_exchange_d2(cmdb_bank *b, int B, const PeerPtrs &peers, int world, int rank, int slot, unsigned long long epoch,
+int score_shard_exchange_keys(const ScoreCall &c, int B, int P_img, const PeerPtrs &peers, int world, int rank, int slot, unsigned long long epoch);
+int score_shard_exchange_d2(const ScoreCall &c, int B, const PeerPtrs &peers, int world, int rank, int slot, unsigned long long epoch,
                             const float *contrib_dev, float *d2_sum_dev);
 int upsample_blur_launch(cudaStream_t stream, int n_img, int img_first, int img_step, size_t map_stride, const float *map_dev,
                          int fh, int fw, int out_hw, float *pre_dev, float *out_dev, unsigned char *u8_dev,

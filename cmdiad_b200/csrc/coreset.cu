@@ -753,7 +753,7 @@ static int launch_coreset(cmdb_bank *b, CoresetParams p) {
         int per_sm = 0;
         CMDB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kCsThreads, smem));
         CMDB_REQUIRE(per_sm >= 1, CMDB_ERR_CUDA, "coreset: persistent kernel does not fit on an SM (smem %zu)", smem);
-        CMDB_CUDA(cudaMemsetAsync(p.slots, 0, sizeof(PickSlot) * 2 * grid, b->stream));
+        CMDB_CUDA(cudaMemsetAsync(p.slots, 0, sizeof(PickSlot) * 2 * grid, b->handle_stream()));
         // The projected bank is re-read once per pick.  B200's L2 (126 MB) cannot hold a 120 MB cyclic sweep under its
         // default replacement (measured: 20 % hit rate), so pin as much of it as the persisting carve-out allows and
         // stream the rest: DRAM traffic per pick drops to roughly (1 - hitRatio) of the bank.
@@ -777,15 +777,15 @@ static int launch_coreset(cmdb_bank *b, CoresetParams p) {
                     (float)std::min(1.0, (double)carve / (double)attr.accessPolicyWindow.num_bytes);
                 attr.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
                 attr.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-                persisting = cudaStreamSetAttribute(b->stream, cudaStreamAttributeAccessPolicyWindow, &attr) == cudaSuccess;
+                persisting = cudaStreamSetAttribute(b->handle_stream(), cudaStreamAttributeAccessPolicyWindow, &attr) == cudaSuccess;
             }
             (void)cudaGetLastError();
         }
         void *args[] = {&p};
-        cudaError_t le = cudaLaunchCooperativeKernel((void *)kern, dim3(grid), dim3(kCsThreads), args, smem, b->stream);
+        cudaError_t le = cudaLaunchCooperativeKernel((void *)kern, dim3(grid), dim3(kCsThreads), args, smem, b->handle_stream());
         if (persisting) {
             attr.accessPolicyWindow.num_bytes = 0;
-            cudaStreamSetAttribute(b->stream, cudaStreamAttributeAccessPolicyWindow, &attr);
+            cudaStreamSetAttribute(b->handle_stream(), cudaStreamAttributeAccessPolicyWindow, &attr);
             // the carve-out is released by the caller after the kernel has finished (coreset_greedy_dev)
         }
         CMDB_CUDA(le);
@@ -816,7 +816,7 @@ int coreset_greedy_dev(cmdb_bank *b, const double *z_dev, int64_t N, int d, int6
                  "coreset: unknown dtype_mode %d", dtype_mode);
     CMDB_REQUIRE(!sharded || (!force_idx_host && N > 0), CMDB_ERR_UNSUPPORTED,
                  "coreset: the row-sharded loop needs non-empty shards and does not support teacher forcing");
-    cudaStream_t st = b->stream;
+    cudaStream_t st = b->handle_stream();
     long long *idx_dev = nullptr, *force_dev = nullptr;
     PickSlot *slots = nullptr;
     __half *zh_alloc = nullptr;

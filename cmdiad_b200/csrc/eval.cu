@@ -251,9 +251,9 @@ int cmdb_debug_eval_load(cmdb_bank *b, const double *maps_host, int64_t n_images
                  f.acc_n, (long long)n_images, f.acc_cap);
     CMDB_CUDA(cudaSetDevice(b->device));
     CMDB_CUDA(cudaMemcpyAsync(f.acc_maps + (size_t)f.acc_n * f.acc_npix, maps_host, sizeof(double) * (size_t)n_images * f.acc_npix,
-                              cudaMemcpyHostToDevice, b->stream));
-    CMDB_CUDA(cudaMemsetAsync(f.acc_scores + f.acc_n, 0, sizeof(double) * (size_t)n_images, b->stream));
-    CMDB_CUDA(cudaStreamSynchronize(b->stream));
+                              cudaMemcpyHostToDevice, b->handle_stream()));
+    CMDB_CUDA(cudaMemsetAsync(f.acc_scores + f.acc_n, 0, sizeof(double) * (size_t)n_images, b->handle_stream()));
+    CMDB_CUDA(cudaStreamSynchronize(b->handle_stream()));
     f.acc_n += n_images;
     return CMDB_OK;
 }
@@ -281,7 +281,7 @@ int cmdb_eval_pixel_metrics(cmdb_bank *b, const int32_t *labels_host, int64_t n_
         CMDB_REQUIRE(ok_rank_pos_host[t] >= 0 && ok_rank_pos_host[t] < n_neg && (t == 0 || ok_rank_pos_host[t] >= ok_rank_pos_host[t - 1]),
                      CMDB_ERR_INVALID, "cmdb_eval_pixel_metrics: threshold ranks must be ascending and inside [0, %lld)", n_neg);
     CMDB_CUDA(cudaSetDevice(b->device));
-    cudaStream_t st = b->stream;
+    cudaStream_t st = b->handle_stream();
     const int n_blocks = (int)std::min<long long>((n + kSortThreads * 32 - 1) / (kSortThreads * 32), (long long)b->num_sms * 8);
     const int n_warps = n_blocks * kSortWarps;
     const long long per_warp = ((n + n_warps - 1) / n_warps + 31) / 32 * 32;

@@ -86,7 +86,7 @@ int project_rows(cmdb_bank *b, const float *x_dev, int64_t n_rows, int D, const 
     double *data_d = nullptr;  // [nnz] doubles followed by [nnz] int32 indices (generic path)
     cudaError_t e = cudaMalloc(&indptr_d, sizeof(int) * (d_proj + 1));
     if (e == cudaSuccess)
-        e = cudaMemcpyAsync(indptr_d, indptr_h, sizeof(int) * (d_proj + 1), cudaMemcpyHostToDevice, b->stream);
+        e = cudaMemcpyAsync(indptr_d, indptr_h, sizeof(int) * (d_proj + 1), cudaMemcpyHostToDevice, b->handle_stream());
     unsigned short *packed_h = nullptr;
     if (e == cudaSuccess && uniform) {
         packed_h = (unsigned short *)malloc(sizeof(unsigned short) * (size_t)nnz);
@@ -95,14 +95,14 @@ int project_rows(cmdb_bank *b, const float *x_dev, int64_t n_rows, int D, const 
         e = cudaMalloc(&packed_d, sizeof(unsigned short) * (size_t)nnz);
         if (e == cudaSuccess)
             e = cudaMemcpyAsync(packed_d, packed_h, sizeof(unsigned short) * (size_t)nnz, cudaMemcpyHostToDevice,
-                                b->stream);
+                                b->handle_stream());
     } else if (e == cudaSuccess) {
         e = cudaMalloc(&data_d, (sizeof(double) + sizeof(int)) * (size_t)(nnz > 0 ? nnz : 1));
         if (e == cudaSuccess && nnz > 0)
-            e = cudaMemcpyAsync(data_d, data_h, sizeof(double) * (size_t)nnz, cudaMemcpyHostToDevice, b->stream);
+            e = cudaMemcpyAsync(data_d, data_h, sizeof(double) * (size_t)nnz, cudaMemcpyHostToDevice, b->handle_stream());
         if (e == cudaSuccess && nnz > 0)
             e = cudaMemcpyAsync(reinterpret_cast<int *>(data_d + nnz), indices_h, sizeof(int) * (size_t)nnz,
-                                cudaMemcpyHostToDevice, b->stream);
+                                cudaMemcpyHostToDevice, b->handle_stream());
     }
     if (e == cudaSuccess) {
         const size_t csr_bytes = sizeof(int) * (d_proj + 1) + (uniform ? sizeof(unsigned short) * (size_t)nnz : 0) + 16;
@@ -118,7 +118,7 @@ int project_rows(cmdb_bank *b, const float *x_dev, int64_t n_rows, int D, const 
             const int grid = (int)std::min<int64_t>(n_tiles, (int64_t)b->num_sms);
             auto launch = [&](auto kern) {
                 cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                kern<<<grid, 256, smem, b->stream>>>(x_dev, n_rows, D, indptr_d, packed_d, data_d, mag, d_proj, nnz, z_dev);
+                kern<<<grid, 256, smem, b->handle_stream()>>>(x_dev, n_rows, D, indptr_d, packed_d, data_d, mag, d_proj, nnz, z_dev);
             };
             if (rt == 32) launch(project_kernel<32>);
             else if (rt == 16) launch(project_kernel<16>);
@@ -126,7 +126,7 @@ int project_rows(cmdb_bank *b, const float *x_dev, int64_t n_rows, int D, const 
             e = cudaGetLastError();
         }
     }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(b->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(b->handle_stream());
     free(packed_h);
     cudaFree(indptr_d);
     cudaFree(packed_d);

@@ -604,37 +604,37 @@ void gemm_prefer_carveout() {
     (void)cudaGetLastError();
 }
 
-static void free_lane(ScoreScratch &s) {
-    cudaFree(s.q_hi), cudaFree(s.q_lo), cudaFree(s.q_scale_exp);
-    cudaFree(s.cand), cudaFree(s.topk_keys);   // s_key lives inside the fail_ctl allocation
-    cudaFree(s.map_tmp), cudaFree(s.map_max), cudaFree(s.m_test), cudaFree(s.m_star);
-    cudaFree(s.top3), cudaFree(s.done_counter);
-    cudaFree(s.q_norm), cudaFree(s.q_eps), cudaFree(s.fail_list), cudaFree(s.fail_ctl);
-    cudaFree(s.work_list), cudaFree(s.best_key);
-    if (s.fail_count_host) cudaFreeHost(s.fail_count_host);
-    free(s.tmap_qhi), free(s.tmap_qlo);
+template <typename... T>
+static void free_dev(T *&...p) {
+    ((cudaFree(p), p = nullptr), ...);
 }
 
+static void free_lane(Lane &l) {
+    free_dev(l.q_hi, l.q_lo, l.q_scale_exp, l.cand, l.topk_keys, l.map_tmp, l.map_max, l.m_test, l.m_star, l.top3,
+             l.done_counter, l.q_norm, l.q_eps, l.fail_list, l.fail_ctl, l.work_list, l.best_key);
+    l.s_key = nullptr;   // lives inside the fail_ctl allocation
+    if (l.fail_count_host) cudaFreeHost(l.fail_count_host);
+    free(l.tmap_qhi), free(l.tmap_qlo);
+    l.fail_count_host = nullptr, l.tmap_qhi = l.tmap_qlo = nullptr;
+}
+
+// callers make sure that no submitted call is outstanding: its results would be lost
 void score_scratch_free(cmdb_bank *b) {
     // no copy or kernel may still be in flight into / out of the buffers
     if (b->copy_stream) cudaStreamSynchronize(b->copy_stream);
     if (b->d2h_stream) cudaStreamSynchronize(b->d2h_stream);
-    for (auto st : b->lane_stream)
-        if (st) cudaStreamSynchronize(st);
-    for (auto st : b->lane_aux)
-        if (st) cudaStreamSynchronize(st);
-    // query / result blocks are per SLOT and shared by both lane copies (slot i is only ever used by lane i)
-    ScoreScratch &s0 = b->ss_store[0];
-    for (int i = 0; i < kResultSlots; ++i) {
-        cudaFree(s0.q_f32_buf[i]), cudaFree(s0.out_block_buf[i]);
-        if (s0.out_block_host_buf[i]) cudaFreeHost(s0.out_block_host_buf[i]);
-        b->pending[i].active = false;
+    for (const Lane &l : b->lane) {
+        if (l.stream) cudaStreamSynchronize(l.stream);
+        if (l.aux) cudaStreamSynchronize(l.aux);
     }
-    for (auto &s : b->ss_store) {
-        free_lane(s);
-        s = ScoreScratch();
+    for (ResultSlot &s : b->slot) {
+        free_dev(s.q_f32, s.out_block);
+        if (s.out_block_host) cudaFreeHost(s.out_block_host);
+        s.out_block_host = nullptr;
     }
-    b->ss = ScoreScratch();
+    for (Lane &l : b->lane) free_lane(l);
+    b->layout = ScoreLayout();
+    b->round.open = false;   // an open sharded round lived in these buffers
     b->last_fail_host = nullptr;
     b->fail_pending = false;
 }
@@ -645,34 +645,32 @@ int score_max_batch(const cmdb_bank *b) {
     return std::max(1, std::min(32, by_smem));
 }
 
-// lane == slot: points b->ss / b->stream at that lane's scratch copy and stream, and at the slot's query / result blocks
-void score_select_slot(cmdb_bank *b, int lane, int rslot) {
-    b->ss = b->ss_store[lane];
-    b->stream = b->lane_stream[lane];
-    b->cur_slot = lane;
-    ScoreScratch &s = b->ss;
-    s.q_f32 = s.q_f32_buf[rslot];
-    s.out_block = s.out_block_buf[rslot];
-    s.out_block_host = s.out_block_host_buf[rslot];
-    s.tail = s.out_block;
-    s.min_val = reinterpret_cast<float *>(s.out_block + s.off_min_val);
-    s.min_idx = reinterpret_cast<long long *>(s.out_block + s.off_min_idx);
-    s.map_out = reinterpret_cast<float *>(s.out_block + s.off_map_out);
-    s.map_pre = reinterpret_cast<float *>(s.out_block + s.off_map_pre);
-    s.map_u8 = s.out_block + s.off_map_u8;
+ScoreCall score_call(cmdb_bank *b, int lane, int slot) {
+    const ScoreLayout &L = b->layout;
+    ResultSlot &rs = b->slot[slot];
+    unsigned char *blk = rs.out_block;
+    b->last_lane = lane;
+    return ScoreCall{b, lane, slot, &b->lane[lane], &rs, b->lane[lane].stream, reinterpret_cast<TailResult *>(blk),
+                     reinterpret_cast<float *>(blk + L.off_min_val), reinterpret_cast<long long *>(blk + L.off_min_idx),
+                     reinterpret_cast<float *>(blk + L.off_map_out), reinterpret_cast<float *>(blk + L.off_map_pre),
+                     blk + L.off_map_u8};
+}
+
+int score_mark(const ScoreCall &c, int stage, cudaStream_t st) {
+    const cmdb_bank *b = c.b;
+    if (b->timing && stage >= 0) CMDB_CUDA(cudaEventRecord(b->timing == 2 ? c.lane->ev_tl[stage] : b->ev[stage], st));
+    return CMDB_OK;
 }
 
 int score_scratch_alloc(cmdb_bank *b, int B, int P_img, int out_hw) {
     const int p_pad = (B * P_img + BM - 1) / BM * BM;
     const int map_n = out_hw * out_hw;
-    {
-        const ScoreScratch &cur = b->ss_store[0];
-        if (cur.cap_p >= p_pad && cur.cap_b >= B && (int)cur.map_stride >= map_n) return CMDB_OK;
-    }
+    ScoreLayout &L = b->layout;
+    if (L.cap_p >= p_pad && L.cap_b >= B && (int)L.map_stride >= map_n) return CMDB_OK;
     CMDB_REQUIRE(!b->any_pending(), CMDB_ERR_STATE,
                  "scoring: the scratch buffers have to grow while a submitted batch is outstanding; wait for it first");
-    const int cap_p = std::max(p_pad, b->ss_store[0].cap_p), cap_b = std::max(B, b->ss_store[0].cap_b);
-    const int map_cap = std::max(map_n, (int)b->ss_store[0].map_stride);
+    const int cap_p = std::max(p_pad, L.cap_p), cap_b = std::max(B, L.cap_b);
+    const int map_cap = std::max(map_n, (int)L.map_stride);
     score_scratch_free(b);
     {
         static bool once = false;
@@ -683,73 +681,70 @@ int score_scratch_alloc(cmdb_bank *b, int B, int P_img, int out_hw) {
     }
     const size_t D = b->dim;
     auto up = [](size_t v) { return (v + 255) & ~size_t(255); };
-    // shared per-slot blocks: queries in, results out (mirrored by a pinned host block)
-    ScoreScratch shared;
-    shared.map_stride = map_cap;
-    shared.off_min_val = up(sizeof(TailResult) * cap_b);
-    shared.off_min_idx = shared.off_min_val + up(sizeof(float) * cap_p);
-    shared.off_map_out = shared.off_min_idx + up(sizeof(long long) * cap_p);
-    shared.off_map_pre = shared.off_map_out + up(sizeof(float) * map_cap * cap_b);
-    shared.off_map_u8 = shared.off_map_pre + up(sizeof(float) * map_cap * cap_b);
-    shared.out_block_bytes = shared.off_map_u8 + up((size_t)map_cap * cap_b);
-    for (int i = 0; i < kResultSlots; ++i) {
-        CMDB_CUDA(cudaMalloc(&shared.q_f32_buf[i], sizeof(float) * cap_p * D));
-        CMDB_CUDA(cudaMalloc(&shared.out_block_buf[i], shared.out_block_bytes));
-        CMDB_CUDA(cudaMallocHost(&shared.out_block_host_buf[i], shared.out_block_bytes));
+    L.map_stride = map_cap;
+    L.off_min_val = up(sizeof(TailResult) * cap_b);
+    L.off_min_idx = L.off_min_val + up(sizeof(float) * cap_p);
+    L.off_map_out = L.off_min_idx + up(sizeof(long long) * cap_p);
+    L.off_map_pre = L.off_map_out + up(sizeof(float) * map_cap * cap_b);
+    L.off_map_u8 = L.off_map_pre + up(sizeof(float) * map_cap * cap_b);
+    L.out_block_bytes = L.off_map_u8 + up((size_t)map_cap * cap_b);
+    L.n_topk_blocks = b->num_sms * 4;
+    // per slot: queries in, results out (mirrored by a pinned host block)
+    for (ResultSlot &s : b->slot) {
+        CMDB_CUDA(cudaMalloc(&s.q_f32, sizeof(float) * cap_p * D));
+        CMDB_CUDA(cudaMalloc(&s.out_block, L.out_block_bytes));
+        CMDB_CUDA(cudaMallocHost(&s.out_block_host, L.out_block_bytes));
     }
-    for (int lane = 0; lane < 2; ++lane) {
-        ScoreScratch &s = b->ss_store[lane];
-        s = shared;
-        s.n_topk_blocks = b->num_sms * 4;
-        CMDB_CUDA(cudaMalloc(&s.q_hi, sizeof(__half) * cap_p * D));
-        CMDB_CUDA(cudaMalloc(&s.q_lo, sizeof(__half) * cap_p * D));
-        CMDB_CUDA(cudaMalloc(&s.q_scale_exp, sizeof(int) * cap_p));
-        CMDB_CUDA(cudaMalloc(&s.q_norm, sizeof(float) * cap_p));
-        CMDB_CUDA(cudaMalloc(&s.q_eps, sizeof(float) * cap_p));
-        CMDB_CUDA(cudaMalloc(&s.fail_list, sizeof(int) * cap_p));
+    for (Lane &l : b->lane) {
+        CMDB_CUDA(cudaMalloc(&l.q_hi, sizeof(__half) * cap_p * D));
+        CMDB_CUDA(cudaMalloc(&l.q_lo, sizeof(__half) * cap_p * D));
+        CMDB_CUDA(cudaMalloc(&l.q_scale_exp, sizeof(int) * cap_p));
+        CMDB_CUDA(cudaMalloc(&l.q_norm, sizeof(float) * cap_p));
+        CMDB_CUDA(cudaMalloc(&l.q_eps, sizeof(float) * cap_p));
+        CMDB_CUDA(cudaMalloc(&l.fail_list, sizeof(int) * cap_p));
         // control block (8 ints) and the per-image argmax keys behind it: one allocation, cleared by ONE memset per call
-        CMDB_CUDA(cudaMalloc(&s.fail_ctl, 8 * sizeof(int) + sizeof(unsigned long long) * cap_b));
-        s.s_key = reinterpret_cast<unsigned long long *>(s.fail_ctl + 8);
-        CMDB_CUDA(cudaMalloc(&s.work_list, sizeof(int2) * kWorkCap));
-        CMDB_CUDA(cudaMalloc(&s.best_key, sizeof(unsigned long long) * cap_p));
-        CMDB_CUDA(cudaMallocHost(&s.fail_count_host, 2 * sizeof(int)));
-        s.fail_count_host[0] = s.fail_count_host[1] = 0;
-        CMDB_CUDA(cudaMalloc(&s.done_counter, sizeof(unsigned int)));
-        CMDB_CUDA(cudaMemset(s.done_counter, 0, sizeof(unsigned int)));
+        CMDB_CUDA(cudaMalloc(&l.fail_ctl, 8 * sizeof(int) + sizeof(unsigned long long) * cap_b));
+        l.s_key = reinterpret_cast<unsigned long long *>(l.fail_ctl + 8);
+        CMDB_CUDA(cudaMalloc(&l.work_list, sizeof(int2) * kWorkCap));
+        CMDB_CUDA(cudaMalloc(&l.best_key, sizeof(unsigned long long) * cap_p));
+        CMDB_CUDA(cudaMallocHost(&l.fail_count_host, 2 * sizeof(int)));
+        l.fail_count_host[0] = l.fail_count_host[1] = 0;
+        CMDB_CUDA(cudaMalloc(&l.done_counter, sizeof(unsigned int)));
+        CMDB_CUDA(cudaMemset(l.done_counter, 0, sizeof(unsigned int)));
         const size_t cand_bytes = sizeof(float4) * (size_t)cap_p * 2 * b->num_sms;
-        CMDB_CUDA(cudaMalloc(&s.cand, cand_bytes));
-        CMDB_CUDA(cudaMalloc(&s.map_tmp, (size_t)map_cap * cap_b));
-        CMDB_CUDA(cudaMalloc(&s.map_max, sizeof(float) * cap_b * 17));  // [cap_b] maxima, then [cap_b][16] band maxima
-        CMDB_CUDA(cudaMalloc(&s.topk_keys, sizeof(unsigned long long) * 3 * s.n_topk_blocks * cap_b));
-        CMDB_CUDA(cudaMalloc(&s.top3, sizeof(unsigned long long) * 3 * cap_b));
-        CMDB_CUDA(cudaMalloc(&s.m_test, sizeof(float) * D * cap_b));
-        CMDB_CUDA(cudaMalloc(&s.m_star, sizeof(float) * D * cap_b));
-        s.cap_p = cap_p, s.cap_b = cap_b, s.map_cap = map_cap;
-        CMDB_CHECK(make_map(&s.tmap_qhi, s.q_hi, cap_p, b->dim, BM));
-        CMDB_CHECK(make_map(&s.tmap_qlo, s.q_lo, cap_p, b->dim, BM));
+        CMDB_CUDA(cudaMalloc(&l.cand, cand_bytes));
+        CMDB_CUDA(cudaMalloc(&l.map_tmp, (size_t)map_cap * cap_b));
+        CMDB_CUDA(cudaMalloc(&l.map_max, sizeof(float) * cap_b * 17));
+        CMDB_CUDA(cudaMalloc(&l.topk_keys, sizeof(unsigned long long) * 3 * L.n_topk_blocks * cap_b));
+        CMDB_CUDA(cudaMalloc(&l.top3, sizeof(unsigned long long) * 3 * cap_b));
+        CMDB_CUDA(cudaMalloc(&l.m_test, sizeof(float) * D * cap_b));
+        CMDB_CUDA(cudaMalloc(&l.m_star, sizeof(float) * D * cap_b));
+        CMDB_CHECK(make_map(&l.tmap_qhi, l.q_hi, cap_p, b->dim, BM));
+        CMDB_CHECK(make_map(&l.tmap_qlo, l.q_lo, cap_p, b->dim, BM));
     }
-    b->fail_pending = false;
-    score_select_slot(b, 0, 0);
+    L.cap_p = cap_p, L.cap_b = cap_b;   // last: a failed allocation leaves the scratch to be rebuilt by the next call
     return CMDB_OK;
 }
 
-int score_query_prep(cmdb_bank *b, int P, bool compact, int row0) {
-    ScoreScratch &s = b->ss;
+int score_query_prep(const ScoreCall &c, cudaStream_t st, int P, bool compact, int row0) {
+    const cmdb_bank *b = c.b;
+    const Lane &l = *c.lane;
     const int p_pad = (P + BM - 1) / BM * BM;
     const size_t o = (size_t)row0 * b->dim;
-    q_split_kernel<<<std::min(b->num_sms * 2, (p_pad + 7) / 8), 256, 0, b->stream>>>(
-        s.q_f32 + o, P, p_pad, b->dim, s.q_hi + o, s.q_lo + o, s.q_scale_exp + row0, compact ? nullptr : s.q_norm + row0,
-        compact ? nullptr : s.q_eps + row0, compact ? s.fail_list : nullptr, compact ? s.fail_ctl + 2 : nullptr);
+    q_split_kernel<<<std::min(b->num_sms * 2, (p_pad + 7) / 8), 256, 0, st>>>(
+        c.slot->q_f32 + o, P, p_pad, b->dim, l.q_hi + o, l.q_lo + o, l.q_scale_exp + row0, compact ? nullptr : l.q_norm + row0,
+        compact ? nullptr : l.q_eps + row0, compact ? l.fail_list : nullptr, compact ? l.fail_ctl + 2 : nullptr);
     CMDB_CUDA(cudaGetLastError());
     return CMDB_OK;
 }
 
 // fp16 split (+ norms for the certificate) of n explicit rows (n <= cap_p) into rows 0.. of the query operand
-void q_split_rows(cmdb_bank *b, const float *rows_dev, int n) {
-    ScoreScratch &s = b->ss;
+void q_split_rows(const ScoreCall &c, const float *rows_dev, int n) {
+    const cmdb_bank *b = c.b;
+    const Lane &l = *c.lane;
     const int p_pad = (n + BM - 1) / BM * BM;
-    q_split_kernel<<<std::min(b->num_sms * 2, p_pad / 8), 256, 0, b->stream>>>(rows_dev, n, p_pad, b->dim, s.q_hi, s.q_lo, s.q_scale_exp,
-                                                                              s.q_norm, s.q_eps, nullptr, nullptr);
+    q_split_kernel<<<std::min(b->num_sms * 2, p_pad / 8), 256, 0, c.stream>>>(rows_dev, n, p_pad, b->dim, l.q_hi, l.q_lo,
+                                                                              l.q_scale_exp, l.q_norm, l.q_eps, nullptr, nullptr);
 }
 
 int score_tile_stride(int mt, int G) {  // == tile_stride() of the kernel
@@ -778,22 +773,22 @@ int score_gemm_run(int nt, int mt_units, int G) {
     return 1;
 }
 
-int score_gemm_candidates(cmdb_bank *b, int P, int terms, bool compact, int *n_cand_out, int row0) {
-    ScoreScratch &s = b->ss;
+int score_gemm_candidates(const ScoreCall &c, cudaStream_t st, int P, int terms, bool compact, GemmSched *sched, int row0) {
+    const cmdb_bank *b = c.b;
+    const Lane &l = *c.lane;
     const int p_pad = (P + BM - 1) / BM * BM;
-    cudaStream_t st = b->stream;
 
     GemmParams p{};
     p.nt = (int)(b->fin_rows_pad / BN);
     p.kb = b->dim / BK;
     p.bnorm = b->norm;
-    p.q_scale_exp = s.q_scale_exp;
+    p.q_scale_exp = l.q_scale_exp;
     p.b_scale_exp = b->scale_exp;
-    p.cand = s.cand;
-    p.cand_stride = s.cap_p;
+    p.cand = l.cand;
+    p.cand_stride = b->layout.cap_p;
     p.mt = p_pad / BM;
     p.m_base = row0 / BM;
-    p.m_count = compact ? s.fail_ctl + 2 : nullptr;
+    p.m_count = compact ? l.fail_ctl + 2 : nullptr;
     // CTA pairs (cta_group::2), measured at 16 images x 200k x 768: the 3-term kernel gains 5 % from pairs (7.84 -> 7.42 ms),
     // the 1-term pre-filter loses 3 % (2.81 -> 2.90 ms; it is not limited by shared-memory reads, and a pair halves the
     // producers per query)
@@ -803,9 +798,6 @@ int score_gemm_candidates(cmdb_bank *b, int P, int terms, bool compact, int *n_c
         // compact launches size themselves on the device (m_count): single tiles there
         p.run = compact ? 1 : score_gemm_run(p.nt, (p.mt + cg - 1) / cg, b->num_sms / cg);
     }
-    if (!compact && row0 == 0) s.sched_pair = pair;   // the first-pass schedule (the exact rescan needs it)
-    s.sched_pair_last = pair;
-    s.sched_run_last = p.run;
     const int threads = kGemmCtlThreads + 128 * kGemmEpiGroups;
     auto launch = [&](auto kern, size_t smem, bool cluster2) -> int {
         CMDB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -818,14 +810,14 @@ int score_gemm_candidates(cmdb_bank *b, int P, int terms, bool compact, int *n_c
         // the pair kernels load HALF bank tiles (box of 128 rows)
         const CUtensorMap &mh = *reinterpret_cast<CUtensorMap *>(cluster2 ? b->tmap_hi2 : b->tmap_hi);
         const CUtensorMap &ml = *reinterpret_cast<CUtensorMap *>(cluster2 ? b->tmap_lo2 : b->tmap_lo);
-        CMDB_CUDA(cudaLaunchKernelEx(&cfg, kern, *reinterpret_cast<CUtensorMap *>(s.tmap_qhi),
-                                     *reinterpret_cast<CUtensorMap *>(s.tmap_qlo), mh, ml, p));
+        CMDB_CUDA(cudaLaunchKernelEx(&cfg, kern, *reinterpret_cast<CUtensorMap *>(l.tmap_qhi),
+                                     *reinterpret_cast<CUtensorMap *>(l.tmap_qlo), mh, ml, p));
         return CMDB_OK;
     };
     if (pair) CMDB_CHECK(launch(score_gemm_kernel<3, kGemmEpiGroups, 2>, GemmSmem<3, 2>::total + 1024, true));
     else if (terms == 1) CMDB_CHECK(launch(score_gemm_kernel<1, kGemmEpiGroups, 1>, GemmSmem<1, 1>::total + 1024, false));
     else CMDB_CHECK(launch(score_gemm_kernel<3, kGemmEpiGroups, 1>, GemmSmem<3, 1>::total + 1024, false));
-    *n_cand_out = kGemmEpiGroups * b->num_sms;  // (CTA, column group) producers
+    *sched = GemmSched{kGemmEpiGroups * b->num_sms, pair, p.run};
     return CMDB_OK;
 }
 

@@ -449,7 +449,7 @@ __global__ void __launch_bounds__(256) exact_scan_kernel(const float *__restrict
 int score_exact_scan(cmdb_bank *b, const float *q_dev, int P, unsigned long long *keys_dev) {
     const long long chunk = std::max<long long>(64, (b->fin_rows + 4 * b->num_sms - 1) / (4 * b->num_sms));
     const int gx = (int)((b->fin_rows + chunk - 1) / chunk);
-    exact_scan_kernel<<<dim3(gx, (P + 7) / 8), 256, 0, b->stream>>>(q_dev, P, b->data, b->fin_rows, b->dim, chunk, keys_dev);
+    exact_scan_kernel<<<dim3(gx, (P + 7) / 8), 256, 0, b->handle_stream()>>>(q_dev, P, b->data, b->fin_rows, b->dim, chunk, keys_dev);
     CMDB_CUDA(cudaGetLastError());
     return CMDB_OK;
 }
@@ -532,24 +532,27 @@ __global__ void __launch_bounds__(256) simt_min_kernel(const float *__restrict__
     }
 }
 
-int score_simt_candidates(cmdb_bank *b, int P, int *n_cand_out) {
+int score_simt_candidates(const ScoreCall &c, int P, int *n_cand_out) {
+    const cmdb_bank *b = c.b;
     const int q_tiles = (P + 63) / 64;
     int slices = std::max(1, std::min(b->num_sms, (2 * b->num_sms + q_tiles - 1) / q_tiles));
     slices = (int)std::min<long long>(slices, (b->fin_rows + 63) / 64);
-    simt_min_kernel<<<dim3(q_tiles, slices), 256, 0, b->stream>>>(b->ss.q_f32, P, b->data, b->fin_rows, b->dim, b->ss.cand,
-                                                                 b->ss.cap_p);
+    simt_min_kernel<<<dim3(q_tiles, slices), 256, 0, c.stream>>>(c.slot->q_f32, P, b->data, b->fin_rows, b->dim, c.lane->cand,
+                                                                b->layout.cap_p);
     CMDB_CUDA(cudaGetLastError());
     *n_cand_out = slices;
     return CMDB_OK;
 }
 
-int score_refine(cmdb_bank *b, int B, int P_img, int n_cand, bool compact) {
+int score_refine(const ScoreCall &c, cudaStream_t st, int B, int P_img, int n_cand, bool compact) {
+    const cmdb_bank *b = c.b;
+    const Lane &l = *c.lane;
     const int P = B * P_img;
-    // compact mode follows score_refine_certified, which already reset s_key and published the certified queries
-    if (!compact) CMDB_CUDA(cudaMemsetAsync(b->ss.s_key, 0, sizeof(unsigned long long) * B, b->stream));
-    refine_kernel<<<(P + 7) / 8, 256, 0, b->stream>>>(b->ss.cand, n_cand, b->ss.cap_p, b->ss.q_f32, b->data, b->dim, P, P_img,
-                                                      b->row_offset, b->ss.min_val, b->ss.min_idx, b->ss.s_key,
-                                                      compact ? b->ss.fail_list : nullptr, compact ? b->ss.fail_ctl + 2 : nullptr);
+    // compact mode follows score_certify, which already reset s_key and published the certified queries
+    if (!compact) CMDB_CUDA(cudaMemsetAsync(l.s_key, 0, sizeof(unsigned long long) * B, st));
+    refine_kernel<<<(P + 7) / 8, 256, 0, st>>>(l.cand, n_cand, b->layout.cap_p, c.slot->q_f32, b->data, b->dim, P, P_img,
+                                               b->row_offset, c.min_val, c.min_idx, l.s_key, compact ? l.fail_list : nullptr,
+                                               compact ? l.fail_ctl + 2 : nullptr);
     CMDB_CUDA(cudaGetLastError());
     return CMDB_OK;
 }
@@ -562,71 +565,71 @@ static int mod_inverse(int a, int m) {
     return 0;
 }
 
-static int score_certify(cmdb_bank *b, int B, int P_img, int n_cand) {
+static int score_certify(const ScoreCall &c, int B, int P_img, int n_cand) {
+    const cmdb_bank *b = c.b;
+    const Lane &s = *c.lane;
     const int P = B * P_img;
-    ScoreScratch &s = b->ss;
-    cudaStream_t st = b->stream;
+    cudaStream_t st = c.stream;
     CMDB_CUDA(cudaMemsetAsync(s.fail_ctl, 0, 8 * sizeof(int) + sizeof(unsigned long long) * B, st));  // control block + s_key
     const float acc_model = (float)(b->dim / 16 + 1) * 17.f * 1.1920929e-7f;
-    if (b->timing == 2) CMDB_CUDA(cudaEventRecord(b->ev_dbg[b->cur_slot][0], st));
+    if (b->timing == 2) CMDB_CUDA(cudaEventRecord(s.ev_dbg[0], st));
     // queries per block: 8 = one query per warp in phase 3 and 10 list entries per thread held in registers (measured best)
     constexpr int QB = 8;
-    refine_cert_kernel<QB><<<(P + QB - 1) / QB, kCertThreads, 0, st>>>(s.cand, n_cand, s.cap_p, s.q_f32, b->data, b->dim, P, P_img,
-                                                                       b->row_offset, s.q_norm, s.q_eps, b->cert_bmax, b->cert_eb_max,
-                                                                       acc_model, s.min_val, s.min_idx, s.s_key, s.fail_list,
-                                                                       s.fail_ctl, s.work_list, s.best_key);
-    if (b->timing == 2) CMDB_CUDA(cudaEventRecord(b->ev_dbg[b->cur_slot][1], st));
+    refine_cert_kernel<QB><<<(P + QB - 1) / QB, kCertThreads, 0, st>>>(s.cand, n_cand, b->layout.cap_p, c.slot->q_f32, b->data, b->dim,
+                                                                       P, P_img, b->row_offset, s.q_norm, s.q_eps, b->cert_bmax,
+                                                                       b->cert_eb_max, acc_model, c.min_val, c.min_idx, s.s_key,
+                                                                       s.fail_list, s.fail_ctl, s.work_list, s.best_key);
+    if (b->timing == 2) CMDB_CUDA(cudaEventRecord(s.ev_dbg[1], st));
     CMDB_CUDA(cudaGetLastError());
     return CMDB_OK;
 }
 
-static int score_rescan(cmdb_bank *b, int P_img) {
-    ScoreScratch &s = b->ss;
-    cudaStream_t st = b->stream;
+static int score_rescan(const ScoreCall &c, int P_img) {
+    const cmdb_bank *b = c.b;
+    const Lane &s = *c.lane;
+    cudaStream_t st = c.stream;
     CMDB_CUDA(cudaGetLastError());
-    // tier 1: few uncertified (query, producer) pairs -> exact rescan of those producers' rows
-    const int cg = s.sched_pair ? 2 : 1, n_units = b->num_sms / cg, EG = kGemmEpiGroups;
-    const int last_tiles = s.mt_total - (s.mt_total - 1) / s.chunk_tiles * s.chunk_tiles;
+    // tier 1: few uncertified (query, producer) pairs -> exact rescan of those producers' rows, along the first-pass schedule
+    const int cg = c.pair ? 2 : 1, n_units = b->num_sms / cg, EG = kGemmEpiGroups;
+    const int last_tiles = c.mt_total - (c.mt_total - 1) / c.chunk_tiles * c.chunk_tiles;
     const int nt = (int)(b->fin_rows_pad / kScoreBN);
-    rescan_kernel<<<b->num_sms * 8, 256, 0, st>>>(s.work_list, s.fail_ctl + 3, s.q_f32, b->data, b->dim, b->fin_rows, n_units, cg, EG,
-                                                  nt, s.chunk_tiles, s.mt_total,
-                                                  mod_inverse(score_tile_stride((s.chunk_tiles + cg - 1) / cg, n_units), n_units),
+    rescan_kernel<<<b->num_sms * 8, 256, 0, st>>>(s.work_list, s.fail_ctl + 3, c.slot->q_f32, b->data, b->dim, b->fin_rows, n_units, cg,
+                                                  EG, nt, c.chunk_tiles, c.mt_total,
+                                                  mod_inverse(score_tile_stride((c.chunk_tiles + cg - 1) / cg, n_units), n_units),
                                                   mod_inverse(score_tile_stride((last_tiles + cg - 1) / cg, n_units), n_units),
-                                                  score_gemm_run(nt, (s.chunk_tiles + cg - 1) / cg, n_units),
+                                                  score_gemm_run(nt, (c.chunk_tiles + cg - 1) / cg, n_units),
                                                   score_gemm_run(nt, (last_tiles + cg - 1) / cg, n_units), s.best_key,
-                                                  s.fail_list, s.fail_ctl, P_img, b->row_offset, s.min_val, s.min_idx, s.s_key);
+                                                  s.fail_list, s.fail_ctl, P_img, b->row_offset, c.min_val, c.min_idx, s.s_key);
     CMDB_CUDA(cudaGetLastError());
-    if (b->timing == 2) CMDB_CUDA(cudaEventRecord(b->ev_dbg[b->cur_slot][2], st));
+    if (b->timing == 2) CMDB_CUDA(cudaEventRecord(s.ev_dbg[2], st));
     return CMDB_OK;
 }
 
-// min_val / min_idx / s_key of a sub-batch in the bank's GEMM mode: stages the queries into ss.q_f32, builds the
+// min_val / min_idx / s_key of a sub-batch in the bank's GEMM mode: stages the queries into the slot's q_f32, builds the
 // candidate lists, refines.  ev_gemm / ev_refine: timing event slots recorded before the (first) GEMM and before the
 // (first) refine, or -1.
 // Host queries are staged in up to kMaxStageChunks chunks on a copy stream; chunk c is split and multiplied while chunk
 // c + 1 is still crossing PCIe.  (One GEMM launch per chunk: each streams the fp16 bank once more, which is cheap next to
 // the host link.)  Device-resident queries use one chunk.
-int score_local_min(cmdb_bank *b, const float *src, int src_is_device, int B, int P_img, int ev_gemm, int ev_refine,
+int score_local_min(ScoreCall &c, const float *src, int src_is_device, int B, int P_img, int ev_gemm, int ev_refine,
                     cudaEvent_t stage_after) {
-    ScoreScratch &s = b->ss;
-    cudaStream_t st = b->stream;
+    cmdb_bank *b = c.b;
+    const Lane &l = *c.lane;
+    float *q_f32 = c.slot->q_f32;
+    cudaStream_t st = c.stream;
     const int P = B * P_img;
     const size_t D = b->dim;
     int n_cand = 0;
-    auto mark = [&](int i) -> int {
-        if (b->timing && i >= 0) CMDB_CUDA(cudaEventRecord(b->timing == 2 ? b->ev_tl[b->cur_slot][i] : b->ev[i], st));
-        return CMDB_OK;
-    };
     const int64_t prev_queries = b->last_queries;
     b->last_queries = P;
     if (b->score_impl != CMDB_SCORE_TCGEN05) {
         b->last_mode = 3;
-        CMDB_CUDA(cudaMemcpyAsync(s.q_f32, src, sizeof(float) * P * D, src_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
-        if (b->q_norm_enabled) launch_normalize(st, b->num_sms, s.q_f32, (int64_t)P * D, b->q_mean, b->q_std);
-        CMDB_CHECK(mark(ev_gemm));
-        CMDB_CHECK(score_simt_candidates(b, P, &n_cand));
-        CMDB_CHECK(mark(ev_refine));
-        return score_refine(b, B, P_img, n_cand, false);
+        CMDB_CUDA(cudaMemcpyAsync(q_f32, src, sizeof(float) * P * D, src_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
+        if (b->q_norm_enabled) launch_normalize(st, b->num_sms, q_f32, (int64_t)P * D, b->q_mean, b->q_std);
+        CMDB_CHECK(score_mark(c, ev_gemm, st));
+        CMDB_CHECK(score_simt_candidates(c, P, &n_cand));
+        CMDB_CHECK(score_mark(c, ev_refine, st));
+        return score_refine(c, st, B, P_img, n_cand, false);
     }
     int mode = b->prefilter_terms;
     if (mode == 0) {
@@ -656,7 +659,7 @@ int score_local_min(cmdb_bank *b, const float *src, int src_is_device, int B, in
     n_chunks = std::max(1, std::min(std::min(n_chunks, kMaxStageChunks), mt_total));
     const int chunk_tiles = (mt_total + n_chunks - 1) / n_chunks;
     n_chunks = (mt_total + chunk_tiles - 1) / chunk_tiles;
-    s.chunk_tiles = chunk_tiles, s.mt_total = mt_total;
+    c.chunk_tiles = chunk_tiles, c.mt_total = mt_total;
     if (via_copy_stream) {
         // the copy stream may only overwrite q_f32 once its previous readers are done: the event the caller names, or
         // everything queued on the compute stream so far
@@ -666,58 +669,58 @@ int score_local_min(cmdb_bank *b, const float *src, int src_is_device, int B, in
         }
         CMDB_CUDA(cudaStreamWaitEvent(b->copy_stream, stage_after, 0));
     }
-    for (int c = 0; c < n_chunks; ++c) {
-        const int row0 = c * chunk_tiles * kScoreBM, rows = std::min(P, (c + 1) * chunk_tiles * kScoreBM) - row0;
+    for (int k = 0; k < n_chunks; ++k) {
+        const int row0 = k * chunk_tiles * kScoreBM, rows = std::min(P, (k + 1) * chunk_tiles * kScoreBM) - row0;
         const size_t o = (size_t)row0 * D;
         if (!via_copy_stream) {
-            CMDB_CUDA(cudaMemcpyAsync(s.q_f32, src, sizeof(float) * P * D, src_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
+            CMDB_CUDA(cudaMemcpyAsync(q_f32, src, sizeof(float) * P * D, src_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
         } else {
-            CMDB_CUDA(cudaMemcpyAsync(s.q_f32 + o, src + o, sizeof(float) * rows * D, cudaMemcpyHostToDevice, b->copy_stream));
-            CMDB_CUDA(cudaEventRecord(b->ev_chunk[c], b->copy_stream));
+            CMDB_CUDA(cudaMemcpyAsync(q_f32 + o, src + o, sizeof(float) * rows * D, cudaMemcpyHostToDevice, b->copy_stream));
+            CMDB_CUDA(cudaEventRecord(b->ev_chunk[k], b->copy_stream));
         }
     }
-    for (int c = 0; c < n_chunks; ++c) {
-        const int row0 = c * chunk_tiles * kScoreBM, rows = std::min(P, (c + 1) * chunk_tiles * kScoreBM) - row0;
-        if (via_copy_stream) CMDB_CUDA(cudaStreamWaitEvent(st, b->ev_chunk[c], 0));
+    GemmSched sched{};
+    for (int k = 0; k < n_chunks; ++k) {
+        const int row0 = k * chunk_tiles * kScoreBM, rows = std::min(P, (k + 1) * chunk_tiles * kScoreBM) - row0;
+        if (via_copy_stream) CMDB_CUDA(cudaStreamWaitEvent(st, b->ev_chunk[k], 0));
         // (patch - mean) / std on the device (multiple_features.py:90): without chunking the one copy above covers all rows
         if (b->q_norm_enabled)
-            launch_normalize(st, b->num_sms, s.q_f32 + (size_t)row0 * D, (int64_t)(via_copy_stream ? rows : P) * D, b->q_mean, b->q_std);
-        CMDB_CHECK(score_query_prep(b, rows, false, row0));
-        if (c == 0) CMDB_CHECK(mark(ev_gemm));
-        CMDB_CHECK(score_gemm_candidates(b, rows, mode == 3 ? 3 : 1, false, &n_cand, row0));
+            launch_normalize(st, b->num_sms, q_f32 + (size_t)row0 * D, (int64_t)(via_copy_stream ? rows : P) * D, b->q_mean, b->q_std);
+        CMDB_CHECK(score_query_prep(c, st, rows, false, row0));
+        if (k == 0) CMDB_CHECK(score_mark(c, ev_gemm, st));
+        CMDB_CHECK(score_gemm_candidates(c, st, rows, mode == 3 ? 3 : 1, false, &sched, row0));
+        if (k == 0) c.pair = sched.pair;
     }
-    CMDB_CHECK(mark(ev_refine));
-    if (mode != 0) return score_refine(b, B, P_img, n_cand, false);
+    n_cand = sched.producers;
+    CMDB_CHECK(score_mark(c, ev_refine, st));
+    if (mode != 0) return score_refine(c, st, B, P_img, n_cand, false);
     // certificate kernel (takes the tier decision), then the two tiers side by side: the exact rescan on the lane's stream,
     // the counters copy and the tier-2 launches on the lane's side stream.  The tiers are exclusive (the control block
     // enables one of them) and touch disjoint buffers, so nothing orders them against each other; the side stream's launches
     // are empty in the common case and their launch latencies (27 us in a row) disappear behind the rescan.
-    const int lane = b->cur_slot;
-    cudaStream_t aux = b->lane_aux[lane];
-    CMDB_CHECK(score_certify(b, B, P_img, n_cand));
-    CMDB_CUDA(cudaEventRecord(b->ev_fork[lane], st));
-    CMDB_CUDA(cudaStreamWaitEvent(aux, b->ev_fork[lane], 0));
-    CMDB_CHECK(score_rescan(b, P_img));
-    b->stream = aux;
+    cudaStream_t aux = l.aux;
+    CMDB_CHECK(score_certify(c, B, P_img, n_cand));
+    CMDB_CUDA(cudaEventRecord(l.ev_fork, st));
+    CMDB_CUDA(cudaStreamWaitEvent(aux, l.ev_fork, 0));
+    CMDB_CHECK(score_rescan(c, P_img));
     int rc = CMDB_OK;
-    if (cudaMemcpyAsync(s.fail_count_host, s.fail_ctl, 2 * sizeof(int), cudaMemcpyDeviceToHost, aux) != cudaSuccess ||
+    if (cudaMemcpyAsync(l.fail_count_host, l.fail_ctl, 2 * sizeof(int), cudaMemcpyDeviceToHost, aux) != cudaSuccess ||
         cudaEventRecord(b->ev_fail, aux) != cudaSuccess)
         rc = CMDB_ERR_CUDA;
     b->fail_pending = true;
-    b->last_fail_host = s.fail_count_host;   // this lane's pinned counters
+    b->last_fail_host = l.fail_count_host;   // this lane's pinned counters
     // tier 2 (many uncertified pairs): FP32-equivalent GEMM over the compacted uncertified queries; every launch sizes
     // itself from the device-side control block and returns at once in the common case
-    if (rc == CMDB_OK) rc = score_query_prep(b, P, true);
-    if (rc == CMDB_OK) rc = score_gemm_candidates(b, P, 3, true, &n_cand);
-    if (rc == CMDB_OK) rc = score_refine(b, B, P_img, n_cand, true);
-    b->stream = st;
+    if (rc == CMDB_OK) rc = score_query_prep(c, aux, P, true);
+    if (rc == CMDB_OK) rc = score_gemm_candidates(c, aux, P, 3, true, &sched);
+    if (rc == CMDB_OK) rc = score_refine(c, aux, B, P_img, sched.producers, true);
     if (rc != CMDB_OK) {
         if (rc == CMDB_ERR_CUDA) set_error("scoring: CUDA error while enqueuing the fallback tier: %s", cudaGetErrorString(cudaGetLastError()));
         return rc;
     }
-    CMDB_CUDA(cudaEventRecord(b->ev_join[lane], aux));
-    CMDB_CUDA(cudaStreamWaitEvent(st, b->ev_join[lane], 0));
-    if (b->timing == 2) CMDB_CUDA(cudaEventRecord(b->ev_dbg[lane][3], st));
+    CMDB_CUDA(cudaEventRecord(l.ev_join, aux));
+    CMDB_CUDA(cudaStreamWaitEvent(st, l.ev_join, 0));
+    if (b->timing == 2) CMDB_CUDA(cudaEventRecord(l.ev_dbg[3], st));
     return CMDB_OK;
 }
 
@@ -1252,26 +1255,27 @@ static_assert(kCommScoreFlagsOff + kShardSlots * 2 * kMaxRanks * 8 <= kCommScore
 static_assert(kCommScoreD2Off + (size_t)kShardSlots * kMaxRanks * kShardD2Cap * 4 <= kCommScoreKeysOff, "d2 slots overlap the key slots");
 static_assert(kCommScoreKeysOff + (size_t)kShardSlots * kMaxRanks * kShardKeysCap * 8 <= kCommHeaderBytes, "key slots exceed the header");
 
-int score_shard_exchange_keys(cmdb_bank *b, int B, int P_img, const PeerPtrs &peers, int world, int rank, int slot,
+int score_shard_exchange_keys(const ScoreCall &c, int B, int P_img, const PeerPtrs &peers, int world, int rank, int slot,
                               unsigned long long epoch) {
-    ScoreScratch &s = b->ss;
-    cudaStream_t st = b->stream;
+    const cmdb_bank *b = c.b;
+    cudaStream_t st = c.stream;
     const int n = B * P_img;
     CMDB_REQUIRE(n <= kShardKeysCap, CMDB_ERR_UNSUPPORTED, "sharded round: %d queries exceed the exchange slot (%d)", n, kShardKeysCap);
     const size_t keys_off = kCommScoreKeysOff + (size_t)slot * kMaxRanks * kShardKeysCap * 8;
     const int blocks = std::min((n + 255) / 256, 2 * b->num_sms);
-    shard_push_keys_kernel<<<blocks, 256, 0, st>>>(s.min_val, s.min_idx, n, peers, world, rank, keys_off, shard_flag_off(slot, 0), epoch,
+    shard_push_keys_kernel<<<blocks, 256, 0, st>>>(c.min_val, c.min_idx, n, peers, world, rank, keys_off, shard_flag_off(slot, 0), epoch,
                                                    b->shard_ctr + (slot & 1));  // consecutive rounds (= the two lanes) use different counters
-    CMDB_CUDA(cudaMemsetAsync(s.s_key, 0, sizeof(unsigned long long) * B, st));
-    shard_reduce_keys_kernel<<<blocks, 256, 0, st>>>(peers.p[rank], keys_off, shard_flag_off(slot, 0), world, epoch, n, P_img, s.min_val,
-                                                     s.min_idx, s.s_key, b->shard_abort_dev);
+    CMDB_CUDA(cudaMemsetAsync(c.lane->s_key, 0, sizeof(unsigned long long) * B, st));
+    shard_reduce_keys_kernel<<<blocks, 256, 0, st>>>(peers.p[rank], keys_off, shard_flag_off(slot, 0), world, epoch, n, P_img, c.min_val,
+                                                     c.min_idx, c.lane->s_key, b->shard_abort_dev);
     CMDB_CUDA(cudaGetLastError());
     return CMDB_OK;
 }
 
-int score_shard_exchange_d2(cmdb_bank *b, int B, const PeerPtrs &peers, int world, int rank, int slot, unsigned long long epoch,
-                            const float *contrib_dev, float *d2_sum_dev) {
-    cudaStream_t st = b->stream;
+int score_shard_exchange_d2(const ScoreCall &c, int B, const PeerPtrs &peers, int world, int rank, int slot,
+                            unsigned long long epoch, const float *contrib_dev, float *d2_sum_dev) {
+    const cmdb_bank *b = c.b;
+    cudaStream_t st = c.stream;
     CMDB_REQUIRE(2 * B <= kShardD2Cap, CMDB_ERR_UNSUPPORTED, "sharded round: batch %d exceeds the exchange slot", B);
     const size_t d2_off = kCommScoreD2Off + (size_t)slot * kMaxRanks * kShardD2Cap * 4;
     shard_push_d2_kernel<<<1, 64, 0, st>>>(contrib_dev, 2 * B, peers, world, rank, d2_off, shard_flag_off(slot, 1), epoch);
@@ -1439,36 +1443,37 @@ __global__ void __launch_bounds__(kBlurThreads) vblur_kernel(const unsigned char
     }
 }
 
-int score_select(cmdb_bank *b, int B, int P_img, bool local_m_star) {
-    select_kernel<<<B, 256, 0, b->stream>>>(b->ss.s_key, b->ss.min_idx, P_img, b->ss.q_f32, b->data, b->dim, b->row_offset,
-                                            b->fin_rows, b->ss.m_test, local_m_star ? b->ss.m_star : nullptr,
-                                            reinterpret_cast<TailResult *>(b->ss.tail));
+int score_select(const ScoreCall &c, int B, int P_img, bool local_m_star) {
+    const cmdb_bank *b = c.b;
+    const Lane &l = *c.lane;
+    select_kernel<<<B, 256, 0, c.stream>>>(l.s_key, c.min_idx, P_img, c.slot->q_f32, b->data, b->dim, b->row_offset, b->fin_rows,
+                                           l.m_test, local_m_star ? l.m_star : nullptr, c.tail);
     CMDB_CUDA(cudaGetLastError());
     return CMDB_OK;
 }
 
 // tensor-core variant: select -> fp16 split of the m_star rows -> hi.hi GEMM with one M tile -> reweight_cert_kernel
-static int score_reweight_tensor(cmdb_bank *b, int B, int P_img) {
-    ScoreScratch &s = b->ss;
-    cudaStream_t st = b->stream;
-    CMDB_CHECK(score_select(b, B, P_img, true));  // m_test, m_star, s*, s_idx, m_star_row
+static int score_reweight_tensor(const ScoreCall &c, int B, int P_img) {
+    const cmdb_bank *b = c.b;
+    const Lane &s = *c.lane;
+    CMDB_CHECK(score_select(c, B, P_img, true));  // m_test, m_star, s*, s_idx, m_star_row
     // the min/argmin phase is complete: its query operand buffers and candidate lists are free again
-    q_split_rows(b, s.m_star, B);
+    q_split_rows(c, s.m_star, B);
     CMDB_CUDA(cudaGetLastError());
-    int n_cand = 0;
-    CMDB_CHECK(score_gemm_candidates(b, B, 1, false, &n_cand));
+    GemmSched sched{};
+    CMDB_CHECK(score_gemm_candidates(c, c.stream, B, 1, false, &sched));
     ReweightCertParams p{};
-    p.cand = s.cand, p.n_cand = n_cand, p.cand_stride = s.cap_p;
+    p.cand = s.cand, p.n_cand = sched.producers, p.cand_stride = b->layout.cap_p;
     p.m_star = s.m_star, p.m_test = s.m_test, p.bank = b->data, p.rows = b->fin_rows, p.row_offset = b->row_offset;
     p.dim = b->dim, p.q_norm = s.q_norm, p.q_eps = s.q_eps;
     p.bmax = b->cert_bmax, p.eb_max = b->cert_eb_max, p.acc_model = (float)(b->dim / 16 + 1) * 17.f * 1.1920929e-7f;
-    p.cg = s.sched_pair_last ? 2 : 1, p.n_units = b->num_sms / p.cg, p.EG = kGemmEpiGroups;
+    p.cg = sched.pair ? 2 : 1, p.n_units = b->num_sms / p.cg, p.EG = kGemmEpiGroups;
     p.stride = score_tile_stride(1, p.n_units);
     p.nt = (int)(b->fin_rows_pad / kScoreBN);
-    p.run = s.sched_run_last;
-    p.s_key = s.s_key, p.top3 = s.top3, p.res = reinterpret_cast<TailResult *>(s.tail), p.fuse_final = 1;
-    CMDB_REQUIRE(n_cand <= 320, CMDB_ERR_UNSUPPORTED, "scoring: %d GEMM producers exceed reweight_cert_kernel's limit", n_cand);
-    reweight_cert_kernel<<<B, 256, 0, st>>>(p);
+    p.run = sched.run;
+    p.s_key = s.s_key, p.top3 = s.top3, p.res = c.tail, p.fuse_final = 1;
+    CMDB_REQUIRE(p.n_cand <= 320, CMDB_ERR_UNSUPPORTED, "scoring: %d GEMM producers exceed reweight_cert_kernel's limit", p.n_cand);
+    reweight_cert_kernel<<<B, 256, 0, c.stream>>>(p);
     CMDB_CUDA(cudaGetLastError());
     return CMDB_OK;
 }
@@ -1476,12 +1481,13 @@ static int score_reweight_tensor(cmdb_bank *b, int B, int P_img) {
 // SURVEY 8f-1: three nearest bank rows of every bank row.  The bank is its own query set: chunks of rows go through the
 // fp16 split, the certified pre-filter GEMM and reweight_cert_kernel (one block per row, keys only).
 int score_build_knn_table(cmdb_bank *b, long long row_first, long long row_count) {
-    ScoreScratch &s = b->ss;
     const int chunk = 64 * kScoreBM;  // 8192 rows: 64 M tiles per GEMM launch
     // scratch for `chunk` query rows; sized like a 32-image batch so that later scoring calls do not have to grow it
-    CMDB_CHECK(score_scratch_alloc(b, 32, chunk / 32, s.map_stride ? (int)lround(sqrt((double)s.map_stride)) : 224));
-    score_select_slot(b, 0, 0);
-    cudaStream_t st = b->stream;  // lane 0 (only valid after the selection)
+    const size_t map_stride = b->layout.map_stride;
+    CMDB_CHECK(score_scratch_alloc(b, 32, chunk / 32, map_stride ? (int)lround(sqrt((double)map_stride)) : 224));
+    const ScoreCall c = score_call(b, 0, 0);   // lane 0; the result slot is not used
+    const Lane &s = *c.lane;
+    cudaStream_t st = c.stream;
     if (!b->knn_table || b->knn_rows != b->fin_rows) {
         cudaFree(b->knn_table);
         b->knn_table = nullptr;
@@ -1493,22 +1499,22 @@ int score_build_knn_table(cmdb_bank *b, long long row_first, long long row_count
     for (long long r0 = row_first; r0 < row_end; r0 += chunk) {
         const int n = (int)std::min<long long>(chunk, row_end - r0);
         const float *rows = b->data + (size_t)r0 * b->dim;
-        q_split_rows(b, rows, n);
+        q_split_rows(c, rows, n);
         CMDB_CUDA(cudaGetLastError());
-        int n_cand = 0;
-        CMDB_CHECK(score_gemm_candidates(b, n, 1, false, &n_cand));
+        GemmSched sched{};
+        CMDB_CHECK(score_gemm_candidates(c, st, n, 1, false, &sched));
         ReweightCertParams p{};
-        p.cand = s.cand, p.n_cand = n_cand, p.cand_stride = s.cap_p;
+        p.cand = s.cand, p.n_cand = sched.producers, p.cand_stride = b->layout.cap_p;
         p.m_star = rows, p.m_test = nullptr, p.bank = b->data, p.rows = b->fin_rows, p.row_offset = 0;
         p.dim = b->dim, p.q_norm = s.q_norm, p.q_eps = s.q_eps;
         p.bmax = b->cert_bmax, p.eb_max = b->cert_eb_max, p.acc_model = (float)(b->dim / 16 + 1) * 17.f * 1.1920929e-7f;
-        p.cg = s.sched_pair_last ? 2 : 1, p.n_units = b->num_sms / p.cg, p.EG = kGemmEpiGroups;
+        p.cg = sched.pair ? 2 : 1, p.n_units = b->num_sms / p.cg, p.EG = kGemmEpiGroups;
         const int mt = (n + kScoreBM - 1) / kScoreBM;
         p.stride = score_tile_stride((mt + p.cg - 1) / p.cg, p.n_units);
         p.nt = (int)(b->fin_rows_pad / kScoreBN);
-        p.run = s.sched_run_last;
+        p.run = sched.run;
         p.s_key = nullptr, p.top3 = b->knn_table + (size_t)r0 * 3, p.res = nullptr, p.fuse_final = 0;
-        CMDB_REQUIRE(n_cand <= 320, CMDB_ERR_UNSUPPORTED, "scoring: %d GEMM producers exceed reweight_cert_kernel's limit", n_cand);
+        CMDB_REQUIRE(p.n_cand <= 320, CMDB_ERR_UNSUPPORTED, "scoring: %d GEMM producers exceed reweight_cert_kernel's limit", p.n_cand);
         reweight_cert_kernel<<<n, 256, 0, st>>>(p);
         CMDB_CUDA(cudaGetLastError());
     }
@@ -1516,29 +1522,30 @@ int score_build_knn_table(cmdb_bank *b, long long row_first, long long row_count
     return CMDB_OK;
 }
 
-int score_reweight(cmdb_bank *b, int B, int P_img) {
+int score_reweight(const ScoreCall &c, int B, int P_img) {
+    const cmdb_bank *b = c.b;
+    const Lane &l = *c.lane;
     if (b->knn_table && b->row_offset == 0 && b->knn_rows == b->fin_rows) {  // the bank's neighbour table: the w_dist pass is a lookup
-        CMDB_CHECK(score_select(b, B, P_img, true));
-        reweight_lookup_kernel<<<B, 64, 0, b->stream>>>(b->knn_table, b->ss.m_test, b->data, b->dim, b->ss.s_key, b->ss.top3,
-                                                        reinterpret_cast<TailResult *>(b->ss.tail));
+        CMDB_CHECK(score_select(c, B, P_img, true));
+        reweight_lookup_kernel<<<B, 64, 0, c.stream>>>(b->knn_table, l.m_test, b->data, b->dim, l.s_key, l.top3, c.tail);
         CMDB_CUDA(cudaGetLastError());
         return CMDB_OK;
     }
     // a single image: the one-launch CUDA-core sweep is as fast as a one-tile GEMM over the whole bank; batches go to the
     // tensor cores, whose cost does not grow with B (identical keys either way).
     if (b->score_impl == CMDB_SCORE_TCGEN05 && b->prefilter_terms == 0 && B >= 2 && B <= kScoreBM)
-        return score_reweight_tensor(b, B, P_img);
+        return score_reweight_tensor(c, B, P_img);
     ReweightParams p{};
     p.bank = b->data, p.rows = b->fin_rows, p.row_offset = b->row_offset, p.dim = b->dim, p.B = B, p.P_img = P_img;
-    p.q = b->ss.q_f32, p.s_key = b->ss.s_key, p.min_idx = b->ss.min_idx;
-    p.block_keys = b->ss.topk_keys, p.top3 = b->ss.top3, p.done_counter = b->ss.done_counter;
-    p.res = reinterpret_cast<TailResult *>(b->ss.tail);
+    p.q = c.slot->q_f32, p.s_key = l.s_key, p.min_idx = c.min_idx;
+    p.block_keys = l.topk_keys, p.top3 = l.top3, p.done_counter = l.done_counter;
+    p.res = c.tail;
     const size_t smem = sizeof(float) * (size_t)B * b->dim + sizeof(unsigned long long) * 8 * B * 3;
-    const int blocks = b->ss.n_topk_blocks;
+    const int blocks = b->layout.n_topk_blocks;
 #define CMDB_RW(DVV)                                                                                              \
     case DVV:                                                                                                     \
         CMDB_CUDA(cudaFuncSetAttribute(reweight_kernel<DVV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        reweight_kernel<DVV><<<blocks, 256, smem, b->stream>>>(p);                                                \
+        reweight_kernel<DVV><<<blocks, 256, smem, c.stream>>>(p);                                                 \
         break;
     switch ((b->dim / 4 + 31) / 32) {
         CMDB_RW(1) CMDB_RW(2) CMDB_RW(3) CMDB_RW(4) CMDB_RW(5) CMDB_RW(6) CMDB_RW(7) CMDB_RW(8) CMDB_RW(9) CMDB_RW(10)
@@ -1552,15 +1559,16 @@ int score_reweight(cmdb_bank *b, int B, int P_img) {
     return CMDB_OK;
 }
 
-int score_shard_lookup(cmdb_bank *b, int B, float *contrib_dev) {
-    shard_lookup_kernel<<<B, 64, 0, b->stream>>>(b->knn_table, b->ss.m_test, b->data, b->fin_rows, b->row_offset, b->dim, b->ss.top3,
-                                                 reinterpret_cast<TailResult *>(b->ss.tail), contrib_dev);
+int score_shard_lookup(const ScoreCall &c, int B, float *contrib_dev) {
+    const cmdb_bank *b = c.b;
+    shard_lookup_kernel<<<B, 64, 0, c.stream>>>(b->knn_table, c.lane->m_test, b->data, b->fin_rows, b->row_offset, b->dim,
+                                                c.lane->top3, c.tail, contrib_dev);
     CMDB_CUDA(cudaGetLastError());
     return CMDB_OK;
 }
 
-int score_shard_final(cmdb_bank *b, int B, const float *d2_sum_dev) {
-    shard_final_kernel<<<1, 64, 0, b->stream>>>(b->ss.top3, d2_sum_dev, b->dim, B, reinterpret_cast<TailResult *>(b->ss.tail));
+int score_shard_final(const ScoreCall &c, int B, const float *d2_sum_dev) {
+    shard_final_kernel<<<1, 64, 0, c.stream>>>(c.lane->top3, d2_sum_dev, c.b->dim, B, c.tail);
     CMDB_CUDA(cudaGetLastError());
     return CMDB_OK;
 }

@@ -101,7 +101,8 @@ int cmdb_bank_set_option(cmdb_bank *bank, int option, int value);
  * out_sum / out_sumsq (optional) return the float64 sum and sum of squares (the latter rebuilt as
  * sum((x - mean)^2) + sum * mean) so that shards can be combined on the host. */
 int cmdb_bank_stats(cmdb_bank *bank, double *out_mean, double *out_std_unbiased, double *out_sum, double *out_sumsq);
-/* lib = (lib - mean) / std in float32, in place (multiple_features.py:41); one IEEE subtract and one IEEE divide. */
+/* lib = (lib - mean) / std in float32, in place (multiple_features.py:41); one IEEE subtract and one IEEE divide.
+ * normalize, gather and finalize return CMDB_ERR_STATE while a submitted call (batch, round, fused batch) is outstanding. */
 int cmdb_bank_normalize(cmdb_bank *bank, float mean, float std);
 /* lib = lib[idx] (multiple_features.py:48): keeps n rows in the given order; idx are LOCAL row numbers. */
 int cmdb_bank_gather(cmdb_bank *bank, const int64_t *idx_host, int64_t n);
@@ -112,8 +113,9 @@ int cmdb_bank_read_device(cmdb_bank *bank, int64_t row0, int64_t n_rows, float *
 /* Builds the scoring layout (fp16 hi/lo split, row norms) for the current rows. Must precede cmdb_score*. */
 int cmdb_bank_finalize(cmdb_bank *bank);
 /* A handle has two compute lanes (stream + private scratch each); scoring calls alternate between them so that the tail of
- * one batch / round overlaps the distance GEMM of the next.  cmdb_bank_stream: the cudaStream_t the NEXT scoring call on this
- * handle will run on (order producer work / collectives against it); cmdb_bank_lane_streams: both of them. */
+ * one batch / round overlaps the distance GEMM of the next.  Everything else runs on lane 0.  cmdb_bank_stream: the
+ * cudaStream_t the NEXT scoring call on this handle will run on, or during a sharded round the round's (order producer work /
+ * collectives against it); cmdb_bank_lane_streams: both of them. */
 int cmdb_bank_stream(cmdb_bank *bank, void **out_stream);
 int cmdb_bank_lane_streams(cmdb_bank *bank, void **out_streams2);
 /* milliseconds of each stage (CMDB_T_*) of the last cmdb_score call on this handle; needs CMDB_OPT_TIMING = 1.
@@ -324,7 +326,8 @@ int cmdb_eval_read(cmdb_bank *bank, int64_t first, int64_t n, double *maps_host 
  *      of the other outs[] entries are left untouched).
  * Phases 1 and 2 only enqueue work on the handle's stream (cmdb_bank_stream) and return; run the collectives on that same
  * stream.  Nothing synchronises the host between the phases, and three rounds can be outstanding per handle (the result
- * copy of round k and the host work for the next rounds overlap the kernels of the other lane).
+ * copy of round k and the host work for the next rounds overlap the kernels of the other lane).  cmdb_score_shard_min opens
+ * the round and cmdb_score_shard_finish_submit closes it; phases 2 and 3 return CMDB_ERR_STATE when no round is open.
  * Results are bit-identical to cmdb_score_batch on the un-sharded bank.
  */
 int cmdb_score_shard_min(cmdb_bank *bank, const float *patches, int B, int P, int patch_is_device, int out_hw,
