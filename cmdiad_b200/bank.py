@@ -357,18 +357,21 @@ class Bank:
         return (np.ascontiguousarray(indptr, dtype=np.int32), np.ascontiguousarray(indices, dtype=np.int32),
                 np.ascontiguousarray(data, dtype=np.float64), int(d_proj))
 
-    def coreset_select(self, n_select, csr, dtype_mode=L.CORESET_FP16, force_idx=None, return_min=False):
-        """Greedy k-center selection on the projected bank; csr = (indptr, indices, data, d_proj) or None."""
+    def coreset_select(self, n_select, csr, dtype_mode=L.CORESET_FP16, force_idx=None, return_min=False,
+                       _mind_global=False):
+        """Greedy k-center selection on the projected bank; csr = (indptr, indices, data, d_proj) or None.
+        _mind_global (tests): keep the kernel's min-distance vector in global memory even where it fits shared memory."""
         indptr, indices, data, d_proj = self._csr(csr)
         out = np.zeros(int(n_select), dtype=np.int64)
-        if force_idx is None and not return_min:
+        if force_idx is None and not return_min and not _mind_global:
             L.check(self._lib.cmdb_coreset_select(self._h, int(n_select), _ptr(indptr), _ptr(indices), _ptr(data), d_proj,
                                                   int(dtype_mode), _ptr(out)))
             return out
         fi = None if force_idx is None else np.ascontiguousarray(force_idx, dtype=np.int64)
         mn = np.zeros(self.rows, dtype=np.float16 if dtype_mode == L.CORESET_FP16 else np.float64)
         L.check(self._lib.cmdb_coreset_select_debug(self._h, int(n_select), _ptr(indptr), _ptr(indices), _ptr(data),
-                                                    d_proj, int(dtype_mode), _ptr(out), _ptr(fi), _ptr(mn)))
+                                                    d_proj, int(dtype_mode), _ptr(out), _ptr(fi), _ptr(mn),
+                                                    int(bool(_mind_global))))
         return (out, mn) if return_min else out
 
     def coreset_select_sharded(self, comm, n_total_rows, n_select, csr, dtype_mode=L.CORESET_FP16):

@@ -212,7 +212,7 @@ int cmdb_project(cmdb_bank *b, const int32_t *indptr, const int32_t *indices, co
 
 static int coreset_impl(cmdb_bank *b, int64_t n_select, const int32_t *indptr, const int32_t *indices, const double *data,
                         int d_proj, int dtype_mode, int64_t *out_idx_host, const int64_t *force_idx, void *out_min_last,
-                        ShardCtx *sh = nullptr) {
+                        ShardCtx *sh = nullptr, bool force_mind_global = false) {
     CMDB_REQUIRE(b && out_idx_host, CMDB_ERR_INVALID, "cmdb_coreset_select: NULL argument");
     CMDB_REQUIRE(b->rows > 0, CMDB_ERR_STATE, "cmdb_coreset_select: bank is empty");
     const int64_t n_total = sh ? sh->n_total : b->rows;
@@ -223,8 +223,12 @@ static int coreset_impl(cmdb_bank *b, int64_t n_select, const int32_t *indptr, c
                  d_proj, b->dim);
     CMDB_CUDA(cudaSetDevice(b->device));
     const int d = d_proj > 0 ? d_proj : b->dim;
-    // the shard's projected rows start (row_offset*d) & 3 elements past a 32-byte boundary (see coreset_greedy_dev)
-    const int pad = (int)((b->row_offset * d) & 3);
+    // The kernels' 16-byte vector loads assume that address alignment follows the alignment class they compute for a
+    // row.  The row-sharded loop (world > 1) computes it from the GLOBAL row, so the shard's projected rows start
+    // (row_offset*d) & 3 elements past a 32-byte boundary (see coreset_greedy_dev).  Every other call runs with
+    // row_offset 0 -- also on a handle whose row_offset is set -- and its rows start on the boundary.
+    const bool sharded = sh && sh->world > 1;
+    const int pad = sharded ? (int)((b->row_offset * d) & 3) : 0;
     double *z_alloc = nullptr;
     CMDB_CUDA(cudaMalloc(&z_alloc, sizeof(double) * ((size_t)b->rows * d + 4)));
     double *z = z_alloc + pad;
@@ -236,7 +240,9 @@ static int coreset_impl(cmdb_bank *b, int64_t n_select, const int32_t *indptr, c
         f32_to_f64_kernel<<<b->num_sms * 4, 512, 0, b->handle_stream()>>>(b->data, (long long)b->rows * d, z);
         rc = cudaGetLastError() == cudaSuccess ? CMDB_OK : CMDB_ERR_CUDA;
     }
-    if (rc == CMDB_OK) rc = coreset_greedy_dev(b, z, b->rows, d, n_select, dtype_mode, out_idx_host, force_idx, out_min_last, sh);
+    if (rc == CMDB_OK)
+        rc = coreset_greedy_dev(b, z, b->rows, d, n_select, dtype_mode, out_idx_host, force_idx, out_min_last, sh,
+                                force_mind_global);
     cudaFree(z_alloc);
     return rc;
 }
@@ -246,12 +252,19 @@ int cmdb_coreset_select(cmdb_bank *b, int64_t n_select, const int32_t *indptr, c
     return coreset_impl(b, n_select, indptr, indices, data, d_proj, dtype_mode, out_idx_host, nullptr, nullptr);
 }
 
-// test hook (not in the public header): teacher forcing and the final min-distance vector
+// test hook (not in the public header): teacher forcing, the final min-distance vector, and (mind_global != 0) the
+// min-distance vector kept in global memory at any bank size
 int cmdb_coreset_select_debug(cmdb_bank *b, int64_t n_select, const int32_t *indptr, const int32_t *indices,
                               const double *data, int d_proj, int dtype_mode, int64_t *out_idx_host,
-                              const int64_t *force_idx_host, void *out_min_last_host) {
+                              const int64_t *force_idx_host, void *out_min_last_host, int mind_global) {
     return coreset_impl(b, n_select, indptr, indices, data, d_proj, dtype_mode, out_idx_host, force_idx_host,
-                        out_min_last_host);
+                        out_min_last_host, nullptr, mind_global != 0);
+}
+
+// host-only test hook (not in the public header): the coreset kernel's rows per CTA on num_sms SMs and whether their
+// min-distances live in shared memory (1) or global memory (0) -- the rule launch_coreset applies
+int cmdb_debug_coreset_plan(int num_sms, int64_t N, int d, int dtype_mode, int64_t *rows_per_cta, int *mind_in_smem) {
+    return coreset_plan_info(num_sms, N, d, dtype_mode, rows_per_cta, mind_in_smem);
 }
 
 size_t cmdb_coreset_mailbox_bytes(int world, int d_proj_max) {

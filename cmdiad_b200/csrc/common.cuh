@@ -275,7 +275,10 @@ struct ShardCtx {  // row-sharded coreset loop
     const double *z0_host;  // float64 projection of global row 0
 };
 int coreset_greedy_dev(cmdb_bank *b, const double *z_dev, int64_t N, int d, int64_t n_select, int dtype_mode,
-                       int64_t *out_idx_host, const int64_t *force_idx_host, void *out_min_last_host, const ShardCtx *sh);
+                       int64_t *out_idx_host, const int64_t *force_idx_host, void *out_min_last_host, const ShardCtx *sh,
+                       bool force_mind_global);
+// host only: rows per CTA of the persistent kernel on num_sms SMs and whether their min-distances fit shared memory
+int coreset_plan_info(int num_sms, int64_t N, int d, int dtype_mode, int64_t *rows_per_cta, int *mind_in_smem);
 int coreset_greedy(cmdb_bank *b, const double *z_dev, int64_t N, int d, int64_t n_select, int dtype_mode,
                    int64_t *out_idx_host);
 int coreset_rownorms(int device, const void *z_host, const void *last_host, int64_t n_rows, int d, int dtype_mode,

@@ -738,17 +738,48 @@ static int launch_rownorm(cudaStream_t st, int num_sms, const T *z, const T *las
     return CMDB_OK;
 }
 
+// Where coreset_kernel keeps the running min-distance vector.  CTA c of `grid` owns rows [c * rows_per_cta,
+// (c + 1) * rows_per_cta) and holds their min-distances in shared memory, behind the fixed part of its layout (transpose
+// tiles, `last`, up to 16 bytes of alignment, the 64 reduction slots), as long as the whole block stays within 200 KB;
+// otherwise they stay in global memory and every access goes through L2 (.cg).  force_global picks the second
+// placement at any size (tests compare the two on the same bank).
+struct CoresetPlan {
+    long long rows_per_cta;
+    bool mind_in_smem;
+    size_t smem;  // dynamic shared memory of the launch
+};
 template <typename T>
-static int launch_coreset(cmdb_bank *b, CoresetParams p) {
+static CoresetPlan coreset_plan(int grid, long long N, int d, bool force_global) {
+    const size_t fixed = sizeof(typename Traits<T>::acc_t) * kCsWarps * 32 * 33 + sizeof(T) * (size_t)d + 16 + 64 * 8;
+    CoresetPlan pl;
+    pl.rows_per_cta = (N + grid - 1) / grid;
+    pl.smem = fixed + sizeof(T) * (size_t)pl.rows_per_cta;
+    pl.mind_in_smem = !force_global && pl.smem <= 200 * 1024;
+    if (!pl.mind_in_smem) pl.smem = fixed;
+    return pl;
+}
+
+int coreset_plan_info(int num_sms, int64_t N, int d, int dtype_mode, int64_t *rows_per_cta, int *mind_in_smem) {
+    CMDB_REQUIRE(num_sms >= 1 && N >= 1 && d >= 1 && rows_per_cta && mind_in_smem, CMDB_ERR_INVALID, "coreset plan: bad arguments");
+    CMDB_REQUIRE(dtype_mode == CMDB_CORESET_FP16 || dtype_mode == CMDB_CORESET_FP64, CMDB_ERR_INVALID,
+                 "coreset plan: unknown dtype_mode %d", dtype_mode);
+    const CoresetPlan pl = dtype_mode == CMDB_CORESET_FP16 ? coreset_plan<__half>(num_sms, N, d, false)
+                                                           : coreset_plan<double>(num_sms, N, d, false);
+    *rows_per_cta = pl.rows_per_cta;
+    *mind_in_smem = pl.mind_in_smem ? 1 : 0;
+    return CMDB_OK;
+}
+
+template <typename T>
+static int launch_coreset(cmdb_bank *b, CoresetParams p, bool force_mind_global) {
     const int d = p.d;
     const int nv = d >= 128 ? (d / 4 + 31) / 32 : 1;
     int grid = b->num_sms;
-    const size_t fixed = sizeof(typename Traits<T>::acc_t) * kCsWarps * 32 * 33 + sizeof(T) * (size_t)d + 16 + 64 * 8;
     auto run = [&](auto kern) -> int {
-        p.rows_per_cta = (p.N + grid - 1) / grid;
-        size_t smem = fixed + sizeof(T) * (size_t)p.rows_per_cta;
-        p.mind_in_smem = smem <= 200 * 1024;
-        if (!p.mind_in_smem) smem = fixed;
+        const CoresetPlan pl = coreset_plan<T>(grid, p.N, d, force_mind_global);
+        p.rows_per_cta = pl.rows_per_cta;
+        p.mind_in_smem = pl.mind_in_smem;
+        const size_t smem = pl.smem;
         CMDB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         int per_sm = 0;
         CMDB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kCsThreads, smem));
@@ -805,8 +836,10 @@ static int launch_coreset(cmdb_bank *b, CoresetParams p) {
 
 // z_dev: float64 [N,d] projected rows of THIS shard; for a shard with row_offset != 0 the caller places row 0 of the
 // buffer (row_offset*d) & 3 elements past a 32-byte boundary so that address alignment == global alignment class.
+// force_mind_global: keep the min-distance vector in global memory even where it would fit shared memory (coreset_plan).
 int coreset_greedy_dev(cmdb_bank *b, const double *z_dev, int64_t N, int d, int64_t n_select, int dtype_mode,
-                       int64_t *out_idx_host, const int64_t *force_idx_host, void *out_min_last_host, const ShardCtx *sh) {
+                       int64_t *out_idx_host, const int64_t *force_idx_host, void *out_min_last_host, const ShardCtx *sh,
+                       bool force_mind_global) {
     const bool sharded = sh && sh->world > 1;
     const long long n_total = sharded ? sh->n_total : N;
     CMDB_REQUIRE(N >= 0 && n_total > 0 && d >= 32 && n_select >= 1 && n_select <= n_total, CMDB_ERR_INVALID,
@@ -906,7 +939,7 @@ int coreset_greedy_dev(cmdb_bank *b, const double *z_dev, int64_t N, int d, int6
             CS_TRY(cudaGetLastError());
             if (sharded) CS_TRY(publish_shard());
             p.z = zh, p.mind = mind;
-            rc = launch_coreset<__half>(b, p);
+            rc = launch_coreset<__half>(b, p, force_mind_global);
         }
     } else {
         CS_TRY(cudaMalloc(&mind, sizeof(double) * (size_t)N));
@@ -918,7 +951,7 @@ int coreset_greedy_dev(cmdb_bank *b, const double *z_dev, int64_t N, int d, int6
                 CS_TRY(publish_shard());
                 p.z = mine_in_replica;
             }
-            rc = launch_coreset<double>(b, p);
+            rc = launch_coreset<double>(b, p, force_mind_global);
         }
     }
     if (rc != CMDB_OK) {
@@ -945,7 +978,7 @@ int coreset_greedy_dev(cmdb_bank *b, const double *z_dev, int64_t N, int d, int6
 
 int coreset_greedy(cmdb_bank *b, const double *z_dev, int64_t N, int d, int64_t n_select, int dtype_mode,
                    int64_t *out_idx_host) {
-    return coreset_greedy_dev(b, z_dev, N, d, n_select, dtype_mode, out_idx_host, nullptr, nullptr, nullptr);
+    return coreset_greedy_dev(b, z_dev, N, d, n_select, dtype_mode, out_idx_host, nullptr, nullptr, nullptr, false);
 }
 
 int coreset_rownorms(int device, const void *z_host, const void *last_host, int64_t n_rows, int d, int dtype_mode,
