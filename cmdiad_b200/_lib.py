@@ -132,6 +132,7 @@ DEBUG_SYMBOLS = {
     "cmdb_debug_eval_load": (_I, [_VP, _VP, _I64]),
     "cmdb_coreset_select_debug": (_I, [_VP, _I64, _VP, _VP, _VP, _I, _I, _VP, _VP, _VP, _I]),
     "cmdb_debug_coreset_plan": (_I, [_I, _I64, _I, _I, c_i64_p, ctypes.POINTER(_I)]),
+    "cmdb_debug_producer_tiles": (_I, [_I, _I, _I, _I, _I, _I, c_i32_p, _I, ctypes.POINTER(_I)]),
 }
 
 _lib = None

@@ -13,25 +13,21 @@ __global__ void __launch_bounds__(512) f32_to_f64_kernel(const float *__restrict
         z[i] = (double)x[i];
 }
 
-// keys[p] = (float_bits(min_val[p]) << 32) | global_row ; and the inverse
+// keys[p] = exchange_key(min_val[p], global row); and the inverse
 __global__ void pack_keys_kernel(const float *__restrict__ min_val, const long long *__restrict__ min_idx, int P,
                                  long long *__restrict__ keys) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < P) {
-        const long long g = min_idx[i];
-        keys[i] = g < 0 ? 0x7fffffffffffffffLL
-                        : (long long)(((unsigned long long)__float_as_uint(min_val[i]) << 32) | (unsigned long long)g);
-    }
+    if (i < P) keys[i] = exchange_key(min_val[i], min_idx[i]);
 }
 __global__ void unpack_keys_kernel(const long long *__restrict__ keys, int P, int P_img, float *__restrict__ min_val,
                                    long long *__restrict__ min_idx, unsigned long long *s_key) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < P) {
         const unsigned long long k = (unsigned long long)keys[i];
-        const float v = __uint_as_float((unsigned int)(k >> 32));
+        const float v = key_value(k);
         min_val[i] = v;
-        min_idx[i] = (long long)(k & 0xffffffffULL);
-        atomicMax(s_key + i / P_img, ((unsigned long long)__float_as_uint(v) << 32) | (0xffffffffu - (unsigned int)(i % P_img)));
+        min_idx[i] = key_row(k);
+        argmax_publish(s_key, i, P_img, v);
     }
 }
 
@@ -621,7 +617,30 @@ int cmdb_debug_lane_timeline(cmdb_bank *b, float *out) {
     return CMDB_OK;
 }
 
-int cmdb_debug_tile_stride(int mt, int G) { return score_tile_stride(mt, G); }
+int cmdb_debug_tile_stride(int mt, int G) { return tile_stride(mt, G); }
+
+// host-only test hook (not in the public header): the N tiles the exact rescan visits for (M tile mtile of a batch whose
+// first-pass GEMM ran in launches of chunk_tiles out of mt_total M tiles on num_sms CTAs, producer CTA c), in slot order --
+// the schedules gemm_sched records, walked by rescan_tile.  One chunk (chunk_tiles == mt_total) is the walk of the
+// re-weighting certificate over a launch of mt_total M tiles.
+int cmdb_debug_producer_tiles(int num_sms, int nt, int chunk_tiles, int mt_total, int mtile, int c, int32_t *tiles, int cap,
+                              int *n_out) {
+    CMDB_REQUIRE(num_sms >= 1 && nt >= 1 && chunk_tiles >= 1 && chunk_tiles <= mt_total && mtile >= 0 && mtile < mt_total && c >= 0 &&
+                     c < num_sms && tiles && n_out,
+                 CMDB_ERR_INVALID, "cmdb_debug_producer_tiles: bad arguments");
+    const int last_tiles = mt_total - (mt_total - 1) / chunk_tiles * chunk_tiles;
+    const GemmSched full = gemm_sched(nt, chunk_tiles, num_sms, false);
+    const GemmSched last = gemm_sched(nt, last_tiles, num_sms, false);
+    int n = 0;
+    for (int kt = 0; kt < producer_slots(full, last); ++kt) {
+        const int t = rescan_tile(full, last, chunk_tiles, mt_total, mtile, c, kt);
+        if (t >= nt) continue;
+        CMDB_REQUIRE(n < cap, CMDB_ERR_CAPACITY, "cmdb_debug_producer_tiles: more than %d tiles", cap);
+        tiles[n++] = t;
+    }
+    *n_out = n;
+    return CMDB_OK;
+}
 int cmdb_debug_fallback_use_rescan(int fails, int pairs) { return fallback_use_rescan(fails, pairs) ? 1 : 0; }
 
 // test hook (not in the public header): rows [r0, r0 + n) of the neighbour table as packed (d^2 bits << 32 | row) keys

@@ -291,6 +291,78 @@ struct TailResult {  // head of a result block (ScoreCall::tail), one per image
     long long m_star_row;  // global row of m_star
 };
 
+// Launch schedule of one distance-GEMM launch, decided by score_gemm_candidates alone (gemm_sched).  N tiles go in order,
+// dealt as runs of `run` consecutive tiles: run j of M tile m (M tile pair when pair) goes to unit (j * stride + m) % units.
+struct GemmSched {
+    int producers;  // (CTA, column group) candidate lists
+    bool pair;      // CTA pairs (cta_group::2)
+    int units;      // scheduling units G: CTAs, or CTA pairs
+    int stride;     // tile_stride(M tiles per unit, G); 0 for a compact launch, which sizes itself on the device
+    int inv;        // stride^-1 mod G
+    int run;        // N tiles per visit of an M tile (score_gemm_run)
+    int nt;         // N tiles of the launch
+};
+
+// Smallest s >= mt with gcd(s mod G, G) == 1: the stride of the GEMM's tile schedule (score_gemm.cu, TileIter).
+__host__ __device__ __forceinline__ int tile_stride(int mt, int G) {
+    for (int s = mt;; ++s) {
+        int a = s % G, b = G;
+        if (a == 0) a = G;
+        while (b) {
+            const int t = a % b;
+            a = b, b = t;
+        }
+        if (a == 1 || G == 1) return s;
+    }
+}
+
+// Which rows a producer (unit c, column group) saw for M tile m of a launch with schedule s: the runs j, j + G, j + 2G,
+// ... with j * stride = c - m (mod G), i.e. j = (c - m) * stride^-1 mod G.  The certificate consumers walk them in tile
+// slots `width` >= s.run tiles wide: slot kt is the (kt % width)-th tile of the (kt / width)-th run.  Returns the N tile,
+// or >= s.nt for an empty slot.
+__host__ __device__ __forceinline__ int producer_tile(const GemmSched &s, int width, int c, int m, int kt) {
+    const int G = s.units, k = kt / width, t = kt % width;
+    const int want = ((c - m % G) % G + G) % G;
+    const int jrun = (int)(((long long)want * s.inv) % G) + k * G;
+    return t < s.run ? jrun * s.run + t : s.nt;
+}
+// Slots that cover the longest producer of two launches over the same N tiles (of one launch: a == b): runs counted at
+// the shorter run length, slots as wide as the longer one.
+__host__ __device__ __forceinline__ int producer_slots(const GemmSched &a, const GemmSched &b) {
+    const int run_min = a.run < b.run ? a.run : b.run, run_max = a.run < b.run ? b.run : a.run;
+    return ((a.nt + run_min - 1) / run_min + a.units - 1) / a.units * run_max;
+}
+// Slot kt of the exact rescan of (M tile mtile of a batch, unit c): the batch's first-pass GEMM ran in chunks of
+// chunk_tiles M tiles with schedule `full`; the last chunk, which may be shorter, with schedule `last`.
+__host__ __device__ __forceinline__ int rescan_tile(const GemmSched &full, const GemmSched &last, int chunk_tiles, int mt_total,
+                                                    int mtile, int c, int kt) {
+    const int chunk = mtile / chunk_tiles;
+    const bool is_last = (chunk + 1) * chunk_tiles >= mt_total;
+    return producer_tile(is_last ? last : full, full.run < last.run ? last.run : full.run, c, mtile - chunk * chunk_tiles, kt);
+}
+
+// Packed 64-bit keys: a non-negative float's bits above an index, so that the integer order is the (value, index) order.
+// The value of any of them:
+__device__ __forceinline__ float key_value(unsigned long long k) { return __uint_as_float((unsigned int)(k >> 32)); }
+// (d^2 or distance, row): the minimum is the nearest row, the lowest row on ties; ~0ULL = no row
+__device__ __forceinline__ unsigned long long pack_min_key(float v, unsigned int row) {
+    return ((unsigned long long)__float_as_uint(v) << 32) | row;
+}
+__device__ __forceinline__ long long key_row(unsigned long long k) { return (long long)(k & 0xffffffffULL); }
+// exchange key of a sharded round: (min distance, global row) as a signed integer, INT64_MAX where there is no row, so
+// that a MIN over the ranks is the global argmin (decoded with key_value / key_row)
+__device__ __forceinline__ long long exchange_key(float v, long long row) {
+    return row < 0 ? 0x7fffffffffffffffLL : (long long)(((unsigned long long)__float_as_uint(v) << 32) | (unsigned long long)row);
+}
+// argmax key of an image: an atomicMax over (min_val bits, ~query) keeps the largest value, the lowest query on ties
+__device__ __forceinline__ void argmax_publish(unsigned long long *s_key, int qi, int P_img, float v) {
+    atomicMax(s_key + qi / P_img, ((unsigned long long)__float_as_uint(v) << 32) | (0xffffffffu - (unsigned int)(qi % P_img)));
+}
+__device__ __forceinline__ int argmax_query(unsigned long long k) { return (int)(0xffffffffu - (unsigned int)(k & 0xffffffffu)); }
+
+// alpha of the certificate's error bound: the tensor core's accumulation of D/16 MMAs of 16 exact fp16 products
+inline float cert_acc_model(int dim) { return (float)(dim / 16 + 1) * 17.f * 1.1920929e-7f; }
+
 // One scoring call: the handle, the compute lane and result slot it uses, and where in the slot's result block its
 // results go.  The submit paths take the next lane and slot (api.cu); the neighbour-table build uses lane 0.
 struct ScoreCall {
@@ -304,15 +376,10 @@ struct ScoreCall {
     long long *min_idx;    // [cap_p]
     float *map_out, *map_pre;   // [cap_b][map_stride]
     unsigned char *map_u8;
-    // first-pass GEMM schedule of score_local_min (the exact rescan walks it): M tiles, chunks of chunk_tiles tiles, CTA pairs
+    // first-pass GEMM of score_local_min, which the exact rescan walks: M tiles, chunks of chunk_tiles tiles, and the
+    // schedules of the first and the last chunk launch
     int mt_total = 0, chunk_tiles = 0;
-    bool pair = false;
-};
-// launch schedule of one distance-GEMM launch
-struct GemmSched {
-    int producers;  // (CTA, column group) candidate lists
-    bool pair;      // CTA pairs (cta_group::2)
-    int run;        // N tiles per visit of an M tile (score_gemm_run)
+    GemmSched first{}, last{};
 };
 
 // score_gemm.cu
@@ -329,8 +396,7 @@ int score_query_prep(const ScoreCall &c, cudaStream_t st, int P, bool compact, i
 // the device-side fail count
 int score_gemm_candidates(const ScoreCall &c, cudaStream_t st, int P, int terms, bool compact, GemmSched *sched, int row0 = 0);
 void q_split_rows(const ScoreCall &c, const float *rows_dev, int n);
-int score_tile_stride(int mt, int G); // host copy of the GEMM's tile schedule stride
-int score_gemm_run(int nt, int mt_units, int G);  // N tiles per visit of an M tile for a launch of that shape
+GemmSched gemm_sched(int nt, int mt, int num_sms, bool pair);  // schedule of a non-compact launch over mt M tiles
 // stage the queries (src: host or device, [B*P_img, dim]) + candidates + refine, all modes
 // stage_after: event the copy stream waits for before it overwrites q_f32 (nullptr: everything queued so far)
 int score_local_min(ScoreCall &c, const float *src, int src_is_device, int B, int P_img, int ev_gemm, int ev_refine,

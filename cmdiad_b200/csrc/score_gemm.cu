@@ -193,18 +193,7 @@ constexpr uint32_t kIdescPair = (1u << 4) | ((uint32_t)(BN >> 3) << 17) | ((uint
 // With s == mt this is plain round-robin dealing; making s coprime with G keeps the load balanced (every G N-tiles each
 // CTA receives exactly mt tiles) AND lets every CTA see ~R/G rows of every query whatever gcd(mt, G) is -- the
 // certificate of the pre-filter (score_tail.cu) needs the rows inside a query's error band to land in different CTAs'
-// top-2 lists.
-__device__ __forceinline__ int tile_stride(int mt, int G) {
-    for (int s = mt;; ++s) {
-        int a = s % G, b = G;
-        if (a == 0) a = G;
-        while (b) {
-            const int t = a % b;
-            a = b, b = t;
-        }
-        if (a == 1 || G == 1) return s;
-    }
-}
+// top-2 lists.  (tile_stride, common.cuh; the host records the same schedule in GemmSched.)
 // c: this CTA (or CTA pair), G: number of CTAs (pairs), mt: M tiles (M tile pairs) per N tile
 struct TileIter {  // n, m: current tile; base: first M tile of this CTA inside N tile n
     int n, m, base, smod, G;
@@ -747,21 +736,9 @@ void q_split_rows(const ScoreCall &c, const float *rows_dev, int n) {
                                                                               l.q_scale_exp, l.q_norm, l.q_eps, nullptr, nullptr);
 }
 
-int score_tile_stride(int mt, int G) {  // == tile_stride() of the kernel
-    for (int s = mt;; ++s) {
-        int a = s % G, b = G;
-        if (a == 0) a = G;
-        while (b) {
-            const int t = a % b;
-            a = b, b = t;
-        }
-        if (a == 1 || G == 1) return s;
-    }
-}
-
 // N tiles per visit of an M tile.  Longer runs cut the traffic of the candidate lists (read + written once per run instead of
 // once per tile) but coarsen the work units: take the longest run whose busiest unit stays within 2 % of the ideal share.
-int score_gemm_run(int nt, int mt_units, int G) {
+static int score_gemm_run(int nt, int mt_units, int G) {
     // at least G runs per M tile, so that EVERY producer keeps seeing a share of every query's rows (the certificate wants the
     // rows near a query's minimum spread over many producers; idle producers made 1.7x more queries need a rescan)
     const double ideal = (double)nt * mt_units / G;
@@ -771,6 +748,20 @@ int score_gemm_run(int nt, int mt_units, int G) {
         if ((double)makespan <= ideal * 1.02) return run;
     }
     return 1;
+}
+
+// x with (a * x) % m == 1 (a coprime with m; m = scheduling units of the GEMM, <= a few hundred); 0 for m == 1
+static int mod_inverse(int a, int m) {
+    a %= m;
+    for (int x = 0; x < m; ++x)
+        if ((a * x) % m == 1 % m) return x;
+    return 0;
+}
+
+GemmSched gemm_sched(int nt, int mt, int num_sms, bool pair) {
+    const int cg = pair ? 2 : 1, mt_units = (mt + cg - 1) / cg, G = num_sms / cg;
+    const int stride = tile_stride(mt_units, G);
+    return GemmSched{kGemmEpiGroups * num_sms, pair, G, stride, mod_inverse(stride, G), score_gemm_run(nt, mt_units, G), nt};
 }
 
 int score_gemm_candidates(const ScoreCall &c, cudaStream_t st, int P, int terms, bool compact, GemmSched *sched, int row0) {
@@ -793,11 +784,9 @@ int score_gemm_candidates(const ScoreCall &c, cudaStream_t st, int P, int terms,
     // the 1-term pre-filter loses 3 % (2.81 -> 2.90 ms; it is not limited by shared-memory reads, and a pair halves the
     // producers per query)
     const bool pair = !compact && b->num_sms % 2 == 0 && terms == 3 && p.mt >= 8;
-    {
-        const int cg = pair ? 2 : 1;
-        // compact launches size themselves on the device (m_count): single tiles there
-        p.run = compact ? 1 : score_gemm_run(p.nt, (p.mt + cg - 1) / cg, b->num_sms / cg);
-    }
+    GemmSched s = gemm_sched(p.nt, p.mt, b->num_sms, pair);
+    if (compact) s.stride = s.inv = 0, s.run = 1;  // sized on the device (m_count): single tiles, stride unknown here
+    p.run = s.run;
     const int threads = kGemmCtlThreads + 128 * kGemmEpiGroups;
     auto launch = [&](auto kern, size_t smem, bool cluster2) -> int {
         CMDB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -817,7 +806,7 @@ int score_gemm_candidates(const ScoreCall &c, cudaStream_t st, int P, int terms,
     if (pair) CMDB_CHECK(launch(score_gemm_kernel<3, kGemmEpiGroups, 2>, GemmSmem<3, 2>::total + 1024, true));
     else if (terms == 1) CMDB_CHECK(launch(score_gemm_kernel<1, kGemmEpiGroups, 1>, GemmSmem<1, 1>::total + 1024, false));
     else CMDB_CHECK(launch(score_gemm_kernel<3, kGemmEpiGroups, 1>, GemmSmem<3, 1>::total + 1024, false));
-    *sched = GemmSched{kGemmEpiGroups * b->num_sms, pair, p.run};
+    *sched = s;
     return CMDB_OK;
 }
 

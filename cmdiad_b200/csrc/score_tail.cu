@@ -15,10 +15,6 @@
 
 namespace cmdb {
 
-__device__ __forceinline__ unsigned long long pack_min_key(float v, unsigned int idx) {
-    return ((unsigned long long)__float_as_uint(v) << 32) | idx;  // v >= 0: unsigned order == float order
-}
-
 // exact ||a - b||^2 in float32, one warp: lanes stride over float4s, xor-shuffle tree
 __device__ __forceinline__ float warp_sqdist(const float *__restrict__ a, const float *__restrict__ b, int dim4, int lane) {
     float acc = 0.f;
@@ -139,9 +135,7 @@ __global__ void __launch_bounds__(256) refine_kernel(const float4 *__restrict__ 
         const float dv = sqrtf(best);
         min_val[qi] = dv;
         min_idx[qi] = best_i < 0 ? -1 : (long long)best_i + row_offset;
-        // argmax over the image's queries, ties -> lowest query: max of (value bits, ~query)
-        atomicMax(s_key + qi / P_img,
-                  ((unsigned long long)__float_as_uint(dv) << 32) | (0xffffffffu - (unsigned int)(qi % P_img)));
+        argmax_publish(s_key, qi, P_img, dv);
     }
 }
 
@@ -174,6 +168,20 @@ __global__ void __launch_bounds__(256) refine_kernel(const float4 *__restrict__ 
 // The last block of the grid to finish also takes the tier decision for the launches behind it (ctl[2..4]).
 constexpr int kCertThreads = 256;
 constexpr int kCertRows = 24;    // rows per query list; a query with more in-band first values hands the surplus to the rescan
+
+// v_ref + 2E(q) with slack for the float32 evaluation of E itself, rounded up; +inf where that is not orderable (NaN,
+// overflow): nothing is certified then
+__device__ __forceinline__ float cert_threshold(float v_ref, float qn, float qe, float bmax, float eb_max, float acc_model, int dim) {
+    const float bh = __fadd_ru(bmax, eb_max);
+    float E = __fmul_ru(qe, bh);
+    E = __fmaf_ru(qn, eb_max, E);
+    E = __fmaf_ru(__fmul_ru(acc_model, __fadd_ru(qn, qe)), bh, E);
+    E = __fmul_ru(2.f, E);
+    const float span = __fadd_ru(qn, bmax);
+    E = __fmaf_ru(__fmul_ru((float)(dim + 16) * 5.9604645e-8f, span), span, E);
+    const float t = __fadd_ru(v_ref, __fmul_ru(2.0625f, E));
+    return v_ref < INFINITY && t < INFINITY ? t : INFINITY;
+}
 
 // exact re-check of a query's listed rows (the smallest (d^2, row) wins: the order of the list does not matter)
 __device__ __forceinline__ void cert_recheck(const int *list, int n_list, const float *__restrict__ qrow, const float *__restrict__ bank,
@@ -246,19 +254,8 @@ __global__ void __launch_bounds__(kCertThreads) refine_cert_kernel(const float4 
 #pragma unroll
         for (int k = 1; k < CSTEP; ++k) v1min = fminf(v1min, part_s[k][threadIdx.x]);
         const int qq = q0 + threadIdx.x;
-        float thr = INFINITY;  // +inf also stands for "not orderable" (NaN / overflow): everything is inside the band then
-        if (qq < P) {
-            const float qn = q_norm[qq], qe = q_eps[qq];
-            const float bh = __fadd_ru(bmax, eb_max);
-            float E = __fmul_ru(qe, bh);
-            E = __fmaf_ru(qn, eb_max, E);
-            E = __fmaf_ru(__fmul_ru(acc_model, __fadd_ru(qn, qe)), bh, E);
-            E = __fmul_ru(2.f, E);
-            const float span = __fadd_ru(qn, bmax);
-            E = __fmaf_ru(__fmul_ru((float)(dim + 16) * 5.9604645e-8f, span), span, E);
-            const float t = __fadd_ru(v1min, __fmul_ru(2.0625f, E));  // 2E plus slack for the float32 evaluation of E itself
-            if (v1min < INFINITY && t < INFINITY) thr = t;            // false for NaN / overflow: never certify those
-        }
+        float thr = INFINITY;  // +inf: everything is inside the band
+        if (qq < P) thr = cert_threshold(v1min, q_norm[qq], q_eps[qq], bmax, eb_max, acc_model, dim);
         thr_s[threadIdx.x] = thr;
     }
     __syncthreads();
@@ -305,11 +302,10 @@ __global__ void __launch_bounds__(kCertThreads) refine_cert_kernel(const float4 
                 const float dv = sqrtf(best);
                 min_val[qq] = dv;
                 min_idx[qq] = (long long)best_i + row_offset;
-                atomicMax(s_key + qq / P_img,
-                          ((unsigned long long)__float_as_uint(dv) << 32) | (0xffffffffu - (unsigned int)(qq % P_img)));
+                argmax_publish(s_key, qq, P_img, dv);
             } else {
                 fail_list[atomicAdd(ctl + 0, 1)] = qq;
-                best_key[qq] = best_i < 0 ? ~0ULL : (((unsigned long long)__float_as_uint(best) << 32) | (unsigned int)best_i);
+                best_key[qq] = best_i < 0 ? ~0ULL : pack_min_key(best, (unsigned int)best_i);
             }
         }
     }
@@ -329,41 +325,23 @@ __global__ void __launch_bounds__(kCertThreads) refine_cert_kernel(const float4 
     }
 }
 
-// exact rescan: work item = (query, producer); the producer (CTA c, column group g) saw, for the query's M tile m (counted
-// inside its GEMM launch), the N tiles n with n * stride = c - m (mod G) and of each the columns [g, g+1) * 256 / EG (tile schedule of
-// score_gemm.cu).  Unit = (item, k-th such N tile): one block computes the exact distances of its <= 256/EG rows and
-// folds the smallest (d^2 bits, row) into best_key[query] (atomicMin; d^2 >= 0 so the bits order like the value).
-// first N tile that CTA c processes for M tile m under the GEMM's schedule: smallest n with n * stride = c - m (mod G);
-// the others follow every G tiles (stride is coprime with G)
-__device__ __forceinline__ int producer_first_tile(int c, int m, int G, int stride) {
-    const int want = ((c - m % G) % G + G) % G, smod = stride % G;
-    int n0 = 0;
-    for (int x = 0; x != want; ++n0) {  // x = (n0 * stride) % G, stepped without a division
-        x += smod;
-        if (x >= G) x -= G;
-    }
-    return n0;
-}
-
+// exact rescan: work item = (query, producer); the producer (CTA c, column group g) saw, for the query's M tile, the N
+// tiles rescan_tile names and of each the columns [g, g+1) * 256 / EG.  Unit = (item, tile slot, 32-row slice): the
+// exact distances of its rows, the smallest (d^2 bits, row) folded into best_key[query] (atomicMin).  The first-pass
+// GEMM launches are single CTAs (certified mode runs the 1-term GEMM), checked by score_rescan.
 __global__ void __launch_bounds__(256) rescan_kernel(const int2 *__restrict__ work, const int *__restrict__ n_items_ptr,
                                                      const float *__restrict__ q, const float *__restrict__ bank, int dim,
-                                                     long long rows, int n_units, int cg, int EG, int nt, int chunk_tiles,
-                                                     int mt_total, int inv_full, int inv_last, int run_full,
-                                                     int run_last, unsigned long long *best_key,
+                                                     long long rows, GemmSched full, GemmSched last, int chunk_tiles,
+                                                     int mt_total, unsigned long long *best_key,
                                                      const int *__restrict__ fail_list, int *__restrict__ ctl, int P_img,
                                                      long long row_offset, float *__restrict__ min_val,
                                                      long long *__restrict__ min_idx, unsigned long long *s_key) {
     __shared__ int last_block;
     const int n_items = min(*n_items_ptr, kWorkCap);
-    // n_units scheduling units (CTAs, or CTA pairs when cg == 2) share the runs of N tiles of one M tile (pair); a chunk's
-    // schedule deals runs of `run` consecutive N tiles, so a producer's rows are runs_per runs of run tiles each.  Both
-    // chunk shapes are covered with the larger of the two unit counts (units beyond a producer's real tiles are empty).
-    const int run_max = max(run_full, run_last), run_min = min(run_full, run_last);
-    const int runs_per = ((nt + run_min - 1) / run_min + n_units - 1) / n_units;
-    const int tiles_per = runs_per * run_max;
+    const int tiles_per = producer_slots(full, last);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int cols = kScoreBN / EG;
-    // warp unit = (item, k-th tile of the producer, 32-row slice of the tile's column group, warp slot): four exact
+    const int cols = kScoreBN / kGemmEpiGroups;
+    // warp unit = (item, tile slot of the producer, 32-row slice of the tile's column group, warp slot): four exact
     // distances (rows r, r + 8, r + 16, r + 24) with all loads in flight together, one atomicMin per warp; no block barrier
     constexpr int kUnitRows = 32;
     const int units_per_tile = cols / kUnitRows;
@@ -377,20 +355,9 @@ __global__ void __launch_bounds__(256) rescan_kernel(const int2 *__restrict__ wo
         const int rem = (int)(u / n_items);
         const int kt = rem / units_per_tile, sub = rem % units_per_tile;
         const int2 w = work[item];
-        const int qi = w.x, c = w.y / EG, g = w.y % EG;
-        // the first-pass GEMM ran in chunks of chunk_tiles M tiles (the last one may be shorter), each with its own schedule
-        const int mtile = qi / kScoreBM, chunk = mtile / chunk_tiles;
-        const bool last = (chunk + 1) * chunk_tiles >= mt_total;
-        const int m_in = mtile - chunk * chunk_tiles;  // pair mode: CTA 2u + r handled the M tiles 2*mp + r of pair u
-        const int run = last ? run_last : run_full;
-        const int k = kt / run_max, t = kt % run_max;   // k-th run of this producer, t-th tile inside it
-        // first run that unit c / cg processes for M tile m_in / cg under the GEMM's schedule: the smallest j with
-        // j * stride = c - m (mod G); stride is coprime with G, so j = (c - m) * stride^-1 mod G (inverse from the host)
-        const int G = n_units;
-        const int want = (((c / cg) - (m_in / cg) % G) % G + G) % G;
-        const int jrun = (int)(((long long)want * (last ? inv_last : inv_full)) % G) + k * n_units;
-        const int n = t < run ? jrun * run + t : nt;
-        if (n < nt && (long long)jrun * run < nt) {
+        const int qi = w.x, c = w.y / kGemmEpiGroups, g = w.y % kGemmEpiGroups;
+        const int n = rescan_tile(full, last, chunk_tiles, mt_total, qi / kScoreBM, c, kt);
+        if (n < full.nt) {
             const long long r0 = (long long)n * kScoreBN + g * cols + sub * kUnitRows + wsub;
             if (r0 < rows) {
                 const long long rl = rows - 1;
@@ -401,7 +368,7 @@ __global__ void __launch_bounds__(256) rescan_kernel(const int2 *__restrict__ wo
                 unsigned long long key = ~0ULL;
 #pragma unroll
                 for (int kk4 = 0; kk4 < 4; ++kk4) {  // rows clamped to the last one repeat its key: harmless for a minimum
-                    const unsigned long long kk = ((unsigned long long)__float_as_uint(d[kk4]) << 32) | (unsigned int)min(r0 + 8 * kk4, rl);
+                    const unsigned long long kk = pack_min_key(d[kk4], (unsigned int)min(r0 + 8 * kk4, rl));
                     key = kk < key ? kk : key;
                 }
                 if (lane == 0) atomicMin(best_key + qi, key);
@@ -421,11 +388,10 @@ __global__ void __launch_bounds__(256) rescan_kernel(const int2 *__restrict__ wo
     for (int i = threadIdx.x; i < n_fin; i += blockDim.x) {
         const int qi = fail_list[i];
         const unsigned long long key = __ldcg(best_key + qi);
-        const float dv = sqrtf(__uint_as_float((unsigned int)(key >> 32)));
+        const float dv = sqrtf(key_value(key));
         min_val[qi] = dv;
-        min_idx[qi] = key == ~0ULL ? -1 : (long long)(key & 0xffffffffULL) + row_offset;
-        atomicMax(s_key + qi / P_img,
-                  ((unsigned long long)__float_as_uint(dv) << 32) | (0xffffffffu - (unsigned int)(qi % P_img)));
+        min_idx[qi] = key == ~0ULL ? -1 : key_row(key) + row_offset;
+        argmax_publish(s_key, qi, P_img, dv);
     }
 }
 
@@ -440,7 +406,7 @@ __global__ void __launch_bounds__(256) exact_scan_kernel(const float *__restrict
     unsigned long long key = ~0ULL;
     for (long long r = r0; r < r1; ++r) {
         const float d2 = warp_sqdist(q + (size_t)qi * dim, bank + (size_t)r * dim, dim >> 2, lane);
-        const unsigned long long kk = ((unsigned long long)__float_as_uint(d2) << 32) | (unsigned int)r;
+        const unsigned long long kk = pack_min_key(d2, (unsigned int)r);
         key = kk < key ? kk : key;
     }
     if (lane == 0 && key != ~0ULL) atomicMin(best_key + qi, key);
@@ -557,21 +523,13 @@ int score_refine(const ScoreCall &c, cudaStream_t st, int B, int P_img, int n_ca
     return CMDB_OK;
 }
 
-// x with (a * x) % m == 1 (a coprime with m; m = scheduling units of the GEMM, <= a few hundred); 0 for m == 1
-static int mod_inverse(int a, int m) {
-    a %= m;
-    for (int x = 0; x < m; ++x)
-        if ((a * x) % m == 1 % m) return x;
-    return 0;
-}
-
 static int score_certify(const ScoreCall &c, int B, int P_img, int n_cand) {
     const cmdb_bank *b = c.b;
     const Lane &s = *c.lane;
     const int P = B * P_img;
     cudaStream_t st = c.stream;
     CMDB_CUDA(cudaMemsetAsync(s.fail_ctl, 0, 8 * sizeof(int) + sizeof(unsigned long long) * B, st));  // control block + s_key
-    const float acc_model = (float)(b->dim / 16 + 1) * 17.f * 1.1920929e-7f;
+    const float acc_model = cert_acc_model(b->dim);
     if (b->timing == 2) CMDB_CUDA(cudaEventRecord(s.ev_dbg[0], st));
     // queries per block: 8 = one query per warp in phase 3 and 10 list entries per thread held in registers (measured best)
     constexpr int QB = 8;
@@ -590,16 +548,10 @@ static int score_rescan(const ScoreCall &c, int P_img) {
     cudaStream_t st = c.stream;
     CMDB_CUDA(cudaGetLastError());
     // tier 1: few uncertified (query, producer) pairs -> exact rescan of those producers' rows, along the first-pass schedule
-    const int cg = c.pair ? 2 : 1, n_units = b->num_sms / cg, EG = kGemmEpiGroups;
-    const int last_tiles = c.mt_total - (c.mt_total - 1) / c.chunk_tiles * c.chunk_tiles;
-    const int nt = (int)(b->fin_rows_pad / kScoreBN);
-    rescan_kernel<<<b->num_sms * 8, 256, 0, st>>>(s.work_list, s.fail_ctl + 3, c.slot->q_f32, b->data, b->dim, b->fin_rows, n_units, cg,
-                                                  EG, nt, c.chunk_tiles, c.mt_total,
-                                                  mod_inverse(score_tile_stride((c.chunk_tiles + cg - 1) / cg, n_units), n_units),
-                                                  mod_inverse(score_tile_stride((last_tiles + cg - 1) / cg, n_units), n_units),
-                                                  score_gemm_run(nt, (c.chunk_tiles + cg - 1) / cg, n_units),
-                                                  score_gemm_run(nt, (last_tiles + cg - 1) / cg, n_units), s.best_key,
-                                                  s.fail_list, s.fail_ctl, P_img, b->row_offset, c.min_val, c.min_idx, s.s_key);
+    CMDB_REQUIRE(!c.first.pair && !c.last.pair, CMDB_ERR_UNSUPPORTED, "scoring: the exact rescan cannot walk a CTA-pair GEMM schedule");
+    rescan_kernel<<<b->num_sms * 8, 256, 0, st>>>(s.work_list, s.fail_ctl + 3, c.slot->q_f32, b->data, b->dim, b->fin_rows, c.first,
+                                                  c.last, c.chunk_tiles, c.mt_total, s.best_key, s.fail_list, s.fail_ctl, P_img,
+                                                  b->row_offset, c.min_val, c.min_idx, s.s_key);
     CMDB_CUDA(cudaGetLastError());
     if (b->timing == 2) CMDB_CUDA(cudaEventRecord(s.ev_dbg[2], st));
     return CMDB_OK;
@@ -689,8 +641,9 @@ int score_local_min(ScoreCall &c, const float *src, int src_is_device, int B, in
         CMDB_CHECK(score_query_prep(c, st, rows, false, row0));
         if (k == 0) CMDB_CHECK(score_mark(c, ev_gemm, st));
         CMDB_CHECK(score_gemm_candidates(c, st, rows, mode == 3 ? 3 : 1, false, &sched, row0));
-        if (k == 0) c.pair = sched.pair;
+        if (k == 0) c.first = sched;
     }
+    c.last = sched;
     n_cand = sched.producers;
     CMDB_CHECK(score_mark(c, ev_refine, st));
     if (mode != 0) return score_refine(c, st, B, P_img, n_cand, false);
@@ -733,7 +686,7 @@ __global__ void __launch_bounds__(256) select_kernel(const unsigned long long *s
                                                      TailResult *res) {
     const int b = blockIdx.x;
     const unsigned long long key = s_key[b];
-    const int s_idx = (int)(0xffffffffu - (unsigned int)(key & 0xffffffffu));
+    const int s_idx = argmax_query(key);
     const long long g = min_idx[(size_t)b * P_img + s_idx];
     for (int c = threadIdx.x; c < dim; c += blockDim.x) {
         m_test[(size_t)b * dim + c] = q[((size_t)b * P_img + s_idx) * dim + c];
@@ -742,7 +695,7 @@ __global__ void __launch_bounds__(256) select_kernel(const unsigned long long *s
     }
     if (threadIdx.x == 0) {
         res[b].s_idx = s_idx;
-        res[b].s_star = __uint_as_float((unsigned int)(key >> 32));
+        res[b].s_star = key_value(key);
         res[b].m_star_row = g;
     }
 }
@@ -781,6 +734,16 @@ __device__ __forceinline__ void warp_top3(unsigned long long (&t)[3], unsigned l
     }
 }
 
+// m_star_knn, w and s of an image (features.py:275-290) from s* and the distances to m_star's two nearest other rows
+__device__ __forceinline__ void reweight_final(TailResult *res, float s_star, float knn0, float knn1, int dim) {
+    const float Dn = sqrtf((float)dim);  // torch.sqrt(torch.tensor(patch.shape[1]))  (features.py:285)
+    const float den = expf(knn0 / Dn) + expf(knn1 / Dn);
+    const float w = 1.f - expf(s_star / Dn) / den;  // features.py:287
+    res->w = w;
+    res->s = w * s_star;  // features.py:290
+    res->knn0 = knn0, res->knn1 = knn1;
+}
+
 struct ReweightParams {
     const float *bank;               // [rows, dim] float32 (local shard)
     long long rows, row_offset;
@@ -809,7 +772,7 @@ __global__ void __launch_bounds__(256) reweight_kernel(ReweightParams p) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     if (threadIdx.x < B) {
         const unsigned long long skey = p.s_key[threadIdx.x];
-        const int s_idx = (int)(0xffffffffu - (unsigned int)(skey & 0xffffffffu));
+        const int s_idx = argmax_query(skey);
         s_idx_sh[threadIdx.x] = s_idx;
         g_sh[threadIdx.x] = p.min_idx[(size_t)threadIdx.x * p.P_img + s_idx];
     }
@@ -899,29 +862,22 @@ __global__ void __launch_bounds__(256) reweight_kernel(ReweightParams p) {
         const unsigned long long *src = p.block_keys + (size_t)b * gridDim.x * 3;
         for (int i = lane; i < (int)gridDim.x * 3; i += 32) top3_insert(t, __ldcg(src + i));
         warp_top3(t, f);
-        const unsigned long long skey = p.s_key[b];
-        const float s_star = __uint_as_float((unsigned int)(skey >> 32));
+        const float s_star = key_value(p.s_key[b]);
         const int s_idx = s_idx_sh[b];
         float knn[2] = {NAN, NAN};  // features.py:275-283: m_star_knn = ||m_test - bank[nn_idx[1:]]||, m_test = patch[s_idx]
 #pragma unroll
         for (int k = 0; k < 2; ++k)
             if (f[1 + k] != ~0ULL)
                 knn[k] = sqrtf(warp_sqdist(p.q + ((size_t)b * p.P_img + s_idx) * dim,
-                                           p.bank + (size_t)((long long)(f[1 + k] & 0xffffffffULL) - p.row_offset) * dim,
-                                           dim4, lane));
+                                           p.bank + (size_t)(key_row(f[1 + k]) - p.row_offset) * dim, dim4, lane));
         if (lane == 0) {
             TailResult *res = p.res + b;
             p.top3[b * 3 + 0] = f[0], p.top3[b * 3 + 1] = f[1], p.top3[b * 3 + 2] = f[2];
             res->s_idx = s_idx;
             res->s_star = s_star;
             res->m_star_row = g_sh[b];
-            for (int k = 0; k < 3; ++k) res->nn_idx[k] = f[k] == ~0ULL ? -1 : (long long)(f[k] & 0xffffffffULL);
-            const float Dn = sqrtf((float)dim);  // torch.sqrt(torch.tensor(patch.shape[1]))  (features.py:285)
-            const float den = expf(knn[0] / Dn) + expf(knn[1] / Dn);
-            const float w = 1.f - expf(s_star / Dn) / den;  // features.py:287
-            res->w = w;
-            res->s = w * s_star;  // features.py:290
-            res->knn0 = knn[0], res->knn1 = knn[1];
+            for (int k = 0; k < 3; ++k) res->nn_idx[k] = f[k] == ~0ULL ? -1 : key_row(f[k]);
+            reweight_final(res, s_star, knn[0], knn[1], dim);
         }
     }
 }
@@ -939,17 +895,16 @@ struct ReweightCertParams {
     const float4 *cand;
     int n_cand, cand_stride;
     const float *m_star;             // [B, dim]
-    const float *m_test;             // [B, dim] (fused final only)
+    const float *m_test;             // [B, dim] (with res only)
     const float *bank;
     long long rows, row_offset;
     int dim;
     const float *q_norm, *q_eps;     // of the m_star rows (q_split_kernel)
     float bmax, eb_max, acc_model;
-    int n_units, cg, EG, stride, nt, run; // tile schedule of the GEMM launch: units = CTAs or CTA pairs, run = N tiles per visit
+    GemmSched sched;                 // of the GEMM launch (single CTAs)
     const unsigned long long *s_key;
     unsigned long long *top3;
-    TailResult *res;
-    int fuse_final;
+    TailResult *res;                 // nullptr: only the keys (table build)
 };
 
 __device__ __forceinline__ unsigned int float_order_bits(float v) {  // monotone float -> uint (handles negatives)
@@ -987,19 +942,9 @@ __global__ void __launch_bounds__(256) reweight_cert_kernel(ReweightCertParams p
         for (int w = 0; w < 8; ++w)
             for (int k = 0; k < 3; ++k) top3_insert(g3, wkeys[w][k]);
         float thr = INFINITY;  // fewer than three real rows: everything is a candidate
-        if (g3[2] != ~0ULL) {
-            const float v3 = float_from_order_bits((unsigned int)(g3[2] >> 32));
-            const float qn = p.q_norm[b], qe = p.q_eps[b];
-            const float bh = __fadd_ru(p.bmax, p.eb_max);
-            float E = __fmul_ru(qe, bh);
-            E = __fmaf_ru(qn, p.eb_max, E);
-            E = __fmaf_ru(__fmul_ru(p.acc_model, __fadd_ru(qn, qe)), bh, E);
-            E = __fmul_ru(2.f, E);
-            const float span = __fadd_ru(qn, p.bmax);
-            E = __fmaf_ru(__fmul_ru((float)(dim + 16) * 5.9604645e-8f, span), span, E);
-            thr = __fadd_ru(v3, __fmul_ru(2.0625f, E));
-            if (!(thr == thr)) thr = INFINITY;  // NaN: certify nothing, scan everything
-        }
+        if (g3[2] != ~0ULL)
+            thr = cert_threshold(float_from_order_bits((unsigned int)(g3[2] >> 32)), p.q_norm[b], p.q_eps[b], p.bmax, p.eb_max,
+                                 p.acc_model, dim);
         thr_sh = thr;
     }
     __syncthreads();
@@ -1022,19 +967,14 @@ __global__ void __launch_bounds__(256) reweight_cert_kernel(ReweightCertParams p
     };
     const int n_rows = n_rows_sh, n_bad = n_bad_sh;
     for (int i = warp; i < n_rows; i += 8) visit(cand_rows[i]);
-    const int cols = kScoreBN / p.EG;
-    const int nruns = (p.nt + p.run - 1) / p.run, runs_per = (nruns + p.n_units - 1) / p.n_units;
+    const int cols = kScoreBN / kGemmEpiGroups, slots = producer_slots(p.sched, p.sched);
     for (int i = 0; i < n_bad; ++i) {
-        const int c = bad_prod[i] / p.EG, g = bad_prod[i] % p.EG;
-        // M tile of this query row inside the GEMM launch (0 for the re-weighting of a batch; the table build has many);
-        // the producer visited runs j0, j0 + n_units, ... of p.run consecutive N tiles each
-        const int j0 = producer_first_tile(c / p.cg, (b / kScoreBM) / p.cg, p.n_units, p.stride);
-        for (int j = warp; j < runs_per * p.run * cols; j += 8) {
-            const int k = j / (p.run * cols), t = (j / cols) % p.run;
-            const int jrun = j0 + k * p.n_units;
-            const int n = jrun * p.run + t;
+        const int c = bad_prod[i] / kGemmEpiGroups, g = bad_prod[i] % kGemmEpiGroups;
+        // the query row's M tile inside the GEMM launch: 0 for the re-weighting of a batch, the table build has many
+        for (int j = warp; j < slots * cols; j += 8) {
+            const int n = producer_tile(p.sched, p.sched.run, c, b / kScoreBM, j / cols);
             const long long r = (long long)n * kScoreBN + g * cols + j % cols;
-            if (jrun < nruns && n < p.nt && r < p.rows) visit(r);
+            if (n < p.sched.nt && r < p.rows) visit(r);
         }
     }
     if (lane == 0) wkeys[warp][0] = w3[0], wkeys[warp][1] = w3[1], wkeys[warp][2] = w3[2];
@@ -1048,27 +988,20 @@ __global__ void __launch_bounds__(256) reweight_cert_kernel(ReweightCertParams p
         }
     float s_star = 0.f;
     float knn[2] = {NAN, NAN};
-    if (p.fuse_final) {  // features.py:275-283: m_star_knn = ||m_test - bank[nn_idx[1:]]||, m_test = patch[s_idx]
-        s_star = __uint_as_float((unsigned int)(p.s_key[b] >> 32));
+    if (p.res) {  // features.py:275-283: m_star_knn = ||m_test - bank[nn_idx[1:]]||, m_test = patch[s_idx]
+        s_star = key_value(p.s_key[b]);
 #pragma unroll
         for (int k = 0; k < 2; ++k)
             if (f[1 + k] != ~0ULL)
                 knn[k] = sqrtf(warp_sqdist(p.m_test + (size_t)b * dim,
-                                           p.bank + (size_t)((long long)(f[1 + k] & 0xffffffffULL) - p.row_offset) * dim, dim4, lane));
+                                           p.bank + (size_t)(key_row(f[1 + k]) - p.row_offset) * dim, dim4, lane));
     }
     if (lane == 0) {
         p.top3[(size_t)b * 3 + 0] = f[0], p.top3[(size_t)b * 3 + 1] = f[1], p.top3[(size_t)b * 3 + 2] = f[2];
         if (!p.res) return;  // table build: only the keys
         TailResult *res = p.res + b;
-        for (int k = 0; k < 3; ++k) res->nn_idx[k] = f[k] == ~0ULL ? -1 : (long long)(f[k] & 0xffffffffULL);
-        if (p.fuse_final) {
-            const float Dn = sqrtf((float)dim);  // torch.sqrt(torch.tensor(patch.shape[1]))  (features.py:285)
-            const float den = expf(knn[0] / Dn) + expf(knn[1] / Dn);
-            const float w = 1.f - expf(s_star / Dn) / den;  // features.py:287
-            res->w = w;
-            res->s = w * s_star;  // features.py:290
-            res->knn0 = knn[0], res->knn1 = knn[1];
-        }
+        for (int k = 0; k < 3; ++k) res->nn_idx[k] = f[k] == ~0ULL ? -1 : key_row(f[k]);
+        reweight_final(res, s_star, knn[0], knn[1], dim);
     }
 }
 
@@ -1085,21 +1018,16 @@ __global__ void __launch_bounds__(64) reweight_lookup_kernel(const unsigned long
     const unsigned long long *keys3 = table + (size_t)res->m_star_row * 3;
     const unsigned long long key = keys3[1 + warp];
     float v = NAN;
-    if (key != ~0ULL) v = sqrtf(warp_sqdist(m_test + (size_t)b * dim, bank + (size_t)(key & 0xffffffffULL) * dim, dim >> 2, lane));
+    if (key != ~0ULL) v = sqrtf(warp_sqdist(m_test + (size_t)b * dim, bank + (size_t)key_row(key) * dim, dim >> 2, lane));
     if (lane == 0) knn[warp] = v;
     __syncthreads();
     if (threadIdx.x == 0) {
-        const float s_star = __uint_as_float((unsigned int)(s_key[b] >> 32));
+        const float s_star = key_value(s_key[b]);
         for (int k = 0; k < 3; ++k) {
             top3[b * 3 + k] = keys3[k];
-            res->nn_idx[k] = keys3[k] == ~0ULL ? -1 : (long long)(keys3[k] & 0xffffffffULL);
+            res->nn_idx[k] = keys3[k] == ~0ULL ? -1 : key_row(keys3[k]);
         }
-        const float Dn = sqrtf((float)dim);  // torch.sqrt(torch.tensor(patch.shape[1]))  (features.py:285)
-        const float den = expf(knn[0] / Dn) + expf(knn[1] / Dn);
-        const float w = 1.f - expf(s_star / Dn) / den;  // features.py:287
-        res->w = w;
-        res->s = w * s_star;  // features.py:290
-        res->knn0 = knn[0], res->knn1 = knn[1];
+        reweight_final(res, s_star, knn[0], knn[1], dim);
     }
 }
 
@@ -1115,14 +1043,14 @@ __global__ void __launch_bounds__(64) shard_lookup_kernel(const unsigned long lo
     TailResult *res = res_all + b;
     const unsigned long long *keys3 = table + (size_t)res->m_star_row * 3;
     const unsigned long long key = keys3[1 + warp];
-    const long long l = (long long)(key & 0xffffffffULL) - row_offset;
+    const long long l = key_row(key) - row_offset;
     float v = 0.f;
     if (key != ~0ULL && l >= 0 && l < rows) v = warp_sqdist(m_test + (size_t)b * dim, bank + (size_t)l * dim, dim >> 2, lane);
     if (lane == 0) contrib[b * 2 + warp] = v;
     if (threadIdx.x == 0)
         for (int k = 0; k < 3; ++k) {
             top3[b * 3 + k] = keys3[k];
-            res->nn_idx[k] = keys3[k] == ~0ULL ? -1 : (long long)(keys3[k] & 0xffffffffULL);
+            res->nn_idx[k] = keys3[k] == ~0ULL ? -1 : key_row(keys3[k]);
         }
 }
 
@@ -1134,13 +1062,7 @@ __global__ void shard_final_kernel(const unsigned long long *__restrict__ top3, 
     TailResult *res = res_all + b;
     float knn[2];
     for (int k = 0; k < 2; ++k) knn[k] = top3[b * 3 + 1 + k] == ~0ULL ? NAN : sqrtf(d2_sum[b * 2 + k]);
-    const float Dn = sqrtf((float)dim);
-    const float s_star = res->s_star;
-    const float den = expf(knn[0] / Dn) + expf(knn[1] / Dn);
-    const float w = 1.f - expf(s_star / Dn) / den;
-    res->w = w;
-    res->s = w * s_star;
-    res->knn0 = knn[0], res->knn1 = knn[1];
+    reweight_final(res, res->s_star, knn[0], knn[1], dim);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -1168,9 +1090,7 @@ __global__ void __launch_bounds__(256) shard_push_keys_kernel(const float *__res
                                                               int n, PeerPtrs peers, int world, int rank, size_t keys_off,
                                                               size_t flag_off, unsigned long long epoch, unsigned int *ctr) {
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        const long long g = min_idx[i];
-        const long long key = g < 0 ? 0x7fffffffffffffffLL
-                                    : (long long)(((unsigned long long)__float_as_uint(min_val[i]) << 32) | (unsigned long long)g);
+        const long long key = exchange_key(min_val[i], min_idx[i]);
         for (int r = 0; r < world; ++r)
             reinterpret_cast<long long *>(peers.p[r] + keys_off)[(size_t)rank * kShardKeysCap + i] = key;
     }
@@ -1220,10 +1140,10 @@ __global__ void __launch_bounds__(256) shard_reduce_keys_kernel(const unsigned c
             const long long v = __ldcg(keys + (size_t)r * kShardKeysCap + i);
             k = v < k ? v : k;
         }
-        const float v = __uint_as_float((unsigned int)((unsigned long long)k >> 32));
+        const float v = key_value((unsigned long long)k);
         min_val[i] = v;
-        min_idx[i] = (long long)((unsigned long long)k & 0xffffffffULL);
-        atomicMax(s_key + i / P_img, ((unsigned long long)__float_as_uint(v) << 32) | (0xffffffffu - (unsigned int)(i % P_img)));
+        min_idx[i] = key_row((unsigned long long)k);
+        argmax_publish(s_key, i, P_img, v);
     }
 }
 
@@ -1452,9 +1372,29 @@ int score_select(const ScoreCall &c, int B, int P_img, bool local_m_star) {
     return CMDB_OK;
 }
 
+// reweight_cert_kernel over the n m_star rows of the GEMM launch `sched` on the call's lane, one block per row: the three
+// nearest rows as keys into top3 and, with res, the final re-weighting (m_test, s_key) into res
+static int launch_reweight_cert(const ScoreCall &c, const GemmSched &sched, int n, const float *m_star, long long row_offset,
+                                unsigned long long *top3, TailResult *res) {
+    const cmdb_bank *b = c.b;
+    const Lane &s = *c.lane;
+    CMDB_REQUIRE(!sched.pair, CMDB_ERR_UNSUPPORTED, "scoring: the re-weighting certificate cannot walk a CTA-pair GEMM schedule");
+    CMDB_REQUIRE(sched.producers <= 320, CMDB_ERR_UNSUPPORTED, "scoring: %d GEMM producers exceed reweight_cert_kernel's limit",
+                 sched.producers);
+    ReweightCertParams p{};
+    p.cand = s.cand, p.n_cand = sched.producers, p.cand_stride = b->layout.cap_p;
+    p.m_star = m_star, p.m_test = res ? s.m_test : nullptr, p.bank = b->data, p.rows = b->fin_rows, p.row_offset = row_offset;
+    p.dim = b->dim, p.q_norm = s.q_norm, p.q_eps = s.q_eps;
+    p.bmax = b->cert_bmax, p.eb_max = b->cert_eb_max, p.acc_model = cert_acc_model(b->dim);
+    p.sched = sched;
+    p.s_key = res ? s.s_key : nullptr, p.top3 = top3, p.res = res;
+    reweight_cert_kernel<<<n, 256, 0, c.stream>>>(p);
+    CMDB_CUDA(cudaGetLastError());
+    return CMDB_OK;
+}
+
 // tensor-core variant: select -> fp16 split of the m_star rows -> hi.hi GEMM with one M tile -> reweight_cert_kernel
 static int score_reweight_tensor(const ScoreCall &c, int B, int P_img) {
-    const cmdb_bank *b = c.b;
     const Lane &s = *c.lane;
     CMDB_CHECK(score_select(c, B, P_img, true));  // m_test, m_star, s*, s_idx, m_star_row
     // the min/argmin phase is complete: its query operand buffers and candidate lists are free again
@@ -1462,20 +1402,7 @@ static int score_reweight_tensor(const ScoreCall &c, int B, int P_img) {
     CMDB_CUDA(cudaGetLastError());
     GemmSched sched{};
     CMDB_CHECK(score_gemm_candidates(c, c.stream, B, 1, false, &sched));
-    ReweightCertParams p{};
-    p.cand = s.cand, p.n_cand = sched.producers, p.cand_stride = b->layout.cap_p;
-    p.m_star = s.m_star, p.m_test = s.m_test, p.bank = b->data, p.rows = b->fin_rows, p.row_offset = b->row_offset;
-    p.dim = b->dim, p.q_norm = s.q_norm, p.q_eps = s.q_eps;
-    p.bmax = b->cert_bmax, p.eb_max = b->cert_eb_max, p.acc_model = (float)(b->dim / 16 + 1) * 17.f * 1.1920929e-7f;
-    p.cg = sched.pair ? 2 : 1, p.n_units = b->num_sms / p.cg, p.EG = kGemmEpiGroups;
-    p.stride = score_tile_stride(1, p.n_units);
-    p.nt = (int)(b->fin_rows_pad / kScoreBN);
-    p.run = sched.run;
-    p.s_key = s.s_key, p.top3 = s.top3, p.res = c.tail, p.fuse_final = 1;
-    CMDB_REQUIRE(p.n_cand <= 320, CMDB_ERR_UNSUPPORTED, "scoring: %d GEMM producers exceed reweight_cert_kernel's limit", p.n_cand);
-    reweight_cert_kernel<<<B, 256, 0, c.stream>>>(p);
-    CMDB_CUDA(cudaGetLastError());
-    return CMDB_OK;
+    return launch_reweight_cert(c, sched, B, s.m_star, c.b->row_offset, s.top3, c.tail);
 }
 
 // SURVEY 8f-1: three nearest bank rows of every bank row.  The bank is its own query set: chunks of rows go through the
@@ -1486,7 +1413,6 @@ int score_build_knn_table(cmdb_bank *b, long long row_first, long long row_count
     const size_t map_stride = b->layout.map_stride;
     CMDB_CHECK(score_scratch_alloc(b, 32, chunk / 32, map_stride ? (int)lround(sqrt((double)map_stride)) : 224));
     const ScoreCall c = score_call(b, 0, 0);   // lane 0; the result slot is not used
-    const Lane &s = *c.lane;
     cudaStream_t st = c.stream;
     if (!b->knn_table || b->knn_rows != b->fin_rows) {
         cudaFree(b->knn_table);
@@ -1503,20 +1429,7 @@ int score_build_knn_table(cmdb_bank *b, long long row_first, long long row_count
         CMDB_CUDA(cudaGetLastError());
         GemmSched sched{};
         CMDB_CHECK(score_gemm_candidates(c, st, n, 1, false, &sched));
-        ReweightCertParams p{};
-        p.cand = s.cand, p.n_cand = sched.producers, p.cand_stride = b->layout.cap_p;
-        p.m_star = rows, p.m_test = nullptr, p.bank = b->data, p.rows = b->fin_rows, p.row_offset = 0;
-        p.dim = b->dim, p.q_norm = s.q_norm, p.q_eps = s.q_eps;
-        p.bmax = b->cert_bmax, p.eb_max = b->cert_eb_max, p.acc_model = (float)(b->dim / 16 + 1) * 17.f * 1.1920929e-7f;
-        p.cg = sched.pair ? 2 : 1, p.n_units = b->num_sms / p.cg, p.EG = kGemmEpiGroups;
-        const int mt = (n + kScoreBM - 1) / kScoreBM;
-        p.stride = score_tile_stride((mt + p.cg - 1) / p.cg, p.n_units);
-        p.nt = (int)(b->fin_rows_pad / kScoreBN);
-        p.run = sched.run;
-        p.s_key = nullptr, p.top3 = b->knn_table + (size_t)r0 * 3, p.res = nullptr, p.fuse_final = 0;
-        CMDB_REQUIRE(p.n_cand <= 320, CMDB_ERR_UNSUPPORTED, "scoring: %d GEMM producers exceed reweight_cert_kernel's limit", p.n_cand);
-        reweight_cert_kernel<<<n, 256, 0, st>>>(p);
-        CMDB_CUDA(cudaGetLastError());
+        CMDB_CHECK(launch_reweight_cert(c, sched, n, rows, 0, b->knn_table + (size_t)r0 * 3, nullptr));
     }
     CMDB_CUDA(cudaStreamSynchronize(st));
     return CMDB_OK;

@@ -1,7 +1,9 @@
-"""CPU suite: the distance GEMM's tile schedule with runs of N tiles, restated on the host, and the two places that
-rebuild "the rows producer (CTA c, column group g) saw for M tile m" from it -- the exact rescan (rescan_kernel, closed
-form) and the re-weighting certificate (reweight_cert_kernel, first-run walk) -- checked against it for the launch shapes
-of large banks.  tests/test_gpu_schedule.py checks the same restatement against the candidate lists the GPU writes."""
+"""CPU suite: the distance GEMM's tile schedule with runs of N tiles, restated on the host, and the library's one
+enumeration of "the rows producer (CTA c, column group g) saw for M tile m", which the exact rescan (rescan_kernel) and
+the re-weighting certificate (reweight_cert_kernel) share -- checked against it for the launch shapes of large banks
+through the host-only hook cmdb_debug_producer_tiles.  tests/test_gpu_schedule.py checks the same restatement against
+the candidate lists the GPU writes."""
+import ctypes
 from math import gcd
 
 import numpy as np
@@ -100,63 +102,22 @@ class Launch:
         return self.owner[r // BN // self.run, m]
 
 
-def mod_inverse(a, m):
-    a %= m
-    for x in range(m):
-        if (a * x) % m == 1 % m:
-            return x
-    return 0
+# ---- the library's enumeration ----------------------------------------------------------------------------------------
+class ProducerTiles:
+    """cmdb_debug_producer_tiles: the N tiles the exact rescan visits for (query in M tile `mtile` of a batch whose
+    first-pass GEMM ran in launches of chunk_tiles out of mt_total M tiles, CTA c), from the schedules the library records
+    for the full and the last chunk launch, in slot order -- so a slot bound that misses part of a producer shows as
+    missing tiles.  A single chunk (chunk_tiles == mt_total) is reweight_cert_kernel's walk over a launch of that size."""
 
+    def __init__(self, G=G_B200):
+        from cmdiad_b200 import _lib as L
+        self.L, self.lib, self.G = L, L.load(), G
+        self.buf, self.n = (ctypes.c_int32 * 65536)(), ctypes.c_int()
 
-# ---- the two enumerations, transcribed from the kernels ---------------------------------------------------------------
-def rescan_tiles(c, mtile, nt, chunk_tiles, mt_total, G):
-    """rescan_kernel's tiles of work item (query in M tile `mtile` of the batch, CTA c) for cg == 1; the host arguments as
-    score_rescan computes them"""
-    last_tiles = mt_total - (mt_total - 1) // chunk_tiles * chunk_tiles
-    inv_full, inv_last = mod_inverse(tile_stride(chunk_tiles, G), G), mod_inverse(tile_stride(last_tiles, G), G)
-    run_full, run_last = gemm_run(nt, chunk_tiles, G), gemm_run(nt, last_tiles, G)
-    run_max, run_min = max(run_full, run_last), min(run_full, run_last)
-    runs_per = ((nt + run_min - 1) // run_min + G - 1) // G
-    tiles_per = runs_per * run_max
-    chunk = mtile // chunk_tiles
-    last = (chunk + 1) * chunk_tiles >= mt_total
-    m_in = mtile - chunk * chunk_tiles
-    run = run_last if last else run_full
-    out = []
-    for kt in range(tiles_per):
-        k, t = kt // run_max, kt % run_max
-        want = ((c - m_in % G) % G + G) % G
-        jrun = (want * (inv_last if last else inv_full)) % G + k * G
-        n = jrun * run + t if t < run else nt
-        if n < nt and jrun * run < nt:
-            out.append(n)
-    return sorted(out)
-
-
-def producer_first_tile(c, m, G, stride):
-    want, smod = ((c - m % G) % G + G) % G, stride % G
-    n0, x = 0, 0
-    while x != want:
-        x += smod
-        if x >= G:
-            x -= G
-        n0 += 1
-    return n0
-
-
-def reweight_cert_tiles(c, m, nt, run, G, stride):
-    """reweight_cert_kernel's walk over a bad producer (CTA c) of a query row in M tile m (cg == 1), at tile level"""
-    nruns = (nt + run - 1) // run
-    runs_per = (nruns + G - 1) // G
-    j0 = producer_first_tile(c, m, G, stride)
-    out = []
-    for k in range(runs_per):
-        for t in range(run):
-            jrun = j0 + k * G
-            n = jrun * run + t
-            if jrun < nruns and n < nt:
-                out.append(n)
-    return out
+    def __call__(self, c, mtile, nt, chunk_tiles, mt_total):
+        self.L.check(self.lib.cmdb_debug_producer_tiles(self.G, nt, chunk_tiles, mt_total, mtile, c, self.buf,
+                                                        len(self.buf), ctypes.byref(self.n)))
+        return self.buf[:self.n.value]
 
 
 # ---- shapes -----------------------------------------------------------------------------------------------------------
@@ -229,10 +190,11 @@ def test_tile_schedule_with_runs_partitions_the_bank():
                 assert all(len(set(la.owner[:, m])) == la.G for m in sorted({0, mt - 1}))
 
 
-def test_rescan_enumeration_equals_the_gemm_schedule():
-    """rescan_kernel's closed form (stride inverse, run_full / run_last, runs_per / tiles_per sized from run_min /
-    run_max) names exactly the N tiles the GEMM's iterator gave each producer, for every producer and every M tile of
-    every chunk, full and last"""
+def test_rescan_enumeration_equals_the_gemm_schedule(built):
+    """the rescan's closed form (stride inverse, run_full / run_last, tile slots sized from run_min / run_max) names
+    exactly the N tiles the GEMM's iterator gave each producer, each once, for every producer and every M tile of every
+    chunk, full and last"""
+    rescan_tiles = ProducerTiles()
     n_diff_runs = 0
     for rows in ROWS:
         nt = (rows + BN - 1) // BN
@@ -244,17 +206,18 @@ def test_rescan_enumeration_equals_the_gemm_schedule():
                 la = launches[mt]
                 for m in range(mt):
                     for c in range(la.G):
-                        assert rescan_tiles(c, first + m, nt, ct, mt_total, la.G) == la.tiles(c, m), (rows, what, first, m, c)
+                        assert sorted(rescan_tiles(c, first + m, nt, ct, mt_total)) == la.tiles(c, m), (rows, what, first, m, c)
     assert n_diff_runs >= 6   # run_full != run_last is exercised
 
 
-def test_reweight_certificate_walk_equals_the_gemm_schedule():
+def test_reweight_certificate_walk_equals_the_gemm_schedule(built):
     """reweight_cert_kernel's bad-producer walk (first run, then every G runs, `run` tiles each) names exactly the GEMM
-    iterator's tiles: table-build launches (full and ragged last chunk, chunks starting anywhere) and the one-M-tile
-    re-weighting launch"""
+    iterator's tiles, in order: table-build launches (full and ragged last chunk, chunks starting anywhere) and the
+    one-M-tile re-weighting launch"""
+    producer_tiles = ProducerTiles()
     for rows, mts in _launch_shapes():
         for mt in mts:
             la = Launch(rows, mt)
             for m in sorted({0, 1 % mt, mt // 2, mt - 1}):
                 for c in range(la.G):
-                    assert reweight_cert_tiles(c, m, la.nt, la.run, la.G, la.stride) == la.tiles(c, m), (rows, mt, m, c)
+                    assert producer_tiles(c, m, la.nt, mt, mt) == la.tiles(c, m), (rows, mt, m, c)
