@@ -326,7 +326,7 @@ static int submit_sub_batch(ScoreCall &c, const float *src, int is_device, int b
     CMDB_CUDA(cudaMemcpyAsync(s.out_block_host, s.out_block, L.off_min_val, cudaMemcpyDeviceToHost, b->d2h_stream));
     CMDB_CHECK(publish_call(c, bc, P, out_hw, want, host_maps, 0, 1));
     CMDB_CHECK(score_mark(c, CMDB_T_COUNT, b->d2h_stream));
-    if (b->timing == 1) b->ev_valid = true;  // only batches record the stage events, sharded rounds do not
+    if (b->timing) b->ev_valid = true;  // only batches record the stage events, sharded rounds do not
     return CMDB_OK;
 }
 
@@ -579,9 +579,8 @@ int cmdb_debug_exact_min(cmdb_bank *b, const float *patch_host, int P, float *mi
     if (e == cudaSuccess) e = cudaMalloc(&keys, sizeof(unsigned long long) * (size_t)P);
     cudaStream_t st = b->handle_stream();
     if (e == cudaSuccess) e = cudaMemcpyAsync(q, patch_host, sizeof(float) * (size_t)P * b->dim, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaMemsetAsync(keys, 0xff, sizeof(unsigned long long) * (size_t)P, st);
     int rc = CMDB_OK;
-    if (e == cudaSuccess) rc = score_exact_scan(b, q, P, keys);
+    if (e == cudaSuccess) rc = score_exact_scan(b, st, q, P, keys);
     if (e == cudaSuccess && rc == CMDB_OK) e = cudaMemcpyAsync(h.data(), keys, sizeof(unsigned long long) * (size_t)P, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess && rc == CMDB_OK) e = cudaStreamSynchronize(st);
     cudaFree(q), cudaFree(keys);
@@ -598,25 +597,6 @@ int cmdb_debug_exact_min(cmdb_bank *b, const float *patch_host, int P, float *mi
 }
 
 // host-only test hooks (not in the public header): the GEMM's tile-schedule stride and the fallback-tier rule
-// CMDB_OPT_TIMING = 2: milliseconds since the time base of every stage mark of the last batch on each lane
-// (out: float [2][CMDB_T_COUNT + 1 + 4]: the stage marks, then the four marks inside the refine stage); all submitted
-// batches must have been waited for
-int cmdb_debug_lane_timeline(cmdb_bank *b, float *out) {
-    CMDB_REQUIRE(b && out && b->timing == 2 && b->ev_base, CMDB_ERR_STATE, "cmdb_debug_lane_timeline: set CMDB_OPT_TIMING = 2 first");
-    CMDB_CUDA(cudaSetDevice(b->device));
-    CMDB_CUDA(cudaDeviceSynchronize());
-    constexpr int kN = CMDB_T_COUNT + 1 + 4;
-    for (int l = 0; l < 2; ++l)
-        for (int i = 0; i < kN; ++i) {
-            cudaEvent_t e = i <= CMDB_T_COUNT ? b->lane[l].ev_tl[i] : b->lane[l].ev_dbg[i - CMDB_T_COUNT - 1];
-            if (cudaEventElapsedTime(out + l * kN + i, b->ev_base, e) != cudaSuccess) {
-                (void)cudaGetLastError();
-                out[l * kN + i] = -1.f;
-            }
-        }
-    return CMDB_OK;
-}
-
 int cmdb_debug_tile_stride(int mt, int G) { return tile_stride(mt, G); }
 
 // host-only test hook (not in the public header): the N tiles the exact rescan visits for (M tile mtile of a batch whose

@@ -323,12 +323,7 @@ void cmdb_bank_destroy(cmdb_bank *b) {
     cudaFree(b->cert_buf);
     for (auto &e : b->ev)
         if (e) cudaEventDestroy(e);
-    if (b->ev_base) cudaEventDestroy(b->ev_base);
     for (Lane &l : b->lane) {
-        for (auto &e : l.ev_tl)
-            if (e) cudaEventDestroy(e);
-        for (auto &e : l.ev_dbg)
-            if (e) cudaEventDestroy(e);
         if (l.stream) cudaStreamDestroy(l.stream);
         if (l.aux) cudaStreamDestroy(l.aux);
         if (l.ev_fork) cudaEventDestroy(l.ev_fork);
@@ -396,22 +391,10 @@ int cmdb_bank_set_option(cmdb_bank *b, int option, int value) {
         return CMDB_OK;
     }
     if (option == CMDB_OPT_TIMING) {
-        b->timing = value == 2 ? 2 : (value != 0);
+        b->timing = value != 0;
         if (b->timing && !b->ev[0]) {
             CMDB_CUDA(cudaSetDevice(b->device));
             for (auto &e : b->ev) CMDB_CUDA(cudaEventCreate(&e));
-        }
-        if (b->timing == 2) {  // lane timeline (diagnostics): per-lane events against a common base
-            CMDB_CUDA(cudaSetDevice(b->device));
-            if (!b->ev_base) {
-                CMDB_CUDA(cudaEventCreate(&b->ev_base));
-                for (Lane &l : b->lane) {
-                    for (auto &e : l.ev_tl) CMDB_CUDA(cudaEventCreate(&e));
-                    for (auto &e : l.ev_dbg) CMDB_CUDA(cudaEventCreate(&e));
-                }
-            }
-            CMDB_CUDA(cudaDeviceSynchronize());
-            CMDB_CUDA(cudaEventRecord(b->ev_base, b->lane[0].stream));
         }
         b->ev_valid = false;
         return CMDB_OK;

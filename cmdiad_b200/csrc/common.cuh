@@ -78,10 +78,6 @@ struct Lane {
     cudaStream_t stream = nullptr;
     cudaStream_t aux = nullptr;     // side stream of the (normally empty) tier-2 launches and the counters copy, beside the rescan
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-    // CMDB_OPT_TIMING = 2 (diagnostics): this lane's stage marks and the four marks inside the refine stage (before / after
-    // the certificate kernel, after the rescan, after the tier-2 launches), read by cmdb_debug_lane_timeline
-    cudaEvent_t ev_tl[CMDB_T_COUNT + 1] = {};
-    cudaEvent_t ev_dbg[4] = {};
     __half *q_hi = nullptr;         // [cap_p, D]  split-fp16 query operand
     __half *q_lo = nullptr;
     int *q_scale_exp = nullptr;     // device [cap_p]: per-row exponent e_q with q_hi + q_lo = q * 2^e_q
@@ -97,7 +93,8 @@ struct Lane {
     unsigned long long *s_key = nullptr;    // [cap_b] packed argmax key of min_val
     int *fail_count_host = nullptr; // pinned copy of [0..1] (statistics / adaptive mode)
     int2 *work_list = nullptr;      // [kWorkCap] (query row, producer) pairs whose producer may hide rows inside the band
-    unsigned long long *best_key = nullptr;  // [cap_p] running exact (d^2 bits << 32 | row) of the uncertified queries
+    // [cap_p] running exact (d^2 bits << 32 | row) of the uncertified queries; of every query in the CUDA-core mode
+    unsigned long long *best_key = nullptr;
     unsigned int *done_counter = nullptr;  // last-block-done counter of reweight_kernel
     float4 *cand = nullptr;         // [n_ctas, cap_p] per-CTA running top-2 (val1, idx1, val2, idx2) of the GEMM epilogue
     unsigned char *map_tmp = nullptr;  // horizontally blurred 8-bit images between the two blur kernels
@@ -224,9 +221,6 @@ struct cmdb_bank {
     int timing = 0;
     cudaEvent_t ev[CMDB_T_COUNT + 1] = {};
     bool ev_valid = false;
-    // CMDB_OPT_TIMING = 2 (diagnostics): common time base of the lanes' stage events (Lane::ev_tl), so that the overlap of
-    // the two lanes can be read (cmdb_debug_lane_timeline)
-    cudaEvent_t ev_base = nullptr;
     double *stats_buf = nullptr;  // 2 + num_sms * 4 doubles on device (cmdb_bank_stats)
     unsigned int *absmax_buf = nullptr;
 };
@@ -413,12 +407,12 @@ void api_prefer_carveout();    // api.cu
 void bank_prefer_carveout();   // bank.cu
 
 // score_tail.cu
-int score_simt_candidates(const ScoreCall &c, int P, int *n_cand_out);
 int score_refine(const ScoreCall &c, cudaStream_t st, int B, int P_img, int n_cand, bool compact);
 int score_select(const ScoreCall &c, int B, int P_img, bool local_m_star);
 int score_reweight(const ScoreCall &c, int B, int P_img);
 int score_build_knn_table(cmdb_bank *b, long long row_first, long long row_count);
-int score_exact_scan(cmdb_bank *b, const float *q_dev, int P, unsigned long long *keys_dev);
+// keys_dev[0, P) = smallest (d^2 bits << 32 | local row) of each query over the whole bank, on st
+int score_exact_scan(const cmdb_bank *b, cudaStream_t st, const float *q_dev, int P, unsigned long long *keys_dev);
 int score_shard_lookup(const ScoreCall &c, int B, float *contrib_dev);
 int score_shard_final(const ScoreCall &c, int B, const float *d2_sum_dev);
 // peer-memory form of the two exchanges of a sharded round (no NCCL): see score_tail.cu

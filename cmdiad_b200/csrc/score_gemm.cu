@@ -647,7 +647,7 @@ ScoreCall score_call(cmdb_bank *b, int lane, int slot) {
 
 int score_mark(const ScoreCall &c, int stage, cudaStream_t st) {
     const cmdb_bank *b = c.b;
-    if (b->timing && stage >= 0) CMDB_CUDA(cudaEventRecord(b->timing == 2 ? c.lane->ev_tl[stage] : b->ev[stage], st));
+    if (b->timing && stage >= 0) CMDB_CUDA(cudaEventRecord(b->ev[stage], st));
     return CMDB_OK;
 }
 

@@ -2,7 +2,8 @@
 //   refine_cert certificate of the pre-filter GEMM + exact float32 re-check of every candidate inside the error band
 //               -> min_val / min_idx (:227) and the packed argmax key of min_val -> s_star / s_idx (:228-231);
 //               rescan / fallback_decide / rescan_finish: exact rescan of producers the certificate could not clear
-//   refine      (3-term and diagnostics modes) exact re-check of the 4 best candidates
+//   refine      (3-term and 1-term modes, tier 2) exact re-check of the 4 best candidates
+//   exact_scan  (CUDA-core mode, cmdb_debug_exact_min) exact distances to every bank row
 //   select      m_test = patch[s_idx], m_star = bank[min_idx[s_idx]] (:235-251)
 //   reweight    w_dist = ||m_star - bank_r|| for every bank row, 3 smallest (:239-254), m_star_knn, w, s (:275-290):
 //               reweight_lookup (bank neighbour table), reweight_cert (batch through the tensor cores) or reweight_kernel
@@ -395,14 +396,14 @@ __global__ void __launch_bounds__(256) rescan_kernel(const int2 *__restrict__ wo
     }
 }
 
-// test hook: the exact scan the certificate promises equality with -- every (query, bank row) distance by warp_sqdist, smallest
-// (d^2 bits, row) key per query.  grid (row chunks, query groups of 8); one warp per query.
+// the exact scan the certificate promises equality with (CMDB_SCORE_SIMT, cmdb_debug_exact_min) -- every (query, bank row)
+// distance by warp_sqdist, smallest (d^2 bits, row) key per query.  grid (query groups of 8, row chunks); one warp per query.
 __global__ void __launch_bounds__(256) exact_scan_kernel(const float *__restrict__ q, int P, const float *__restrict__ bank,
                                                          long long rows, int dim, long long chunk,
                                                          unsigned long long *__restrict__ best_key) {
-    const int lane = threadIdx.x & 31, qi = blockIdx.y * 8 + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31, qi = blockIdx.x * 8 + (threadIdx.x >> 5);
     if (qi >= P) return;
-    const long long r0 = (long long)blockIdx.x * chunk, r1 = min(rows, r0 + chunk);
+    const long long r0 = (long long)blockIdx.y * chunk, r1 = min(rows, r0 + chunk);
     unsigned long long key = ~0ULL;
     for (long long r = r0; r < r1; ++r) {
         const float d2 = warp_sqdist(q + (size_t)qi * dim, bank + (size_t)r * dim, dim >> 2, lane);
@@ -412,102 +413,26 @@ __global__ void __launch_bounds__(256) exact_scan_kernel(const float *__restrict
     if (lane == 0 && key != ~0ULL) atomicMin(best_key + qi, key);
 }
 
-int score_exact_scan(cmdb_bank *b, const float *q_dev, int P, unsigned long long *keys_dev) {
+int score_exact_scan(const cmdb_bank *b, cudaStream_t st, const float *q_dev, int P, unsigned long long *keys_dev) {
     const long long chunk = std::max<long long>(64, (b->fin_rows + 4 * b->num_sms - 1) / (4 * b->num_sms));
-    const int gx = (int)((b->fin_rows + chunk - 1) / chunk);
-    exact_scan_kernel<<<dim3(gx, (P + 7) / 8), 256, 0, b->handle_stream()>>>(q_dev, P, b->data, b->fin_rows, b->dim, chunk, keys_dev);
+    const int n_chunks = (int)((b->fin_rows + chunk - 1) / chunk);
+    CMDB_CUDA(cudaMemsetAsync(keys_dev, 0xff, sizeof(unsigned long long) * (size_t)P, st));
+    exact_scan_kernel<<<dim3((P + 7) / 8, n_chunks), 256, 0, st>>>(q_dev, P, b->data, b->fin_rows, b->dim, chunk, keys_dev);
     CMDB_CUDA(cudaGetLastError());
     return CMDB_OK;
 }
 
-// ---------------------------------------------------------------------------------------------------------------
-// diagnostics scorer: exact direct-form float32 distances on CUDA cores, same candidate format as the GEMM epilogue.
-// grid (query tiles of 64, bank slices); block 256 = 16x16 threads, 4x4 outputs each, K chunks of 32 through smem.
-// ---------------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) simt_min_kernel(const float *__restrict__ q, int P, const float *__restrict__ bank,
-                                                       long long R, int dim, float4 *__restrict__ cand, int cand_stride) {
-    __shared__ float qs[64][33], bs[64][33];
-    __shared__ float rv[64][16][2];
-    __shared__ int ri[64][16][2];
-    const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-    const int q0 = blockIdx.x * 64;
-    const long long rows_per_slice = ((R + gridDim.y - 1) / gridDim.y + 63) / 64 * 64;
-    const long long r_begin = (long long)blockIdx.y * rows_per_slice, r_end = min(R, r_begin + rows_per_slice);
-    float b1[4], b2[4];
-    int i1[4], i2[4];
-#pragma unroll
-    for (int a = 0; a < 4; ++a) b1[a] = b2[a] = INFINITY, i1[a] = i2[a] = -1;
-    for (long long r0 = r_begin; r0 < r_end; r0 += 64) {
-        float acc[4][4] = {};
-        for (int k0 = 0; k0 < dim; k0 += 32) {
-            __syncthreads();
-            for (int i = threadIdx.x; i < 64 * 32; i += 256) {
-                const int r = i >> 5, c = i & 31;
-                qs[r][c] = (q0 + r < P) ? q[(size_t)(q0 + r) * dim + k0 + c] : 0.f;
-                bs[r][c] = (r0 + r < r_end) ? bank[(size_t)(r0 + r) * dim + k0 + c] : 0.f;
-            }
-            __syncthreads();
-#pragma unroll 8
-            for (int k = 0; k < 32; ++k) {
-                float qa[4], ba[4];
-#pragma unroll
-                for (int a = 0; a < 4; ++a) qa[a] = qs[ty * 4 + a][k], ba[a] = bs[tx * 4 + a][k];
-#pragma unroll
-                for (int a = 0; a < 4; ++a)
-#pragma unroll
-                    for (int c = 0; c < 4; ++c) {
-                        const float d = qa[a] - ba[c];
-                        acc[a][c] = fmaf(d, d, acc[a][c]);
-                    }
-            }
-        }
-#pragma unroll
-        for (int a = 0; a < 4; ++a)
-#pragma unroll
-            for (int c = 0; c < 4; ++c) {
-                const long long r = r0 + tx * 4 + c;
-                if (r >= r_end) continue;
-                const float v = acc[a][c];
-                const int ri_ = (int)r;
-                if (v < b1[a] || (v == b1[a] && ri_ < i1[a]) || i1[a] < 0) {
-                    b2[a] = b1[a], i2[a] = i1[a], b1[a] = v, i1[a] = ri_;
-                } else if (v < b2[a] || (v == b2[a] && ri_ < i2[a]) || i2[a] < 0) {
-                    b2[a] = v, i2[a] = ri_;
-                }
-            }
-    }
-    __syncthreads();
-#pragma unroll
-    for (int a = 0; a < 4; ++a) {
-        rv[ty * 4 + a][tx][0] = b1[a], rv[ty * 4 + a][tx][1] = b2[a];
-        ri[ty * 4 + a][tx][0] = i1[a], ri[ty * 4 + a][tx][1] = i2[a];
-    }
-    __syncthreads();
-    if (threadIdx.x < 64 && q0 + threadIdx.x < P) {
-        float c1 = INFINITY, c2 = INFINITY;
-        int j1 = -1, j2 = -1;
-        for (int t = 0; t < 16; ++t)
-            for (int u = 0; u < 2; ++u) {
-                const float v = rv[threadIdx.x][t][u];
-                const int i = ri[threadIdx.x][t][u];
-                if (i < 0) continue;
-                if (j1 < 0 || v < c1 || (v == c1 && i < j1)) c2 = c1, j2 = j1, c1 = v, j1 = i;
-                else if (j2 < 0 || v < c2 || (v == c2 && i < j2)) c2 = v, j2 = i;
-            }
-        cand[(size_t)blockIdx.y * cand_stride + q0 + threadIdx.x] = make_float4(c1, __int_as_float(j1), c2, __int_as_float(j2));
-    }
-}
-
-int score_simt_candidates(const ScoreCall &c, int P, int *n_cand_out) {
-    const cmdb_bank *b = c.b;
-    const int q_tiles = (P + 63) / 64;
-    int slices = std::max(1, std::min(b->num_sms, (2 * b->num_sms + q_tiles - 1) / q_tiles));
-    slices = (int)std::min<long long>(slices, (b->fin_rows + 63) / 64);
-    simt_min_kernel<<<dim3(q_tiles, slices), 256, 0, c.stream>>>(c.slot->q_f32, P, b->data, b->fin_rows, b->dim, c.lane->cand,
-                                                                b->layout.cap_p);
-    CMDB_CUDA(cudaGetLastError());
-    *n_cand_out = slices;
-    return CMDB_OK;
+// the exact scan's keys -> min_val / min_idx / argmax keys, with the arithmetic of refine_kernel's epilogue
+__global__ void __launch_bounds__(256) exact_decode_kernel(const unsigned long long *__restrict__ keys, int P, int P_img,
+                                                           long long row_offset, float *__restrict__ min_val,
+                                                           long long *__restrict__ min_idx, unsigned long long *s_key) {
+    const int qi = blockIdx.x * blockDim.x + threadIdx.x;
+    if (qi >= P) return;
+    const unsigned long long key = keys[qi];
+    const float dv = sqrtf(key_value(key));
+    min_val[qi] = dv;
+    min_idx[qi] = key_row(key) + row_offset;   // a finalized bank has rows: every query has a key
+    argmax_publish(s_key, qi, P_img, dv);
 }
 
 int score_refine(const ScoreCall &c, cudaStream_t st, int B, int P_img, int n_cand, bool compact) {
@@ -530,14 +455,12 @@ static int score_certify(const ScoreCall &c, int B, int P_img, int n_cand) {
     cudaStream_t st = c.stream;
     CMDB_CUDA(cudaMemsetAsync(s.fail_ctl, 0, 8 * sizeof(int) + sizeof(unsigned long long) * B, st));  // control block + s_key
     const float acc_model = cert_acc_model(b->dim);
-    if (b->timing == 2) CMDB_CUDA(cudaEventRecord(s.ev_dbg[0], st));
     // queries per block: 8 = one query per warp in phase 3 and 10 list entries per thread held in registers (measured best)
     constexpr int QB = 8;
     refine_cert_kernel<QB><<<(P + QB - 1) / QB, kCertThreads, 0, st>>>(s.cand, n_cand, b->layout.cap_p, c.slot->q_f32, b->data, b->dim,
                                                                        P, P_img, b->row_offset, s.q_norm, s.q_eps, b->cert_bmax,
                                                                        b->cert_eb_max, acc_model, c.min_val, c.min_idx, s.s_key,
                                                                        s.fail_list, s.fail_ctl, s.work_list, s.best_key);
-    if (b->timing == 2) CMDB_CUDA(cudaEventRecord(s.ev_dbg[1], st));
     CMDB_CUDA(cudaGetLastError());
     return CMDB_OK;
 }
@@ -553,7 +476,6 @@ static int score_rescan(const ScoreCall &c, int P_img) {
                                                   c.last, c.chunk_tiles, c.mt_total, s.best_key, s.fail_list, s.fail_ctl, P_img,
                                                   b->row_offset, c.min_val, c.min_idx, s.s_key);
     CMDB_CUDA(cudaGetLastError());
-    if (b->timing == 2) CMDB_CUDA(cudaEventRecord(s.ev_dbg[2], st));
     return CMDB_OK;
 }
 
@@ -571,7 +493,6 @@ int score_local_min(ScoreCall &c, const float *src, int src_is_device, int B, in
     cudaStream_t st = c.stream;
     const int P = B * P_img;
     const size_t D = b->dim;
-    int n_cand = 0;
     const int64_t prev_queries = b->last_queries;
     b->last_queries = P;
     if (b->score_impl != CMDB_SCORE_TCGEN05) {
@@ -579,9 +500,12 @@ int score_local_min(ScoreCall &c, const float *src, int src_is_device, int B, in
         CMDB_CUDA(cudaMemcpyAsync(q_f32, src, sizeof(float) * P * D, src_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
         if (b->q_norm_enabled) launch_normalize(st, b->num_sms, q_f32, (int64_t)P * D, b->q_mean, b->q_std);
         CMDB_CHECK(score_mark(c, ev_gemm, st));
-        CMDB_CHECK(score_simt_candidates(c, P, &n_cand));
+        CMDB_CHECK(score_exact_scan(b, st, q_f32, P, l.best_key));
         CMDB_CHECK(score_mark(c, ev_refine, st));
-        return score_refine(c, st, B, P_img, n_cand, false);
+        CMDB_CUDA(cudaMemsetAsync(l.s_key, 0, sizeof(unsigned long long) * B, st));
+        exact_decode_kernel<<<(P + 255) / 256, 256, 0, st>>>(l.best_key, P, P_img, b->row_offset, c.min_val, c.min_idx, l.s_key);
+        CMDB_CUDA(cudaGetLastError());
+        return CMDB_OK;
     }
     int mode = b->prefilter_terms;
     if (mode == 0) {
@@ -644,7 +568,7 @@ int score_local_min(ScoreCall &c, const float *src, int src_is_device, int B, in
         if (k == 0) c.first = sched;
     }
     c.last = sched;
-    n_cand = sched.producers;
+    const int n_cand = sched.producers;
     CMDB_CHECK(score_mark(c, ev_refine, st));
     if (mode != 0) return score_refine(c, st, B, P_img, n_cand, false);
     // certificate kernel (takes the tier decision), then the two tiers side by side: the exact rescan on the lane's stream,
@@ -673,7 +597,6 @@ int score_local_min(ScoreCall &c, const float *src, int src_is_device, int B, in
     }
     CMDB_CUDA(cudaEventRecord(l.ev_join, aux));
     CMDB_CUDA(cudaStreamWaitEvent(st, l.ev_join, 0));
-    if (b->timing == 2) CMDB_CUDA(cudaEventRecord(l.ev_dbg[3], st));
     return CMDB_OK;
 }
 

@@ -51,7 +51,8 @@ typedef enum cmdb_status {
 
 /* scoring implementation selector (cmdb_bank_set_option(CMDB_OPT_SCORE_IMPL)) */
 #define CMDB_SCORE_TCGEN05 0 /* tcgen05/TMEM split-fp16 distance GEMM (default, the product path) */
-#define CMDB_SCORE_SIMT 1    /* plain fp32 CUDA-core kernel, diagnostics only (same outputs, ~10x slower) */
+#define CMDB_SCORE_SIMT 1    /* exact float32 scan of the whole bank on CUDA cores (warp_sqdist, lowest row on ties);
+                                diagnostics and test reference */
 
 #define CMDB_OPT_SCORE_IMPL 1
 /* Mode of the distance GEMM behind calculate_dist (features.py:186-190):
@@ -68,11 +69,11 @@ typedef enum cmdb_status {
  *              another one of them -- equal up to the resolution of a float32 |a|^2 + |b|^2 - 2ab evaluation, not necessarily the lowest row).
  *  1           uncertified hi.hi pre-filter + exact re-check of the 4 best candidates (diagnostics). */
 #define CMDB_OPT_PREFILTER_TERMS 3
-#define CMDB_OPT_TIMING 2 /* 1 = record CUDA events between the stages of cmdb_score (see cmdb_bank_get_timings) */
+#define CMDB_OPT_TIMING 2 /* non-zero = record CUDA events between the stages of cmdb_score (see cmdb_bank_get_timings) */
 
 /* stage indices of cmdb_bank_get_timings */
 #define CMDB_T_STAGE_IN 0   /* patch copy + fp16 split of the queries */
-#define CMDB_T_GEMM 1       /* tcgen05 distance GEMM + fused top-2 epilogue (or the SIMT diagnostics kernel) */
+#define CMDB_T_GEMM 1       /* tcgen05 distance GEMM + fused top-2 epilogue (or the exact CUDA-core scan) */
 #define CMDB_T_REFINE 2     /* exact re-check -> min_val / min_idx / s_star */
 #define CMDB_T_MAP 3        /* bilinear upsample + Gaussian blur (then the maps start their device -> host copy) */
 #define CMDB_T_REWEIGHT 4   /* m_star selection, w_dist top-3 over the bank, w and s (overlaps the copy of the maps) */
@@ -118,7 +119,7 @@ int cmdb_bank_finalize(cmdb_bank *bank);
  * collectives against it); cmdb_bank_lane_streams: both of them. */
 int cmdb_bank_stream(cmdb_bank *bank, void **out_stream);
 int cmdb_bank_lane_streams(cmdb_bank *bank, void **out_streams2);
-/* milliseconds of each stage (CMDB_T_*) of the last cmdb_score call on this handle; needs CMDB_OPT_TIMING = 1.
+/* milliseconds of each stage (CMDB_T_*) of the last cmdb_score call on this handle; needs CMDB_OPT_TIMING on.
  * out_ms: float [CMDB_T_COUNT].  Measured with CUDA events on the handle's stream. */
 int cmdb_bank_get_timings(cmdb_bank *bank, float *out_ms);
 /* Optional (SURVEY 8f-1): the three nearest bank rows of EVERY bank row, computed once after cmdb_bank_finalize with the

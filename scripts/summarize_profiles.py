@@ -6,6 +6,9 @@ import subprocess
 import sys
 
 TAG = sys.argv[1] if len(sys.argv) > 1 else "r01"
+# the scoring workload of the captures: the bench bank with its neighbour table, four batches of 16 images
+SCORE_RUN = ('python -c "import bench, torch; b = bench.build_bank(0, bench.BANK_ROWS, 0); b.finalize(); b.build_knn(); '
+             'p = torch.stack(bench.test_patches(16)).cuda(); [b.score_batch(p, (28, 28), 224) for _ in range(4)]"')
 KEYS = ["gpu__time_duration.sum", "sm__cycles_elapsed.max.per_second", "dram__bytes_read.sum", "dram__bytes_write.sum",
         "dram__bytes_read.sum.per_second", "gpu__dram_throughput.avg.pct_of_peak_sustained_elapsed", "lts__t_sector_hit_rate.pct",
         "sm__pipe_tensor_cycles_active.avg.pct_of_peak_sustained_active", "sm__throughput.avg.pct_of_peak_sustained_elapsed",
@@ -73,8 +76,8 @@ if __name__ == "__main__":
     if os.path.exists(f"{g}/launches.csv"):
         launches(f"{g}/launches.csv", f"profiles/{TAG}_launches_bench.txt",
                  "ncu --metrics gpu__time_duration.sum --clock-control none -c 2500 python bench.py --steps 2 --warmup 3 --skip-cpu "
-                 "--skip-extras --skip-dropin   (scripts/final_check.sh)")
-    cap = "ncu --set full --clock-control none --import-source on -k regex:%s -s 1 -c 1 python scripts/profile_target.py score 16"
+                 "--skip-extras --skip-dropin")
+    cap = "ncu --set full --clock-control none --import-source on -k regex:%s -s 1 -c 1 " + SCORE_RUN
     for rep, out, title in (
             ("prof_score_gemm", "prof_gemm", "score_gemm_kernel<1,2,1>, batch of 16 images x 784 patches vs 200k x 768 bank"),
             ("prof_gemm", "prof_gemm", "score_gemm_kernel<1,2,1>, batch of 16 images x 784 patches vs 200k x 768 bank"),

@@ -123,7 +123,7 @@ def test_score_shapes_vs_oracle(env, R, P, fm, D):
 
 
 def test_score_tcgen05_equals_simt(env):
-    """both candidate generators feed the same exact re-check, so outputs must be identical bit for bit"""
+    """the certified tensor-core path and the exact CUDA-core scan must give identical outputs bit for bit"""
     from cmdiad_b200 import synth
     L = env["L"]
     lib = synth.patches(30000, 768, seed=5, dist="G")
@@ -305,6 +305,30 @@ def _exact_scan(b, patch):
     return ex_val, ex_idx
 
 
+@pytest.mark.parametrize("B,fm", [(3, 28), (32, 128)])
+def test_exact_scan_mode_on_a_row_offset_handle(env, B, fm):
+    """The CUDA-core mode on a handle holding global rows [k, k + R): min_idx are global rows, equal to the exact scan of
+    the same rows at offset 0 plus k; every row is stored twice and the lower copy wins.  32 images of 128 x 128 patches
+    are 524 288 query rows, more than 65 535 groups of 8."""
+    L = env["L"]
+    D, R, k = 64, 1000, 123_457
+    g = np.random.Generator(np.random.PCG64(B))
+    half = g.standard_normal((R // 2, D), dtype=np.float32)
+    patches = half[g.integers(0, R // 2, (B, fm * fm))] + 0.3 * g.standard_normal((B, fm * fm, D), dtype=np.float32)
+    b = env["Bank"](D, R, row_offset=k)
+    b.append(np.concatenate([half, half]))
+    b.finalize()
+    b.set_score_impl(L.SCORE_SIMT)
+    res = b.score_batch(patches, (fm, fm), 64)
+    b.set_row_offset(0)
+    ex_val, ex_idx = _exact_scan(b, patches.reshape(-1, D))
+    assert (ex_idx < R // 2).all()
+    assert (np.concatenate([r.min_idx for r in res]) == ex_idx + k).all()
+    assert (np.concatenate([r.min_val for r in res]) == ex_val).all()
+    assert all(r.s_star[0] == r.min_val.max() and r.s_idx[0] == int(np.argmax(r.min_val)) for r in res)
+    b.close()
+
+
 def test_certificate_fallback_on_near_duplicates(env):
     """Groups of near-duplicate bank rows defeat an 11-bit pre-filter: the certificate must notice (fallback > 0).  While the
     unresolved (query, producer) pairs fit the work list they are rescanned exactly and the answers equal the exact scan of
@@ -481,8 +505,7 @@ def test_certificate_under_adversarial_inputs(env, kind, D):
     cert = b.score(patch, (fm, fm), 224)
     stats = b.score_stats()
     # the exact scan the certificate promises equality with: every (query, row) distance by the re-check arithmetic
-    # (warp_sqdist), lowest row on ties.  (The CUDA-core diagnostics scorer is NOT that reference here: it re-checks only
-    # its 4 best candidates, and these inputs have up to 8 rows within one float32 ulp of each other.)
+    # (warp_sqdist), lowest row on ties
     ex_val, ex_idx = _exact_scan(b, patch)
     bad = np.nonzero((cert.min_idx != ex_idx) | (cert.min_val != ex_val))[0]
     assert bad.size == 0, (kind, D, stats, bad[:5], cert.min_idx[bad[:5]], ex_idx[bad[:5]], cert.min_val[bad[:5]], ex_val[bad[:5]])
