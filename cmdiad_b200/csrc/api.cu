@@ -13,18 +13,19 @@ __global__ void __launch_bounds__(512) f32_to_f64_kernel(const float *__restrict
         z[i] = (double)x[i];
 }
 
-// keys[p] = exchange_key(min_val[p], global row); and the inverse
-__global__ void pack_keys_kernel(const float *__restrict__ min_val, const long long *__restrict__ min_idx, int P,
+// keys[p] = exchange_key(local min d^2, global row) -- a round's local min_val holds d^2 (ScoreCall::sq_min); and the
+// inverse, which takes the root: min_val = sqrtf(d^2) as a single bank computes it
+__global__ void pack_keys_kernel(const float *__restrict__ min_d2, const long long *__restrict__ min_idx, int P,
                                  long long *__restrict__ keys) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < P) keys[i] = exchange_key(min_val[i], min_idx[i]);
+    if (i < P) keys[i] = exchange_key(min_d2[i], min_idx[i]);
 }
 __global__ void unpack_keys_kernel(const long long *__restrict__ keys, int P, int P_img, float *__restrict__ min_val,
                                    long long *__restrict__ min_idx, unsigned long long *s_key) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < P) {
         const unsigned long long k = (unsigned long long)keys[i];
-        const float v = key_value(k);
+        const float v = sqrtf(key_value(k));
         min_val[i] = v;
         min_idx[i] = key_row(k);
         argmax_publish(s_key, i, P_img, v);
@@ -447,6 +448,7 @@ int cmdb_score_shard_min(cmdb_bank *b, const float *patches, int B, int P, int p
     // rounds may be outstanding (three result slots on the two lanes)
     ScoreCall c{};
     CMDB_CHECK(begin_call(b, B, P, out_hw, "cmdb_score_shard_min", &c));
+    c.sq_min = true;   // the keys carry d^2
     CMDB_CHECK(score_local_min(c, patches, patch_is_device, B, P, -1, -1, c.slot->ev_compute));
     pack_keys_kernel<<<(B * P + 255) / 256, 256, 0, c.stream>>>(c.min_val, c.min_idx, B * P, (long long *)keys_device);
     CMDB_CUDA(cudaGetLastError());
@@ -528,6 +530,7 @@ int cmdb_score_shard_round_submit(cmdb_bank *b, const float *patches, int B, int
     CMDB_CHECK(comm_info(b->comm, &rank, &world, &local, peers.p, &bytes));
     ScoreCall c{};
     CMDB_CHECK(begin_call(b, B, P, out_hw, "cmdb_score_shard_round_submit", &c));
+    c.sq_min = true;   // the keys carry d^2
     CMDB_CHECK(score_local_min(c, patches, patch_is_device, B, P, -1, -1, c.slot->ev_compute));
     const unsigned long long epoch = comm_next_score_epoch(b->comm);  // per buffer, not per bank: several banks may share it
     const int xslot = (int)(epoch % kShardSlots);

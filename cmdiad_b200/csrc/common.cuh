@@ -252,7 +252,7 @@ constexpr size_t kCommCoresetBytes = 256 * 1024;  // coreset flags + key slots (
 // row-sharded SCORING rounds exchange through the same buffer (never cleared: every word is rewritten with the round's epoch):
 //   flags  [4 slots][2 kinds][kMaxRanks] u64 at kCommScoreFlagsOff
 //   d2     [4 slots][kMaxRanks][kShardD2Cap] float at kCommScoreD2Off        (squared neighbour distances, 2 per image)
-//   keys   [4 slots][kMaxRanks][kShardKeysCap] int64 at kCommScoreKeysOff    (packed (min distance, global row) per query)
+//   keys   [4 slots][kMaxRanks][kShardKeysCap] int64 at kCommScoreKeysOff    (packed (min d^2, global row) per query)
 // (4 slots, round r uses slot r & 3: with two lanes per rank a rank may start round r + 2 while a peer still reads round r)
 constexpr size_t kCommScoreFlagsOff = kCommCoresetBytes;
 constexpr size_t kCommScoreD2Off = kCommScoreFlagsOff + 4096;
@@ -343,10 +343,12 @@ __device__ __forceinline__ unsigned long long pack_min_key(float v, unsigned int
     return ((unsigned long long)__float_as_uint(v) << 32) | row;
 }
 __device__ __forceinline__ long long key_row(unsigned long long k) { return (long long)(k & 0xffffffffULL); }
-// exchange key of a sharded round: (min distance, global row) as a signed integer, INT64_MAX where there is no row, so
-// that a MIN over the ranks is the global argmin (decoded with key_value / key_row)
-__device__ __forceinline__ long long exchange_key(float v, long long row) {
-    return row < 0 ? 0x7fffffffffffffffLL : (long long)(((unsigned long long)__float_as_uint(v) << 32) | (unsigned long long)row);
+// exchange key of a sharded round: (local min d^2, global row) as a signed integer, INT64_MAX where there is no row, so
+// that a MIN over the ranks is the global argmin with the order and ties of a single bank's (d^2, row) keys (sqrtf maps
+// neighbouring d^2 to one distance: packing distances would let the lower row win where the other row is nearer).
+// Decoded with key_row and min_val = sqrtf(key_value).
+__device__ __forceinline__ long long exchange_key(float d2, long long row) {
+    return row < 0 ? 0x7fffffffffffffffLL : (long long)(((unsigned long long)__float_as_uint(d2) << 32) | (unsigned long long)row);
 }
 // argmax key of an image: an atomicMax over (min_val bits, ~query) keeps the largest value, the lowest query on ties
 __device__ __forceinline__ void argmax_publish(unsigned long long *s_key, int qi, int P_img, float v) {
@@ -374,6 +376,9 @@ struct ScoreCall {
     // schedules of the first and the last chunk launch
     int mt_total = 0, chunk_tiles = 0;
     GemmSched first{}, last{};
+    // sharded rounds: score_local_min leaves the SQUARED minimum distance in min_val, which the exchange key packs; the
+    // decode after the exchange takes the root and publishes the argmax keys again
+    bool sq_min = false;
 };
 
 // score_gemm.cu

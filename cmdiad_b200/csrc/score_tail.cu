@@ -72,9 +72,10 @@ __global__ void __launch_bounds__(256) refine_kernel(const float4 *__restrict__ 
                                                      const float *__restrict__ q, const float *__restrict__ bank, int dim,
                                                      int P, int P_img, long long row_offset, float *__restrict__ min_val,
                                                      long long *__restrict__ min_idx, unsigned long long *s_key,
-                                                     const int *__restrict__ list, const int *__restrict__ count) {
+                                                     const int *__restrict__ list, const int *__restrict__ count, bool sq) {
     // P = total query rows of the batch (B images of P_img patches each); s_key[b] is image b's packed argmax.
-    // Compact mode (list != nullptr): candidate column c belongs to query list[c], c < *count.
+    // Compact mode (list != nullptr): candidate column c belongs to query list[c], c < *count.  sq: min_val gets d^2
+    // (ScoreCall::sq_min).
     const int lane = threadIdx.x & 31;
     const int qc = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);  // candidate column
     if (qc >= (count ? __ldg(count) : P)) return;
@@ -133,7 +134,7 @@ __global__ void __launch_bounds__(256) refine_kernel(const float4 *__restrict__ 
         if (best_i < 0 || d2 < best || (d2 == best && i < best_i)) best = d2, best_i = i;
     }
     if (lane == 0) {
-        const float dv = sqrtf(best);
+        const float dv = sq ? best : sqrtf(best);
         min_val[qi] = dv;
         min_idx[qi] = best_i < 0 ? -1 : (long long)best_i + row_offset;
         argmax_publish(s_key, qi, P_img, dv);
@@ -214,7 +215,8 @@ __global__ void __launch_bounds__(kCertThreads) refine_cert_kernel(const float4 
                                                           float *__restrict__ min_val,
                                                           long long *__restrict__ min_idx, unsigned long long *s_key,
                                                           int *__restrict__ fail_list, int *__restrict__ ctl,
-                                                          int2 *__restrict__ work_list, unsigned long long *__restrict__ best_key) {
+                                                          int2 *__restrict__ work_list, unsigned long long *__restrict__ best_key,
+                                                          bool sq) {
     constexpr int kWarps = kCertThreads / 32;
     constexpr int PL = 32 / QB;            // producers covered by one warp-wide load
     constexpr int CSTEP = kWarps * PL;     // producers covered by one block-wide load
@@ -300,7 +302,7 @@ __global__ void __launch_bounds__(kCertThreads) refine_cert_kernel(const float4 
         cert_recheck(list_s[k], min(cnt_s[k], kCertRows), q + (size_t)qq * dim, bank, dim, lane, best, best_i);
         if (lane == 0) {
             if (bad_s[k] == 0 && best_i >= 0) {
-                const float dv = sqrtf(best);
+                const float dv = sq ? best : sqrtf(best);
                 min_val[qq] = dv;
                 min_idx[qq] = (long long)best_i + row_offset;
                 argmax_publish(s_key, qq, P_img, dv);
@@ -336,7 +338,7 @@ __global__ void __launch_bounds__(256) rescan_kernel(const int2 *__restrict__ wo
                                                      int mt_total, unsigned long long *best_key,
                                                      const int *__restrict__ fail_list, int *__restrict__ ctl, int P_img,
                                                      long long row_offset, float *__restrict__ min_val,
-                                                     long long *__restrict__ min_idx, unsigned long long *s_key) {
+                                                     long long *__restrict__ min_idx, unsigned long long *s_key, bool sq) {
     __shared__ int last_block;
     const int n_items = min(*n_items_ptr, kWorkCap);
     const int tiles_per = producer_slots(full, last);
@@ -389,7 +391,7 @@ __global__ void __launch_bounds__(256) rescan_kernel(const int2 *__restrict__ wo
     for (int i = threadIdx.x; i < n_fin; i += blockDim.x) {
         const int qi = fail_list[i];
         const unsigned long long key = __ldcg(best_key + qi);
-        const float dv = sqrtf(key_value(key));
+        const float dv = sq ? key_value(key) : sqrtf(key_value(key));
         min_val[qi] = dv;
         min_idx[qi] = key == ~0ULL ? -1 : key_row(key) + row_offset;
         argmax_publish(s_key, qi, P_img, dv);
@@ -425,11 +427,11 @@ int score_exact_scan(const cmdb_bank *b, cudaStream_t st, const float *q_dev, in
 // the exact scan's keys -> min_val / min_idx / argmax keys, with the arithmetic of refine_kernel's epilogue
 __global__ void __launch_bounds__(256) exact_decode_kernel(const unsigned long long *__restrict__ keys, int P, int P_img,
                                                            long long row_offset, float *__restrict__ min_val,
-                                                           long long *__restrict__ min_idx, unsigned long long *s_key) {
+                                                           long long *__restrict__ min_idx, unsigned long long *s_key, bool sq) {
     const int qi = blockIdx.x * blockDim.x + threadIdx.x;
     if (qi >= P) return;
     const unsigned long long key = keys[qi];
-    const float dv = sqrtf(key_value(key));
+    const float dv = sq ? key_value(key) : sqrtf(key_value(key));
     min_val[qi] = dv;
     min_idx[qi] = key_row(key) + row_offset;   // a finalized bank has rows: every query has a key
     argmax_publish(s_key, qi, P_img, dv);
@@ -443,7 +445,7 @@ int score_refine(const ScoreCall &c, cudaStream_t st, int B, int P_img, int n_ca
     if (!compact) CMDB_CUDA(cudaMemsetAsync(l.s_key, 0, sizeof(unsigned long long) * B, st));
     refine_kernel<<<(P + 7) / 8, 256, 0, st>>>(l.cand, n_cand, b->layout.cap_p, c.slot->q_f32, b->data, b->dim, P, P_img,
                                                b->row_offset, c.min_val, c.min_idx, l.s_key, compact ? l.fail_list : nullptr,
-                                               compact ? l.fail_ctl + 2 : nullptr);
+                                               compact ? l.fail_ctl + 2 : nullptr, c.sq_min);
     CMDB_CUDA(cudaGetLastError());
     return CMDB_OK;
 }
@@ -460,7 +462,7 @@ static int score_certify(const ScoreCall &c, int B, int P_img, int n_cand) {
     refine_cert_kernel<QB><<<(P + QB - 1) / QB, kCertThreads, 0, st>>>(s.cand, n_cand, b->layout.cap_p, c.slot->q_f32, b->data, b->dim,
                                                                        P, P_img, b->row_offset, s.q_norm, s.q_eps, b->cert_bmax,
                                                                        b->cert_eb_max, acc_model, c.min_val, c.min_idx, s.s_key,
-                                                                       s.fail_list, s.fail_ctl, s.work_list, s.best_key);
+                                                                       s.fail_list, s.fail_ctl, s.work_list, s.best_key, c.sq_min);
     CMDB_CUDA(cudaGetLastError());
     return CMDB_OK;
 }
@@ -474,7 +476,7 @@ static int score_rescan(const ScoreCall &c, int P_img) {
     CMDB_REQUIRE(!c.first.pair && !c.last.pair, CMDB_ERR_UNSUPPORTED, "scoring: the exact rescan cannot walk a CTA-pair GEMM schedule");
     rescan_kernel<<<b->num_sms * 8, 256, 0, st>>>(s.work_list, s.fail_ctl + 3, c.slot->q_f32, b->data, b->dim, b->fin_rows, c.first,
                                                   c.last, c.chunk_tiles, c.mt_total, s.best_key, s.fail_list, s.fail_ctl, P_img,
-                                                  b->row_offset, c.min_val, c.min_idx, s.s_key);
+                                                  b->row_offset, c.min_val, c.min_idx, s.s_key, c.sq_min);
     CMDB_CUDA(cudaGetLastError());
     return CMDB_OK;
 }
@@ -503,7 +505,8 @@ int score_local_min(ScoreCall &c, const float *src, int src_is_device, int B, in
         CMDB_CHECK(score_exact_scan(b, st, q_f32, P, l.best_key));
         CMDB_CHECK(score_mark(c, ev_refine, st));
         CMDB_CUDA(cudaMemsetAsync(l.s_key, 0, sizeof(unsigned long long) * B, st));
-        exact_decode_kernel<<<(P + 255) / 256, 256, 0, st>>>(l.best_key, P, P_img, b->row_offset, c.min_val, c.min_idx, l.s_key);
+        exact_decode_kernel<<<(P + 255) / 256, 256, 0, st>>>(l.best_key, P, P_img, b->row_offset, c.min_val, c.min_idx, l.s_key,
+                                                             c.sq_min);
         CMDB_CUDA(cudaGetLastError());
         return CMDB_OK;
     }
@@ -991,12 +994,13 @@ __global__ void shard_final_kernel(const unsigned long long *__restrict__ top3, 
 // ---------------------------------------------------------------------------------------------------------------
 // NCCL-free exchanges of a sharded round over peer-mapped memory (CUDA IPC / NVLink, cmdb_comm): the collective is fused
 // into the kernels on both sides of it.
-//   push   every rank packs its local (min distance, global row) keys and stores them straight into the round's slot
+//   push   every rank packs its local (min d^2, global row) keys and stores them straight into the round's slot
 //          [slot][rank][query] of EVERY rank's buffer (coalesced 8-byte NVLink stores); the last block to finish raises
 //          the rank's flag (the round's epoch) in every buffer: threadfence_system by all writers, then a release store
 //   reduce every rank waits for the world flags in its LOCAL buffer, takes the MIN over the world key arrays (non-negative
-//          distance bits << 32 | global row: integer MIN == argmin with lowest-row tie-break) and decodes min_val / min_idx /
-//          the per-image argmax key -- what ncclAllReduce(MIN) + unpack did in two launches and ~60 us at 8 ranks.
+//          d^2 bits << 32 | global row: integer MIN == argmin with lowest-row tie-break, the order of a single bank's
+//          keys) and decodes min_val = sqrtf(d^2) / min_idx / the per-image argmax key -- what ncclAllReduce(MIN) + unpack
+//          did in two launches and ~60 us at 8 ranks.
 // Slots alternate by round parity; a rank can be at most one round ahead of the slowest rank (it needs everybody's flag
 // of round r + 1 before it can finish that round), so a slot is never overwritten while someone still reads it.
 // ---------------------------------------------------------------------------------------------------------------
@@ -1009,11 +1013,12 @@ __device__ __forceinline__ unsigned long long ld_acquire_sys_u64(const unsigned 
     return v;
 }
 
-__global__ void __launch_bounds__(256) shard_push_keys_kernel(const float *__restrict__ min_val, const long long *__restrict__ min_idx,
+// min_d2: the local min_val of a round, which holds d^2 (ScoreCall::sq_min)
+__global__ void __launch_bounds__(256) shard_push_keys_kernel(const float *__restrict__ min_d2, const long long *__restrict__ min_idx,
                                                               int n, PeerPtrs peers, int world, int rank, size_t keys_off,
                                                               size_t flag_off, unsigned long long epoch, unsigned int *ctr) {
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        const long long key = exchange_key(min_val[i], min_idx[i]);
+        const long long key = exchange_key(min_d2[i], min_idx[i]);
         for (int r = 0; r < world; ++r)
             reinterpret_cast<long long *>(peers.p[r] + keys_off)[(size_t)rank * kShardKeysCap + i] = key;
     }
@@ -1063,7 +1068,7 @@ __global__ void __launch_bounds__(256) shard_reduce_keys_kernel(const unsigned c
             const long long v = __ldcg(keys + (size_t)r * kShardKeysCap + i);
             k = v < k ? v : k;
         }
-        const float v = key_value((unsigned long long)k);
+        const float v = sqrtf(key_value((unsigned long long)k));
         min_val[i] = v;
         min_idx[i] = key_row((unsigned long long)k);
         argmax_publish(s_key, i, P_img, v);

@@ -21,17 +21,20 @@ def owner_of(row, n_rows, world):
     return r
 
 
-def pack_keys(dist_f32, global_rows):
-    """key = float_bits(d) << 32 | row.  d >= 0, so signed int64 order == (d, row) lexicographic order: an integer MIN
-    all-reduce is argmin with lowest-global-row tie-break."""
-    bits = np.ascontiguousarray(dist_f32, dtype=np.float32).view(np.uint32).astype(np.int64)
+def pack_keys(d2_f32, global_rows):
+    """key = float_bits(d2) << 32 | row, with d2 the float32 SQUARED distance.  d2 >= 0, so signed int64 order == (d2, row)
+    lexicographic order: an integer MIN all-reduce is argmin d2 with lowest-global-row tie-break, the order of a single
+    bank's keys.  (Distances would not do: sqrt maps neighbouring float32 d2 to one value, and the MIN would then pick
+    the lower row where the other one is strictly nearer.)"""
+    bits = np.ascontiguousarray(d2_f32, dtype=np.float32).view(np.uint32).astype(np.int64)
     return (bits << 32) | np.asarray(global_rows, dtype=np.int64)
 
 
 def unpack_keys(keys):
+    """(d2, rows) of packed keys; the device decodes min_val as np.sqrt(d2) in float32 (correctly rounded, == sqrtf)"""
     keys = np.asarray(keys, dtype=np.int64)
-    d = (keys >> 32).astype(np.uint32).view(np.float32)
-    return d, keys & 0xFFFFFFFF
+    d2 = (keys >> 32).astype(np.uint32).view(np.float32)
+    return d2, keys & 0xFFFFFFFF
 
 
 def stage_slice(n_rows, world, rank):

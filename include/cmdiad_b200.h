@@ -314,9 +314,10 @@ int cmdb_eval_read(cmdb_bank *bank, int64_t first, int64_t n, double *maps_host 
  * batch of patches.  All buffers named *_device are device memory on the bank's GPU, owned by the caller (torch tensors),
  * so the collectives between the phases run on them directly.  A round scores B images (B <= 32 and B*dim*4 <= 160 KB)
  * in three phases with TWO small collectives; all phases of one round use the same B, P, out_hw:
- *   1. cmdb_score_shard_min            keys[b*P+p] = (float_bits(local min distance) << 32) | global_row
- *      (non-negative, so integer MIN == argmin with lowest-global-row tie-break)               -> all-reduce MIN (int64[B*P])
- *   2. cmdb_score_shard_lookup         decodes the reduced keys (min_val, min_idx, s*, s_idx, m_star row), reads the three
+ *   1. cmdb_score_shard_min            keys[b*P+p] = (float_bits(local min SQUARED distance) << 32) | global_row
+ *      (non-negative, so integer MIN == argmin with lowest-global-row tie-break; squared, because sqrtf maps neighbouring
+ *      float32 d^2 to one distance and the single bank's argmin is that of d^2)              -> all-reduce MIN (int64[B*P])
+ *   2. cmdb_score_shard_lookup         decodes the reduced keys (min_val = sqrtf(d^2), min_idx, s*, s_idx, m_star row), reads the three
  *      nearest rows of m_star from the table and writes, per image, the exact SQUARED distances ||m_test - bank[nn_k]||^2
  *      (k = 1, 2; features.py:275-283) for the neighbour rows this rank owns, 0 for the others     -> all-reduce SUM (float[B*2])
  *   3. cmdb_score_shard_finish_submit  m_star_knn = sqrt(sum), w, s for all images; upsample + blur + device->host copy of

@@ -2,7 +2,8 @@
 
 Covers both transports of the sharded round with the replicated neighbour table (NCCL collectives; exchanges over
 peer-mapped memory), the table itself, replicated and distributed finishing, host and device queries, several rounds per
-call and pipelined rounds.
+call, pipelined rounds, and a witness bank: near-duplicate rows on ranks 0 and N - 1 whose distances to a query are equal
+in float32 while their squared distances are not (the exchange keys must carry d^2 to pick the same row as one bank).
 Prints one line per check and a final SHARD CHECK OK / FAILED (rank 0); exit code 1 on failure."""
 import os
 import sys
@@ -83,6 +84,61 @@ for mode in ("table/nccl", "table/peer-memory"):
         while pending:
             got.extend(pending.pop(0).wait())
         report(f"[{tag}] 8 rounds, three outstanding, {src_name} queries", all(same(got[t], bb[t]) for t in range(64)))
+
+# Witness bank: rows J[t] on the last rank are copies of rows I[t] on rank 0 nudged by 2 ulps in two coordinates.  For a
+# query near such a pair the float32 d^2 differ by about an ulp while sqrtf makes the distances equal ("witnesses"): a
+# single bank returns the nearer row J[t], and so must the exchange of (d^2, row) keys on both transports.
+g = np.random.Generator(np.random.PCG64(77))
+Rw, Dw, n_pairs = 4099, 64, 24
+libw = g.standard_normal((Rw, Dw), dtype=np.float32)
+I = 100 + np.arange(n_pairs)
+J = Rw * (world - 1) // world + 300 + np.arange(n_pairs)
+for i, j in zip(I, J):
+    libw[j] = libw[i]
+    for c in g.choice(Dw, 2, replace=False):
+        step = np.float32(np.inf) if g.random() < 0.5 else np.float32(-np.inf)
+        libw[j, c] = np.nextafter(np.nextafter(libw[j, c], step), step)
+qw = np.concatenate([libw[i] + 0.2 * g.standard_normal((128, Dw), dtype=np.float32) for i in I]).astype(np.float32)
+pair = np.repeat(np.arange(n_pairs), 128)
+fullw = Bank(Dw, Rw, device=local)
+fullw.append(libw)
+fullw.finalize()
+fullw.build_knn()
+
+
+def exact_min(b, q):
+    v, i = np.empty(q.shape[0], np.float32), np.empty(q.shape[0], np.int64)
+    assert b._lib.cmdb_debug_exact_min(b._h, q.ctypes.data, q.shape[0], v.ctypes.data, i.ctypes.data) == 0
+    return v, i
+
+
+pairs_i, pairs_j = Bank(Dw, n_pairs, device=local), Bank(Dw, n_pairs, device=local)
+pairs_i.append(libw[I])
+pairs_j.append(libw[J])
+pairs_i.finalize()
+pairs_j.finalize()
+vi, _ = exact_min(pairs_i, qw)
+vj, _ = exact_min(pairs_j, qw)
+_, jf = exact_min(fullw, qw)
+n_wit = int(((vi == vj) & (jf == J[pair])).sum())
+pairs_i.close()
+pairs_j.close()
+xw = qw.reshape(12, 256, Dw)
+bw = fullw.score_batch(xw, (16, 16), 64, full=True)
+lo_w, hi_w = Rw * rank // world, Rw * (rank + 1) // world
+shardw = Bank(Dw, hi_w - lo_w, device=local, row_offset=lo_w)
+shardw.append(libw[lo_w:hi_w])
+shardw.finalize()
+shardw.build_knn_sharded()
+for tag in ("nccl", "peer-memory"):
+    if tag == "peer-memory":
+        shardw.attach_comm(comm)
+    aw = shardw.score_sharded_batch(xw, (16, 16), 64, full=True)
+    report(f"[witness bank/{tag}] {n_wit} near-tie witnesses across ranks 0 and {world - 1}",
+           all(same(aw[t], bw[t]) for t in range(12)))
+shardw.attach_comm(None)
+shardw.close()
+fullw.close()
 t = torch.tensor([bad], device="cuda")
 dist.all_reduce(t)
 if rank == 0:

@@ -131,8 +131,8 @@ def test_projection_error_branch_keeps_unprojected_bank(env, capsys):
 
 def test_sharded_entry_points_with_one_rank(env):
     """the sharded scoring and the sharded coreset entry points on a 1-rank NCCL group must reproduce the plain
-    single-GPU calls (the multi-rank exchange itself is checked by scripts/shard_check.py and
-    scripts/coreset_shard_check.py under torchrun, and by tests/test_sharding_gloo.py on the host side)"""
+    single-GPU calls (several shards of one round: tests/test_gpu_shards.py on one GPU, scripts/shard_check.py and
+    scripts/coreset_shard_check.py under torchrun, tests/test_sharding_gloo.py on the host side)"""
     import torch.distributed as dist
     from cmdiad_b200 import Bank, Comm
     O = env["O"]
