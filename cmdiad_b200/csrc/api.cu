@@ -196,14 +196,10 @@ int cmdb_project(cmdb_bank *b, const int32_t *indptr, const int32_t *indices, co
                  "cmdb_project: bad row range");
     CMDB_REQUIRE(d_proj > 0, CMDB_ERR_INVALID, "cmdb_project: d_proj must be positive");
     CMDB_CUDA(cudaSetDevice(b->device));
-    double *z = nullptr;
-    CMDB_CUDA(cudaMalloc(&z, sizeof(double) * (size_t)n_rows * d_proj));
-    int rc = project_rows(b, b->data + row0 * b->dim, n_rows, b->dim, indptr, indices, data, d_proj, z);
-    cudaError_t e = cudaSuccess;
-    if (rc == CMDB_OK) e = cudaMemcpy(out_host, z, sizeof(double) * (size_t)n_rows * d_proj, cudaMemcpyDeviceToHost);
-    cudaFree(z);
-    if (rc != CMDB_OK) return rc;
-    CMDB_CUDA(e);
+    Buffer<double> z;
+    CMDB_CUDA(z.alloc((size_t)n_rows * d_proj));
+    CMDB_CHECK(project_rows(b, b->data + row0 * b->dim, n_rows, b->dim, indptr, indices, data, d_proj, z));
+    CMDB_CUDA(cudaMemcpy(out_host, z, sizeof(double) * (size_t)n_rows * d_proj, cudaMemcpyDeviceToHost));
     return CMDB_OK;
 }
 
@@ -226,22 +222,18 @@ static int coreset_impl(cmdb_bank *b, int64_t n_select, const int32_t *indptr, c
     // row_offset 0 -- also on a handle whose row_offset is set -- and its rows start on the boundary.
     const bool sharded = sh && sh->world > 1;
     const int pad = sharded ? (int)((b->row_offset * d) & 3) : 0;
-    double *z_alloc = nullptr;
-    CMDB_CUDA(cudaMalloc(&z_alloc, sizeof(double) * ((size_t)b->rows * d + 4)));
+    Buffer<double> z_alloc;
+    CMDB_CUDA(z_alloc.alloc((size_t)b->rows * d + 4));
     double *z = z_alloc + pad;
-    int rc;
     if (d_proj > 0) {
-        rc = project_rows(b, b->data, b->rows, b->dim, indptr, indices, data, d_proj, z);
+        CMDB_CHECK(project_rows(b, b->data, b->rows, b->dim, indptr, indices, data, d_proj, z));
     } else {
         // features.py:369-370: projection skipped, the float32 bank itself is used
         f32_to_f64_kernel<<<b->num_sms * 4, 512, 0, b->handle_stream()>>>(b->data, (long long)b->rows * d, z);
-        rc = cudaGetLastError() == cudaSuccess ? CMDB_OK : CMDB_ERR_CUDA;
+        CMDB_CUDA(cudaGetLastError());
     }
-    if (rc == CMDB_OK)
-        rc = coreset_greedy_dev(b, z, b->rows, d, n_select, dtype_mode, out_idx_host, force_idx, out_min_last, sh,
-                                force_mind_global);
-    cudaFree(z_alloc);
-    return rc;
+    return coreset_greedy_dev(b, z, b->rows, d, n_select, dtype_mode, out_idx_host, force_idx, out_min_last, sh,
+                              force_mind_global);
 }
 
 int cmdb_coreset_select(cmdb_bank *b, int64_t n_select, const int32_t *indptr, const int32_t *indices, const double *data,
@@ -495,8 +487,10 @@ int cmdb_score_shard_finish_submit(cmdb_bank *b, const float *knn_d2_sum_device,
 int cmdb_bank_attach_comm(cmdb_bank *b, cmdb_comm *comm) {
     CMDB_REQUIRE(b, CMDB_ERR_INVALID, "cmdb_bank_attach_comm: bank is NULL");
     CMDB_REQUIRE(!b->any_pending(), CMDB_ERR_STATE, "cmdb_bank_attach_comm: a submitted round is outstanding");
-    b->comm = comm;
-    if (!comm) return CMDB_OK;
+    if (!comm) {
+        b->comm = nullptr;
+        return CMDB_OK;
+    }
     int rank = 0, world = 1;
     size_t bytes = 0;
     unsigned char *local = nullptr, *peers[kMaxRanks];
@@ -504,14 +498,21 @@ int cmdb_bank_attach_comm(cmdb_bank *b, cmdb_comm *comm) {
     CMDB_REQUIRE(bytes >= kCommHeaderBytes, CMDB_ERR_INVALID, "cmdb_bank_attach_comm: the peer buffer has %zu bytes, need >= %zu", bytes,
                  (size_t)kCommHeaderBytes);
     CMDB_CUDA(cudaSetDevice(b->device));
-    if (!b->shard_ctr) {
-        CMDB_CUDA(cudaMalloc(&b->shard_ctr, 4 * sizeof(unsigned int)));
-        CMDB_CUDA(cudaMemset(b->shard_ctr, 0, 4 * sizeof(unsigned int)));
-        CMDB_CUDA(cudaMalloc(&b->shard_d2, sizeof(float) * 2 * kShardSlots * kShardD2Cap));
-        CMDB_CUDA(cudaHostAlloc(&b->shard_abort_host, sizeof(unsigned int), cudaHostAllocMapped));
-        *b->shard_abort_host = 0u;
-        CMDB_CUDA(cudaHostGetDevicePointer(&b->shard_abort_dev, b->shard_abort_host, 0));
+    if (!b->shard_ctr) {   // the exchange buffers go to the handle only once all of them exist
+        Buffer<unsigned int> ctr;
+        Buffer<float> d2;
+        Buffer<unsigned int, Mem::Mapped> abort_host;
+        unsigned int *abort_dev = nullptr;
+        CMDB_CUDA(ctr.alloc(4));
+        CMDB_CUDA(cudaMemset(ctr, 0, 4 * sizeof(unsigned int)));
+        CMDB_CUDA(d2.alloc(2 * kShardSlots * kShardD2Cap));
+        CMDB_CUDA(abort_host.alloc(1));
+        *abort_host = 0u;
+        CMDB_CUDA(cudaHostGetDevicePointer(&abort_dev, abort_host, 0));
+        b->shard_ctr = std::move(ctr), b->shard_d2 = std::move(d2), b->shard_abort_host = std::move(abort_host);
+        b->shard_abort_dev = abort_dev;
     }
+    b->comm = comm;   // last: a failed attach leaves the handle as it was
     return CMDB_OK;
 }
 
@@ -575,20 +576,16 @@ int cmdb_debug_read_candidates(cmdb_bank *b, float *out_host, int n_cta, int n_q
 int cmdb_debug_exact_min(cmdb_bank *b, const float *patch_host, int P, float *min_val_out, int64_t *min_idx_out) {
     CMDB_REQUIRE(b && patch_host && min_val_out && min_idx_out && P >= 1 && b->finalized, CMDB_ERR_INVALID, "cmdb_debug_exact_min: bad arguments");
     CMDB_CUDA(cudaSetDevice(b->device));
-    float *q = nullptr;
-    unsigned long long *keys = nullptr;
+    Buffer<float> q;
+    Buffer<unsigned long long> keys;
     std::vector<unsigned long long> h((size_t)P);
-    cudaError_t e = cudaMalloc(&q, sizeof(float) * (size_t)P * b->dim);
-    if (e == cudaSuccess) e = cudaMalloc(&keys, sizeof(unsigned long long) * (size_t)P);
+    CMDB_CUDA(q.alloc((size_t)P * b->dim));
+    CMDB_CUDA(keys.alloc(P));
     cudaStream_t st = b->handle_stream();
-    if (e == cudaSuccess) e = cudaMemcpyAsync(q, patch_host, sizeof(float) * (size_t)P * b->dim, cudaMemcpyHostToDevice, st);
-    int rc = CMDB_OK;
-    if (e == cudaSuccess) rc = score_exact_scan(b, st, q, P, keys);
-    if (e == cudaSuccess && rc == CMDB_OK) e = cudaMemcpyAsync(h.data(), keys, sizeof(unsigned long long) * (size_t)P, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess && rc == CMDB_OK) e = cudaStreamSynchronize(st);
-    cudaFree(q), cudaFree(keys);
-    if (rc != CMDB_OK) return rc;
-    CMDB_CUDA(e);
+    CMDB_CUDA(cudaMemcpyAsync(q, patch_host, sizeof(float) * (size_t)P * b->dim, cudaMemcpyHostToDevice, st));
+    CMDB_CHECK(score_exact_scan(b, st, q, P, keys));
+    CMDB_CUDA(cudaMemcpyAsync(h.data(), keys, sizeof(unsigned long long) * (size_t)P, cudaMemcpyDeviceToHost, st));
+    CMDB_CUDA(cudaStreamSynchronize(st));
     for (int i = 0; i < P; ++i) {
         const unsigned int bits = (unsigned int)(h[i] >> 32);
         float d2;
@@ -648,12 +645,9 @@ static int fused_alloc(cmdb_bank *b0, int out_hw) {
     if (f.cap_bytes >= need) return CMDB_OK;
     CMDB_REQUIRE(!f.active[0] && !f.active[1], CMDB_ERR_STATE, "fused scoring: out_hw grows while a submitted batch is outstanding");
     for (int i = 0; i < 2; ++i) {
-        cudaFree(f.dev[i]);
-        if (f.host[i]) cudaFreeHost(f.host[i]);
-        f.dev[i] = f.host[i] = nullptr;
-        CMDB_CUDA(cudaMalloc(&f.dev[i], need));
-        CMDB_CUDA(cudaMallocHost(&f.host[i], need));
-        if (!f.ev_done[i]) CMDB_CUDA(cudaEventCreateWithFlags(&f.ev_done[i], cudaEventDisableTiming));
+        CMDB_CUDA(f.dev[i].alloc(need));
+        CMDB_CUDA(f.host[i].alloc(need));
+        if (!f.ev_done[i]) CMDB_CUDA(f.ev_done[i].create());
     }
     f.cap_bytes = need;
     return CMDB_OK;
@@ -800,10 +794,9 @@ int cmdb_eval_reserve(cmdb_bank *b, int64_t n_images, int out_hw) {
     CMDB_REQUIRE(!f.active[0] && !f.active[1], CMDB_ERR_STATE, "cmdb_eval_reserve: a submitted batch is outstanding");
     CMDB_CUDA(cudaSetDevice(b->device));
     CMDB_CUDA(cudaStreamSynchronize(b->handle_stream()));
-    cudaFree(f.acc_maps), cudaFree(f.acc_scores);
-    f.acc_maps = f.acc_scores = nullptr, f.acc_cap = f.acc_n = 0, f.acc_npix = out_hw * out_hw;
-    CMDB_CUDA(cudaMalloc(&f.acc_maps, sizeof(double) * (size_t)n_images * f.acc_npix));
-    CMDB_CUDA(cudaMalloc(&f.acc_scores, sizeof(double) * (size_t)n_images));
+    f.acc_cap = f.acc_n = 0, f.acc_npix = out_hw * out_hw;
+    CMDB_CUDA(f.acc_maps.alloc((size_t)n_images * f.acc_npix));
+    CMDB_CUDA(f.acc_scores.alloc(n_images));
     f.acc_cap = n_images;
     return CMDB_OK;
 }
@@ -849,23 +842,19 @@ int cmdb_upsample_blur(int device, const float *map_host, int fh, int fw, int ou
     }
     CMDB_CUDA(cudaSetDevice(device));
     const size_t npix = (size_t)out_hw * out_hw;
-    float *in = nullptr, *pre = nullptr, *o = nullptr, *mx = nullptr;
-    unsigned char *u8 = nullptr, *tmp = nullptr;
-    cudaError_t e = cudaMalloc(&in, sizeof(float) * fh * fw);
-    if (e == cudaSuccess) e = cudaMalloc(&tmp, npix);
-    if (e == cudaSuccess) e = cudaMalloc(&mx, sizeof(float) * 17);
-    if (e == cudaSuccess) e = cudaMalloc(&pre, sizeof(float) * npix);
-    if (e == cudaSuccess) e = cudaMalloc(&o, sizeof(float) * npix);
-    if (e == cudaSuccess) e = cudaMalloc(&u8, npix);
-    if (e == cudaSuccess) e = cudaMemcpy(in, map_host, sizeof(float) * fh * fw, cudaMemcpyHostToDevice);
-    int rc = CMDB_OK;
-    if (e == cudaSuccess) rc = upsample_blur_launch(nullptr, 1, 0, 1, npix, in, fh, fw, out_hw, pre, o, u8, tmp, mx, mx + 1);
-    if (e == cudaSuccess && rc == CMDB_OK) e = cudaMemcpy(out_host, o, sizeof(float) * npix, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess && rc == CMDB_OK && out_pre_host) e = cudaMemcpy(out_pre_host, pre, sizeof(float) * npix, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess && rc == CMDB_OK && out_u8_host) e = cudaMemcpy(out_u8_host, u8, npix, cudaMemcpyDeviceToHost);
-    cudaFree(in), cudaFree(pre), cudaFree(o), cudaFree(u8), cudaFree(tmp), cudaFree(mx);
-    if (rc != CMDB_OK) return rc;
-    CMDB_CUDA(e);
+    Buffer<float> in, pre, o, mx;
+    Buffer<unsigned char> u8, tmp;
+    CMDB_CUDA(in.alloc(fh * fw));
+    CMDB_CUDA(tmp.alloc(npix));
+    CMDB_CUDA(mx.alloc(17));
+    CMDB_CUDA(pre.alloc(npix));
+    CMDB_CUDA(o.alloc(npix));
+    CMDB_CUDA(u8.alloc(npix));
+    CMDB_CUDA(cudaMemcpy(in, map_host, sizeof(float) * fh * fw, cudaMemcpyHostToDevice));
+    CMDB_CHECK(upsample_blur_launch(nullptr, 1, 0, 1, npix, in, fh, fw, out_hw, pre, o, u8, tmp, mx, mx + 1));
+    CMDB_CUDA(cudaMemcpy(out_host, o, sizeof(float) * npix, cudaMemcpyDeviceToHost));
+    if (out_pre_host) CMDB_CUDA(cudaMemcpy(out_pre_host, pre, sizeof(float) * npix, cudaMemcpyDeviceToHost));
+    if (out_u8_host) CMDB_CUDA(cudaMemcpy(out_u8_host, u8, npix, cudaMemcpyDeviceToHost));
     return CMDB_OK;
 }
 

@@ -3,7 +3,7 @@
 // run_coreset (reference multiple_features.py:37-48 and the five other variants).
 #include <math.h>
 
-#include <cstdlib>
+#include <memory>
 
 #include "common.cuh"
 
@@ -214,6 +214,14 @@ int cmdb_version(void) { return 100; }
 
 const char *cmdb_last_error(void) { return cmdb::g_err; }
 
+// host-only test hook (not in the public header): what the library's resource owners hold in this process -- device
+// bytes, pinned host bytes, streams, events
+int cmdb_debug_live_resources(int64_t *out4) {
+    CMDB_REQUIRE(out4, CMDB_ERR_INVALID, "cmdb_debug_live_resources: out4 is NULL");
+    for (int i = 0; i < 4; ++i) out4[i] = live_resources[i];
+    return CMDB_OK;
+}
+
 int cmdb_device_count(int *out_n) {
     CMDB_REQUIRE(out_n != nullptr, CMDB_ERR_INVALID, "cmdb_device_count: out_n is NULL");
     int n = 0;
@@ -232,6 +240,28 @@ int cmdb_device_count(int *out_n) {
     return CMDB_OK;
 }
 
+// the streams, events and buffers a handle holds from creation on, in the order of first use
+static cudaError_t create_handle_resources(cmdb_bank *b) {
+    if (cudaError_t e = b->copy_stream.create()) return e;
+    if (cudaError_t e = b->d2h_stream.create()) return e;
+    for (Lane &l : b->lane) {
+        if (cudaError_t e = l.stream.create()) return e;
+        if (cudaError_t e = l.aux.create()) return e;
+        if (cudaError_t e = l.ev_fork.create()) return e;
+        if (cudaError_t e = l.ev_join.create()) return e;
+    }
+    for (ResultSlot &s : b->slot) {
+        if (cudaError_t e = s.ev_done.create()) return e;
+        if (cudaError_t e = s.ev_compute.create()) return e;
+    }
+    if (cudaError_t e = b->ev_fail.create()) return e;
+    for (Event &ev : b->ev_chunk)
+        if (cudaError_t e = ev.create()) return e;
+    if (cudaError_t e = b->data.alloc((size_t)b->capacity * b->dim)) return e;
+    if (cudaError_t e = b->stats_buf.alloc(2 + (size_t)b->num_sms * 4)) return e;
+    return b->absmax_buf.alloc(1);
+}
+
 int cmdb_bank_create(int device, int dim, int64_t capacity_rows, cmdb_bank **out) {
     CMDB_REQUIRE(out != nullptr, CMDB_ERR_INVALID, "cmdb_bank_create: out is NULL");
     *out = nullptr;
@@ -244,7 +274,7 @@ int cmdb_bank_create(int device, int dim, int64_t capacity_rows, cmdb_bank **out
     if (e != cudaSuccess || ndev == 0) {
         (void)cudaGetLastError();
         set_error("cmdb_bank_create: no CUDA device (%s); this library has no CPU fallback",
-                  e == cudaSuccess ? "device count is 0" : cudaGetErrorString(e));
+                  e != cudaSuccess ? cudaGetErrorString(e) : "device count is 0");
         return CMDB_ERR_CUDA;
     }
     CMDB_REQUIRE(device >= 0 && device < ndev, CMDB_ERR_INVALID, "cmdb_bank_create: device %d out of range [0,%d)", device,
@@ -254,90 +284,26 @@ int cmdb_bank_create(int device, int dim, int64_t capacity_rows, cmdb_bank **out
     CMDB_REQUIRE(major == 10, CMDB_ERR_CUDA, "cmdb_bank_create: device %d is sm_%d0, this library is sm_100a only", device,
                  major);
     CMDB_CUDA(cudaSetDevice(device));
-    cmdb_bank *b = new cmdb_bank();
+    std::unique_ptr<cmdb_bank> b(new cmdb_bank());
     b->device = device;
     b->dim = dim;
     b->capacity = capacity_rows;
     cudaDeviceGetAttribute(&b->num_sms, cudaDevAttrMultiProcessorCount, device);
-    cudaError_t err = cudaStreamCreateWithFlags(&b->copy_stream, cudaStreamNonBlocking);
-    if (err == cudaSuccess) err = cudaStreamCreateWithFlags(&b->d2h_stream, cudaStreamNonBlocking);
-    for (Lane &l : b->lane) {
-        if (err == cudaSuccess) err = cudaStreamCreateWithFlags(&l.stream, cudaStreamNonBlocking);
-        if (err == cudaSuccess) err = cudaStreamCreateWithFlags(&l.aux, cudaStreamNonBlocking);
-        if (err == cudaSuccess) err = cudaEventCreateWithFlags(&l.ev_fork, cudaEventDisableTiming);
-        if (err == cudaSuccess) err = cudaEventCreateWithFlags(&l.ev_join, cudaEventDisableTiming);
-    }
-    for (ResultSlot &s : b->slot) {
-        if (err == cudaSuccess) err = cudaEventCreateWithFlags(&s.ev_done, cudaEventDisableTiming);
-        if (err == cudaSuccess) err = cudaEventCreateWithFlags(&s.ev_compute, cudaEventDisableTiming);
-    }
-    if (err == cudaSuccess) err = cudaEventCreateWithFlags(&b->ev_fail, cudaEventDisableTiming);
-    for (auto &e : b->ev_chunk)
-        if (err == cudaSuccess) err = cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
-    if (err == cudaSuccess) err = cudaMalloc(&b->data, sizeof(float) * (size_t)capacity_rows * dim);
-    if (err == cudaSuccess) err = cudaMalloc(&b->stats_buf, sizeof(double) * (2 + (size_t)b->num_sms * 4));
-    if (err == cudaSuccess) err = cudaMalloc(&b->absmax_buf, sizeof(unsigned int));
+    const cudaError_t err = create_handle_resources(b.get());
     if (err != cudaSuccess) {
         set_error("cmdb_bank_create: allocation of %lld x %d floats failed: %s", (long long)capacity_rows, dim,
                   cudaGetErrorString(err));
         (void)cudaGetLastError();
-        cmdb_bank_destroy(b);
         return CMDB_ERR_CUDA;
     }
-    *out = b;
+    *out = b.release();
     return CMDB_OK;
-}
-
-static void free_scoring_layout(cmdb_bank *b) {
-    cudaFree(b->hi);
-    cudaFree(b->lo);
-    cudaFree(b->norm);
-    cudaFree(b->knn_table);
-    b->knn_table = nullptr, b->knn_rows = 0;
-    b->hi = b->lo = nullptr;
-    b->norm = nullptr;
-    free(b->tmap_hi);
-    free(b->tmap_lo);
-    free(b->tmap_hi2);
-    free(b->tmap_lo2);
-    b->tmap_hi = b->tmap_lo = b->tmap_hi2 = b->tmap_lo2 = nullptr;
-    score_scratch_free(b);
-    b->finalized = false;
 }
 
 void cmdb_bank_destroy(cmdb_bank *b) {
     if (!b) return;
     cudaSetDevice(b->device);
-    free_scoring_layout(b);   // synchronises every stream of the handle first
-    for (int i = 0; i < 2; ++i) {
-        cudaFree(b->fused.dev[i]);
-        if (b->fused.host[i]) cudaFreeHost(b->fused.host[i]);
-        if (b->fused.ev_done[i]) cudaEventDestroy(b->fused.ev_done[i]);
-    }
-    cudaFree(b->fused.acc_maps), cudaFree(b->fused.acc_scores);
-    cudaFree(b->shard_ctr), cudaFree(b->shard_d2);
-    if (b->shard_abort_host) cudaFreeHost(b->shard_abort_host);
-    cudaFree(b->data);
-    cudaFree(b->stats_buf);
-    cudaFree(b->absmax_buf);
-    cudaFree(b->cert_buf);
-    for (auto &e : b->ev)
-        if (e) cudaEventDestroy(e);
-    for (Lane &l : b->lane) {
-        if (l.stream) cudaStreamDestroy(l.stream);
-        if (l.aux) cudaStreamDestroy(l.aux);
-        if (l.ev_fork) cudaEventDestroy(l.ev_fork);
-        if (l.ev_join) cudaEventDestroy(l.ev_join);
-    }
-    if (b->copy_stream) cudaStreamDestroy(b->copy_stream);
-    if (b->d2h_stream) cudaStreamDestroy(b->d2h_stream);
-    for (ResultSlot &s : b->slot) {
-        if (s.ev_done) cudaEventDestroy(s.ev_done);
-        if (s.ev_compute) cudaEventDestroy(s.ev_compute);
-    }
-    if (b->ev_fail) cudaEventDestroy(b->ev_fail);
-    for (auto &e : b->ev_chunk)
-        if (e) cudaEventDestroy(e);
+    b->sync_streams();
     delete b;
 }
 
@@ -391,11 +357,13 @@ int cmdb_bank_set_option(cmdb_bank *b, int option, int value) {
         return CMDB_OK;
     }
     if (option == CMDB_OPT_TIMING) {
-        b->timing = value != 0;
-        if (b->timing && !b->ev[0]) {
+        if (value && !b->ev[0]) {   // all events exist before timing is on
             CMDB_CUDA(cudaSetDevice(b->device));
-            for (auto &e : b->ev) CMDB_CUDA(cudaEventCreate(&e));
+            Event ev[CMDB_T_COUNT + 1];
+            for (Event &e : ev) CMDB_CUDA(e.create(cudaEventDefault));
+            for (int i = 0; i <= CMDB_T_COUNT; ++i) b->ev[i] = std::move(ev[i]);
         }
+        b->timing = value != 0;
         b->ev_valid = false;
         return CMDB_OK;
     }
@@ -477,9 +445,8 @@ int cmdb_bank_set_knn_table(cmdb_bank *b, const uint64_t *keys, int64_t n_rows_t
     CMDB_REQUIRE(!b->any_pending(), CMDB_ERR_STATE, "cmdb_bank_set_knn_table: a submitted batch is outstanding");
     CMDB_CUDA(cudaSetDevice(b->device));
     CMDB_CUDA(cudaStreamSynchronize(b->handle_stream()));
-    cudaFree(b->knn_table);
-    b->knn_table = nullptr, b->knn_rows = 0;
-    CMDB_CUDA(cudaMalloc(&b->knn_table, sizeof(uint64_t) * 3 * (size_t)n_rows_total));
+    b->knn_rows = 0;
+    CMDB_CUDA(b->knn_table.alloc(3 * (size_t)n_rows_total));
     CMDB_CUDA(cudaMemcpyAsync(b->knn_table, keys, sizeof(uint64_t) * 3 * (size_t)n_rows_total,
                               keys_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, b->handle_stream()));
     CMDB_CUDA(cudaStreamSynchronize(b->handle_stream()));
@@ -549,26 +516,16 @@ int cmdb_bank_gather(cmdb_bank *b, const int64_t *idx_host, int64_t n) {
                      (long long)b->rows);
     CMDB_REQUIRE(!b->any_pending(), CMDB_ERR_STATE, "cmdb_bank_gather: a submitted call still reads the rows; wait for it first");
     CMDB_CUDA(cudaSetDevice(b->device));
-    long long *idx_dev = nullptr;
-    float *tmp = nullptr;
-    CMDB_CUDA(cudaMalloc(&idx_dev, sizeof(long long) * (size_t)n));
-    cudaError_t e = cudaMalloc(&tmp, sizeof(float) * (size_t)n * b->dim);
-    if (e != cudaSuccess) {
-        cudaFree(idx_dev);
-        CMDB_CUDA(e);
-    }
-    e = cudaMemcpyAsync(idx_dev, idx_host, sizeof(long long) * (size_t)n, cudaMemcpyHostToDevice, b->handle_stream());
-    if (e == cudaSuccess) {
-        int grid = (int)std::min<int64_t>((n + 7) / 8, (int64_t)b->num_sms * 8);
-        gather_rows_kernel<<<grid, 256, 0, b->handle_stream()>>>(b->data, tmp, idx_dev, n, b->dim / 4);
-        e = cudaGetLastError();
-    }
-    if (e == cudaSuccess)
-        e = cudaMemcpyAsync(b->data, tmp, sizeof(float) * (size_t)n * b->dim, cudaMemcpyDeviceToDevice, b->handle_stream());
-    if (e == cudaSuccess) e = cudaStreamSynchronize(b->handle_stream());
-    cudaFree(idx_dev);
-    cudaFree(tmp);
-    CMDB_CUDA(e);
+    Buffer<long long> idx_dev;
+    Buffer<float> tmp;
+    CMDB_CUDA(idx_dev.alloc(n));
+    CMDB_CUDA(tmp.alloc((size_t)n * b->dim));
+    CMDB_CUDA(cudaMemcpyAsync(idx_dev, idx_host, sizeof(long long) * (size_t)n, cudaMemcpyHostToDevice, b->handle_stream()));
+    int grid = (int)std::min<int64_t>((n + 7) / 8, (int64_t)b->num_sms * 8);
+    gather_rows_kernel<<<grid, 256, 0, b->handle_stream()>>>(b->data, tmp, idx_dev, n, b->dim / 4);
+    CMDB_CUDA(cudaGetLastError());
+    CMDB_CUDA(cudaMemcpyAsync(b->data, tmp, sizeof(float) * (size_t)n * b->dim, cudaMemcpyDeviceToDevice, b->handle_stream()));
+    CMDB_CUDA(cudaStreamSynchronize(b->handle_stream()));
     b->rows = n;
     b->finalized = false;
     return CMDB_OK;
@@ -594,16 +551,18 @@ int cmdb_bank_finalize(cmdb_bank *b) {
     CMDB_REQUIRE(!b->any_pending(), CMDB_ERR_STATE,
                  "cmdb_bank_finalize: a submitted call still uses the scoring layout; wait for it first");
     CMDB_CUDA(cudaSetDevice(b->device));
-    free_scoring_layout(b);
+    score_scratch_free(b);   // synchronises every stream of the handle first
+    static_cast<FinalizeBuffers &>(*b) = FinalizeBuffers();
+    b->finalized = false;
     const int64_t pad = (b->rows + kScoreBN - 1) / kScoreBN * kScoreBN;
-    CMDB_CUDA(cudaMalloc(&b->hi, sizeof(__half) * (size_t)pad * b->dim));
-    CMDB_CUDA(cudaMalloc(&b->lo, sizeof(__half) * (size_t)pad * b->dim));
-    CMDB_CUDA(cudaMalloc(&b->norm, sizeof(float) * (size_t)pad));
+    CMDB_CUDA(b->hi.alloc((size_t)pad * b->dim));
+    CMDB_CUDA(b->lo.alloc((size_t)pad * b->dim));
+    CMDB_CUDA(b->norm.alloc(pad));
     float absmax = 0.f;
     CMDB_CHECK(bank_max_abs(b, b->data, b->rows * b->dim, &absmax));
     CMDB_REQUIRE(isfinite(absmax), CMDB_ERR_INVALID, "cmdb_bank_finalize: bank contains non-finite values");
     b->scale_exp = pick_scale_exp(absmax);
-    if (!b->cert_buf) CMDB_CUDA(cudaMalloc(&b->cert_buf, 2 * sizeof(unsigned int)));
+    if (!b->cert_buf) CMDB_CUDA(b->cert_buf.alloc(2));
     CMDB_CUDA(cudaMemsetAsync(b->cert_buf, 0, 2 * sizeof(unsigned int), b->handle_stream()));
     launch_split_rows(b->handle_stream(), b->num_sms, b->data, b->rows, pad, b->dim, b->scale_exp, b->hi, b->lo, b->norm, INFINITY,
                       b->cert_buf);

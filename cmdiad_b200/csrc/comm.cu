@@ -2,16 +2,23 @@
 // box can write over NVLink (CUDA IPC mapping, one process per GPU).  The persistent coreset kernel uses it for the
 // per-pick exchange of (value,row) candidates and of the winning row itself -- no host launch, no NCCL call per pick.
 #include <algorithm>
+#include <memory>
 
 #include "common.cuh"
 
 struct cmdb_comm {
     int device = 0, rank = 0, world = 1;
     size_t bytes = 0;
-    unsigned char *local = nullptr;                 // this rank's mailbox (device memory)
+    cmdb::Buffer<unsigned char> local;              // this rank's mailbox
     unsigned char *peer[cmdb::kMaxRanks] = {};      // every rank's mailbox as mapped into this process (peer[rank] == local)
     bool imported = false;
     unsigned long long score_epoch = 0;  // round counter of the sharded-scoring exchange (monotone per buffer, same on every rank)
+    ~cmdb_comm() {   // peers may still write into the mailbox: synchronise, close the imported mappings, then free it
+        cudaSetDevice(device);
+        cudaDeviceSynchronize();
+        for (int r = 0; r < world; ++r)
+            if (r != rank && peer[r]) cudaIpcCloseMemHandle(peer[r]);
+    }
 };
 
 using namespace cmdb;
@@ -25,18 +32,16 @@ int cmdb_comm_create(int device, int rank, int world, size_t mailbox_bytes, cmdb
                  "cmdb_comm_create: rank %d / world %d not supported (max %d ranks)", rank, world, kMaxRanks);
     CMDB_REQUIRE(mailbox_bytes >= 64, CMDB_ERR_INVALID, "cmdb_comm_create: mailbox too small");
     CMDB_CUDA(cudaSetDevice(device));
-    cmdb_comm *c = new cmdb_comm();
+    std::unique_ptr<cmdb_comm> c(new cmdb_comm());
     c->device = device, c->rank = rank, c->world = world, c->bytes = (mailbox_bytes + 255) & ~size_t(255);
-    cudaError_t e = cudaMalloc(&c->local, c->bytes);
-    if (e == cudaSuccess) e = cudaMemset(c->local, 0, c->bytes);
-    if (e != cudaSuccess) {
+    cudaError_t e = c->local.alloc(c->bytes);
+    if (e != cudaSuccess || (e = cudaMemset(c->local, 0, c->bytes)) != cudaSuccess) {
         set_error("cmdb_comm_create: %s", cudaGetErrorString(e));
         (void)cudaGetLastError();
-        delete c;
         return CMDB_ERR_CUDA;
     }
     c->peer[rank] = c->local;
-    *out = c;
+    *out = c.release();
     return CMDB_OK;
 }
 
@@ -79,15 +84,7 @@ int cmdb_comm_reset(cmdb_comm *c) {
     return CMDB_OK;
 }
 
-void cmdb_comm_destroy(cmdb_comm *c) {
-    if (!c) return;
-    cudaSetDevice(c->device);
-    cudaDeviceSynchronize();
-    for (int r = 0; r < c->world; ++r)
-        if (r != c->rank && c->peer[r]) cudaIpcCloseMemHandle(c->peer[r]);
-    cudaFree(c->local);
-    delete c;
-}
+void cmdb_comm_destroy(cmdb_comm *c) { delete c; }
 
 }  // extern "C"
 

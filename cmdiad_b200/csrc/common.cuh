@@ -1,12 +1,15 @@
 // Shared declarations of the cmdiad_b200 CUDA library (sm_100a only).
 #pragma once
+#include <cuda.h>
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <atomic>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <utility>
 
 #include "../../include/cmdiad_b200.h"
 
@@ -37,6 +40,82 @@ void set_error(const char *fmt, ...);
             return status;                \
         }                                 \
     } while (0)
+
+// Owners of the library's CUDA resources, move-only: the destructor releases what they hold, so a group of them is
+// released by assigning it a fresh value, and a function's temporaries are freed on every return.  They count what they
+// hold in this process (cmdb_debug_live_resources): device bytes, pinned host bytes, streams, events.
+enum { kLiveDeviceBytes, kLivePinnedBytes, kLiveStreams, kLiveEvents };
+inline std::atomic<long long> live_resources[4];
+
+enum class Mem { Device, Pinned, Mapped };  // cudaMalloc, cudaMallocHost, cudaHostAlloc(cudaHostAllocMapped)
+
+template <typename T, Mem M = Mem::Device>
+class Buffer {
+  public:
+    Buffer() = default;
+    Buffer(Buffer &&o) noexcept { *this = std::move(o); }
+    Buffer &operator=(Buffer &&o) noexcept {
+        if (this != &o) reset(), p_ = std::exchange(o.p_, nullptr), bytes_ = std::exchange(o.bytes_, 0);
+        return *this;
+    }
+    ~Buffer() { reset(); }
+    cudaError_t alloc(size_t n) {  // n elements of T
+        reset();
+        void *p = nullptr;
+        const size_t bytes = sizeof(T) * n;
+        const cudaError_t e = M == Mem::Device   ? cudaMalloc(&p, bytes)
+                              : M == Mem::Pinned ? cudaMallocHost(&p, bytes)
+                                                 : cudaHostAlloc(&p, bytes, cudaHostAllocMapped);
+        if (e != cudaSuccess) return e;
+        p_ = static_cast<T *>(p), bytes_ = bytes;
+        live_resources[kind] += (long long)bytes;
+        return cudaSuccess;
+    }
+    void reset() {
+        if (!p_) return;
+        (void)(M == Mem::Device ? cudaFree(p_) : cudaFreeHost(p_));
+        live_resources[kind] -= (long long)bytes_;
+        p_ = nullptr, bytes_ = 0;
+    }
+    T *get() const { return p_; }
+    operator T *() const { return p_; }
+
+  private:
+    static constexpr int kind = M == Mem::Device ? kLiveDeviceBytes : kLivePinnedBytes;
+    T *p_ = nullptr;
+    size_t bytes_ = 0;
+};
+
+template <typename H, cudaError_t (*Create)(H *, unsigned), cudaError_t (*Destroy)(H), int kind, unsigned kFlags>
+class Handle {
+  public:
+    Handle() = default;
+    Handle(Handle &&o) noexcept { *this = std::move(o); }
+    Handle &operator=(Handle &&o) noexcept {
+        if (this != &o) reset(), h_ = std::exchange(o.h_, nullptr);
+        return *this;
+    }
+    ~Handle() { reset(); }
+    cudaError_t create(unsigned flags = kFlags) {
+        reset();
+        const cudaError_t e = Create(&h_, flags);
+        if (e != cudaSuccess) return h_ = nullptr, e;
+        ++live_resources[kind];
+        return cudaSuccess;
+    }
+    void reset() {
+        if (!h_) return;
+        (void)Destroy(h_);
+        --live_resources[kind];
+        h_ = nullptr;
+    }
+    operator H() const { return h_; }
+
+  private:
+    H h_ = nullptr;
+};
+using Stream = Handle<cudaStream_t, cudaStreamCreateWithFlags, cudaStreamDestroy, kLiveStreams, cudaStreamNonBlocking>;
+using Event = Handle<cudaEvent_t, cudaEventCreateWithFlags, cudaEventDestroy, kLiveEvents, cudaEventDisableTiming>;
 
 constexpr int kNumSMsDefault = 148;
 constexpr int kMaxRanks = 8;         // GPUs of one NVSwitch box
@@ -71,51 +150,60 @@ struct ScoreLayout {
     int n_topk_blocks = 0;  // blocks of reweight_kernel
 };
 
-// A compute lane: the streams a call runs on and every device buffer that lives only while a call computes.  Call k runs on
-// lane k & 1, so the tail of a batch / round -- certificate, rescans, exchanges, re-weighting, maps -- overlaps the
-// distance GEMM of the next one (the GEMM is one persistent CTA per SM; the small tail kernels fit beside it).
-struct Lane {
-    cudaStream_t stream = nullptr;
-    cudaStream_t aux = nullptr;     // side stream of the (normally empty) tier-2 launches and the counters copy, beside the rescan
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-    __half *q_hi = nullptr;         // [cap_p, D]  split-fp16 query operand
-    __half *q_lo = nullptr;
-    int *q_scale_exp = nullptr;     // device [cap_p]: per-row exponent e_q with q_hi + q_lo = q * 2^e_q
-    float *q_norm = nullptr;        // [cap_p] ||q|| (rounded up)            -- certified pre-filter, score_tail.cu
-    float *q_eps = nullptr;         // [cap_p] ||q - q_hi * 2^-e_q|| (rounded up)
-    int *fail_list = nullptr;       // [cap_p] query rows whose pre-filter result could not be certified
+// The scratch of a compute lane: every device buffer that lives only while a call computes (score_scratch_alloc /
+// score_scratch_free).
+struct LaneScratch {
+    Buffer<__half> q_hi;            // [cap_p, D]  split-fp16 query operand
+    Buffer<__half> q_lo;
+    Buffer<int> q_scale_exp;        // device [cap_p]: per-row exponent e_q with q_hi + q_lo = q * 2^e_q
+    Buffer<float> q_norm;           // [cap_p] ||q|| (rounded up)            -- certified pre-filter, score_tail.cu
+    Buffer<float> q_eps;            // [cap_p] ||q - q_hi * 2^-e_q|| (rounded up)
+    Buffer<int> fail_list;          // [cap_p] query rows whose pre-filter result could not be certified
     // device control block of the fallback: [0] uncertified queries, [1] (query, producer) pairs to rescan,
     // [2] rows of the 3-term GEMM fallback, [3] pairs of the exact rescan, [4] queries the rescan finishes
     // ([2..4] are derived from [0..1] by the last block of refine_cert_kernel: pairs that fit the work list -> rescan, more ->
     // GEMM), [5] / [6] last-block tickets of the certificate / rescan kernels; the per-image argmax keys (s_key) follow at
     // fail_ctl + 8 in the same allocation so that one memset clears both
-    int *fail_ctl = nullptr;
+    Buffer<int> fail_ctl;
     unsigned long long *s_key = nullptr;    // [cap_b] packed argmax key of min_val
-    int *fail_count_host = nullptr; // pinned copy of [0..1] (statistics / adaptive mode)
-    int2 *work_list = nullptr;      // [kWorkCap] (query row, producer) pairs whose producer may hide rows inside the band
+    Buffer<int, Mem::Pinned> fail_count_host;  // pinned copy of [0..1] (statistics / adaptive mode)
+    Buffer<int2> work_list;         // [kWorkCap] (query row, producer) pairs whose producer may hide rows inside the band
     // [cap_p] running exact (d^2 bits << 32 | row) of the uncertified queries; of every query in the CUDA-core mode
-    unsigned long long *best_key = nullptr;
-    unsigned int *done_counter = nullptr;  // last-block-done counter of reweight_kernel
-    float4 *cand = nullptr;         // [n_ctas, cap_p] per-CTA running top-2 (val1, idx1, val2, idx2) of the GEMM epilogue
-    unsigned char *map_tmp = nullptr;  // horizontally blurred 8-bit images between the two blur kernels
-    float *map_max = nullptr;       // [cap_b] map maxima, then [cap_b][16] band maxima
-    unsigned long long *topk_keys = nullptr;  // [n_blocks*3] per-block w_dist top-3 packed keys
-    unsigned long long *top3 = nullptr;  // merged 3 smallest w_dist keys
-    float *m_test = nullptr;        // [cap_b, D] patch[s_idx]
-    float *m_star = nullptr;        // [cap_b, D] bank[min_idx[s_idx]]
-    void *tmap_qhi = nullptr;       // host CUtensorMap objects for q_hi / q_lo
-    void *tmap_qlo = nullptr;
+    Buffer<unsigned long long> best_key;
+    Buffer<unsigned int> done_counter;  // last-block-done counter of reweight_kernel
+    Buffer<float4> cand;            // [n_ctas, cap_p] per-CTA running top-2 (val1, idx1, val2, idx2) of the GEMM epilogue
+    Buffer<unsigned char> map_tmp;  // horizontally blurred 8-bit images between the two blur kernels
+    Buffer<float> map_max;          // [cap_b] map maxima, then [cap_b][16] band maxima
+    Buffer<unsigned long long> topk_keys;  // [n_blocks*3] per-block w_dist top-3 packed keys
+    Buffer<unsigned long long> top3;  // merged 3 smallest w_dist keys
+    Buffer<float> m_test;           // [cap_b, D] patch[s_idx]
+    Buffer<float> m_star;           // [cap_b, D] bank[min_idx[s_idx]]
+    CUtensorMap tmap_qhi{}, tmap_qlo{};  // of q_hi / q_lo
+};
+
+// A compute lane: its scratch and the streams a call runs on, which live as long as the handle.  Call k runs on lane k & 1,
+// so the tail of a batch / round -- certificate, rescans, exchanges, re-weighting, maps -- overlaps the distance GEMM of
+// the next one (the GEMM is one persistent CTA per SM; the small tail kernels fit beside it).
+struct Lane : LaneScratch {
+    Stream stream;
+    Stream aux;                     // side stream of the (normally empty) tier-2 launches and the counters copy, beside the rescan
+    Event ev_fork, ev_join;
+};
+
+// The scratch of a result slot: the query and result blocks (score_scratch_alloc / score_scratch_free).
+struct SlotScratch {
+    Buffer<float> q_f32;                    // [cap_p, D] normalised query patches
+    Buffer<unsigned char> out_block;        // device result block (ScoreLayout)
+    Buffer<unsigned char, Mem::Pinned> out_block_host;  // its pinned mirror
 };
 
 // A result slot: what a submitted call holds until the caller has waited for it.  The slots cycle independently of the
 // lanes (call k uses slot k % kResultSlots), so the results of calls k - 1 and k travel to the host / wait for the caller
-// while call k + 1 is already enqueued, and its queries are staged while call k is still scored.
-struct ResultSlot {
-    float *q_f32 = nullptr;                 // [cap_p, D] normalised query patches
-    unsigned char *out_block = nullptr;     // device result block (ScoreLayout)
-    unsigned char *out_block_host = nullptr;  // its pinned mirror
-    cudaEvent_t ev_done = nullptr;          // the block is in the pinned host memory
-    cudaEvent_t ev_compute = nullptr;       // the kernels of the call that used the slot are done (q_f32 may be overwritten)
+// while call k + 1 is already enqueued, and its queries are staged while call k is still scored.  The events live as long
+// as the handle.
+struct ResultSlot : SlotScratch {
+    Event ev_done;                          // the block is in the pinned host memory
+    Event ev_compute;                       // the kernels of the call that used the slot are done (q_f32 may be overwritten)
     struct Pending {
         bool active = false;
         int B = 0, P = 0, out_hw = 0;
@@ -126,9 +214,26 @@ struct ResultSlot {
     } pending;
 };
 
+// The scoring layout that cmdb_bank_finalize builds from the rows, and the neighbour table built on it: a new finalize
+// releases all of it.
+struct FinalizeBuffers {
+    Buffer<__half> hi;        // [fin_rows_pad, dim] fp16(x * 2^scale_exp)
+    Buffer<__half> lo;        // [fin_rows_pad, dim] fp16(x * 2^scale_exp - hi)
+    Buffer<float> norm;       // [fin_rows_pad] ||x * 2^scale_exp||^2 ; +inf on padding rows
+    CUtensorMap tmap_hi{}, tmap_lo{};
+    CUtensorMap tmap_hi2{}, tmap_lo2{};  // box of 128 bank rows (CTA-pair kernels)
+    // optional table of the three nearest bank rows of every bank row, as packed (d^2 bits << 32 | row) keys
+    // (cmdb_bank_build_knn; SURVEY 8f-1): turns the per-image w_dist pass into a lookup
+    Buffer<unsigned long long> knn_table;  // [knn_rows][3]
+    // rows the table covers: fin_rows for a table built on this handle (cmdb_bank_build_knn); the GLOBAL row count for a
+    // replicated table installed on a row-sharded handle (cmdb_bank_set_knn_table)
+    long long knn_rows = 0;
+};
+
 }  // namespace cmdb
 
-struct cmdb_bank {
+// Every other member lives as long as the handle; cmdb_bank_destroy synchronises the streams and deletes it.
+struct cmdb_bank : cmdb::FinalizeBuffers {
     int device = 0;
     int dim = 0;
     int num_sms = cmdb::kNumSMsDefault;
@@ -142,13 +247,7 @@ struct cmdb_bank {
     // error-bound inputs of the certificate, true units, rounded up (cmdb_bank_finalize)
     float cert_bmax = 0.f;    // max ||b||
     float cert_eb_max = 0.f;  // max ||b - b_hi * 2^-scale_exp||
-    unsigned int *cert_buf = nullptr;  // device [2]: the two maxima as float bits
-    // optional table of the three nearest bank rows of every bank row, as packed (d^2 bits << 32 | row) keys
-    // (cmdb_bank_build_knn; SURVEY 8f-1): turns the per-image w_dist pass into a lookup
-    unsigned long long *knn_table = nullptr;  // [knn_rows][3]
-    // rows the table covers: fin_rows for a table built on this handle (cmdb_bank_build_knn); the GLOBAL row count for a
-    // replicated table installed on a row-sharded handle (cmdb_bank_set_knn_table)
-    long long knn_rows = 0;
+    cmdb::Buffer<unsigned int> cert_buf;  // device [2]: the two maxima as float bits
     // statistics of the last scoring call / adaptive fallback to the direct 3-term GEMM
     int64_t last_queries = 0;
     int last_mode = 0;           // GEMM mode the last call actually ran
@@ -166,11 +265,16 @@ struct cmdb_bank {
     // the sharded round opened by cmdb_score_shard_min and closed by cmdb_score_shard_finish_submit
     struct Round { bool open = false; int lane = 0, slot = 0; } round;
     int *last_fail_host = nullptr;   // pinned certificate counters of the most recent certified call (either lane)
-    cudaStream_t copy_stream = nullptr;   // host -> device staging of query chunks, overlapped with the GEMM of earlier chunks
-    cudaEvent_t ev_chunk[cmdb::kMaxStageChunks] = {};
-    cudaStream_t d2h_stream = nullptr;    // device -> host copies of the results
-    cudaEvent_t ev_fail = nullptr;        // the certificate counters of the last certified call are on the host
+    cmdb::Stream copy_stream;   // host -> device staging of query chunks, overlapped with the GEMM of earlier chunks
+    cmdb::Event ev_chunk[cmdb::kMaxStageChunks];
+    cmdb::Stream d2h_stream;    // device -> host copies of the results
+    cmdb::Event ev_fail;        // the certificate counters of the last certified call are on the host
     cudaStream_t handle_stream() const { return lane[0].stream; }
+    void sync_streams() const {  // no copy or kernel of the handle is in flight afterwards
+        const cudaStream_t all[] = {copy_stream, d2h_stream, lane[0].stream, lane[0].aux, lane[1].stream, lane[1].aux};
+        for (cudaStream_t s : all)
+            if (s) cudaStreamSynchronize(s);
+    }
     bool any_pending() const {  // a submitted call (batch, round, fused batch) still uses the handle's buffers
         for (const auto &s : slot)
             if (s.pending.active) return true;
@@ -183,10 +287,10 @@ struct cmdb_bank {
     // late-fusion head on the device (cmdb_score_fused_batch*; this handle is modality 0 of the fused call): per slot the
     // fused float64 maps / image scores / lambda-scaled per-modality s in one device block mirrored by a pinned host block
     struct Fused {
-        unsigned char *dev[2] = {nullptr, nullptr};
-        unsigned char *host[2] = {nullptr, nullptr};
+        cmdb::Buffer<unsigned char> dev[2];
+        cmdb::Buffer<unsigned char, cmdb::Mem::Pinned> host[2];
         size_t cap_bytes = 0;
-        cudaEvent_t ev_done[2] = {};
+        cmdb::Event ev_done[2];
         bool active[2] = {false, false};
         int next_fs = 0;   // fused block of the next fused call (two fused batches may be outstanding)
         int n_modal[2] = {0, 0}, B[2] = {0, 0}, out_hw[2] = {0, 0};
@@ -194,35 +298,28 @@ struct cmdb_bank {
         int slots[2][3] = {};
         long long ticket[2] = {0, 0};
         // device-resident accumulation of the fused maps over predict calls (cmdb_eval_*; SURVEY 8f-3)
-        double *acc_maps = nullptr;     // [acc_cap][npix]
-        double *acc_scores = nullptr;   // [acc_cap]
+        cmdb::Buffer<double> acc_maps;     // [acc_cap][npix]
+        cmdb::Buffer<double> acc_scores;   // [acc_cap]
         long long acc_cap = 0, acc_n = 0;
         int acc_npix = 0;
     } fused;
     long long ticket_counter = 0;
     cmdb_comm *comm = nullptr;             // peer buffers for NCCL-free sharded rounds (cmdb_bank_attach_comm; not owned)
-    unsigned int *shard_ctr = nullptr;     // [0] device: last-block counter of the push kernels
-    unsigned int *shard_abort_host = nullptr;  // pinned + mapped: set by a kernel whose peers never arrived
+    cmdb::Buffer<unsigned int> shard_ctr;  // [0] device: last-block counter of the push kernels
+    cmdb::Buffer<unsigned int, cmdb::Mem::Mapped> shard_abort_host;  // set by a kernel whose peers never arrived
     unsigned int *shard_abort_dev = nullptr;   // device alias of shard_abort_host
-    float *shard_d2 = nullptr;             // device [2][kShardD2Cap]: local contributions / sums of the neighbour distances
-    float *data = nullptr;  // [capacity, dim] float32 row-major
-    // scoring layout (cmdb_bank_finalize)
+    cmdb::Buffer<float> shard_d2;          // device [2][kShardD2Cap]: local contributions / sums of the neighbour distances
+    cmdb::Buffer<float> data;  // [capacity, dim] float32 row-major
+    // scoring layout (cmdb_bank_finalize; its buffers: FinalizeBuffers)
     bool finalized = false;
     int64_t fin_rows = 0;
     int64_t fin_rows_pad = 0;  // multiple of kScoreBN
-    __half *hi = nullptr;      // [fin_rows_pad, dim] fp16(x * 2^scale_exp)
-    __half *lo = nullptr;      // [fin_rows_pad, dim] fp16(x * 2^scale_exp - hi)
-    float *norm = nullptr;     // [fin_rows_pad] ||x * 2^scale_exp||^2 ; +inf on padding rows
     int scale_exp = 0;
-    void *tmap_hi = nullptr;  // host copies of the CUtensorMap objects (128 B each)
-    void *tmap_lo = nullptr;
-    void *tmap_hi2 = nullptr;  // box of 128 bank rows (CTA-pair kernels)
-    void *tmap_lo2 = nullptr;
     int timing = 0;
-    cudaEvent_t ev[CMDB_T_COUNT + 1] = {};
+    cmdb::Event ev[CMDB_T_COUNT + 1];
     bool ev_valid = false;
-    double *stats_buf = nullptr;  // 2 + num_sms * 4 doubles on device (cmdb_bank_stats)
-    unsigned int *absmax_buf = nullptr;
+    cmdb::Buffer<double> stats_buf;  // 2 + num_sms * 4 doubles on device (cmdb_bank_stats)
+    cmdb::Buffer<unsigned int> absmax_buf;
 };
 
 namespace cmdb {
@@ -273,8 +370,6 @@ int coreset_greedy_dev(cmdb_bank *b, const double *z_dev, int64_t N, int d, int6
                        bool force_mind_global);
 // host only: rows per CTA of the persistent kernel on num_sms SMs and whether their min-distances fit shared memory
 int coreset_plan_info(int num_sms, int64_t N, int d, int dtype_mode, int64_t *rows_per_cta, int *mind_in_smem);
-int coreset_greedy(cmdb_bank *b, const double *z_dev, int64_t N, int d, int64_t n_select, int dtype_mode,
-                   int64_t *out_idx_host);
 int coreset_rownorms(int device, const void *z_host, const void *last_host, int64_t n_rows, int d, int dtype_mode,
                      void *out_host);
 

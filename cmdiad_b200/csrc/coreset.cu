@@ -850,48 +850,37 @@ int coreset_greedy_dev(cmdb_bank *b, const double *z_dev, int64_t N, int d, int6
     CMDB_REQUIRE(!sharded || (!force_idx_host && N > 0), CMDB_ERR_UNSUPPORTED,
                  "coreset: the row-sharded loop needs non-empty shards and does not support teacher forcing");
     cudaStream_t st = b->handle_stream();
-    long long *idx_dev = nullptr, *force_dev = nullptr;
-    PickSlot *slots = nullptr;
-    __half *zh_alloc = nullptr;
-    double *z0_dev = nullptr;
-    unsigned int *abort_dev = nullptr;
-    void *mind = nullptr;
-    int rc = CMDB_OK;
-    size_t l2_prev = 0;
-    bool l2_changed = false;
-    auto cleanup = [&]() {  // every exit path: error returns included
-        if (l2_changed) {
-            // hand the persisting-L2 carve-out back exactly as it was found (cudaDeviceSetLimit is process-wide state);
-            // lines other code had pinned are left alone -- only our own window was ever marked persisting
+    Buffer<long long> idx_dev, force_dev;
+    Buffer<PickSlot> slots;
+    Buffer<__half> zh_alloc;
+    Buffer<double> z0_dev;
+    Buffer<unsigned int> abort_dev;
+    Buffer<unsigned char> mind;
+    // Hands the persisting-L2 carve-out back exactly as it was found on every exit (cudaDeviceSetLimit is process-wide
+    // state); lines other code had pinned are left alone -- only our own window was ever marked persisting.  Declared
+    // after the buffers, so it runs before they are freed.
+    struct L2Restore {
+        cudaStream_t st;
+        size_t prev = 0;
+        bool changed = false;
+        ~L2Restore() {
+            if (!changed) return;
             (void)cudaStreamSynchronize(st);
-            (void)cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, l2_prev);
+            (void)cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, prev);
             (void)cudaGetLastError();
-            l2_changed = false;
         }
-        cudaFree(idx_dev), cudaFree(force_dev), cudaFree(slots), cudaFree(zh_alloc), cudaFree(mind);
-        cudaFree(z0_dev), cudaFree(abort_dev);
-    };
-#define CS_TRY(expr)                                                                                         \
-    do {                                                                                                     \
-        cudaError_t _e = (expr);                                                                             \
-        if (_e != cudaSuccess) {                                                                             \
-            set_error("%s:%d %s -> %s", __FILE__, __LINE__, #expr, cudaGetErrorString(_e));                  \
-            (void)cudaGetLastError();                                                                        \
-            cleanup();                                                                                       \
-            return CMDB_ERR_CUDA;                                                                            \
-        }                                                                                                    \
-    } while (0)
-    CS_TRY(cudaMalloc(&idx_dev, sizeof(long long) * (size_t)n_select));
-    CS_TRY(cudaMalloc(&slots, sizeof(PickSlot) * 2 * (size_t)b->num_sms));
-    CS_TRY(cudaMalloc(&abort_dev, sizeof(unsigned int)));
-    CS_TRY(cudaMemsetAsync(abort_dev, 0, sizeof(unsigned int), st));
+    } l2{st};
+    CMDB_CUDA(idx_dev.alloc(n_select));
+    CMDB_CUDA(slots.alloc(2 * (size_t)b->num_sms));
+    CMDB_CUDA(abort_dev.alloc(1));
+    CMDB_CUDA(cudaMemsetAsync(abort_dev, 0, sizeof(unsigned int), st));
     if (force_idx_host) {
-        CS_TRY(cudaMalloc(&force_dev, sizeof(long long) * (size_t)n_select));
-        CS_TRY(cudaMemcpyAsync(force_dev, force_idx_host, sizeof(long long) * (size_t)n_select, cudaMemcpyHostToDevice, st));
+        CMDB_CUDA(force_dev.alloc(n_select));
+        CMDB_CUDA(cudaMemcpyAsync(force_dev, force_idx_host, sizeof(long long) * (size_t)n_select, cudaMemcpyHostToDevice, st));
     }
     CoresetParams p{};
     p.N = N, p.d = d, p.n_select = n_select, p.out_idx = idx_dev, p.force_idx = force_dev, p.slots = slots;
-    p.l2_prev_limit = &l2_prev, p.l2_changed = &l2_changed;
+    p.l2_prev_limit = &l2.prev, p.l2_changed = &l2.changed;
     p.world = 1, p.rank = 0, p.row_offset = 0, p.abort_flag = abort_dev, p.spin_limit = 20LL * 1000 * 1000 * 1000;  // ~10 s
     const double *first_row = z_dev;  // pick 0 = global row 0
     const size_t es = dtype_mode == CMDB_CORESET_FP16 ? sizeof(__half) : sizeof(double);
@@ -901,9 +890,9 @@ int coreset_greedy_dev(cmdb_bank *b, const double *z_dev, int64_t N, int d, int6
         p.mb_keys_off = kCommKeysOff, p.mb_ready_off = kCommReadyOff, p.ready_epoch = 1ULL;
         for (int r = 0; r < kMaxRanks; ++r) p.mb_peer[r] = sh->peers[r];
         CMDB_REQUIRE(b->num_sms <= (int)kCommMaxCtas, CMDB_ERR_UNSUPPORTED, "coreset: %d SMs exceed the mailbox layout", b->num_sms);
-        CS_TRY(cudaMalloc(&z0_dev, sizeof(double) * (d + 1)));
-        CS_TRY(cudaMemcpyAsync(z0_dev, sh->z0_host, sizeof(double) * d, cudaMemcpyHostToDevice, st));
-        CS_TRY(cudaMemcpyAsync(z0_dev + d, &p.ready_epoch, sizeof(unsigned long long), cudaMemcpyHostToDevice, st));
+        CMDB_CUDA(z0_dev.alloc(d + 1));
+        CMDB_CUDA(cudaMemcpyAsync(z0_dev, sh->z0_host, sizeof(double) * d, cudaMemcpyHostToDevice, st));
+        CMDB_CUDA(cudaMemcpyAsync(z0_dev + d, &p.ready_epoch, sizeof(unsigned long long), cudaMemcpyHostToDevice, st));
         first_row = z0_dev;
         p.z_full = sh->peers[sh->rank] + kCommHeaderBytes;
         mine_in_replica = sh->peers[sh->rank] + kCommHeaderBytes + es * (size_t)sh->row_offset * d;
@@ -911,74 +900,58 @@ int coreset_greedy_dev(cmdb_bank *b, const double *z_dev, int64_t N, int d, int6
     // row-sharded: the kernel reads the local rows from the replica (the natural [n_total, d] layout, so address alignment ==
     // global alignment class with no padding); every rank copies its slice into all peers' replicas over NVLink and then
     // raises its flag there (stream order: the flag lands after the rows)
-    auto publish_shard = [&]() -> cudaError_t {
+    auto publish_shard = [&]() -> int {
         for (int r = 0; r < p.world; ++r) {
-            cudaError_t e = cudaSuccess;
             if (r != p.rank)
-                e = cudaMemcpyAsync(sh->peers[r] + kCommHeaderBytes + es * (size_t)sh->row_offset * d, mine_in_replica,
-                                    es * (size_t)N * d, cudaMemcpyDeviceToDevice, st);
-            if (e == cudaSuccess)
-                e = cudaMemcpyAsync(sh->peers[r] + kCommReadyOff + 8 * (size_t)p.rank, z0_dev + d, 8, cudaMemcpyDeviceToDevice, st);
-            if (e != cudaSuccess) return e;
+                CMDB_CUDA(cudaMemcpyAsync(sh->peers[r] + kCommHeaderBytes + es * (size_t)sh->row_offset * d, mine_in_replica,
+                                          es * (size_t)N * d, cudaMemcpyDeviceToDevice, st));
+            CMDB_CUDA(cudaMemcpyAsync(sh->peers[r] + kCommReadyOff + 8 * (size_t)p.rank, z0_dev + d, 8, cudaMemcpyDeviceToDevice, st));
         }
-        return cudaSuccess;
+        return CMDB_OK;
     };
     if (dtype_mode == CMDB_CORESET_FP16) {
         __half *zh;
         if (sharded) {
             zh = reinterpret_cast<__half *>(mine_in_replica);
         } else {
-            CS_TRY(cudaMalloc(&zh_alloc, sizeof(__half) * ((size_t)N * d + 4)));
+            CMDB_CUDA(zh_alloc.alloc((size_t)N * d + 4));
             zh = zh_alloc;
         }
-        CS_TRY(cudaMalloc(&mind, sizeof(__half) * (size_t)std::max<int64_t>(N, 1)));
+        CMDB_CUDA(mind.alloc(sizeof(__half) * (size_t)std::max<int64_t>(N, 1)));
         // features.py:378 initial distances in float64, then .half() (:389-391)
-        rc = launch_rownorm<double>(st, b->num_sms, z_dev, first_row, N, d, nullptr, reinterpret_cast<__half *>(mind), p.row_offset);
-        if (rc == CMDB_OK) {
-            to_half_kernel<<<b->num_sms * 4, 512, 0, st>>>(z_dev, (long long)N * d, zh);
-            CS_TRY(cudaGetLastError());
-            if (sharded) CS_TRY(publish_shard());
-            p.z = zh, p.mind = mind;
-            rc = launch_coreset<__half>(b, p, force_mind_global);
-        }
+        CMDB_CHECK(launch_rownorm<double>(st, b->num_sms, z_dev, first_row, N, d, nullptr, reinterpret_cast<__half *>(mind.get()),
+                                          p.row_offset));
+        to_half_kernel<<<b->num_sms * 4, 512, 0, st>>>(z_dev, (long long)N * d, zh);
+        CMDB_CUDA(cudaGetLastError());
+        if (sharded) CMDB_CHECK(publish_shard());
+        p.z = zh, p.mind = mind;
+        CMDB_CHECK(launch_coreset<__half>(b, p, force_mind_global));
     } else {
-        CS_TRY(cudaMalloc(&mind, sizeof(double) * (size_t)N));
-        rc = launch_rownorm<double>(st, b->num_sms, z_dev, first_row, N, d, reinterpret_cast<double *>(mind), nullptr, p.row_offset);
-        if (rc == CMDB_OK) {
-            p.z = z_dev, p.mind = mind;
-            if (sharded) {
-                CS_TRY(cudaMemcpyAsync(mine_in_replica, z_dev, es * (size_t)N * d, cudaMemcpyDeviceToDevice, st));
-                CS_TRY(publish_shard());
-                p.z = mine_in_replica;
-            }
-            rc = launch_coreset<double>(b, p, force_mind_global);
+        CMDB_CUDA(mind.alloc(sizeof(double) * (size_t)N));
+        CMDB_CHECK(launch_rownorm<double>(st, b->num_sms, z_dev, first_row, N, d, reinterpret_cast<double *>(mind.get()), nullptr,
+                                          p.row_offset));
+        p.z = z_dev, p.mind = mind;
+        if (sharded) {
+            CMDB_CUDA(cudaMemcpyAsync(mine_in_replica, z_dev, es * (size_t)N * d, cudaMemcpyDeviceToDevice, st));
+            CMDB_CHECK(publish_shard());
+            p.z = mine_in_replica;
         }
-    }
-    if (rc != CMDB_OK) {
-        cleanup();
-        return rc;
+        CMDB_CHECK(launch_coreset<double>(b, p, force_mind_global));
     }
     unsigned int aborted = 0;
-    CS_TRY(cudaMemcpyAsync(out_idx_host, idx_dev, sizeof(long long) * (size_t)n_select, cudaMemcpyDeviceToHost, st));
-    CS_TRY(cudaMemcpyAsync(&aborted, abort_dev, sizeof(aborted), cudaMemcpyDeviceToHost, st));
+    CMDB_CUDA(cudaMemcpyAsync(out_idx_host, idx_dev, sizeof(long long) * (size_t)n_select, cudaMemcpyDeviceToHost, st));
+    CMDB_CUDA(cudaMemcpyAsync(&aborted, abort_dev, sizeof(aborted), cudaMemcpyDeviceToHost, st));
     if (out_min_last_host)
-        CS_TRY(cudaMemcpyAsync(out_min_last_host, mind,
-                               (dtype_mode == CMDB_CORESET_FP16 ? sizeof(__half) : sizeof(double)) * (size_t)N,
-                               cudaMemcpyDeviceToHost, st));
-    CS_TRY(cudaStreamSynchronize(st));
-#undef CS_TRY
-    cleanup();
+        CMDB_CUDA(cudaMemcpyAsync(out_min_last_host, mind,
+                                  (dtype_mode == CMDB_CORESET_FP16 ? sizeof(__half) : sizeof(double)) * (size_t)N,
+                                  cudaMemcpyDeviceToHost, st));
+    CMDB_CUDA(cudaStreamSynchronize(st));
     if (aborted) {
         set_error("coreset: a peer rank did not answer within the exchange timeout (all ranks must call "
                   "cmdb_coreset_select_sharded together)");
         return CMDB_ERR_CUDA;
     }
     return CMDB_OK;
-}
-
-int coreset_greedy(cmdb_bank *b, const double *z_dev, int64_t N, int d, int64_t n_select, int dtype_mode,
-                   int64_t *out_idx_host) {
-    return coreset_greedy_dev(b, z_dev, N, d, n_select, dtype_mode, out_idx_host, nullptr, nullptr, nullptr, false);
 }
 
 int coreset_rownorms(int device, const void *z_host, const void *last_host, int64_t n_rows, int d, int dtype_mode,
@@ -988,27 +961,19 @@ int coreset_rownorms(int device, const void *z_host, const void *last_host, int6
     int num_sms = kNumSMsDefault;
     cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, device);
     const size_t es = dtype_mode == CMDB_CORESET_FP16 ? sizeof(__half) : sizeof(double);
-    void *z = nullptr, *last = nullptr, *out = nullptr;
-    cudaError_t e = cudaMalloc(&z, es * (size_t)n_rows * d);
-    if (e == cudaSuccess) e = cudaMalloc(&last, es * (size_t)d);
-    if (e == cudaSuccess) e = cudaMalloc(&out, es * (size_t)n_rows);
-    if (e == cudaSuccess) e = cudaMemcpy(z, z_host, es * (size_t)n_rows * d, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMemcpy(last, last_host, es * (size_t)d, cudaMemcpyHostToDevice);
-    int rc = CMDB_OK;
-    if (e == cudaSuccess) {
-        if (dtype_mode == CMDB_CORESET_FP16)
-            rc = launch_rownorm<__half>(nullptr, num_sms, (const __half *)z, (const __half *)last, n_rows, d, (__half *)out,
-                                        nullptr);
-        else
-            rc = launch_rownorm<double>(nullptr, num_sms, (const double *)z, (const double *)last, n_rows, d, (double *)out,
-                                        nullptr);
-        if (rc == CMDB_OK) e = cudaMemcpy(out_host, out, es * (size_t)n_rows, cudaMemcpyDeviceToHost);
-    }
-    cudaFree(z);
-    cudaFree(last);
-    cudaFree(out);
-    if (rc != CMDB_OK) return rc;
-    CMDB_CUDA(e);
+    Buffer<unsigned char> z, last, out;
+    CMDB_CUDA(z.alloc(es * (size_t)n_rows * d));
+    CMDB_CUDA(last.alloc(es * (size_t)d));
+    CMDB_CUDA(out.alloc(es * (size_t)n_rows));
+    CMDB_CUDA(cudaMemcpy(z, z_host, es * (size_t)n_rows * d, cudaMemcpyHostToDevice));
+    CMDB_CUDA(cudaMemcpy(last, last_host, es * (size_t)d, cudaMemcpyHostToDevice));
+    if (dtype_mode == CMDB_CORESET_FP16)
+        CMDB_CHECK(launch_rownorm<__half>(nullptr, num_sms, (const __half *)z.get(), (const __half *)last.get(), n_rows, d,
+                                          (__half *)out.get(), nullptr));
+    else
+        CMDB_CHECK(launch_rownorm<double>(nullptr, num_sms, (const double *)z.get(), (const double *)last.get(), n_rows, d,
+                                          (double *)out.get(), nullptr));
+    CMDB_CUDA(cudaMemcpy(out_host, out, es * (size_t)n_rows, cudaMemcpyDeviceToHost));
     return CMDB_OK;
 }
 

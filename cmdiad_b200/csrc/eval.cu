@@ -287,50 +287,35 @@ int cmdb_eval_pixel_metrics(cmdb_bank *b, const int32_t *labels_host, int64_t n_
     const long long per_warp = ((n + n_warps - 1) / n_warps + 31) / 32 * 32;
     const int scan_blocks = (int)((n + kScanTile - 1) / kScanTile);
     const size_t hist_cols = (size_t)n_components * (n_thresholds + 1);
-    unsigned long long *keys[2] = {nullptr, nullptr}, *thr_keys = nullptr, *comp_hist = nullptr, *u2 = nullptr;
-    unsigned int *vals[2] = {nullptr, nullptr}, *hist = nullptr, *block_cnt = nullptr, *negprefix = nullptr;
-    long long *pos_dev = nullptr;
-    double *thr_dev = nullptr;
-    int rc = CMDB_OK;
-    auto cleanup = [&]() {
-        cudaFree(keys[0]), cudaFree(keys[1]), cudaFree(vals[0]), cudaFree(vals[1]), cudaFree(hist), cudaFree(block_cnt);
-        cudaFree(negprefix), cudaFree(thr_keys), cudaFree(comp_hist), cudaFree(u2), cudaFree(pos_dev), cudaFree(thr_dev);
-    };
-#define EV_TRY(expr)                                                                          \
-    do {                                                                                      \
-        cudaError_t _e = (expr);                                                              \
-        if (_e != cudaSuccess) {                                                              \
-            set_error("%s:%d %s -> %s", __FILE__, __LINE__, #expr, cudaGetErrorString(_e));   \
-            (void)cudaGetLastError();                                                         \
-            cleanup();                                                                        \
-            return CMDB_ERR_CUDA;                                                             \
-        }                                                                                     \
-    } while (0)
+    Buffer<unsigned long long> keys[2], thr_keys, comp_hist, u2;
+    Buffer<unsigned int> vals[2], hist, block_cnt, negprefix;
+    Buffer<long long> pos_dev;
+    Buffer<double> thr_dev;
     for (int i = 0; i < 2; ++i) {
-        EV_TRY(cudaMalloc(&keys[i], sizeof(unsigned long long) * (size_t)n));
-        EV_TRY(cudaMalloc(&vals[i], sizeof(unsigned int) * (size_t)n));
+        CMDB_CUDA(keys[i].alloc(n));
+        CMDB_CUDA(vals[i].alloc(n));
     }
-    EV_TRY(cudaMalloc(&hist, sizeof(unsigned int) * 256 * (size_t)n_warps));
-    EV_TRY(cudaMalloc(&block_cnt, sizeof(unsigned int) * (size_t)(scan_blocks + 1)));
-    EV_TRY(cudaMalloc(&negprefix, sizeof(unsigned int) * (size_t)n));
-    EV_TRY(cudaMalloc(&thr_keys, sizeof(unsigned long long) * n_thresholds));
-    EV_TRY(cudaMalloc(&thr_dev, sizeof(double) * n_thresholds));
-    EV_TRY(cudaMalloc(&comp_hist, sizeof(unsigned long long) * std::max<size_t>(1, hist_cols)));
-    EV_TRY(cudaMalloc(&u2, sizeof(unsigned long long)));
-    EV_TRY(cudaMalloc(&pos_dev, sizeof(long long) * n_thresholds));
-    EV_TRY(cudaMemsetAsync(comp_hist, 0, sizeof(unsigned long long) * std::max<size_t>(1, hist_cols), st));
-    EV_TRY(cudaMemsetAsync(u2, 0, sizeof(unsigned long long), st));
-    EV_TRY(cudaMemcpyAsync(vals[0], labels_host, sizeof(unsigned int) * (size_t)n, cudaMemcpyHostToDevice, st));
-    EV_TRY(cudaMemcpyAsync(pos_dev, ok_rank_pos_host, sizeof(long long) * n_thresholds, cudaMemcpyHostToDevice, st));
+    CMDB_CUDA(hist.alloc(256 * (size_t)n_warps));
+    CMDB_CUDA(block_cnt.alloc(scan_blocks + 1));
+    CMDB_CUDA(negprefix.alloc(n));
+    CMDB_CUDA(thr_keys.alloc(n_thresholds));
+    CMDB_CUDA(thr_dev.alloc(n_thresholds));
+    CMDB_CUDA(comp_hist.alloc(std::max<size_t>(1, hist_cols)));
+    CMDB_CUDA(u2.alloc(1));
+    CMDB_CUDA(pos_dev.alloc(n_thresholds));
+    CMDB_CUDA(cudaMemsetAsync(comp_hist, 0, sizeof(unsigned long long) * std::max<size_t>(1, hist_cols), st));
+    CMDB_CUDA(cudaMemsetAsync(u2, 0, sizeof(unsigned long long), st));
+    CMDB_CUDA(cudaMemcpyAsync(vals[0], labels_host, sizeof(unsigned int) * (size_t)n, cudaMemcpyHostToDevice, st));
+    CMDB_CUDA(cudaMemcpyAsync(pos_dev, ok_rank_pos_host, sizeof(long long) * n_thresholds, cudaMemcpyHostToDevice, st));
     eval_make_keys_kernel<<<b->num_sms * 8, 256, 0, st>>>(f.acc_maps, n, keys[0]);
-    EV_TRY(cudaGetLastError());
+    CMDB_CUDA(cudaGetLastError());
     int cur = 0;
     for (int pass = 0; pass < 8; ++pass) {  // stable LSD radix sort, 8 bits per pass
         radix_hist_kernel<<<n_blocks, kSortThreads, 0, st>>>(keys[cur], n, per_warp, 8 * pass, hist, n_warps);
         scan_u32_kernel<<<1, 1024, 0, st>>>(hist, 256LL * n_warps);
         radix_scatter_kernel<<<n_blocks, kSortThreads, 0, st>>>(keys[cur], vals[cur], n, per_warp, 8 * pass, hist, n_warps,
                                                                 keys[cur ^ 1], vals[cur ^ 1]);
-        EV_TRY(cudaGetLastError());
+        CMDB_CUDA(cudaGetLastError());
         cur ^= 1;
     }
     neg_block_count_kernel<<<scan_blocks, 256, 0, st>>>(vals[cur], n, block_cnt);
@@ -340,15 +325,13 @@ int cmdb_eval_pixel_metrics(cmdb_bank *b, const int32_t *labels_host, int64_t n_
     eval_count_kernel<<<b->num_sms * 8, 256, sizeof(unsigned long long) * n_thresholds, st>>>(
         keys[cur], vals[cur], negprefix, n, (unsigned int)n_neg, thr_keys, n_thresholds, comp_hist, u2);
     keys_to_double_kernel<<<(n_thresholds + 255) / 256, 256, 0, st>>>(thr_keys, n_thresholds, thr_dev);
-    EV_TRY(cudaGetLastError());
+    CMDB_CUDA(cudaGetLastError());
     std::vector<unsigned long long> h_hist(std::max<size_t>(1, hist_cols));
     unsigned long long h_u2 = 0;
-    EV_TRY(cudaMemcpyAsync(h_hist.data(), comp_hist, sizeof(unsigned long long) * std::max<size_t>(1, hist_cols), cudaMemcpyDeviceToHost, st));
-    EV_TRY(cudaMemcpyAsync(&h_u2, u2, sizeof(h_u2), cudaMemcpyDeviceToHost, st));
-    EV_TRY(cudaMemcpyAsync(out_thresholds, thr_dev, sizeof(double) * n_thresholds, cudaMemcpyDeviceToHost, st));
-    EV_TRY(cudaStreamSynchronize(st));
-#undef EV_TRY
-    cleanup();
+    CMDB_CUDA(cudaMemcpyAsync(h_hist.data(), comp_hist, sizeof(unsigned long long) * std::max<size_t>(1, hist_cols), cudaMemcpyDeviceToHost, st));
+    CMDB_CUDA(cudaMemcpyAsync(&h_u2, u2, sizeof(h_u2), cudaMemcpyDeviceToHost, st));
+    CMDB_CUDA(cudaMemcpyAsync(out_thresholds, thr_dev, sizeof(double) * n_thresholds, cudaMemcpyDeviceToHost, st));
+    CMDB_CUDA(cudaStreamSynchronize(st));
     // cumulative counts: #{scores of component c <= thr[t]}  (GroundTruthComponent.compute_overlap, au_pro_util.py:44-49)
     for (int64_t c = 0; c < n_components; ++c) {
         unsigned long long run = 0;
@@ -361,7 +344,7 @@ int cmdb_eval_pixel_metrics(cmdb_bank *b, const int32_t *labels_host, int64_t n_
     *out_two_u = h_u2;
     *out_n_neg = n_neg;
     *out_n_pos = n - n_neg;
-    return rc;
+    return CMDB_OK;
 }
 
 }  // extern "C"

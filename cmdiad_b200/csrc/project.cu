@@ -7,6 +7,9 @@
 // Layout: a CTA stages RT rows with row stride D+1 floats, so the 32 lanes of a warp (= 32 different rows, same output
 // column j, hence the same CSR index) hit 32 different banks; the CSR (indptr + 16-bit index|sign) sits in shared
 // memory and is read as a warp broadcast.
+#include <memory>
+#include <new>
+
 #include "common.cuh"
 
 namespace cmdb {
@@ -81,58 +84,48 @@ int project_rows(cmdb_bank *b, const float *x_dev, int64_t n_rows, int D, const 
                      indices_h[k], D);
         if (fabs(data_h[k]) != mag) uniform = false;
     }
-    int *indptr_d = nullptr;
-    unsigned short *packed_d = nullptr;
-    double *data_d = nullptr;  // [nnz] doubles followed by [nnz] int32 indices (generic path)
-    cudaError_t e = cudaMalloc(&indptr_d, sizeof(int) * (d_proj + 1));
-    if (e == cudaSuccess)
-        e = cudaMemcpyAsync(indptr_d, indptr_h, sizeof(int) * (d_proj + 1), cudaMemcpyHostToDevice, b->handle_stream());
-    unsigned short *packed_h = nullptr;
-    if (e == cudaSuccess && uniform) {
-        packed_h = (unsigned short *)malloc(sizeof(unsigned short) * (size_t)nnz);
+    const size_t csr_bytes = sizeof(int) * (d_proj + 1) + (uniform ? sizeof(unsigned short) * (size_t)nnz : 0) + 16;
+    const size_t budget = 220 * 1024;
+    int rt = 32;
+    while (rt > 8 && sizeof(float) * (size_t)rt * (D + 1) + csr_bytes > budget) rt >>= 1;
+    const size_t smem = sizeof(float) * (size_t)rt * (D + 1) + csr_bytes;
+    CMDB_REQUIRE(smem <= budget, CMDB_ERR_INVALID, "projection: dim=%d with %d non-zeros does not fit shared memory", D, nnz);
+    cudaStream_t st = b->handle_stream();
+    Buffer<int> indptr_d;
+    Buffer<unsigned short> packed_d;
+    Buffer<unsigned char> data_d;  // [nnz] doubles followed by [nnz] int32 indices (generic path)
+    std::unique_ptr<unsigned short[]> packed_h;
+    CMDB_CUDA(indptr_d.alloc(d_proj + 1));
+    CMDB_CUDA(cudaMemcpyAsync(indptr_d, indptr_h, sizeof(int) * (d_proj + 1), cudaMemcpyHostToDevice, st));
+    if (uniform) {
+        packed_h.reset(new (std::nothrow) unsigned short[nnz]);
+        CMDB_REQUIRE(packed_h, CMDB_ERR_CUDA, "projection: no host memory for %d packed indices", nnz);
         for (int k = 0; k < nnz; ++k)
             packed_h[k] = (unsigned short)(indices_h[k] | (data_h[k] < 0 ? 0x8000 : 0));
-        e = cudaMalloc(&packed_d, sizeof(unsigned short) * (size_t)nnz);
-        if (e == cudaSuccess)
-            e = cudaMemcpyAsync(packed_d, packed_h, sizeof(unsigned short) * (size_t)nnz, cudaMemcpyHostToDevice,
-                                b->handle_stream());
-    } else if (e == cudaSuccess) {
-        e = cudaMalloc(&data_d, (sizeof(double) + sizeof(int)) * (size_t)(nnz > 0 ? nnz : 1));
-        if (e == cudaSuccess && nnz > 0)
-            e = cudaMemcpyAsync(data_d, data_h, sizeof(double) * (size_t)nnz, cudaMemcpyHostToDevice, b->handle_stream());
-        if (e == cudaSuccess && nnz > 0)
-            e = cudaMemcpyAsync(reinterpret_cast<int *>(data_d + nnz), indices_h, sizeof(int) * (size_t)nnz,
-                                cudaMemcpyHostToDevice, b->handle_stream());
-    }
-    if (e == cudaSuccess) {
-        const size_t csr_bytes = sizeof(int) * (d_proj + 1) + (uniform ? sizeof(unsigned short) * (size_t)nnz : 0) + 16;
-        const size_t budget = 220 * 1024;
-        int rt = 32;
-        while (rt > 8 && sizeof(float) * (size_t)rt * (D + 1) + csr_bytes > budget) rt >>= 1;
-        const size_t smem = sizeof(float) * (size_t)rt * (D + 1) + csr_bytes;
-        if (smem > budget) {
-            set_error("projection: dim=%d with %d non-zeros does not fit shared memory", D, nnz);
-            e = cudaErrorInvalidValue;
-        } else {
-            const int64_t n_tiles = (n_rows + rt - 1) / rt;
-            const int grid = (int)std::min<int64_t>(n_tiles, (int64_t)b->num_sms);
-            auto launch = [&](auto kern) {
-                cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                kern<<<grid, 256, smem, b->handle_stream()>>>(x_dev, n_rows, D, indptr_d, packed_d, data_d, mag, d_proj, nnz, z_dev);
-            };
-            if (rt == 32) launch(project_kernel<32>);
-            else if (rt == 16) launch(project_kernel<16>);
-            else launch(project_kernel<8>);
-            e = cudaGetLastError();
+        CMDB_CUDA(packed_d.alloc(nnz));
+        CMDB_CUDA(cudaMemcpyAsync(packed_d, packed_h.get(), sizeof(unsigned short) * (size_t)nnz, cudaMemcpyHostToDevice, st));
+    } else {
+        CMDB_CUDA(data_d.alloc((sizeof(double) + sizeof(int)) * (size_t)(nnz > 0 ? nnz : 1)));
+        if (nnz > 0) {
+            CMDB_CUDA(cudaMemcpyAsync(data_d, data_h, sizeof(double) * (size_t)nnz, cudaMemcpyHostToDevice, st));
+            CMDB_CUDA(cudaMemcpyAsync(data_d + sizeof(double) * nnz, indices_h, sizeof(int) * (size_t)nnz, cudaMemcpyHostToDevice,
+                                      st));
         }
     }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(b->handle_stream());
-    free(packed_h);
-    cudaFree(indptr_d);
-    cudaFree(packed_d);
-    cudaFree(data_d);
-    if (e != cudaSuccess && e != cudaErrorInvalidValue) CMDB_CUDA(e);
-    return e == cudaSuccess ? CMDB_OK : CMDB_ERR_INVALID;
+    const int64_t n_tiles = (n_rows + rt - 1) / rt;
+    const int grid = (int)std::min<int64_t>(n_tiles, (int64_t)b->num_sms);
+    auto launch = [&](auto kern) -> int {
+        CMDB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kern<<<grid, 256, smem, st>>>(x_dev, n_rows, D, indptr_d, packed_d, reinterpret_cast<const double *>(data_d.get()), mag,
+                                      d_proj, nnz, z_dev);
+        CMDB_CUDA(cudaGetLastError());
+        return CMDB_OK;
+    };
+    if (rt == 32) CMDB_CHECK(launch(project_kernel<32>));
+    else if (rt == 16) CMDB_CHECK(launch(project_kernel<16>));
+    else CMDB_CHECK(launch(project_kernel<8>));
+    CMDB_CUDA(cudaStreamSynchronize(st));
+    return CMDB_OK;
 }
 
 }  // namespace cmdb

@@ -20,10 +20,6 @@
 //   * one launch sweeps all M tiles of a batch in n-major order: the bank streams from HBM exactly once per launch and
 //     the (small) query operand is re-read from L2; the tile schedule spreads every query's rows over all CTAs.
 // Algorithmic work: 2*P*R*D FLOP per image (TERMS = 3 issues 3x that).
-#include <cuda.h>
-
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace cmdb {
@@ -565,17 +561,15 @@ static EncodeTiledFn get_encode_fn() {
 }
 
 // fp16 [rows, dim] row-major, box = [box_rows, 64] (128 B inner extent), SWIZZLE_128B
-static int make_map(void **slot, const __half *base, long long rows, int dim, int box_rows) {
+static int make_map(CUtensorMap *map, const __half *base, long long rows, int dim, int box_rows) {
     EncodeTiledFn fn = get_encode_fn();
     CMDB_REQUIRE(fn != nullptr, CMDB_ERR_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
-    if (!*slot) *slot = aligned_alloc(64, sizeof(CUtensorMap));
     cuuint64_t gdim[2] = {(cuuint64_t)dim, (cuuint64_t)rows};
     cuuint64_t gstr[1] = {(cuuint64_t)dim * 2};
     cuuint32_t box[2] = {(cuuint32_t)BK, (cuuint32_t)box_rows};
     cuuint32_t estr[2] = {1, 1};
-    CUresult r = fn(reinterpret_cast<CUtensorMap *>(*slot), CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, (void *)base, gdim, gstr, box,
-                    estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, (void *)base, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                    CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     CMDB_REQUIRE(r == CUDA_SUCCESS, CMDB_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
     return CMDB_OK;
 }
@@ -593,35 +587,11 @@ void gemm_prefer_carveout() {
     (void)cudaGetLastError();
 }
 
-template <typename... T>
-static void free_dev(T *&...p) {
-    ((cudaFree(p), p = nullptr), ...);
-}
-
-static void free_lane(Lane &l) {
-    free_dev(l.q_hi, l.q_lo, l.q_scale_exp, l.cand, l.topk_keys, l.map_tmp, l.map_max, l.m_test, l.m_star, l.top3,
-             l.done_counter, l.q_norm, l.q_eps, l.fail_list, l.fail_ctl, l.work_list, l.best_key);
-    l.s_key = nullptr;   // lives inside the fail_ctl allocation
-    if (l.fail_count_host) cudaFreeHost(l.fail_count_host);
-    free(l.tmap_qhi), free(l.tmap_qlo);
-    l.fail_count_host = nullptr, l.tmap_qhi = l.tmap_qlo = nullptr;
-}
-
 // callers make sure that no submitted call is outstanding: its results would be lost
 void score_scratch_free(cmdb_bank *b) {
-    // no copy or kernel may still be in flight into / out of the buffers
-    if (b->copy_stream) cudaStreamSynchronize(b->copy_stream);
-    if (b->d2h_stream) cudaStreamSynchronize(b->d2h_stream);
-    for (const Lane &l : b->lane) {
-        if (l.stream) cudaStreamSynchronize(l.stream);
-        if (l.aux) cudaStreamSynchronize(l.aux);
-    }
-    for (ResultSlot &s : b->slot) {
-        free_dev(s.q_f32, s.out_block);
-        if (s.out_block_host) cudaFreeHost(s.out_block_host);
-        s.out_block_host = nullptr;
-    }
-    for (Lane &l : b->lane) free_lane(l);
+    b->sync_streams();   // no copy or kernel may still be in flight into / out of the buffers
+    for (ResultSlot &s : b->slot) static_cast<SlotScratch &>(s) = SlotScratch();
+    for (Lane &l : b->lane) static_cast<LaneScratch &>(l) = LaneScratch();
     b->layout = ScoreLayout();
     b->round.open = false;   // an open sharded round lived in these buffers
     b->last_fail_host = nullptr;
@@ -680,34 +650,33 @@ int score_scratch_alloc(cmdb_bank *b, int B, int P_img, int out_hw) {
     L.n_topk_blocks = b->num_sms * 4;
     // per slot: queries in, results out (mirrored by a pinned host block)
     for (ResultSlot &s : b->slot) {
-        CMDB_CUDA(cudaMalloc(&s.q_f32, sizeof(float) * cap_p * D));
-        CMDB_CUDA(cudaMalloc(&s.out_block, L.out_block_bytes));
-        CMDB_CUDA(cudaMallocHost(&s.out_block_host, L.out_block_bytes));
+        CMDB_CUDA(s.q_f32.alloc(cap_p * D));
+        CMDB_CUDA(s.out_block.alloc(L.out_block_bytes));
+        CMDB_CUDA(s.out_block_host.alloc(L.out_block_bytes));
     }
     for (Lane &l : b->lane) {
-        CMDB_CUDA(cudaMalloc(&l.q_hi, sizeof(__half) * cap_p * D));
-        CMDB_CUDA(cudaMalloc(&l.q_lo, sizeof(__half) * cap_p * D));
-        CMDB_CUDA(cudaMalloc(&l.q_scale_exp, sizeof(int) * cap_p));
-        CMDB_CUDA(cudaMalloc(&l.q_norm, sizeof(float) * cap_p));
-        CMDB_CUDA(cudaMalloc(&l.q_eps, sizeof(float) * cap_p));
-        CMDB_CUDA(cudaMalloc(&l.fail_list, sizeof(int) * cap_p));
+        CMDB_CUDA(l.q_hi.alloc(cap_p * D));
+        CMDB_CUDA(l.q_lo.alloc(cap_p * D));
+        CMDB_CUDA(l.q_scale_exp.alloc(cap_p));
+        CMDB_CUDA(l.q_norm.alloc(cap_p));
+        CMDB_CUDA(l.q_eps.alloc(cap_p));
+        CMDB_CUDA(l.fail_list.alloc(cap_p));
         // control block (8 ints) and the per-image argmax keys behind it: one allocation, cleared by ONE memset per call
-        CMDB_CUDA(cudaMalloc(&l.fail_ctl, 8 * sizeof(int) + sizeof(unsigned long long) * cap_b));
+        CMDB_CUDA(l.fail_ctl.alloc(8 + sizeof(unsigned long long) / sizeof(int) * cap_b));
         l.s_key = reinterpret_cast<unsigned long long *>(l.fail_ctl + 8);
-        CMDB_CUDA(cudaMalloc(&l.work_list, sizeof(int2) * kWorkCap));
-        CMDB_CUDA(cudaMalloc(&l.best_key, sizeof(unsigned long long) * cap_p));
-        CMDB_CUDA(cudaMallocHost(&l.fail_count_host, 2 * sizeof(int)));
+        CMDB_CUDA(l.work_list.alloc(kWorkCap));
+        CMDB_CUDA(l.best_key.alloc(cap_p));
+        CMDB_CUDA(l.fail_count_host.alloc(2));
         l.fail_count_host[0] = l.fail_count_host[1] = 0;
-        CMDB_CUDA(cudaMalloc(&l.done_counter, sizeof(unsigned int)));
+        CMDB_CUDA(l.done_counter.alloc(1));
         CMDB_CUDA(cudaMemset(l.done_counter, 0, sizeof(unsigned int)));
-        const size_t cand_bytes = sizeof(float4) * (size_t)cap_p * 2 * b->num_sms;
-        CMDB_CUDA(cudaMalloc(&l.cand, cand_bytes));
-        CMDB_CUDA(cudaMalloc(&l.map_tmp, (size_t)map_cap * cap_b));
-        CMDB_CUDA(cudaMalloc(&l.map_max, sizeof(float) * cap_b * 17));
-        CMDB_CUDA(cudaMalloc(&l.topk_keys, sizeof(unsigned long long) * 3 * L.n_topk_blocks * cap_b));
-        CMDB_CUDA(cudaMalloc(&l.top3, sizeof(unsigned long long) * 3 * cap_b));
-        CMDB_CUDA(cudaMalloc(&l.m_test, sizeof(float) * D * cap_b));
-        CMDB_CUDA(cudaMalloc(&l.m_star, sizeof(float) * D * cap_b));
+        CMDB_CUDA(l.cand.alloc((size_t)cap_p * 2 * b->num_sms));
+        CMDB_CUDA(l.map_tmp.alloc((size_t)map_cap * cap_b));
+        CMDB_CUDA(l.map_max.alloc(cap_b * 17));
+        CMDB_CUDA(l.topk_keys.alloc(3 * L.n_topk_blocks * cap_b));
+        CMDB_CUDA(l.top3.alloc(3 * cap_b));
+        CMDB_CUDA(l.m_test.alloc(D * cap_b));
+        CMDB_CUDA(l.m_star.alloc(D * cap_b));
         CMDB_CHECK(make_map(&l.tmap_qhi, l.q_hi, cap_p, b->dim, BM));
         CMDB_CHECK(make_map(&l.tmap_qlo, l.q_lo, cap_p, b->dim, BM));
     }
@@ -722,7 +691,7 @@ int score_query_prep(const ScoreCall &c, cudaStream_t st, int P, bool compact, i
     const size_t o = (size_t)row0 * b->dim;
     q_split_kernel<<<std::min(b->num_sms * 2, (p_pad + 7) / 8), 256, 0, st>>>(
         c.slot->q_f32 + o, P, p_pad, b->dim, l.q_hi + o, l.q_lo + o, l.q_scale_exp + row0, compact ? nullptr : l.q_norm + row0,
-        compact ? nullptr : l.q_eps + row0, compact ? l.fail_list : nullptr, compact ? l.fail_ctl + 2 : nullptr);
+        compact ? nullptr : l.q_eps + row0, compact ? l.fail_list.get() : nullptr, compact ? l.fail_ctl + 2 : nullptr);
     CMDB_CUDA(cudaGetLastError());
     return CMDB_OK;
 }
@@ -797,10 +766,9 @@ int score_gemm_candidates(const ScoreCall &c, cudaStream_t st, int P, int terms,
         attr.val.clusterDim.x = cluster2 ? 2 : 1, attr.val.clusterDim.y = 1, attr.val.clusterDim.z = 1;
         cfg.attrs = &attr, cfg.numAttrs = 1;
         // the pair kernels load HALF bank tiles (box of 128 rows)
-        const CUtensorMap &mh = *reinterpret_cast<CUtensorMap *>(cluster2 ? b->tmap_hi2 : b->tmap_hi);
-        const CUtensorMap &ml = *reinterpret_cast<CUtensorMap *>(cluster2 ? b->tmap_lo2 : b->tmap_lo);
-        CMDB_CUDA(cudaLaunchKernelEx(&cfg, kern, *reinterpret_cast<CUtensorMap *>(l.tmap_qhi),
-                                     *reinterpret_cast<CUtensorMap *>(l.tmap_qlo), mh, ml, p));
+        const CUtensorMap &mh = cluster2 ? b->tmap_hi2 : b->tmap_hi;
+        const CUtensorMap &ml = cluster2 ? b->tmap_lo2 : b->tmap_lo;
+        CMDB_CUDA(cudaLaunchKernelEx(&cfg, kern, l.tmap_qhi, l.tmap_qlo, mh, ml, p));
         return CMDB_OK;
     };
     if (pair) CMDB_CHECK(launch(score_gemm_kernel<3, kGemmEpiGroups, 2>, GemmSmem<3, 2>::total + 1024, true));

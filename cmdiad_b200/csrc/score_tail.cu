@@ -444,7 +444,7 @@ int score_refine(const ScoreCall &c, cudaStream_t st, int B, int P_img, int n_ca
     // compact mode follows score_certify, which already reset s_key and published the certified queries
     if (!compact) CMDB_CUDA(cudaMemsetAsync(l.s_key, 0, sizeof(unsigned long long) * B, st));
     refine_kernel<<<(P + 7) / 8, 256, 0, st>>>(l.cand, n_cand, b->layout.cap_p, c.slot->q_f32, b->data, b->dim, P, P_img,
-                                               b->row_offset, c.min_val, c.min_idx, l.s_key, compact ? l.fail_list : nullptr,
+                                               b->row_offset, c.min_val, c.min_idx, l.s_key, compact ? l.fail_list.get() : nullptr,
                                                compact ? l.fail_ctl + 2 : nullptr, c.sq_min);
     CMDB_CUDA(cudaGetLastError());
     return CMDB_OK;
@@ -1295,7 +1295,7 @@ int score_select(const ScoreCall &c, int B, int P_img, bool local_m_star) {
     const cmdb_bank *b = c.b;
     const Lane &l = *c.lane;
     select_kernel<<<B, 256, 0, c.stream>>>(l.s_key, c.min_idx, P_img, c.slot->q_f32, b->data, b->dim, b->row_offset, b->fin_rows,
-                                           l.m_test, local_m_star ? l.m_star : nullptr, c.tail);
+                                           l.m_test, local_m_star ? l.m_star.get() : nullptr, c.tail);
     CMDB_CUDA(cudaGetLastError());
     return CMDB_OK;
 }
@@ -1311,7 +1311,7 @@ static int launch_reweight_cert(const ScoreCall &c, const GemmSched &sched, int 
                  sched.producers);
     ReweightCertParams p{};
     p.cand = s.cand, p.n_cand = sched.producers, p.cand_stride = b->layout.cap_p;
-    p.m_star = m_star, p.m_test = res ? s.m_test : nullptr, p.bank = b->data, p.rows = b->fin_rows, p.row_offset = row_offset;
+    p.m_star = m_star, p.m_test = res ? s.m_test.get() : nullptr, p.bank = b->data, p.rows = b->fin_rows, p.row_offset = row_offset;
     p.dim = b->dim, p.q_norm = s.q_norm, p.q_eps = s.q_eps;
     p.bmax = b->cert_bmax, p.eb_max = b->cert_eb_max, p.acc_model = cert_acc_model(b->dim);
     p.sched = sched;
@@ -1343,9 +1343,7 @@ int score_build_knn_table(cmdb_bank *b, long long row_first, long long row_count
     const ScoreCall c = score_call(b, 0, 0);   // lane 0; the result slot is not used
     cudaStream_t st = c.stream;
     if (!b->knn_table || b->knn_rows != b->fin_rows) {
-        cudaFree(b->knn_table);
-        b->knn_table = nullptr;
-        CMDB_CUDA(cudaMalloc(&b->knn_table, sizeof(unsigned long long) * 3 * (size_t)b->fin_rows));
+        CMDB_CUDA(b->knn_table.alloc(3 * (size_t)b->fin_rows));
         CMDB_CUDA(cudaMemsetAsync(b->knn_table, 0xff, sizeof(unsigned long long) * 3 * (size_t)b->fin_rows, st));
         b->knn_rows = b->fin_rows;
     }
